@@ -89,6 +89,12 @@ def parse_args():
                          "the JSON line then carries a shorter rowshard measurement of the same batch as well")
     ap.add_argument("--bm25-mode", type=int, default=-1, help="rse_set_bm25_mode override (see include/rse.h); -1 = library default")
     ap.add_argument("--tc-mode", type=int, default=-1, help="rse_set_tc_mode override (see include/rse.h); -1 = library default")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its LAST step as DIR/<name>.npy "
+                         "(float64; float32 where the path returns float32; integers are exact): hybrid600k = "
+                         "id, score, bm25, semantic (rrf: ranks, -1 = none; weighted: normalised scores), count; "
+                         "bm25_10k = score, doc, count; knn100m = dist, row, movie, count.  The inputs are seeded, so "
+                         "two builds run with the same arguments can be compared output for output.  One process only")
     return ap.parse_args()
 
 
@@ -254,6 +260,32 @@ def postings_touched(bm, terms) -> int:
     return int(bm.df[t].sum())
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict):
+    """--dump-outputs: every array (query-major, one row per query) as out_dir/<name>.npy in float32 (what already
+    is float32) or float64.  Above DUMP_MAX_BYTES a fixed seeded sample of the queries is written, their indices
+    as query_index.npy."""
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.kind in "iu" and a.size and int(np.abs(a.astype(np.int64)).max()) >= 2 ** 53:
+            raise ValueError(f"--dump-outputs: {name} holds integers that float64 cannot represent exactly")
+        conv[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    nq = next(iter(conv.values())).shape[0]
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_MAX_BYTES:
+        keep = int(DUMP_MAX_BYTES // (total / nq + 8))
+        rows = np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+        conv = {name: a[rows] for name, a in conv.items()}
+        conv["query_index"] = rows.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in conv.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def config_dict(args, info, world, par="replicate"):
     return {"workload": "configs[3]: movies_600k-shaped synthetic (S-600k), hybrid rrf_search k=60 limit=10 "
                         "(BM25 top-10 + exact vec0 KNN top-100 + per-movie best chunk + RRF), Gemini disabled",
@@ -309,12 +341,8 @@ def run_reference(args, rank, world):
     import oracle
     oracle.build()
     times = []
-    budget_s = 150.0          # the whole arm must end within a few minutes whatever --steps says
-    t_start = time.perf_counter()
     nq_all = NB * args.batch
     for step in range(args.warmup + args.steps):
-        if step > args.warmup + 1 and time.perf_counter() - t_start > budget_s:
-            break
         off = (step * sample) % max(1, nq_all - sample + 1)
         Qs, tp, tr = batch_slice(tok_indptr, terms, Qh, off, off + sample)
         qps, dt, _ = cpu_hybrid_sample(emb_host, movie_of, bm, se.movie_ids, Qs, tp, tr, args.limit, args.mode, sample, cores)
@@ -376,10 +404,11 @@ def measure_hybrid(idx, tm: Timer, batches, mode, param, limit, steps, warmup, *
         idx.hybrid_stage(Qb, tp, tr)
         idx.hybrid_stash(b)
 
-    def step(i):
+    def step(i, park=True):
         idx.hybrid_stash(i % nb)
         idx.hybrid_run(mode, param, limit)
-        idx.hybrid_stash(i % nb)
+        if park:
+            idx.hybrid_stash(i % nb)
 
     for i in range(max(warmup, 3)):
         step(i)
@@ -393,15 +422,19 @@ def measure_hybrid(idx, tm: Timer, batches, mode, param, limit, steps, warmup, *
     torch.cuda.synchronize(); tm.barrier()
     tm.e0.record(tm.stream)
     for i in range(steps):
-        step(i)                               # (no inline NVML sampling here: one query costs the host ~25 ms and the
-    tm.e1.record(tm.stream)                   #  device would idle; the sampler thread polls concurrently instead)
-    torch.cuda.synchronize(); tm.barrier()
+        step(i, park=i + 1 < steps)           # the last batch stays staged: its results are fetched below
+    tm.e1.record(tm.stream)                   # (no inline NVML sampling in the loop: one query costs the host ~25 ms and
+    torch.cuda.synchronize(); tm.barrier()    #  the device would idle; the sampler thread polls concurrently instead)
     clocks = sampler.stop() if sampler else None
     ms_local = tm.e0.elapsed_time(tm.e1)
     st = idx.stats()
     idx.set_timing(False)
+    last = None
+    if steps > 0:
+        last = idx.hybrid_fetch(limit)        # what the last timed step computed
+        idx.hybrid_stash((steps - 1) % nb)
     out = {"ms": tm.max_over_ranks(ms_local), "ms_local": ms_local, "stats": st, "clocks": clocks, "nq": nq,
-           "survivors": None, "e2e": None, "results": None, "ms_ranks": tm.gather_ranks(ms_local)}
+           "survivors": None, "e2e": None, "results": None, "ms_ranks": tm.gather_ranks(ms_local), "last": last}
     if int(st.tc_filter_launches) > 0:
         try:
             out["survivors"] = idx.tc_last_survivors(min(nq, 256))
@@ -852,6 +885,9 @@ def run_b200(args, rank, world, local_rank):
     Qn, batches = pinned_batches(torch, Q, tok_indptr, terms, nq, qlo, qhi)
     m = measure_hybrid(idx, tm, batches, mode, param, limit, args.steps, args.warmup, sample_clocks=local_rank,
                        e2e=not args.no_e2e)
+    if args.dump_outputs:
+        oid, osc, oa, ob, oc = m["last"]
+        dump_outputs(args.dump_outputs, {"id": oid, "score": osc, "bm25": oa, "semantic": ob, "count": oc})
     ms, st, clocks = m["ms"], m["stats"], m["clocks"]
     launches = int(st.kernel_launches)
     scan_ms = st.scan_ms_total / max(1, st.scan_launches_timed)
@@ -1158,6 +1194,8 @@ def run_bm25_10k(args, local_rank):
     for _ in range(args.steps):
         sc, dc, cnt = idx.bm25(tok_indptr, terms, 10)
     wall = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"score": sc, "doc": dc, "count": cnt})
     launches = int(idx.stats().kernel_launches)
     touched = postings_touched(bm, terms)
     import oracle
@@ -1198,7 +1236,7 @@ KNN100M_UNIT = 313 * 1024            # rows per generation unit (a whole number 
 KNN100M_TOTAL_UNITS = 312            # 99 999 744 rows ("100 M"): 8 shards of 39 units, each aligned to vec0 blocks
 
 
-def knn100m_measure(args, rank, world, local_rank, steps, batch=256, total_units=None):
+def knn100m_measure(args, rank, world, local_rank, steps, batch=256, total_units=None, keep_outputs=False):
     """configs[4] AS SPECIFIED: a FIXED synthetic 100M x 384 fp32 corpus (99 999 744 rows: 312 units of 313 vec0
     blocks, unit u generated from seed 1234+u whatever N is) sharded by row over N GPUs, top-100, candidate
     exchange + merge — STRONG scaling over N = 2, 4, 8 (rows per GPU = 100M / N; 256 queries per step in total).
@@ -1298,6 +1336,10 @@ def knn100m_measure(args, rank, world, local_rank, steps, batch=256, total_units
         dist.all_reduce(sig, op=dist.ReduceOp.SUM)
     ms = float(t.item())
     sig = sig.cpu().tolist()
+    outputs = None
+    if keep_outputs:                                      # this rank's query slice, as the last timed step left it
+        outputs = {"dist": od[:ns].cpu().numpy(), "row": orow[:ns].cpu().numpy(), "movie": om[:ns].cpu().numpy(),
+                   "count": oc[:ns].cpu().numpy()}
     scan_ms = st.scan_ms_total / max(1, st.scan_launches_timed)
     idx.close()
     del emb, movie
@@ -1321,7 +1363,7 @@ def knn100m_measure(args, rank, world, local_rank, steps, batch=256, total_units
             "shadow_stream_gbs_per_gpu": rows * ROW_BYTES_SHADOW / (scan_ms * 1e-3) / 1e9 if scan_ms > 0 else None,
             "flagged_queries_in_timed_steps": int(sig[3]), "self_hits_found": int(sig[4]), "full_k": bool(sig[2] == nq * kp),
             "result_checksum": {"rowid_sum": sig[0], "dist_bits_sum": sig[1]},
-            "gpu_launches": int(st.kernel_launches)}
+            "gpu_launches": int(st.kernel_launches), **({"outputs": outputs} if keep_outputs else {})}
 
 
 def run_knn100m(args, rank, world, local_rank):
@@ -1329,9 +1371,15 @@ def run_knn100m(args, rank, world, local_rank):
     units = None
     if args.shard_rows:                                   # a smaller corpus for experiments: units per GPU given
         units = max(1, args.shard_rows // KNN100M_UNIT) * (2 if world == 1 else world)
-    r = knn100m_measure(args, rank, world, local_rank, args.steps, args.batch, total_units=units)
+    r = knn100m_measure(args, rank, world, local_rank, args.steps, args.batch, total_units=units,
+                        keep_outputs=bool(args.dump_outputs))
     if rank != 0:
         return
+    outputs = r.pop("outputs", None)
+    if args.dump_outputs:
+        if outputs is None:
+            raise SystemExit(f"--dump-outputs: nothing was measured ({r.get('skipped')})")
+        dump_outputs(args.dump_outputs, outputs)
     line = {"metric": "kNN top-100 queries/sec x corpus chunks (row-sharded, candidate exchange + merge)",
             "value": r.get("value"), "unit": "query-chunks/s", "n_gpus": world, "steps": args.steps,
             "warmup": max(args.warmup, 3), "ms_per_step": r.get("ms_per_step"), "higher_is_better": True,
@@ -1347,6 +1395,10 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (world > 1 or args.impl == "reference"):
+        raise SystemExit("--dump-outputs: the b200 arm in one process only")
+    if args.dump_outputs and args.steps < 1:
+        raise SystemExit("--dump-outputs: needs --steps >= 1 (it writes what the last timed step computed)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

@@ -1,10 +1,10 @@
-"""Import the UNMODIFIED reference (``/root/reference``) with stub modules for the
-third-party packages that are absent from this image.
+"""Import the UNMODIFIED reference (a checkout of rag-search-engine under ``oracle/_ref``,
+or wherever ``RSE_REFERENCE_ROOT`` points) with stub modules for those of its third-party
+packages that are not installed.
 
-TEST INFRASTRUCTURE ONLY, and only usable in the build container: the GPU box
-has no /root/reference.  Used by oracle/make_golden.py to generate the golden
-fixtures under tests/golden/ and by tests that are skipped when the reference
-is not present.
+TEST INFRASTRUCTURE ONLY.  The checkout is not part of this repository (``oracle/_ref`` is
+git-ignored).  Used by oracle/make_golden.py to generate the golden fixtures under
+tests/golden/ and by tests that are skipped when the reference is not present.
 
 Stubbed (never reached by the arithmetic under test): spacy, rapidfuzz,
 sqlite_vec, sentence_transformers, google.genai.  ``preprocess`` is replaced by
@@ -18,11 +18,14 @@ import sys
 import types
 from pathlib import Path
 
-REFERENCE_ROOT = Path(os.environ.get("RSE_REFERENCE_ROOT", "/root/reference"))
+REFERENCE_ROOT = Path(os.environ.get("RSE_REFERENCE_ROOT") or Path(__file__).resolve().parent / "_ref")
 
 
 def available() -> bool:
-    return (REFERENCE_ROOT / "rag_search_engine" / "utils" / "keyword_search.py").exists()
+    try:
+        return (REFERENCE_ROOT / "rag_search_engine" / "utils" / "keyword_search.py").is_file()
+    except OSError:                   # a path this user may not enter counts as absent
+        return False
 
 
 def frozen_preprocess(texts, n_process=1, batch_size=256):

@@ -41,7 +41,8 @@ def build(force: bool = False, verbose: bool = False) -> Path:
     extra = os.environ.get("RSE_EXTRA_NVCC_FLAGS", "").split()
     cmd = ["nvcc", *NVCC_FLAGS, *extra, "-o", str(LIB), *map(str, SOURCES)]
     proc = subprocess.run(cmd, capture_output=True, text=True)
-    # the log is tracked (register / spill counts per kernel are evidence); drop the lines that differ on every build
+    # the log (register / spill counts per kernel) is a build product, kept beside the library and out of git;
+    # drop the lines that differ on every build
     log = "\n".join(l for l in (proc.stdout + proc.stderr).splitlines() if "Compile time" not in l) + "\n"
     (CSRC / "build.log").write_text(log)
     if proc.returncode != 0:

@@ -6,6 +6,9 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+import pytest
+
 ROOT = Path(__file__).resolve().parents[1]
 
 SHARED_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -33,3 +36,27 @@ def test_reference_arm_prints_one_contract_line():
     assert e2e == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     # value = queries of the timed steps / their time
     assert abs(d["value"] * d["ms_per_step"] / 1e3 - int(cb["sample"].split()[0])) < 1e-6 * max(1, d["value"])
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_above_the_cap(tmp_path, monkeypatch):
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {"id": rng.integers(10, 2 ** 40, (300, 10)), "score": rng.standard_normal((300, 10)),
+              "dist": rng.standard_normal((300, 10)).astype(np.float32), "count": rng.integers(0, 11, 300).astype(np.int32)}
+    bench.dump_outputs(tmp_path / "all", arrays)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "all" / f"{name}.npy")
+        assert got.dtype == (np.float32 if a.dtype == np.float32 else np.float64)
+        assert (got == a).all()
+    assert not (tmp_path / "all" / "query_index.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 8000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(tmp_path / d, arrays)
+    rows = np.load(tmp_path / "s1" / "query_index.npy").astype(np.int64)
+    assert 0 < len(rows) < 300 and (np.diff(rows) > 0).all()
+    assert sum((tmp_path / "s1" / f"{n}.npy").stat().st_size for n in list(arrays) + ["query_index"]) < 8000 + 5 * 256
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "s1" / f"{name}.npy")
+        assert (got == a[rows]).all() and (got == np.load(tmp_path / "s2" / f"{name}.npy")).all()
+    with pytest.raises(ValueError):
+        bench.dump_outputs(tmp_path / "big", {"id": np.array([2 ** 53 + 1], np.int64)})

@@ -446,3 +446,27 @@ def test_sampled_probe_bound_is_verified_and_results_stay_exact(distribution, kn
         finally:
             idx.close()
     assert same(out[1], out[2])
+
+
+def test_bench_resident_loop_returns_the_last_timed_batch(small_world, tmp_path):
+    """bench.py --dump-outputs: measure_hybrid's last timed step is left staged, fetched after the timer and parked
+    again — its results are those of rse_hybrid on batch (steps - 1) % nb, in both fusion modes, and every batch
+    is back in its own stash slot afterwards."""
+    import torch
+    import bench
+    idx, se, bm, batches = small_world
+    stream = torch.cuda.current_stream()
+    tm = bench.Timer(stream, 1, torch.device("cuda", 0))
+    for mode, param, steps in ((0, 60.0, 5), (1, 0.5, 3), (0, 60.0, 1)):
+        m = bench.measure_hybrid(idx, tm, batches, mode, param, 10, steps, 3, e2e=False)
+        assert same(m["last"], idx.hybrid(mode, param, 10, *batches[(steps - 1) % len(batches)])), (mode, steps)
+        for b in (2, 0, 1):
+            idx.hybrid_stash(b)
+            idx.hybrid_run(mode, param, 10)
+            got = idx.hybrid_fetch(10)
+            idx.hybrid_stash(b)
+            assert same(got, idx.hybrid(mode, param, 10, *batches[b])), f"batch {b} not back in its slot"
+    oid, osc, oa, ob, oc = m["last"]
+    bench.dump_outputs(tmp_path, {"id": oid, "score": osc, "bm25": oa, "semantic": ob, "count": oc})
+    assert (np.load(tmp_path / "id.npy") == oid).all() and (np.load(tmp_path / "count.npy") == oc).all()
+    assert np.load(tmp_path / "score.npy").tobytes() == osc.tobytes()

@@ -2,6 +2,7 @@
 (no compute), the SQLite exporter/writer round trip, the text helpers against the reference's own
 functions, the CPython-set emulation against the real set, and the oracle-stays-out-of-the-product rule."""
 import ctypes
+import json
 import random
 import re
 import sqlite3
@@ -15,6 +16,7 @@ from oracle import ref_import
 from helpers.corpus import build_postings, to_csr
 
 ROOT = Path(__file__).resolve().parents[1]
+GOLDEN = ROOT / "tests" / "golden"
 
 
 # ----------------------------------------------------------------------------- C-ABI surface
@@ -102,24 +104,31 @@ def test_window_chunks_known_shapes():
 @pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (GPU box)")
 def test_text_helpers_match_reference():
     _, _, ref_utils = ref_import.load()
+    from oracle.make_golden import chunk_inputs
     from rag_search_engine_b200.textutil import sentence_chunks, window_chunks
-    rnd = random.Random(4)
-    for _ in range(400):
-        n = rnd.randint(0, 14)
-        items = [f"w{i}" for i in range(n)]
-        cs, ov = rnd.randint(1, 5), rnd.randint(0, 6)
-        assert window_chunks(items, cs, ov) == ref_utils.chunk(list(items), cs, ov)
-        text = " ".join(rnd.choice(["Alpha beta.", "What now?", "Go!", "no stop", "x. "]) for _ in range(n))
-        assert sentence_chunks(text, cs, ov) == ref_utils.semantic_chunk(text, cs, ov)
+    want = json.loads((GOLDEN / "live_ref.json").read_text())["chunks"]
+    for (items, cs, ov, text), pinned in zip(chunk_inputs(), want):
+        ref = [ref_utils.chunk(list(items), cs, ov), ref_utils.semantic_chunk(text, cs, ov)]
+        assert window_chunks(items, cs, ov) == ref[0]
+        assert sentence_chunks(text, cs, ov) == ref[1]
+        assert ref == pinned                                  # the pinned answers are the reference's
+
+
+def test_text_helpers_match_pinned_answers():
+    """test_text_helpers_match_reference against its pinned answers (tests/golden/live_ref.json)."""
+    from oracle.make_golden import chunk_inputs
+    from rag_search_engine_b200.textutil import sentence_chunks, window_chunks
+    want = json.loads((GOLDEN / "live_ref.json").read_text())["chunks"]
+    cases = chunk_inputs()
+    assert len(cases) == len(want) == 400
+    for (items, cs, ov, text), pinned in zip(cases, want):
+        assert [window_chunks(items, cs, ov), sentence_chunks(text, cs, ov)] == pinned, (items, cs, ov, text)
 
 
 # ----------------------------------------------------------------------------- SQLite exporter / writer
 def _docs(seed=3, n=60):
-    from oracle.make_golden import make_corpus
-    docs, words, weights = make_corpus(seed, n, 30)
-    for d in docs:                                            # sentence structure for the chunker
-        d["description"] = ". ".join(d["description"].split()[i] for i in range(min(7, len(d["description"].split())))) + "."
-    return docs, words, weights
+    from oracle.make_golden import sentence_corpus
+    return sentence_corpus(seed, n)
 
 
 def test_export_bm25_round_trip_matches_reference_layout(tmp_path, monkeypatch):
@@ -157,17 +166,13 @@ def test_export_bm25_round_trip_matches_reference_layout(tmp_path, monkeypatch):
 
 @pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (GPU box)")
 def test_writer_produces_the_tables_the_reference_build_produces(tmp_path):
-    import json
+    from oracle.make_golden import encode_tables, reference_tables
     from rag_search_engine_b200 import store
     from rag_search_engine_b200.textutil import whitespace_tokenizer
     ref_kw, _, _ = ref_import.load()
     docs, _, _ = _docs(5, 40)
-    p = tmp_path / "movies.json"
-    p.write_text(json.dumps({"movies": docs}))
-    ks = ref_kw.KeywordSearch.build_from_docs(docs_path=p, db_path=tmp_path / "ref.db", force=True)
-    ks.close()
+    a = reference_tables(ref_kw, docs, tmp_path)
     store.write_reference_db(tmp_path / "ours.db", docs, whitespace_tokenizer)
-    a = store.export_bm25(sqlite3.connect(tmp_path / "ref.db"))
     b = store.export_bm25(sqlite3.connect(tmp_path / "ours.db"))
     assert a.n_movies == b.n_movies and a.avgdl == b.avgdl and (a.dl == b.dl).all() and (a.doc_ids == b.doc_ids).all()
     assert set(a.term_row) == set(b.term_row)
@@ -175,6 +180,22 @@ def test_writer_produces_the_tables_the_reference_build_produces(tmp_path):
         ra, rb = a.term_row[t], b.term_row[t]
         sa, sb = slice(a.indptr[ra], a.indptr[ra + 1]), slice(b.indptr[rb], b.indptr[rb + 1])
         assert (a.doc_idx[sa] == b.doc_idx[sb]).all() and (a.tf[sa] == b.tf[sb]).all()
+    assert encode_tables(a) == json.loads((GOLDEN / "live_ref.json").read_text())["tables"]   # pinned = reference
+
+
+def test_writer_tables_match_pinned_answers(tmp_path):
+    """test_writer_produces_the_tables_the_reference_build_produces against its pinned answers
+    (tests/golden/live_ref.json): documents, lengths, and every term's postings and term frequencies."""
+    from oracle.make_golden import encode_tables
+    from rag_search_engine_b200 import store
+    from rag_search_engine_b200.textutil import whitespace_tokenizer
+    docs, _, _ = _docs(5, 40)
+    store.write_reference_db(tmp_path / "ours.db", docs, whitespace_tokenizer)
+    got = encode_tables(store.export_bm25(sqlite3.connect(tmp_path / "ours.db")))
+    want = json.loads((GOLDEN / "live_ref.json").read_text())["tables"]
+    assert got["n_movies"] == want["n_movies"] == 40 and got["avgdl"] == want["avgdl"]
+    assert got["dl"] == want["dl"] and got["doc_ids"] == want["doc_ids"]
+    assert got["postings"] == want["postings"]
 
 
 def test_export_embeddings_physical_layout(tmp_path):
@@ -485,6 +506,8 @@ def test_rebuild_in_place_under_a_live_handle_is_reloaded(tmp_path, monkeypatch)
             return 8
 
     monkeypatch.setattr(_lib, "Index", FakeIndex)
+    # a registry of its own: handles adopted by earlier tests in this process (HybridSearch.from_loaded) stay registered
+    monkeypatch.setattr(runtime, "_handles", {})
     docs, _, _ = _docs(5, 40)
     rng = np.random.default_rng(0)
     embed = lambda texts: rng.standard_normal((len(texts), 8)).astype(np.float32)      # noqa: E731

@@ -3,22 +3,28 @@
 ``movies.json`` is absent from the reference checkout (.MISSING_LARGE_BLOBS) and sentence-transformers / spaCy /
 sqlite-vec are not installable in the build container, so this known-answer run SKIPS there.  It enables itself
 the day the data and the reference's dependencies are present (set ``RSE_MOVIES_JSON`` or drop the file at
-``data/movies.json`` / ``/root/reference/data/movies.json``): the database is built by the REFERENCE's own build,
-queried through this package's GPU classes, and compared with the 4-decimal values the README prints.
+``data/movies.json`` or at ``data/movies.json`` of the reference checkout, see oracle/ref_import.py): the database
+is built by the REFERENCE's own build, queried through this package's GPU classes, and compared with the 4-decimal
+values the README prints.
 """
 import os
 from pathlib import Path
 
 import pytest
 
+from oracle import ref_import
+
 ROOT = Path(__file__).resolve().parents[1]
 
 
 def _movies_json():
-    for p in (os.environ.get("RSE_MOVIES_JSON"), ROOT / "data" / "movies.json", "/root/reference/data/movies.json",
-              ROOT / "baseline" / "_ref" / "data" / "movies.json"):
-        if p and Path(p).exists():
-            return Path(p)
+    for p in (os.environ.get("RSE_MOVIES_JSON"), ROOT / "data" / "movies.json",
+              ref_import.REFERENCE_ROOT / "data" / "movies.json"):
+        try:
+            if p and Path(p).is_file():
+                return Path(p)
+        except OSError:               # a path this user may not enter counts as absent
+            pass
     return None
 
 

@@ -93,22 +93,31 @@ def test_reference_utils_unit_tests_hold_for_pyref():
     assert [x["id"] for x in pyref.rrf_fuse([], [(2, 0.2), (4, 0.4)], 60, 3)][:2] == [2, 4]
 
 
+def live_fixture():
+    return json.loads((GOLDEN / "live_ref.json").read_text())
+
+
 @pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (GPU box)")
 def test_pyref_matches_live_reference_bm25(tmp_path):
     ref_kw, _, _ = ref_import.load()
-    from oracle.make_golden import make_corpus, make_queries
-    docs, words, weights = make_corpus(77, 120, 40)
-    p = tmp_path / "m.json"
-    p.write_text(json.dumps({"movies": docs}))
-    ks = ref_kw.KeywordSearch.build_from_docs(docs_path=p, db_path=tmp_path / "k.db", force=True)
-    try:
-        postings, doclen = build_postings(docs)
-        for q in make_queries(78, words, weights, 25):
-            ref = [(r["id"], r["score"]) for r in ks.search(q, k=7)]
-            got = pyref.bm25_search(postings, doclen, len(doclen), q.lower().split(), k=7)
-            assert got == ref
-    finally:
-        ks.close()
+    from oracle.make_golden import encode_hits, live_bm25_inputs, reference_bm25
+    docs, queries = live_bm25_inputs()
+    refs = reference_bm25(ref_kw, docs, queries, 7, tmp_path)
+    postings, doclen = build_postings(docs)
+    for q, ref in zip(queries, refs):
+        got = pyref.bm25_search(postings, doclen, len(doclen), q.lower().split(), k=7)
+        assert got == ref
+    assert [encode_hits(h) for h in refs] == live_fixture()["bm25"]["hits"]      # the pinned answers are the reference's
+
+
+def test_pyref_bm25_matches_pinned_live_answers():
+    """test_pyref_matches_live_reference_bm25 against its pinned answers (tests/golden/live_ref.json)."""
+    from oracle.make_golden import encode_hits, live_bm25_inputs
+    docs, queries = live_bm25_inputs()
+    fx = live_fixture()["bm25"]
+    postings, doclen = build_postings(docs)
+    got = [encode_hits(pyref.bm25_search(postings, doclen, len(doclen), q.lower().split(), k=fx["k"])) for q in queries]
+    assert got == fx["hits"]
 
 
 @pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (GPU box)")
@@ -116,56 +125,30 @@ def test_pyref_matches_live_reference_fusion(tmp_path):
     """1500 more random fusion cases than the committed fixture holds, straight against the reference's own
     HybridSearch through its dummy-retriever seam (tests/test_hybrid_search.py:73-76): empty sides, overlapping
     hit lists, huge and negative ids (CPython set order), exact score / distance ties, int and float k."""
-    import random
     _, ref_hs, _ = ref_import.load()
-    rnd = random.Random(2026)
+    from oracle.make_golden import encode_fusion, live_fusion_inputs, reference_fusion
+    cases = live_fusion_inputs()
+    refs = reference_fusion(ref_hs, cases, tmp_path)
+    for case, ((bm, sem, alpha, k, limit), (w, r)) in enumerate(zip(cases, refs)):
+        pw = pyref.weighted_fuse(bm, sem, alpha, limit)
+        pr = pyref.rrf_fuse(bm, sem, k, limit)
+        assert [(x["id"], x["bm25"], x["semantic"], x["score"]) for x in w] == \
+               [(x["id"], x["bm25"], x["semantic"], x["score"]) for x in pw], case
+        assert [(x["id"], x["score"], x["bm25_rank"], x["sem_rank"]) for x in r] == \
+               [(x["id"], x["score"], x["bm25_rank"], x["sem_rank"]) for x in pr], case
+    fx = live_fixture()["fusion"]
+    assert [list(encode_fusion(w, r)) for w, r in refs[::fx["stride"]]] == fx["cases"]
 
-    class KW:
-        hits = []
-        def __init__(self, *a, **k): pass
-        def search(self, query, k=10, k1=1.5, b=0.75): return [dict(h) for h in KW.hits]
-        def close(self): pass
 
-    class SEM:
-        hits = []
-        def __init__(self, *a, **k): pass
-        def query_top_k(self, query_text, k=10, knn_multiplier=10): return [dict(h) for h in SEM.hits]
-        def close(self): pass
-
-    old = ref_hs.KeywordSearch, ref_hs.SemanticSearch
-    ref_hs.KeywordSearch, ref_hs.SemanticSearch = KW, SEM
-    try:
-        hs = ref_hs.HybridSearch(docs_path=None, db_path=tmp_path / "h.db")
-        for case in range(1500):
-            limit = rnd.choice([1, 2, 3, 5, 10, 10, 20])
-            space = rnd.choice([3 * limit + 2, 70, 10**6, 2**40, 2**62])
-            nb, ns = rnd.randint(0, limit), rnd.randint(0, limit)
-            bids = rnd.sample(range(-3 if space > 70 else 0, space), nb) if nb else []
-            pool = [i for i in bids]
-            sids = []
-            while len(sids) < ns:
-                c = pool.pop(rnd.randrange(len(pool))) if pool and rnd.random() < 0.5 else rnd.randrange(space)
-                if c not in sids:
-                    sids.append(c)
-            bs = [rnd.choice([rnd.uniform(0.1, 30.0), float(rnd.randint(1, 3))]) for _ in bids]
-            ds = [float(np.float32(rnd.choice([rnd.uniform(0.0, 1.4), rnd.randint(0, 4) / 8.0]))) for _ in sids]
-            bs.sort(reverse=True); ds.sort()
-            alpha = rnd.choice([0.0, 0.3, 0.5, 1.0, rnd.random()])
-            k = rnd.choice([60, 60.0, 1, 0.5, 1000])
-            KW.hits = [{"id": i, "title": "t", "description": "d", "score": s} for i, s in zip(bids, bs)]
-            SEM.hits = [{"chunk_id": 0, "distance": d, "chunk": "", "movie_id": i, "title": "t", "description": "d"}
-                        for i, d in zip(sids, ds)]
-            w = hs.weighted_search("q", alpha=alpha, limit=limit)
-            r = hs.rrf_search("q", k=k, limit=limit)
-            pw = pyref.weighted_fuse(list(zip(bids, bs)), list(zip(sids, ds)), alpha, limit)
-            pr = pyref.rrf_fuse(list(zip(bids, bs)), list(zip(sids, ds)), k, limit)
-            assert [(x["id"], x["bm25"], x["semantic"], x["score"]) for x in w] == \
-                   [(x["id"], x["bm25"], x["semantic"], x["score"]) for x in pw], case
-            assert [(x["id"], x["score"], x["bm25_rank"], x["sem_rank"]) for x in r] == \
-                   [(x["id"], x["score"], x["bm25_rank"], x["sem_rank"]) for x in pr], case
-        hs.close()
-    finally:
-        ref_hs.KeywordSearch, ref_hs.SemanticSearch = old
+def test_pyref_fusion_matches_pinned_live_answers():
+    """test_pyref_matches_live_reference_fusion against its pinned answers: every stride-th of its cases."""
+    from oracle.make_golden import encode_fusion, live_fusion_inputs
+    fx = live_fixture()["fusion"]
+    cases = live_fusion_inputs()[::fx["stride"]]
+    assert len(cases) == len(fx["cases"]) == 300
+    for i, ((bm, sem, alpha, k, limit), want) in enumerate(zip(cases, fx["cases"])):
+        got = encode_fusion(pyref.weighted_fuse(bm, sem, alpha, limit), pyref.rrf_fuse(bm, sem, k, limit))
+        assert list(got) == want, i
 
 
 def test_vec0_literal_scan_equals_key_order():
