@@ -281,6 +281,33 @@ int rse_encode(rse_index *h, int32_t slot, const int32_t *ids, const int32_t *ty
                int32_t n_seq, float *out_host);
 int rse_encode_dev(rse_index *h, int32_t slot, const int32_t *ids, const int32_t *type_ids,
                    const int32_t *cu_seqlens, int32_t n_seq, float *out_dev);
+
+/* ------------------------------------------------------------------ §10 f4: the CLIP towers of the image search
+ * The reference's MultimodalSearch runs SentenceTransformer("clip-ViT-B-32") (llm/multimodal.py:35-42 encodes every
+ * document text, :46-58 every query image): HuggingFace CLIPTextModelWithProjection / CLIPVisionModelWithProjection,
+ * fp32, output not normalised.  rse_clip_create puts one tower into an encoder slot (csrc/clip.cuh); the slot then
+ * takes rse_encoder_set_tensor (names "vision_model.*" + "visual_projection.weight", or "text_model.*" +
+ * "text_projection.weight"; q / k / v projections are fused on the device; a prefix such as "model." is ignored),
+ * rse_encoder_finalize (fails while a tensor is missing) and rse_encoder_set_mode like a BERT slot.
+ *   text tower   : rse_encode / rse_encode_dev with type_ids = NULL -> [n_seq, projection_dim]; sequences of
+ *                  1 .. max_positions tokens (truncate on the host).  The pooled token follows transformers:
+ *                  eos_token_id == 2 -> first argmax of the ids, else first position of eos_token_id (0 if none).
+ *   vision tower : rse_encode_images(_dev) with the image processor's pixel_values [n, 3, image_size, image_size]
+ *                  (NCHW fp32) -> [n, projection_dim].
+ * Shapes: hidden % 32 == 0 and <= 1024, head_dim 32 or 64, image_size % patch_size == 0, at most RSE_CLIP_MAX_TOKENS
+ * tokens per sequence (text max_positions, vision (image_size / patch_size)^2 + 1); else RSE_ERR_UNSUPPORTED. */
+#define RSE_CLIP_MAX_TOKENS 1024
+typedef struct rse_clip_config {
+  int32_t tower; /* 0 = vision, 1 = text */
+  int32_t hidden, layers, heads, intermediate, projection_dim;
+  int32_t vocab_size, max_positions;  /* text */
+  int32_t image_size, patch_size;     /* vision */
+  int32_t eos_token_id;               /* text */
+  float ln_eps;
+} rse_clip_config;
+int rse_clip_create(rse_index *h, int32_t slot, const rse_clip_config *cfg);
+int rse_encode_images(rse_index *h, int32_t slot, const float *pixels_host, int32_t n, float *out_host);
+int rse_encode_images_dev(rse_index *h, int32_t slot, const float *pixels_dev, int32_t n, float *out_dev);
 /* rse_hybrid_stage with the query vectors already ON THE DEVICE ([nq, dim] fp32, e.g. rse_encode_dev's output);
  * tokens still come from the host.  Followed by rse_hybrid_run / rse_hybrid_fetch as usual. */
 int rse_hybrid_stage_dev(rse_index *h, int32_t nq, const float *q_dev, const int32_t *tok_indptr,

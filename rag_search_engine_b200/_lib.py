@@ -63,6 +63,14 @@ class RseEncoderConfig(ctypes.Structure):
                 ("ln_eps", c_float), ("head", c_int32)]
 
 
+class RseClipConfig(ctypes.Structure):
+    """include/rse.h rse_clip_config."""
+    _fields_ = [("tower", c_int32), ("hidden", c_int32), ("layers", c_int32), ("heads", c_int32),
+                ("intermediate", c_int32), ("projection_dim", c_int32), ("vocab_size", c_int32),
+                ("max_positions", c_int32), ("image_size", c_int32), ("patch_size", c_int32),
+                ("eos_token_id", c_int32), ("ln_eps", c_float)]
+
+
 _SIGNATURES = {
     "rse_abi_version": (ctypes.c_int, []),
     "rse_create": (ctypes.c_int, [c_int32, POINTER(c_void_p)]),
@@ -126,6 +134,9 @@ _SIGNATURES = {
                                   POINTER(c_float)]),
     "rse_encode_dev": (ctypes.c_int, [c_void_p, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_int32), c_int32,
                                       c_void_p]),
+    "rse_clip_create": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseClipConfig)]),
+    "rse_encode_images": (ctypes.c_int, [c_void_p, c_int32, POINTER(c_float), c_int32, POINTER(c_float)]),
+    "rse_encode_images_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
     "rse_hybrid_stage_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "rse_comm_unique_id": (ctypes.c_int, [c_void_p]),
     "rse_comm_init": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32]),
@@ -487,6 +498,34 @@ class Index:
         self._check(self._L.rse_encoder_create(self._h, int(slot), ctypes.byref(cfg)))
         self.__dict__.setdefault("_enc_cfg", {})[int(slot)] = cfg
 
+    def clip_create(self, slot: int, *, tower: int, hidden: int, layers: int, heads: int, intermediate: int,
+                    projection_dim: int, ln_eps: float, vocab_size: int = 0, max_positions: int = 0,
+                    image_size: int = 0, patch_size: int = 0, eos_token_id: int = 0):
+        """A CLIP tower (0 = vision, 1 = text) in encoder slot ``slot``; weights then go through encoder_set_tensor /
+        encoder_finalize like a BERT slot's."""
+        cfg = RseClipConfig(int(tower), int(hidden), int(layers), int(heads), int(intermediate), int(projection_dim),
+                            int(vocab_size), int(max_positions), int(image_size), int(patch_size), int(eos_token_id),
+                            float(ln_eps))
+        self._check(self._L.rse_clip_create(self._h, int(slot), ctypes.byref(cfg)))
+        self.__dict__.setdefault("_enc_cfg", {})[int(slot)] = cfg
+
+    def encode_images(self, slot: int, pixel_values):
+        """pixel_values [n, 3, S, S] float32 (NCHW, the image processor's output) -> [n, projection_dim] float32."""
+        px = _c(pixel_values, np.float32)
+        if px.ndim != 4 or px.shape[1] != 3:
+            raise ValueError("pixel_values must be [n, 3, image_size, image_size]")
+        cfg = self._enc_cfg.get(int(slot))
+        if isinstance(cfg, RseClipConfig) and cfg.tower == 0 and px.shape[2:] != (cfg.image_size, cfg.image_size):
+            raise ValueError(f"pixel_values must be {cfg.image_size} x {cfg.image_size} (the tower's image_size)")
+        n = px.shape[0]
+        out = np.zeros((n, cfg.projection_dim if isinstance(cfg, RseClipConfig) else 1), np.float32)
+        self._check(self._L.rse_encode_images(self._h, int(slot), _ptr(px, c_float), n, _ptr(out, c_float)))
+        return out
+
+    def encode_images_dev(self, slot: int, pixels_ptr: int, n: int, out_ptr: int):
+        """Same with the pixels on the device and the result left there (asynchronous on the handle's stream)."""
+        self._check(self._L.rse_encode_images_dev(self._h, int(slot), c_void_p(pixels_ptr), int(n), c_void_p(out_ptr)))
+
     def encoder_set_tensor(self, slot: int, name: str, data):
         a = _c(data, np.float32).reshape(-1)
         self._check(self._L.rse_encoder_set_tensor(self._h, int(slot), name.encode(), _ptr(a, c_float), a.size))
@@ -507,11 +546,15 @@ class Index:
         return ids, tt, cu
 
     def encode(self, slot: int, ids, cu_seqlens, type_ids=None):
-        """Packed token ids -> [n_seq, hidden] float32 (head 0) or [n_seq] logits (head 1), on the host."""
+        """Packed token ids -> [n_seq, hidden] float32 (head 0), [n_seq] logits (head 1) or [n_seq, projection_dim]
+        (CLIP text tower), on the host."""
         ids, tt, cu = self._enc_inputs(ids, type_ids, cu_seqlens)
         cfg = self._enc_cfg[int(slot)]
         n_seq = cu.size - 1
-        out = np.zeros((n_seq, cfg.hidden) if cfg.head == 0 else (n_seq,), np.float32)
+        if isinstance(cfg, RseClipConfig):
+            out = np.zeros((n_seq, cfg.projection_dim), np.float32)
+        else:
+            out = np.zeros((n_seq, cfg.hidden) if cfg.head == 0 else (n_seq,), np.float32)
         self._check(self._L.rse_encode(self._h, int(slot), _ptr(ids, c_int32), _ptr(tt, c_int32), _ptr(cu, c_int32),
                                        n_seq, _ptr(out, c_float)))
         return out

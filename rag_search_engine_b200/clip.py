@@ -1,0 +1,163 @@
+"""The CLIP model of the image search on the GPU (§10 f4).
+
+``GpuClipModel`` stands in for ``SentenceTransformer("clip-ViT-B-32")`` where ``MultimodalSearch`` uses it
+(llm/multimodal.py:35-42 encodes every document text, :46-58 every query image): pass it as
+``MultimodalSearch(documents, model=GpuClipModel(...))``.  Both towers run csrc/clip.cuh through the C-ABI
+(``rse_clip_create``, ``rse_encode`` for text, ``rse_encode_images`` for images) in fp32; the output is what
+sentence-transformers' CLIP ``encode`` returns: ``get_text_features`` / ``get_image_features``, not normalised.
+
+Tokenisation (BPE) and image decoding / resizing / cropping stay on the host: the tokenizer is any callable
+``texts -> token-id lists`` (or a HuggingFace tokenizer), the image processor any callable ``images ->
+pixel_values [n, 3, S, S]`` (or a HuggingFace image processor).  ``from_sentence_transformer`` takes the weights,
+the tokenizer and the image processor from a loaded reference model.  No weights are bundled and nothing is
+downloaded.
+"""
+from __future__ import annotations
+
+from typing import Iterator, Optional, Sequence, Tuple
+
+import numpy as np
+
+from .encoder import pack
+
+VISION_SLOT, TEXT_SLOT = 0, 1
+_TOWER_KEYS = {0: ("vision_model.", "visual_projection."), 1: ("text_model.", "text_projection.")}
+
+
+def _vision_config(v, projection_dim: int) -> dict:
+    if getattr(v, "hidden_act", "quick_gelu") != "quick_gelu":
+        raise ValueError(f"CLIP vision tower: only hidden_act='quick_gelu' is implemented, not {v.hidden_act!r}")
+    if getattr(v, "num_channels", 3) != 3:
+        raise ValueError("CLIP vision tower: only 3-channel images are implemented")
+    if v.image_size % v.patch_size:
+        raise ValueError("CLIP vision tower: image_size must be a multiple of patch_size")
+    return dict(tower=0, hidden=v.hidden_size, layers=v.num_hidden_layers, heads=v.num_attention_heads,
+                intermediate=v.intermediate_size, projection_dim=int(projection_dim), image_size=v.image_size,
+                patch_size=v.patch_size, ln_eps=v.layer_norm_eps)
+
+
+def _text_config(t, projection_dim: int) -> dict:
+    if getattr(t, "hidden_act", "quick_gelu") != "quick_gelu":
+        raise ValueError(f"CLIP text tower: only hidden_act='quick_gelu' is implemented, not {t.hidden_act!r}")
+    return dict(tower=1, hidden=t.hidden_size, layers=t.num_hidden_layers, heads=t.num_attention_heads,
+                intermediate=t.intermediate_size, projection_dim=int(projection_dim), vocab_size=t.vocab_size,
+                max_positions=t.max_position_embeddings, eos_token_id=int(t.eos_token_id), ln_eps=t.layer_norm_eps)
+
+
+def clip_configs_from_hf(cfg) -> Tuple[Optional[dict], Optional[dict]]:
+    """transformers ``CLIPConfig`` -> ``(vision, text)`` keyword arguments of ``Index.clip_create``; a
+    ``CLIPVisionConfig`` or ``CLIPTextConfig`` alone gives ``(vision, None)`` / ``(None, text)``.  A CLIPModel
+    projects both towers to the top-level ``projection_dim``.  Raises ValueError for what is not implemented."""
+    if hasattr(cfg, "vision_config") and hasattr(cfg, "text_config"):
+        pd = cfg.projection_dim
+        return _vision_config(cfg.vision_config, pd), _text_config(cfg.text_config, pd)
+    model_type = getattr(cfg, "model_type", "")
+    if model_type == "clip_vision_model":
+        return _vision_config(cfg, cfg.projection_dim), None
+    if model_type == "clip_text_model":
+        return None, _text_config(cfg, cfg.projection_dim)
+    raise ValueError(f"not a CLIP config: {type(cfg).__name__}")
+
+
+def tower_tensors(state_dict, tower: int) -> Iterator[Tuple[str, np.ndarray]]:
+    """The float tensors of one tower (0 = vision, 1 = text) of a CLIPModel / CLIP*ModelWithProjection state_dict,
+    as float32 arrays; the other tower, ``logit_scale`` and the integer ``position_ids`` buffers are left out."""
+    keys = _TOWER_KEYS[int(tower)]
+    for name, t in state_dict.items():
+        if not any(k in name for k in keys) or name.endswith("position_ids"):
+            continue
+        a = t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+        if a.dtype.kind != "f":
+            continue
+        yield name, a.astype(np.float32, copy=False)
+
+
+def _is_image(x) -> bool:
+    return not isinstance(x, (str, bytes)) and hasattr(x, "size") and hasattr(x, "mode")      # a PIL image
+
+
+class GpuClipModel:
+    """``encode(items) -> float32[n, projection_dim]`` like sentence-transformers' CLIP model: strings through the
+    text tower, PIL images through the vision tower, a mixed list split and returned in input order."""
+
+    def __init__(self, index, state_dict, vision_config: dict, text_config: dict, tokenizer=None,
+                 image_processor=None, *, vision_slot: int = VISION_SLOT, text_slot: int = TEXT_SLOT):
+        if vision_config["projection_dim"] != text_config["projection_dim"]:
+            raise ValueError("the two towers must project to the same projection_dim")
+        self.index, self.vision_slot, self.text_slot = index, int(vision_slot), int(text_slot)
+        self.vision_config, self.text_config = dict(vision_config, tower=0), dict(text_config, tower=1)
+        self.tokenizer, self.image_processor = tokenizer, image_processor
+        self.max_positions = int(self.text_config["max_positions"])
+        sd = dict(state_dict)
+        for slot, cfg in ((self.vision_slot, self.vision_config), (self.text_slot, self.text_config)):
+            index.clip_create(slot, **cfg)
+            for name, a in tower_tensors(sd, cfg["tower"]):
+                index.encoder_set_tensor(slot, name, a)
+            index.encoder_finalize(slot)
+
+    @classmethod
+    def from_sentence_transformer(cls, index, st_model, **kw) -> "GpuClipModel":
+        """From a loaded ``SentenceTransformer("clip-ViT-B-32")`` (llm/multimodal.py:28): its transformers
+        ``CLIPModel`` weights, its processor's tokenizer (truncating to the text tower's length, as the
+        processor does) and its image processor."""
+        mod = st_model[0]
+        model, proc = mod.model, mod.processor
+        vision, text = clip_configs_from_hf(model.config)
+        ml = int(text["max_positions"])
+        tok = lambda texts: proc.tokenizer(list(texts), truncation=True, max_length=ml)["input_ids"]   # noqa: E731
+        img = lambda images: proc.image_processor(list(images), return_tensors="np")["pixel_values"]   # noqa: E731
+        return cls(index, model.state_dict(), vision, text, tok, img, **kw)
+
+    def get_sentence_embedding_dimension(self) -> int:
+        return int(self.text_config["projection_dim"])
+
+    def encode_ids(self, id_lists: Sequence[Sequence[int]], max_tokens_per_call: int = 1 << 16) -> np.ndarray:
+        """Token-id lists -> text embeddings.  Sequences are cut to max_positions; a bulk input (the document texts
+        of an index build) goes through in slices of at most ``max_tokens_per_call`` tokens."""
+        mp = self.max_positions
+        id_lists = [x if len(x) <= mp else list(x)[:mp] for x in id_lists]
+        out = np.empty((len(id_lists), self.get_sentence_embedding_dimension()), np.float32)
+        lo = 0
+        while lo < len(id_lists):
+            hi, tok = lo, 0
+            while hi < len(id_lists) and (hi == lo or tok + len(id_lists[hi]) <= max_tokens_per_call):
+                tok += len(id_lists[hi]); hi += 1
+            ids, _, cu = pack(id_lists[lo:hi])
+            out[lo:hi] = self.index.encode(self.text_slot, ids, cu)
+            lo = hi
+        return out
+
+    def encode_pixels(self, pixel_values, max_images_per_call: int = 256) -> np.ndarray:
+        """pixel_values [n, 3, S, S] (the image processor's output) -> image embeddings, in slices of
+        ``max_images_per_call`` images."""
+        px = np.ascontiguousarray(pixel_values, np.float32)
+        out = np.empty((px.shape[0], self.get_sentence_embedding_dimension()), np.float32)
+        for lo in range(0, px.shape[0], max_images_per_call):
+            out[lo:lo + max_images_per_call] = self.index.encode_images(self.vision_slot, px[lo:lo + max_images_per_call])
+        return out
+
+    def _tokenize(self, texts):
+        if self.tokenizer is None:
+            raise RuntimeError("GpuClipModel has no tokenizer: pass tokenizer=<texts -> token-id lists> "
+                               "(e.g. the reference model's CLIP tokenizer) or call encode_ids")
+        ids = self.tokenizer(list(texts))
+        return ids["input_ids"] if hasattr(ids, "keys") else ids
+
+    def _preprocess(self, images):
+        if self.image_processor is None:
+            raise RuntimeError("GpuClipModel has no image processor: pass image_processor=<images -> pixel_values> "
+                               "(e.g. the reference model's CLIP image processor) or call encode_pixels")
+        px = self.image_processor(list(images))
+        return np.asarray(px["pixel_values"] if hasattr(px, "keys") else px, np.float32)
+
+    def encode(self, items, convert_to_numpy: bool = True, show_progress_bar: bool = False, **_kw) -> np.ndarray:
+        single = isinstance(items, str) or _is_image(items)
+        items = [items] if single else list(items)
+        out = np.empty((len(items), self.get_sentence_embedding_dimension()), np.float32)
+        img_at = [i for i, x in enumerate(items) if _is_image(x)]
+        txt_at = [i for i, x in enumerate(items) if not _is_image(x)]
+        if txt_at:
+            out[txt_at] = self.encode_ids(self._tokenize([items[i] for i in txt_at]))
+        if img_at:
+            out[img_at] = self.encode_pixels(self._preprocess([items[i] for i in img_at]))
+        return out[0] if single else out

@@ -123,10 +123,13 @@ enc_add_ln_kernel(const float* __restrict__ x, const float* __restrict__ residua
 // ---------------------------------------------------------------- GEMM: C[M, N] = A[M, K] . W[N, K]^T + bias
 // (torch.nn.Linear layout: both operands K-contiguous.)  fp32 SIMT, fmaf accumulation: 128 x 128 x 16 tiles, 256
 // threads, 8 x 8 outputs per thread as two 4-wide groups in each dimension (conflict-free float4 reads of the
-// k-major shared tiles), register-prefetched double buffering.  K % 16 == 0.  EPI: 0 = bias, 1 = bias + GELU(erf).
+// k-major shared tiles), register-prefetched double buffering.  K % 16 == 0.  EPI: 0 = bias, 1 = bias + GELU(erf),
+// 2 = bias + quick_gelu (CLIP, clip.cuh).
 constexpr int kGemmBM = 128, kGemmBN = 128, kGemmBK = 16, kGemmPad = 4;
 
 __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f)); }
+// transformers' QuickGELUActivation: x * sigmoid(1.702 x)
+__device__ __forceinline__ float quick_gelu(float x) { return x * (1.0f / (1.0f + expf(-1.702f * x))); }
 
 template <int EPI>
 __global__ void __launch_bounds__(256, 2)
@@ -200,6 +203,7 @@ enc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ W, const 
         if (gn + j < N) {
           float v = acc[i][jg * 4 + j] + bias[gn + j];
           if (EPI == 1) v = gelu_erf(v);
+          if (EPI == 2) v = quick_gelu(v);
           C[static_cast<int64_t>(gm) * N + gn + j] = v;
         }
       }
@@ -211,8 +215,9 @@ enc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ W, const 
 // qkv: packed [T, 3*hidden] rows = [q | k | v], head h at columns h*HD.  One CTA per (sequence, head) of 32..256 threads (the
 // longest sequence of the batch, rse.cu): thread t owns query row t (+blockDim, ... for longer sequences), keys / values stream through shared memory 64 at a time;
 // online softmax (running max / sum), fp32, expf.  Keys beyond the sequence do not exist in the packed layout, which
-// IS the reference's padding mask (BertModel's extended attention mask adds -inf to padded keys).
-template <int HD>
+// IS the reference's padding mask (BertModel's extended attention mask adds -inf to padded keys).  CAUSAL (the CLIP
+// text tower): query i of a sequence attends to its keys j <= i only.
+template <int HD, bool CAUSAL = false>
 __global__ void __launch_bounds__(256)
 enc_attention_kernel(const float* __restrict__ qkv, const int32_t* __restrict__ cu_seqlens, int hidden,
                      float* __restrict__ ctx, float* __restrict__ ctx_lo) {   // ctx_lo != NULL: ctx <- hi, ctx_lo <- lo
@@ -246,7 +251,8 @@ enc_attention_kernel(const float* __restrict__ qkv, const int32_t* __restrict__ 
       }
       __syncthreads();
       if (active) {
-        for (int j = 0; j < nk; ++j) {
+        const int jn = CAUSAL ? min(nk, qi - k0 + 1) : nk;
+        for (int j = 0; j < jn; ++j) {
           float s = 0.0f;
 #pragma unroll
           for (int d = 0; d < HD; ++d) s = fmaf(q[d], sK[j][d], s);
@@ -432,6 +438,7 @@ __device__ __forceinline__ void eg_mma_tf32(uint32_t tmem_d, uint64_t adesc, uin
 }
 
 // EPI 0: C = acc + bias (fp32).  EPI 1: g = GELU(acc + bias) -> C_hi / C_lo (the operand of the next GEMM).
+// EPI 2: the same with quick_gelu (CLIP).
 template <int EPI, int BN>
 __global__ void __launch_bounds__(kEgThreads, BN == 128 ? 1 : 2)
 enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_constant__ CUtensorMap tmap_a_lo,
@@ -553,22 +560,24 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
       if (row < M) {
         const int col = n0 + c0;
         float* dst = C + static_cast<int64_t>(row) * N + col;
-        float* dst_lo = (EPI == 1) ? C_lo + static_cast<int64_t>(row) * N + col : nullptr;
+        float* dst_lo = (EPI != 0) ? C_lo + static_cast<int64_t>(row) * N + col : nullptr;
 #pragma unroll
         for (int j = 0; j < 32; j += 4) {
           float o[4], l[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
             float x = (acc[c0 + j + e] + __uint_as_float(v[j + e])) + (col + j + e < N ? __ldg(bias + col + j + e) : 0.0f);
-            if (EPI == 1) { x = gelu_erf(x); tf32_split(x, o[e], l[e]); } else { o[e] = x; }
+            if (EPI == 1) { x = gelu_erf(x); tf32_split(x, o[e], l[e]); }
+            else if (EPI == 2) { x = quick_gelu(x); tf32_split(x, o[e], l[e]); }
+            else { o[e] = x; }
           }
           if (col + j + 3 < N) {
             *reinterpret_cast<float4*>(dst + j) = make_float4(o[0], o[1], o[2], o[3]);
-            if (EPI == 1) *reinterpret_cast<float4*>(dst_lo + j) = make_float4(l[0], l[1], l[2], l[3]);
+            if (EPI != 0) *reinterpret_cast<float4*>(dst_lo + j) = make_float4(l[0], l[1], l[2], l[3]);
           } else {
 #pragma unroll
             for (int e = 0; e < 4; ++e)
-              if (col + j + e < N) { dst[j + e] = o[e]; if (EPI == 1) dst_lo[j + e] = l[e]; }
+              if (col + j + e < N) { dst[j + e] = o[e]; if (EPI != 0) dst_lo[j + e] = l[e]; }
           }
         }
       }

@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "bm25.cuh"
+#include "clip.cuh"
 #include "comm.h"
 #include "common.cuh"
 #include "encoder.cuh"
@@ -61,6 +62,17 @@ struct Encoder {
   cudaEvent_t pin_ev[2] = {nullptr, nullptr};
   int pin_next = 0;
   int max_len = 128;                  // longest sequence of the batch being encoded (sizes the attention CTA)
+  // ---- §10 f4: a CLIP tower in this slot (rse_clip_create, clip.cuh).  word = token_embedding, pos =
+  // position_embedding, elng / elnb = pre_layrnorm; layer ln1 / ln2 = layer_norm1 / layer_norm2 (pre-LN), wi / wo2 =
+  // mlp.fc1 / fc2.  The patch weight is [hidden, patch_k] with its columns zero-padded to a multiple of 128.
+  bool clip = false;
+  rse_clip_config ccfg{};
+  int patch_k = 0;
+  float *cls_emb = nullptr, *patch_w = nullptr, *patch_w_h = nullptr, *patch_w_l = nullptr;
+  float *flng = nullptr, *flnb = nullptr, *proj = nullptr, *zero_bias = nullptr;
+  DevBuf y, pix, patch, patch_l;      // LayerNorm output (the GEMM operand), device pixels, patch rows (+ lo half)
+  float* pin_px[2] = {nullptr, nullptr};
+  size_t pin_px_n[2] = {0, 0};
 };
 
 }  // namespace
@@ -305,6 +317,8 @@ void release_bm25(rse_index* h) {
 
 void enc_release(Encoder& e) {
   for (float** p : {&e.word, &e.pos, &e.type, &e.elng, &e.elnb, &e.poolw, &e.poolb, &e.clsw, &e.clsb}) free_ptr(*p);
+  for (float** p : {&e.cls_emb, &e.patch_w, &e.patch_w_h, &e.patch_w_l, &e.flng, &e.flnb, &e.proj, &e.zero_bias}) free_ptr(*p);
+  for (DevBuf* b : {&e.y, &e.pix, &e.patch, &e.patch_l}) free_buf(*b);
   for (auto& l : e.layers)
     for (float** p : {&l.wqkv, &l.bqkv, &l.wo, &l.bo, &l.ln1g, &l.ln1b, &l.wi, &l.bi, &l.wo2, &l.bo2, &l.ln2g, &l.ln2b,
                       &l.wqkv_h, &l.wqkv_l, &l.wo_h, &l.wo_l, &l.wi_h, &l.wi_l, &l.wo2_h, &l.wo2_l}) free_ptr(*p);
@@ -316,8 +330,10 @@ void enc_release(Encoder& e) {
     if (e.pin_in[i]) cudaFreeHost(e.pin_in[i]);
     if (e.pin_ev[i]) cudaEventDestroy(e.pin_ev[i]);
     e.pin_in[i] = nullptr; e.pin_in_n[i] = 0; e.pin_ev[i] = nullptr;
+    if (e.pin_px[i]) cudaFreeHost(e.pin_px[i]);
+    e.pin_px[i] = nullptr; e.pin_px_n[i] = 0;
   }
-  e.created = e.finalized = false;
+  e.created = e.finalized = e.clip = false;
 }
 
 // ------------------------------------------------------------------ scan launch
@@ -2155,7 +2171,7 @@ int make_tmap_f32(rse_index* h, CUtensorMap* out, const float* base, int64_t row
   return RSE_OK;
 }
 
-// tensor-core GEMM: C[M, N] = (A_hi + A_lo)[M, K] . (W_hi + W_lo)[N, K]^T + bias; EPI 1: GELU -> C (hi), C_lo
+// tensor-core GEMM: C[M, N] = (A_hi + A_lo)[M, K] . (W_hi + W_lo)[N, K]^T + bias; EPI 1 / 2: GELU / quick_gelu -> C (hi), C_lo
 extern "C++" {
 template <int EPI>
 int enc_gemm_tc(rse_index* h, const float* A_hi, const float* A_lo, const float* W_hi, const float* W_lo, const float* bias,
@@ -2165,6 +2181,8 @@ int enc_gemm_tc(rse_index* h, const float* A_hi, const float* A_lo, const float*
     CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<1, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(128)));
     CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<0, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
     CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
+    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<2, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(128)));
+    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
     h->attr_mask |= 1u << 17;
   }
   // 64-wide tiles, two CTAs per SM (r02, 256 queries / 2.5 k tokens, ms per host-buffer encode call: 64-wide
@@ -2261,6 +2279,141 @@ int enc_forward(rse_index* h, Encoder& e, int n_seq, int T, bool has_types, floa
   return RSE_OK;
 }
 
+// ---- §10 f4: the CLIP towers (clip.cuh).  Scratch for T tokens; y_h / y_l live in x_h / x_l.
+int clip_buffers(rse_index* h, Encoder& e, int T, bool tc) {
+  const size_t H = e.ccfg.hidden, I = e.ccfg.intermediate, t = static_cast<size_t>(T);
+  ENSURE(e.x, sizeof(float) * t * H);
+  ENSURE(e.y, sizeof(float) * t * H);
+  ENSURE(e.qkv, sizeof(float) * t * 3 * H);
+  ENSURE(e.ctx, sizeof(float) * t * H);
+  ENSURE(e.tmp, sizeof(float) * t * H);
+  ENSURE(e.ff, sizeof(float) * t * I);
+  if (tc) {
+    ENSURE(e.x_h, sizeof(float) * t * H);
+    ENSURE(e.x_l, sizeof(float) * t * H);
+    ENSURE(e.ctx_l, sizeof(float) * t * H);
+    ENSURE(e.ff_l, sizeof(float) * t * I);
+  }
+  return RSE_OK;
+}
+
+// the pre-LN layers: on entry x = the embeddings and y = layer 0's layer_norm1(x); on exit x = the last hidden state
+int clip_layers(rse_index* h, Encoder& e, int n_seq, int T, bool tc, bool causal) {
+  const rse_clip_config& c = e.ccfg;
+  const int H = c.hidden, I = c.intermediate, hd = H / c.heads;
+  float* x = static_cast<float*>(e.x.p);
+  float* y = static_cast<float*>(e.y.p);
+  float* qkv = static_cast<float*>(e.qkv.p);
+  float* ctx = static_cast<float*>(e.ctx.p);
+  float* tmp = static_cast<float*>(e.tmp.p);
+  float* ff = static_cast<float*>(e.ff.p);
+  float* y_h = tc ? static_cast<float*>(e.x_h.p) : nullptr;
+  float* y_l = tc ? static_cast<float*>(e.x_l.p) : nullptr;
+  float* ctx_l = tc ? static_cast<float*>(e.ctx_l.p) : nullptr;
+  float* ff_l = tc ? static_cast<float*>(e.ff_l.p) : nullptr;
+  const int32_t* cu = static_cast<const int32_t*>(e.cu.p);
+  const int tok_grid = (T + 3) / 4;
+  for (size_t li = 0; li < e.layers.size(); ++li) {
+    const EncLayer& l = e.layers[li];
+    int rc = tc ? enc_gemm_tc<0>(h, y_h, y_l, l.wqkv_h, l.wqkv_l, l.bqkv, qkv, nullptr, T, 3 * H, H)
+                : enc_gemm<0>(h, y, l.wqkv, l.bqkv, qkv, T, 3 * H, H);
+    if (rc != RSE_OK) return rc;
+    dim3 agrid(n_seq, c.heads);
+    const int acap = static_cast<int64_t>(n_seq) * c.heads < 2ll * h->sm_count ? 256 : 128;   // as enc_forward
+    const int athreads = std::min(acap, std::max(32, (e.max_len + 31) / 32 * 32));
+    if (hd == 32) {
+      if (causal) enc_attention_kernel<32, true><<<agrid, athreads, 0, h->stream>>>(qkv, cu, H, ctx, ctx_l);
+      else enc_attention_kernel<32><<<agrid, athreads, 0, h->stream>>>(qkv, cu, H, ctx, ctx_l);
+    } else {
+      if (causal) enc_attention_kernel<64, true><<<agrid, athreads, 0, h->stream>>>(qkv, cu, H, ctx, ctx_l);
+      else enc_attention_kernel<64><<<agrid, athreads, 0, h->stream>>>(qkv, cu, H, ctx, ctx_l);
+    }
+    LAUNCHED(h);
+    rc = tc ? enc_gemm_tc<0>(h, ctx, ctx_l, l.wo_h, l.wo_l, l.bo, tmp, nullptr, T, H, H)
+            : enc_gemm<0>(h, ctx, l.wo, l.bo, tmp, T, H, H);
+    if (rc != RSE_OK) return rc;
+    clip_residual_ln_kernel<<<tok_grid, 128, 0, h->stream>>>(x, tmp, T, H, l.ln2g, l.ln2b, c.ln_eps, y, y_h, y_l);
+    LAUNCHED(h);
+    rc = tc ? enc_gemm_tc<2>(h, y_h, y_l, l.wi_h, l.wi_l, l.bi, ff, ff_l, T, I, H)
+            : enc_gemm<2>(h, y, l.wi, l.bi, ff, T, I, H);
+    if (rc != RSE_OK) return rc;
+    rc = tc ? enc_gemm_tc<0>(h, ff, ff_l, l.wo2_h, l.wo2_l, l.bo2, tmp, nullptr, T, H, I)
+            : enc_gemm<0>(h, ff, l.wo2, l.bo2, tmp, T, H, I);
+    if (rc != RSE_OK) return rc;
+    const EncLayer* nx = li + 1 < e.layers.size() ? &e.layers[li + 1] : nullptr;    // the next layer's layer_norm1
+    clip_residual_ln_kernel<<<tok_grid, 128, 0, h->stream>>>(x, tmp, T, H, nx ? nx->ln1g : nullptr,
+                                                             nx ? nx->ln1b : nullptr, c.ln_eps, y, y_h, y_l);
+    LAUNCHED(h);
+  }
+  return RSE_OK;
+}
+
+// pixels_dev [n, 3, S, S] on the device -> out_dev [n, projection_dim]
+int clip_vision_forward(rse_index* h, Encoder& e, int n, const float* pixels_dev, float* out_dev) {
+  const rse_clip_config& c = e.ccfg;
+  const int H = c.hidden, S = c.image_size, P = c.patch_size, G = S / P, L = G * G + 1, Kp = e.patch_k;
+  const int T = n * L, Mp = n * G * G;
+  const bool tc = e.mode == 0 && e.tc_ok;
+  int rc = clip_buffers(h, e, T, tc);
+  if (rc != RSE_OK) return rc;
+  ENSURE(e.cu, sizeof(int32_t) * (n + 1));
+  ENSURE(e.patch, sizeof(float) * static_cast<size_t>(Mp) * Kp);
+  if (tc) ENSURE(e.patch_l, sizeof(float) * static_cast<size_t>(Mp) * Kp);
+  int32_t* cu = static_cast<int32_t*>(e.cu.p);
+  float* patch = static_cast<float*>(e.patch.p);
+  float* tmp = static_cast<float*>(e.tmp.p);
+  clip_fixed_cu_kernel<<<(n + 256) / 256, 256, 0, h->stream>>>(n, L, cu);
+  LAUNCHED(h);
+  const int64_t n_elem = static_cast<int64_t>(Mp) * Kp;
+  clip_patchify_kernel<<<static_cast<unsigned int>((n_elem + 255) / 256), 256, 0, h->stream>>>(
+      pixels_dev, n_elem, S, P, G, Kp, tc ? nullptr : patch, tc ? patch : nullptr,
+      tc ? static_cast<float*>(e.patch_l.p) : nullptr);
+  LAUNCHED(h);
+  // the patch conv (no bias) as one GEMM: [n*G*G, Kp] . [hidden, Kp]^T -> tmp
+  rc = tc ? enc_gemm_tc<0>(h, patch, static_cast<float*>(e.patch_l.p), e.patch_w_h, e.patch_w_l, e.zero_bias, tmp,
+                           nullptr, Mp, H, Kp)
+          : enc_gemm<0>(h, patch, e.patch_w, e.zero_bias, tmp, Mp, H, Kp);
+  if (rc != RSE_OK) return rc;
+  const EncLayer& l0 = e.layers[0];
+  clip_vision_embed_kernel<<<(T + 3) / 4, 128, 0, h->stream>>>(
+      tmp, T, L, H, e.cls_emb, e.pos, e.elng, e.elnb, l0.ln1g, l0.ln1b, c.ln_eps, static_cast<float*>(e.x.p),
+      static_cast<float*>(e.y.p), tc ? static_cast<float*>(e.x_h.p) : nullptr, tc ? static_cast<float*>(e.x_l.p) : nullptr);
+  LAUNCHED(h);
+  e.max_len = L;
+  rc = clip_layers(h, e, n, T, tc, false);
+  if (rc != RSE_OK) return rc;
+  clip_head_kernel<<<n, 128, 0, h->stream>>>(static_cast<const float*>(e.x.p), cu, nullptr, 0, H, e.flng, e.flnb,
+                                             c.ln_eps, e.proj, c.projection_dim, out_dev);
+  LAUNCHED(h);
+  return RSE_OK;
+}
+
+// ids / cu_seqlens on the device already (enc_run) -> out_dev [n_seq, projection_dim]
+int clip_text_forward(rse_index* h, Encoder& e, int n_seq, int T, float* out_dev) {
+  const rse_clip_config& c = e.ccfg;
+  const int H = c.hidden;
+  const bool tc = e.mode == 0 && e.tc_ok;
+  int rc = clip_buffers(h, e, T, tc);
+  if (rc != RSE_OK) return rc;
+  ENSURE(e.posidx, sizeof(int32_t) * T);
+  const int32_t* cu = static_cast<const int32_t*>(e.cu.p);
+  const int32_t* ids = static_cast<const int32_t*>(e.ids.p);
+  enc_positions_kernel<<<(T + 255) / 256, 256, 0, h->stream>>>(cu, n_seq, T, static_cast<int32_t*>(e.posidx.p));
+  LAUNCHED(h);
+  const EncLayer& l0 = e.layers[0];
+  clip_text_embed_kernel<<<(T + 3) / 4, 128, 0, h->stream>>>(
+      ids, static_cast<const int32_t*>(e.posidx.p), T, H, c.vocab_size, c.max_positions, e.word, e.pos, l0.ln1g,
+      l0.ln1b, c.ln_eps, static_cast<float*>(e.x.p), static_cast<float*>(e.y.p),
+      tc ? static_cast<float*>(e.x_h.p) : nullptr, tc ? static_cast<float*>(e.x_l.p) : nullptr);
+  LAUNCHED(h);
+  rc = clip_layers(h, e, n_seq, T, tc, true);
+  if (rc != RSE_OK) return rc;
+  clip_head_kernel<<<n_seq, 128, 0, h->stream>>>(static_cast<const float*>(e.x.p), cu, ids, c.eos_token_id, H, e.flng,
+                                                 e.flnb, c.ln_eps, e.proj, c.projection_dim, out_dev);
+  LAUNCHED(h);
+  return RSE_OK;
+}
+
 int enc_check(rse_index* h, int32_t slot, bool need_final) {
   if (slot < 0 || slot >= RSE_MAX_ENCODERS) return fail(h, RSE_ERR_INVALID, "encoder: slot out of range");
   if (!h->enc[slot].created) return fail(h, RSE_ERR_STATE, "encoder: rse_encoder_create has not been called for this slot");
@@ -2274,6 +2427,9 @@ int enc_run(rse_index* h, int32_t slot, const int32_t* ids, const int32_t* type_
   int rc = enc_check(h, slot, true);
   if (rc != RSE_OK) return rc;
   Encoder& e = h->enc[slot];
+  if (e.clip && e.ccfg.tower != 1)
+    return fail(h, RSE_ERR_INVALID, "rse_encode: the slot holds a CLIP vision tower (use rse_encode_images)");
+  if (e.clip && type_ids) return fail(h, RSE_ERR_INVALID, "rse_encode: type_ids must be NULL for a CLIP text tower");
   if (n_seq < 1 || !ids || !cu || !out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode: bad arguments");
   if (cu[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_encode: cu_seqlens must start at 0");
   int max_len = 1;
@@ -2309,6 +2465,7 @@ int enc_run(rse_index* h, int32_t slot, const int32_t* ids, const int32_t* type_
   CK(cudaEventRecord(e.pin_ev[pb], h->stream));
   h->stats.h2d_bytes += static_cast<int64_t>(sizeof(int32_t)) * (static_cast<int64_t>(T) * (type_ids ? 2 : 1) + n_seq + 1);
   e.max_len = max_len;
+  if (e.clip) return clip_text_forward(h, e, n_seq, T, out_dev);
   return enc_forward(h, e, n_seq, T, type_ids != nullptr, out_dev);
 }
 
@@ -2342,12 +2499,138 @@ int rse_encoder_create(rse_index* h, int32_t slot, const rse_encoder_config* cfg
   return RSE_OK;
 }
 
+int rse_clip_create(rse_index* h, int32_t slot, const rse_clip_config* cfg) {
+  if (!h) return RSE_ERR_INVALID;
+  if (slot < 0 || slot >= RSE_MAX_ENCODERS || !cfg) return fail(h, RSE_ERR_INVALID, "rse_clip_create: bad arguments");
+  const rse_clip_config& c = *cfg;
+  const bool vision = c.tower == 0;
+  bool ok = (c.tower == 0 || c.tower == 1) && c.hidden >= 32 && c.hidden <= kEncMaxHidden && c.hidden % 32 == 0 &&
+            c.heads >= 1 && c.hidden % c.heads == 0 && (c.hidden / c.heads == 32 || c.hidden / c.heads == 64) &&
+            c.layers >= 1 && c.layers <= 48 && c.intermediate >= 16 && c.intermediate % 16 == 0 &&
+            c.projection_dim >= 1 && c.projection_dim <= 65536 && c.ln_eps > 0.0f;
+  if (ok && vision)
+    ok = c.patch_size >= 1 && c.image_size >= c.patch_size && c.image_size % c.patch_size == 0 &&
+         c.image_size <= 8192 && static_cast<int64_t>(c.image_size / c.patch_size) * (c.image_size / c.patch_size) + 1 <= RSE_CLIP_MAX_TOKENS;
+  if (ok && !vision) ok = c.vocab_size >= 1 && c.max_positions >= 1 && c.max_positions <= RSE_CLIP_MAX_TOKENS;
+  if (!ok)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_clip_create: unsupported shape (tower 0 / 1, hidden % 32 and <= 1024, head_dim 32 or 64, "
+                                        "intermediate % 16, image_size % patch_size == 0, at most " +
+                                        std::to_string(RSE_CLIP_MAX_TOKENS) + " tokens per sequence)");
+  CK(cudaSetDevice(h->device));
+  Encoder& e = h->enc[slot];
+  enc_release(e);
+  e.clip = true;
+  e.ccfg = c;
+  const int G = vision ? c.image_size / c.patch_size : 0;
+  e.patch_k = vision ? (3 * c.patch_size * c.patch_size + 127) / 128 * 128 : 0;
+  // the BERT view of the shape (finalize's tensor-core check, enc_run's length check)
+  e.cfg = rse_encoder_config{};
+  e.cfg.vocab_size = c.vocab_size; e.cfg.hidden = c.hidden; e.cfg.layers = c.layers; e.cfg.heads = c.heads;
+  e.cfg.intermediate = c.intermediate; e.cfg.max_positions = vision ? G * G + 1 : c.max_positions; e.cfg.ln_eps = c.ln_eps;
+  const size_t H = c.hidden, I = c.intermediate;
+  int rc = RSE_OK;
+  auto A = [&](float** p, size_t n) { if (rc == RSE_OK) rc = enc_alloc(h, p, n); };
+  A(&e.pos, static_cast<size_t>(e.cfg.max_positions) * H);
+  A(&e.flng, H); A(&e.flnb, H); A(&e.proj, static_cast<size_t>(c.projection_dim) * H);
+  if (vision) {
+    A(&e.cls_emb, H); A(&e.elng, H); A(&e.elnb, H); A(&e.patch_w, H * e.patch_k); A(&e.zero_bias, H);
+  } else {
+    A(&e.word, static_cast<size_t>(c.vocab_size) * H);
+  }
+  e.layers.resize(c.layers);
+  for (auto& l : e.layers) {
+    A(&l.wqkv, 3 * H * H); A(&l.bqkv, 3 * H); A(&l.wo, H * H); A(&l.bo, H); A(&l.ln1g, H); A(&l.ln1b, H);
+    A(&l.wi, I * H); A(&l.bi, I); A(&l.wo2, H * I); A(&l.bo2, H); A(&l.ln2g, H); A(&l.ln2b, H);
+  }
+  if (rc == RSE_OK && vision) {
+    if (cudaMemset(e.patch_w, 0, sizeof(float) * H * e.patch_k) != cudaSuccess ||
+        cudaMemset(e.zero_bias, 0, sizeof(float) * H) != cudaSuccess)
+      rc = fail(h, RSE_ERR_CUDA, "rse_clip_create: cudaMemset failed");
+  }
+  if (rc != RSE_OK) { enc_release(e); return rc; }
+  e.created = true;
+  return RSE_OK;
+}
+
+namespace {
+// HuggingFace CLIP state_dict name -> destination in a CLIP slot
+int clip_set_tensor(rse_index* h, Encoder& e, const std::string& full, const float* data, int64_t n_elem) {
+  const rse_clip_config& c = e.ccfg;
+  const bool vision = c.tower == 0;
+  const int64_t H = c.hidden, I = c.intermediate;
+  const char* tower = vision ? "vision_model." : "text_model.";
+  const char* projn = vision ? "visual_projection." : "text_projection.";
+  size_t at = std::string::npos;
+  for (const char* key : {tower, projn}) {
+    const size_t p = full.find(key);
+    if (p != std::string::npos && (at == std::string::npos || p < at)) at = p;
+  }
+  if (at == std::string::npos)
+    return fail(h, RSE_ERR_INVALID, std::string("rse_encoder_set_tensor: not a CLIP ") + (vision ? "vision" : "text") +
+                                         " tower tensor name: " + full);
+  const std::string nm = full.substr(at);
+  const std::string tw(tower);
+  float* dst = nullptr;
+  int64_t want = 0;
+  bool patch = false;
+  auto is = [&](const char* s_) { return nm == s_; };
+  if (is(vision ? "visual_projection.weight" : "text_projection.weight")) { dst = e.proj; want = c.projection_dim * H; }
+  else if (nm == tw + "embeddings.position_embedding.weight") { dst = e.pos; want = e.cfg.max_positions * H; }
+  else if (nm == tw + (vision ? "post_layernorm.weight" : "final_layer_norm.weight")) { dst = e.flng; want = H; }
+  else if (nm == tw + (vision ? "post_layernorm.bias" : "final_layer_norm.bias")) { dst = e.flnb; want = H; }
+  else if (!vision && is("text_model.embeddings.token_embedding.weight")) { dst = e.word; want = c.vocab_size * H; }
+  else if (vision && is("vision_model.embeddings.class_embedding")) { dst = e.cls_emb; want = H; }
+  else if (vision && is("vision_model.embeddings.patch_embedding.weight")) {
+    dst = e.patch_w; want = H * 3 * c.patch_size * c.patch_size; patch = true;
+  }
+  else if (vision && is("vision_model.pre_layrnorm.weight")) { dst = e.elng; want = H; }
+  else if (vision && is("vision_model.pre_layrnorm.bias")) { dst = e.elnb; want = H; }
+  else if (nm.rfind(tw + "encoder.layers.", 0) == 0) {
+    const size_t b = tw.size() + 15, dot = nm.find('.', b);
+    if (dot == std::string::npos) return fail(h, RSE_ERR_INVALID, "rse_encoder_set_tensor: bad layer name: " + full);
+    const int li = std::atoi(nm.substr(b, dot - b).c_str());
+    if (li < 0 || li >= c.layers) return fail(h, RSE_ERR_INVALID, "rse_encoder_set_tensor: layer index out of range: " + full);
+    EncLayer& l = e.layers[li];
+    const std::string t = nm.substr(dot + 1);
+    if (t == "self_attn.q_proj.weight") { dst = l.wqkv; want = H * H; }
+    else if (t == "self_attn.k_proj.weight") { dst = l.wqkv + H * H; want = H * H; }
+    else if (t == "self_attn.v_proj.weight") { dst = l.wqkv + 2 * H * H; want = H * H; }
+    else if (t == "self_attn.q_proj.bias") { dst = l.bqkv; want = H; }
+    else if (t == "self_attn.k_proj.bias") { dst = l.bqkv + H; want = H; }
+    else if (t == "self_attn.v_proj.bias") { dst = l.bqkv + 2 * H; want = H; }
+    else if (t == "self_attn.out_proj.weight") { dst = l.wo; want = H * H; }
+    else if (t == "self_attn.out_proj.bias") { dst = l.bo; want = H; }
+    else if (t == "layer_norm1.weight") { dst = l.ln1g; want = H; }
+    else if (t == "layer_norm1.bias") { dst = l.ln1b; want = H; }
+    else if (t == "mlp.fc1.weight") { dst = l.wi; want = I * H; }
+    else if (t == "mlp.fc1.bias") { dst = l.bi; want = I; }
+    else if (t == "mlp.fc2.weight") { dst = l.wo2; want = H * I; }
+    else if (t == "mlp.fc2.bias") { dst = l.bo2; want = H; }
+    else if (t == "layer_norm2.weight") { dst = l.ln2g; want = H; }
+    else if (t == "layer_norm2.bias") { dst = l.ln2b; want = H; }
+  }
+  if (!dst) return fail(h, RSE_ERR_INVALID, "rse_encoder_set_tensor: unknown tensor: " + full);
+  if (n_elem != want) return fail(h, RSE_ERR_INVALID, "rse_encoder_set_tensor: wrong element count for " + full);
+  CK(cudaSetDevice(h->device));
+  if (patch) {      // [hidden, 3*P*P] into the zero-padded [hidden, patch_k]
+    const size_t k = 3 * static_cast<size_t>(c.patch_size) * c.patch_size;
+    CK(cudaMemcpy2D(dst, sizeof(float) * e.patch_k, data, sizeof(float) * k, sizeof(float) * k, H, cudaMemcpyHostToDevice));
+  } else {
+    CK(cudaMemcpy(dst, data, sizeof(float) * n_elem, cudaMemcpyHostToDevice));
+  }
+  e.seen.insert(nm);
+  e.finalized = false;
+  return RSE_OK;
+}
+}  // namespace
+
 int rse_encoder_set_tensor(rse_index* h, int32_t slot, const char* name, const float* data, int64_t n_elem) {
   if (!h) return RSE_ERR_INVALID;
   int rc = enc_check(h, slot, false);
   if (rc != RSE_OK) return rc;
   if (!name || !data || n_elem < 1) return fail(h, RSE_ERR_INVALID, "rse_encoder_set_tensor: bad arguments");
   Encoder& e = h->enc[slot];
+  if (e.clip) return clip_set_tensor(h, e, name, data, n_elem);
   const rse_encoder_config& c = e.cfg;
   const int64_t H = c.hidden, I = c.intermediate;
   // HuggingFace state_dict names, with whatever prefix the wrapper adds ("bert.", "0.auto_model.", ...)
@@ -2412,7 +2695,8 @@ int rse_encoder_finalize(rse_index* h, int32_t slot) {
   int rc = enc_check(h, slot, false);
   if (rc != RSE_OK) return rc;
   Encoder& e = h->enc[slot];
-  const size_t want = 5 + 16 * static_cast<size_t>(e.cfg.layers) + (e.cfg.head == 1 ? 4 : 0);
+  const size_t want = e.clip ? (e.ccfg.tower == 0 ? 8 : 5) + 16 * static_cast<size_t>(e.cfg.layers)
+                             : 5 + 16 * static_cast<size_t>(e.cfg.layers) + (e.cfg.head == 1 ? 4 : 0);
   if (e.seen.size() != want)
     return fail(h, RSE_ERR_STATE, "rse_encoder_finalize: " + std::to_string(e.seen.size()) + " of " + std::to_string(want) +
                                       " tensors were set");
@@ -2431,6 +2715,13 @@ int rse_encoder_finalize(rse_index* h, int32_t slot) {
         enc_split_kernel<<<static_cast<unsigned int>((p.n + 255) / 256), 256, 0, h->stream>>>(p.w, p.n, *p.hi, *p.lo);
         LAUNCHED(h);
       }
+    }
+    if (e.clip && e.ccfg.tower == 0) {          // the patch conv's weight (its K is padded to a multiple of 128)
+      const int64_t n = H * e.patch_k;
+      if (!e.patch_w_h) { rc = enc_alloc(h, &e.patch_w_h, n); if (rc != RSE_OK) return rc; }
+      if (!e.patch_w_l) { rc = enc_alloc(h, &e.patch_w_l, n); if (rc != RSE_OK) return rc; }
+      enc_split_kernel<<<static_cast<unsigned int>((n + 255) / 256), 256, 0, h->stream>>>(e.patch_w, n, e.patch_w_h, e.patch_w_l);
+      LAUNCHED(h);
     }
     CK(cudaStreamSynchronize(h->stream));
   }
@@ -2460,10 +2751,66 @@ int rse_encode(rse_index* h, int32_t slot, const int32_t* ids, const int32_t* ty
   if (rc != RSE_OK) return rc;
   if (!out_host || n_seq < 1) return fail(h, RSE_ERR_INVALID, "rse_encode: bad arguments");
   Encoder& e = h->enc[slot];
-  const size_t n_out = static_cast<size_t>(n_seq) * (e.cfg.head == 0 ? e.cfg.hidden : 1);
+  const size_t n_out = static_cast<size_t>(n_seq) * (e.clip ? e.ccfg.projection_dim : e.cfg.head == 0 ? e.cfg.hidden : 1);
   CK(cudaSetDevice(h->device));
   ENSURE(e.out, sizeof(float) * n_out);
   rc = enc_run(h, slot, ids, type_ids, cu_seqlens, n_seq, static_cast<float*>(e.out.p));
+  if (rc != RSE_OK) return rc;
+  CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);
+  CK(cudaStreamSynchronize(h->stream));
+  return RSE_OK;
+}
+
+namespace {
+// checks, then (host pixels) pinned staging + upload on the handle's stream, then the vision tower
+int clip_images(rse_index* h, int32_t slot, const float* pixels, int32_t n, float* out_dev, bool host) {
+  int rc = enc_check(h, slot, true);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[slot];
+  if (!e.clip || e.ccfg.tower != 0)
+    return fail(h, RSE_ERR_INVALID, "rse_encode_images: the slot does not hold a CLIP vision tower");
+  if (n < 1 || !pixels || !out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode_images: bad arguments (n < 1 or NULL)");
+  const int64_t per = 3ll * e.ccfg.image_size * e.ccfg.image_size;
+  if (static_cast<int64_t>(n) * e.cfg.max_positions > (1ll << 24))
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_encode_images: more than 2^24 tokens in one call (split the batch)");
+  CK(cudaSetDevice(h->device));
+  if (!host) return clip_vision_forward(h, e, n, pixels, out_dev);
+  const size_t n_px = static_cast<size_t>(n) * per;
+  const int pb = e.pin_next;
+  e.pin_next ^= 1;
+  if (!e.pin_ev[pb]) CK(cudaEventCreateWithFlags(&e.pin_ev[pb], cudaEventDisableTiming));
+  else CK(cudaEventSynchronize(e.pin_ev[pb]));              // the upload out of this buffer (two calls ago) is done
+  if (e.pin_px_n[pb] < n_px) {
+    if (e.pin_px[pb]) CK(cudaFreeHost(e.pin_px[pb]));
+    e.pin_px[pb] = nullptr; e.pin_px_n[pb] = 0;
+    CK(cudaMallocHost(reinterpret_cast<void**>(&e.pin_px[pb]), sizeof(float) * n_px));
+    e.pin_px_n[pb] = n_px;
+  }
+  std::memcpy(e.pin_px[pb], pixels, sizeof(float) * n_px);
+  ENSURE(e.pix, sizeof(float) * n_px);
+  CK(cudaMemcpyAsync(e.pix.p, e.pin_px[pb], sizeof(float) * n_px, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaEventRecord(e.pin_ev[pb], h->stream));
+  h->stats.h2d_bytes += static_cast<int64_t>(sizeof(float) * n_px);
+  return clip_vision_forward(h, e, n, static_cast<const float*>(e.pix.p), out_dev);
+}
+}  // namespace
+
+int rse_encode_images_dev(rse_index* h, int32_t slot, const float* pixels_dev, int32_t n, float* out_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  return clip_images(h, slot, pixels_dev, n, out_dev, false);
+}
+
+int rse_encode_images(rse_index* h, int32_t slot, const float* pixels_host, int32_t n, float* out_host) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = enc_check(h, slot, true);
+  if (rc != RSE_OK) return rc;
+  if (!out_host || n < 1) return fail(h, RSE_ERR_INVALID, "rse_encode_images: bad arguments (n < 1 or NULL)");
+  Encoder& e = h->enc[slot];
+  const size_t n_out = static_cast<size_t>(n) * (e.clip ? e.ccfg.projection_dim : 1);
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.out, sizeof(float) * n_out);
+  rc = clip_images(h, slot, pixels_host, n, static_cast<float*>(e.out.p), true);
   if (rc != RSE_OK) return rc;
   CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
   h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);
