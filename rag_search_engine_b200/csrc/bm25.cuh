@@ -417,11 +417,10 @@ constexpr int kBsMaxGroups = 32;                  // groups per query bm25_fx_fi
 constexpr unsigned int kBsRangeCap = 256;         // documents that may cross theta inside one range
 constexpr int kBsFinalCap = 64;                   // finalists (k + ties) ranked exactly
 
-// out8 (optional): the 8-byte stream bm25_fx_kernel reads, {doc, round(w * wq_scale)} — see the K6'' header
-// out4 (optional): the 4-byte stream, (doc % kBmRange) | round(w * wq4_scale) << 13 — see bm25_fx_body<.., P4 = true>
+// out4 (optional): the 4-byte stream bm25_fx_kernel reads, (doc % kBmRange) | round(w * wq4_scale) << 13 — see the
+// K6'' header
 __global__ void bm25_weight_kernel(const uint2* __restrict__ post, const double* __restrict__ normk, int64_t n,
-                                   double k1p1, Post16* __restrict__ out, uint2* __restrict__ out8, double wq_scale,
-                                   uint32_t* __restrict__ out4, double wq4_scale) {
+                                   double k1p1, Post16* __restrict__ out, uint32_t* __restrict__ out4, double wq4_scale) {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const uint2 e = post[i];
@@ -430,7 +429,6 @@ __global__ void bm25_weight_kernel(const uint2* __restrict__ post, const double*
   o.doc = e.x; o.tf = e.y;
   o.w = __ddiv_rn(__dmul_rn(tfd, k1p1), __dadd_rn(tfd, normk[e.x]));
   out[i] = o;
-  if (out8) out8[i] = make_uint2(e.x, __double2uint_rn(__dmul_rn(o.w, wq_scale)));
   if (out4) {
     unsigned int wq = __double2uint_rn(__dmul_rn(o.w, wq4_scale));
     if (wq > 0x7FFFFu) wq = 0x7FFFFu;                      // (k1+1) * wq4_scale <= 2^19: only a weight at the very top clamps
@@ -680,18 +678,23 @@ bm25_stream_kernel(const int64_t* __restrict__ indptr, const Post16* __restrict_
 // The order only matters for the low bits of a sum.  This kernel accumulates idf*w in 32-bit FIXED POINT with
 // native shared-memory integer atomics (ATOMS.ADD; 64-bit and double shared atomics are CAS loops on sm_100).  The
 // scale is the largest power of two that keeps (k1+1)*log(N+2)*16 below 2^31 (2^21 for the default k1: steps of
-// 4.8e-7).  The kernel is HBM-bound on the posting stream, so it reads an 8-BYTE posting {doc, wq} instead of the
-// 16-byte {doc, tf, double w}: wq = round(w * wq_scale) with wq_scale the largest power of two keeping
-// (k1+1)*wq_scale <= 2^31, i.e. w is known to 2^-32..2^-31 absolute — 1/16 unit of the sum at most.  The sum is
-// exact in that format, independent of the order, and within 9 units (each of <= 16 terms: <= 0.5 unit from its
-// one rounding + <= 1/16 unit from wq) of the reference's double sum times the scale — so all the token slices
-// of a range are cut into 64-posting items (a lane loads one aligned 16-byte PAIR) that the warps take round
-// robin with NO barrier between tokens.  Everything decided on these sums carries a margin of kFxMargin units; the finalists (k plus whatever
-// lies within the margin of the k-th) are RE-SCORED in bm25_fx_finish_kernel with the reference's own
-// expression in query-token order — one thread per (document, token) finds the posting by binary search — which
-// also yields the reference's tie key (first token holding the document).  Scores, order and ties are therefore
-// bit-identical to the general kernel; queries it cannot finish are flagged for it exactly like before.
-constexpr unsigned int kFxMargin = 40u;               // > 2 x (9 units of accumulated rounding + the double sum's own)
+// 4.8e-7).  The kernel is HBM-bound on the posting stream (in a hybrid step it shares the HBM with the tensor-core
+// filter), so it reads a 4-BYTE posting instead of the 16-byte {doc, tf, double w}: 13 bits of document offset
+// inside its range (the range is known from the slice being read) and a 19-bit weight, wq = round(w * wq4_scale)
+// with wq4_scale the largest power of two keeping (k1+1) * wq4_scale <= 2^19.  A weight is known to +-1 unit of wq
+// (0.5 from its rounding, the clamp at the top), i.e. +-idfx units of the sum (idfx = idf * scale / wq4_scale), and
+// each term adds <= 0.5 unit of its own rounding.  The sum is exact in that format and independent of the order, so
+// all the token slices of a range are cut into 128-posting items (a lane loads one aligned 16-byte QUAD) that the
+// warps take round robin with NO barrier between tokens.  Everything decided on these sums carries a margin of
+// 2 * sum_t (idfx_t + 0.5) + 8 units PER QUERY, at least kFxMargin (~1e-3 in score units for a 16-token query with
+// the default k1); the finalists (k plus whatever lies within the margin of the k-th) are RE-SCORED in
+// bm25_fx_finish_kernel with the reference's own expression in query-token order — one thread per (document, token)
+// finds the posting by binary search — which also yields the reference's tie key (first token holding the
+// document).  Scores, order and ties are therefore bit-identical to the general kernel; queries it cannot finish
+// are flagged for it exactly like before.  (r02: the first version read an 8-byte {doc, wq} posting with a 31-bit
+// weight and a constant margin; the 4-byte stream halves the bytes and pays the per-item token lookup half as
+// often, at the price of a few more finalists for the exact finish kernel.)
+constexpr unsigned int kFxMargin = 40u;               // floor of the per-query margin
 constexpr int kFxFinalCap = 48;
 constexpr int kFxRescoreCap = 96;
 
@@ -707,29 +710,19 @@ __host__ __device__ constexpr int fx_smem_bytes(int rpg) {
 // schedulers (3 x 32 x 96 registers = 9216 of 16384), which leaves room for exactly 7 warps of 32 registers per
 // scheduler — 28 warps instead of 16.  (A 768-thread shape does NOT fit: its launch bound lets ptxas take 39
 // registers.)  r02 measurements, all on one box: stand-alone the kernel is thread-parallelism-bound (4 / 3 / 2 / 1
-// CTAs per SM: 0.31 / 0.34 / 0.42 / 0.69 ms, scripts/bm25_occupancy.py), but beside the filter it runs at ~14 % of
-// the stand-alone rate whatever its shape — 28 warps instead of 16 finish 8 us earlier (step 1.078 -> 1.070 ms), and
-// a 55-register variant with four posting loads in flight per lane was slower overall (1.13 ms: only two of those
-// fit an SM once the filter is gone).  What it competes for there is the memory system: the filter streams the
-// shadow at 4.9 TB/s of the 6.5 the HBM gives.
-// P4 (r02): the posting stream is 4 BYTES per posting — 13 bits of document offset inside its range (the range is
-// known from the slice being read) and a 19-bit weight, wq = round(w * wq4_scale), (k1+1) * wq4_scale <= 2^19.  Half
-// the bytes (the kernel shares the HBM with the tensor-core filter in a hybrid step) and 128 postings per warp item
-// instead of 64, so the per-item token lookup is paid half as often.  The price is precision: a weight is known to
-// +-1 unit of wq (0.5 from its rounding, the clamp at the top), i.e. +-idfx units of the sum, so the margin everything
-// is decided with grows from the constant kFxMargin to 2 * sum_t (idfx_t + 0.5) + 8 units PER QUERY (~1e-3 in score
-// units for a 16-token query with the default k1) — a few more finalists for the exact finish kernel, same results.
-template <int THREADS, int DEPTH, bool P4>
+// CTAs per SM, set by padding the shared memory: 0.31 / 0.34 / 0.42 / 0.69 ms), but beside the filter it runs at
+// ~14 % of the stand-alone rate whatever its shape — 28 warps instead of 16 finish 8 us earlier (step 1.078 -> 1.070
+// ms), and a 55-register variant with four posting loads in flight per lane was slower overall (1.13 ms: only two
+// of those fit an SM once the filter is gone).
+// What it competes for there is the memory system: the filter streams the shadow at 4.9 TB/s of the 6.5 the HBM gives.
+// The grid is (queries, groups): the CTAs that are resident together work on the SAME ranges for different queries,
+// so the slices of the hot posting lists they share are read within microseconds of each other.
+template <int THREADS, int DEPTH>
 __device__ __forceinline__ void
-bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8, const uint32_t* __restrict__ roff,
+bm25_fx_body(const int64_t* __restrict__ indptr, const uint32_t* __restrict__ post4, const uint32_t* __restrict__ roff,
              int nr, const int32_t* __restrict__ tok_indptr, const int32_t* __restrict__ term_rows,
-             const double* __restrict__ tok_idf, double scale, int q0, int k, int rpg, int ng, int g0,
+             const double* __restrict__ tok_idf, double scale, int q0, int k, int rpg, int ng,
              uint2* __restrict__ fin, int* __restrict__ fin_cnt, int* __restrict__ status) {
-  // rpg < 0 (host: RSE_BM25_QFAST): the grid is (queries, groups) instead of (groups, queries) — the CTAs that are
-  // resident together then work on the SAME ranges for different queries, so the slices of the hot posting lists
-  // they share are read within microseconds of each other
-  const bool qfast = rpg < 0;
-  if (qfast) rpg = -rpg;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   uint32_t* acc = reinterpret_cast<uint32_t*>(smem_raw);                               // [kBmRange] fixed-point sums
   uint32_t* s_off = acc + kBmRange;                                                    // [kBsMaxTok][rpg + 1]
@@ -737,13 +730,13 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
   uint2* s_cand0 = reinterpret_cast<uint2*>(smem_raw + kBmRange * 4 + ((kBsMaxTok * ostride * 4 + 15) & ~15));
   uint2* s_cand1 = s_cand0 + kBsCandCap;                                               // {sum, doc}
   __shared__ long long s_base[kBsMaxTok];
-  __shared__ double s_idfx[kBsMaxTok];                                                 // idf * scale / wq_scale (exact: powers of two)
+  __shared__ double s_idfx[kBsMaxTok];                                                 // idf * scale / wq4_scale (exact: powers of two)
   __shared__ int s_term[kBsMaxTok];
   __shared__ unsigned int s_ncand, s_nkept;
   __shared__ unsigned int s_min, s_tw, s_margin;
 
-  const int g = g0 + (qfast ? blockIdx.y : blockIdx.x);    // g0: first group of this launch (rse.cu splits the groups)
-  const int q = q0 + (qfast ? blockIdx.x : blockIdx.y);
+  const int g = blockIdx.y;
+  const int q = q0 + blockIdx.x;
   const int t0 = tok_indptr[q], ntok = tok_indptr[q + 1] - t0;
   const int64_t cbase = static_cast<int64_t>(q) * ng + g;
   if (ntok > kBsMaxTok) {                                 // uniform: the whole query goes to the general kernel
@@ -771,14 +764,10 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
     for (int i = threadIdx.x; i < kBmRange / 4; i += blockDim.x) a4[i] = make_uint4(0u, 0u, 0u, 0u);
   }
   if (threadIdx.x == 0) {                         // the margin lives in shared memory: the kernel has no register to spare
-    unsigned int mg = kFxMargin;
-    if (P4) {
-      double m = 0.0;
-      for (int t = 0; t < ntok; ++t) m += s_idfx[t] + 0.5;
-      const unsigned int mq = 2u * static_cast<unsigned int>(ceil(m)) + 8u;
-      if (mq > mg) mg = mq;
-    }
-    s_margin = mg;
+    double m = 0.0;
+    for (int t = 0; t < ntok; ++t) m += s_idfx[t] + 0.5;
+    const unsigned int mq = 2u * static_cast<unsigned int>(ceil(m)) + 8u;
+    s_margin = mq > kFxMargin ? mq : kFxMargin;
   }
   __syncthreads();
 
@@ -818,7 +807,7 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
   constexpr int kVec = kBmRange / 4;                      // accumulators as uint4
   for (int r = r0; r < r1; ++r) {
     const int jr = r - r0;
-    // Items of this range: slice t contributes items of 32 aligned posting PAIRS (one 16-byte load per lane).
+    // Items of this range: slice t contributes items of 32 aligned posting QUADS (one 16-byte load per lane).
     // Every warp derives the same item prefix in registers (lane t owns token t): no shared item table, no
     // barrier before the postings — the two barriers of a range are "sums complete" and "accumulators cleared".
     long long sb = 0;
@@ -827,8 +816,7 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
       const uint32_t a = s_off[lane * ostride + jr];
       sn = s_off[lane * ostride + jr + 1] - a;
       sb = s_base[lane] + a;
-      if (P4) c = sn ? (sn + static_cast<unsigned int>(sb & 3) + 127u) >> 7 : 0u;   // quads start at a multiple of 4
-      else c = sn ? (sn + static_cast<unsigned int>(sb & 1) + 63u) >> 6 : 0u;        // pairs start at an even posting index
+      c = sn ? (sn + static_cast<unsigned int>(sb & 3) + 127u) >> 7 : 0u;   // quads start at a multiple of 4
     }
     unsigned int incl = c;
 #pragma unroll
@@ -845,8 +833,7 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
     const int sb_hi = static_cast<int>(static_cast<unsigned long long>(sb) >> 32);
 
     auto item_load = [&](unsigned int item, uint4& e, double& idfx) {
-      e = P4 ? make_uint4(0u, 0u, 0u, 0u)                 // P4: a zero word adds nothing
-             : make_uint4(0xFFFFFFFFu, 0u, 0xFFFFFFFFu, 0u);   // {doc, wq, doc, wq}; doc = ~0: nothing to add
+      e = make_uint4(0u, 0u, 0u, 0u);                     // a zero word adds nothing
       idfx = 0.0;
       if (item >= n_items) return;                        // warp-uniform
       // token of the item: the highest lane holding items whose first item is <= item
@@ -858,39 +845,24 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
           static_cast<unsigned int>(__shfl_sync(0xFFFFFFFFu, sb_lo, t)));
       const unsigned int tsn = __shfl_sync(0xFFFFFFFFu, sn, t);
       idfx = s_idfx[t];
-      if (P4) {
-        // four packed postings per lane; a word of 0 (weight 0) adds nothing, so that is also the "not mine" mark
-        // (positions relative to the slice start, 32-bit: the kernel has no register to spare)
-        const int len = static_cast<int>(tsn);
-        const int rel = static_cast<int>(chunk * 128u + 4u * lane) - static_cast<int>(tsb & 3);   // of e.x; >= -3
-        if (rel + 3 >= 0 && rel < len) {                  // the quad overlaps the slice (the stream is padded by one quad)
-          e = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const uint32_t*>(post8) + (tsb + rel)));
-          if (rel < 0) e.x = 0u;
-          if (rel + 1 < 0 || rel + 1 >= len) e.y = 0u;
-          if (rel + 2 < 0 || rel + 2 >= len) e.z = 0u;
-          if (rel + 3 >= len) e.w = 0u;
-        }
-        return;
-      }
-      const long long se = tsb + tsn;
-      const long long j0 = (tsb & ~1LL) + chunk * 64u + 2u * lane;
-      if (j0 + 1 >= tsb && j0 < se) {                     // the pair overlaps the slice (the stream is padded by one pair)
-        e = __ldg(reinterpret_cast<const uint4*>(post8 + j0));
-        if (j0 < tsb) e.x = 0xFFFFFFFFu;
-        if (j0 + 1 >= se) e.z = 0xFFFFFFFFu;
+      // four packed postings per lane; a word of 0 (weight 0) adds nothing, so that is also the "not mine" mark
+      // (positions relative to the slice start, 32-bit: the kernel has no register to spare)
+      const int len = static_cast<int>(tsn);
+      const int rel = static_cast<int>(chunk * 128u + 4u * lane) - static_cast<int>(tsb & 3);   // of e.x; >= -3
+      if (rel + 3 >= 0 && rel < len) {                    // the quad overlaps the slice (the stream is padded by one quad)
+        e = __ldg(reinterpret_cast<const uint4*>(post4 + (tsb + rel)));
+        if (rel < 0) e.x = 0u;
+        if (rel + 1 < 0 || rel + 1 >= len) e.y = 0u;
+        if (rel + 2 < 0 || rel + 2 >= len) e.z = 0u;
+        if (rel + 3 >= len) e.w = 0u;
       }
     };
     auto item_apply = [&](const uint4& e, double idfx) {
       // sums only grow and nothing reads them before the barrier: plain reductions, no returned value to wait for
-      if (P4) {
-        const uint32_t w4[4] = {e.x, e.y, e.z, e.w};
+      const uint32_t w4[4] = {e.x, e.y, e.z, e.w};
 #pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (w4[u] >> 13) atomicAdd(&acc[w4[u] & 0x1FFFu], __double2uint_rn(__dmul_rn(idfx, __uint2double_rn(w4[u] >> 13))));
-        return;
-      }
-      if (e.x != 0xFFFFFFFFu) atomicAdd(&acc[e.x - doc_base], __double2uint_rn(__dmul_rn(idfx, __uint2double_rn(e.y))));
-      if (e.z != 0xFFFFFFFFu) atomicAdd(&acc[e.z - doc_base], __double2uint_rn(__dmul_rn(idfx, __uint2double_rn(e.w))));
+      for (int u = 0; u < 4; ++u)
+        if (w4[u] >> 13) atomicAdd(&acc[w4[u] & 0x1FFFu], __double2uint_rn(__dmul_rn(idfx, __uint2double_rn(w4[u] >> 13))));
     };
     {
       // DEPTH loads in flight per lane (a ring of named buffers: every index below is a compile-time constant)
@@ -982,13 +954,13 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8
   if (threadIdx.x == 0) fin_cnt[cbase] = static_cast<int>(n);
 }
 
-template <int THREADS, bool P4>
+template <int THREADS>
 __global__ void __launch_bounds__(THREADS, (THREADS <= 512 ? 4 : 2))
-bm25_fx_kernel(const int64_t* __restrict__ indptr, const uint2* __restrict__ post8, const uint32_t* __restrict__ roff,
+bm25_fx_kernel(const int64_t* __restrict__ indptr, const uint32_t* __restrict__ post4, const uint32_t* __restrict__ roff,
                int nr, const int32_t* __restrict__ tok_indptr, const int32_t* __restrict__ term_rows,
-               const double* __restrict__ tok_idf, double scale, int q0, int k, int rpg, int ng, int g0,
+               const double* __restrict__ tok_idf, double scale, int q0, int k, int rpg, int ng,
                uint2* __restrict__ fin, int* __restrict__ fin_cnt, int* __restrict__ status) {
-  bm25_fx_body<THREADS, 2, P4>(indptr, post8, roff, nr, tok_indptr, term_rows, tok_idf, scale, q0, k, rpg, ng, g0, fin, fin_cnt, status);
+  bm25_fx_body<THREADS, 2>(indptr, post4, roff, nr, tok_indptr, term_rows, tok_idf, scale, q0, k, rpg, ng, fin, fin_cnt, status);
 }
 // K7'': one CTA per query bm25_fx_kernel finished (see the header above).
 __global__ void __launch_bounds__(kBmThreads)
@@ -997,7 +969,7 @@ bm25_fx_finish_kernel(const uint2* __restrict__ fin, const int* __restrict__ fin
                       const uint32_t* __restrict__ roff, int nr, const int32_t* __restrict__ tok_indptr,
                       const int32_t* __restrict__ term_rows, const double* __restrict__ tok_idf, int q0, int k,
                       double* __restrict__ out_score, int* __restrict__ out_doc, int* __restrict__ out_count,
-                      unsigned long long* __restrict__ counters, double idfx_scale) {   // idfx_scale > 0: 4-byte postings
+                      unsigned long long* __restrict__ counters, double idfx_scale) {
   __shared__ uint2 s_c[kBsMaxGroups * kFxFinalCap];       // 12 KB: the groups' candidates {sum, doc}
   __shared__ double s_w[kFxRescoreCap][kBsMaxTok];        // 12 KB: weight of (document, token), 0 = not in the list
   __shared__ uint32_t s_doc[kFxRescoreCap];
@@ -1007,7 +979,7 @@ bm25_fx_finish_kernel(const uint2* __restrict__ fin, const int* __restrict__ fin
   if (status[q] != 0) return;                             // the general path owns this query
   const int t0 = tok_indptr[q], ntok = tok_indptr[q + 1] - t0;
   unsigned int margin = kFxMargin;                        // the same per-query margin bm25_fx_body decided with
-  if (idfx_scale > 0.0) {
+  {
     double m = 0.0;
     for (int t = 0; t < ntok; ++t) m += tok_idf[t0 + t] * idfx_scale + 0.5;
     const unsigned int mq = 2u * static_cast<unsigned int>(ceil(m)) + 8u;

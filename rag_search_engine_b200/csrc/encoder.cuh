@@ -389,24 +389,25 @@ __global__ void enc_positions_kernel(const int32_t* __restrict__ cu_seqlens, int
 //     traffic, no hi/lo copies — was 10 % SLOWER, 1.22 vs 1.11 ms per 256-query batch: the tile is bound by the
 //     latency of a 3-stage ring per CTA and by wave quantisation, not by L2 bandwidth, and the split adds a hop
 //     to every stage.)
-//   * one 128 x 128 output tile per CTA (cta_group::1): warp 0 = TMA producer (3-stage ring, per stage four
-//     128 x 32-float boxes: A_hi, A_lo, W_hi, W_lo, SWIZZLE_128B), warp 1 = single-thread tcgen05.mma issuer
-//     (12 MMAs of 128x128x8 per k-block: 4 k-steps x 3 products), warps 2-5 = epilogue (tcgen05.ld 32x32b, one
-//     TMEM lane = one token row per thread, 128 accumulators in registers): bias (+ GELU + split), 128-byte stores.
-// Output tile 128 x BN, BN = 128 or 64: the narrow tile is for GEMMs whose 128-wide tiling would leave most SMs idle
-// (MiniLM's N = 384 projections on a 2.5 k-token batch: 60 tiles for 148 SMs; 120 with BN = 64).
-constexpr int kEgBM = 128, kEgBN = 128, kEgBK = 32;
-// ring depth: 3 stages of 64 KB for the 128-wide tile (one CTA per SM); 2 stages of 48 KB for the 64-wide tile, which
-// then fits TWICE on an SM (96 KB of shared memory, 256 TMEM columns, 132 registers x 192 threads each): four
-// stages in flight per SM and one CTA's prologue / epilogue under the other's main loop
-__host__ __device__ constexpr int eg_stages(int bn) { return bn == 128 ? 3 : 2; }
+//   * one 128 x 64 output tile per CTA (cta_group::1): warp 0 = TMA producer (2-stage ring, per stage two
+//     128 x 32-float boxes A_hi, A_lo and two 64 x 32-float boxes W_hi, W_lo, SWIZZLE_128B), warp 1 = single-thread
+//     tcgen05.mma issuer (12 MMAs of 128x64x8 per k-block: 4 k-steps x 3 products), warps 2-5 = epilogue
+//     (tcgen05.ld 32x32b, one TMEM lane = one token row per thread, 64 accumulators in registers): bias (+ GELU +
+//     split), 128-byte stores.
+// The tile is 64 wide, not 128, because a 128-wide tiling leaves most SMs idle (MiniLM's N = 384 projections on a
+// 2.5 k-token batch: 60 tiles for 148 SMs; 120 with 64-wide tiles), and the 64-wide tile fits TWICE on an SM (96 KB
+// of shared memory, 256 TMEM columns, 132 registers x 192 threads each): four stages in flight per SM and one CTA's
+// prologue / epilogue under the other's main loop.
+constexpr int kEgBM = 128, kEgBN = 64, kEgBK = 32;
+constexpr int kEgStages = 2;
 constexpr int kEgBox = kEgBM * kEgBK * 4;                       // 16,384 B: one 128-row operand box
+constexpr int kEgWBox = kEgBN * kEgBK * 4;                      // 8,192 B: one 64-row weight box
 constexpr int kEgThreads = 192;
 constexpr int kEgChunkKB = 4;                                   // k-blocks per hi*hi accumulation chunk (K = 128)
-__host__ __device__ constexpr int eg_stage_bytes(int bn) { return 2 * kEgBox + 2 * bn * kEgBK * 4; }
-__host__ __device__ constexpr int eg_smem_bytes(int bn) { return eg_stages(bn) * eg_stage_bytes(bn) + 16 * 8 + 16 + 1024; }
-// kind::tf32: D = f32 (bit 4), A = B = tf32 (format 2), both K-major, N = BN, M = 128
-__host__ __device__ constexpr uint32_t eg_idesc(int bn) { return (1u << 4) | (2u << 7) | (2u << 10) | ((static_cast<uint32_t>(bn) >> 3) << 17) | ((kEgBM >> 4) << 24); }
+constexpr int kEgStageBytes = 2 * kEgBox + 2 * kEgWBox;
+constexpr int kEgSmemBytes = kEgStages * kEgStageBytes + 16 * 8 + 16 + 1024;
+// kind::tf32: D = f32 (bit 4), A = B = tf32 (format 2), both K-major, N = kEgBN, M = 128
+constexpr uint32_t kEgIdesc = (1u << 4) | (2u << 7) | (2u << 10) | ((static_cast<uint32_t>(kEgBN) >> 3) << 17) | ((kEgBM >> 4) << 24);
 
 __global__ void enc_split_kernel(const float* __restrict__ x, int64_t n, float* __restrict__ hi, float* __restrict__ lo) {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -439,20 +440,16 @@ __device__ __forceinline__ void eg_mma_tf32(uint32_t tmem_d, uint64_t adesc, uin
 
 // EPI 0: C = acc + bias (fp32).  EPI 1: g = GELU(acc + bias) -> C_hi / C_lo (the operand of the next GEMM).
 // EPI 2: the same with quick_gelu (CLIP).
-template <int EPI, int BN>
-__global__ void __launch_bounds__(kEgThreads, BN == 128 ? 1 : 2)
+template <int EPI>
+__global__ void __launch_bounds__(kEgThreads, 2)
 enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_constant__ CUtensorMap tmap_a_lo,
                    const __grid_constant__ CUtensorMap tmap_w_hi, const __grid_constant__ CUtensorMap tmap_w_lo,
                    const float* __restrict__ bias, float* __restrict__ C, float* __restrict__ C_lo, int M, int N, int K) {
   extern __shared__ unsigned char smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   unsigned char* smem = smem_raw + (base - smem_u32(smem_raw));
-  constexpr int kStageBytes = eg_stage_bytes(BN);
-  constexpr int kEgStages = eg_stages(BN);
-  constexpr int kWBox = BN * kEgBK * 4;
-  constexpr uint32_t kIdesc = eg_idesc(BN);
-  constexpr uint32_t kTmemCols = BN == 128 ? 512u : 256u;       // 3 x BN columns, rounded up to a power of two
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kEgStages * kStageBytes);
+  constexpr uint32_t kTmemCols = 256u;                          // 3 x kEgBN columns, rounded up to a power of two
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kEgStages * kEgStageBytes);
   uint64_t* full = bars;                       // [stages]
   uint64_t* empty = bars + kEgStages;          // [stages]
   uint64_t* cfull = bars + 2 * kEgStages;      // [2] hi*hi chunk buffer complete
@@ -460,7 +457,7 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
   uint64_t* sfull = bars + 2 * kEgStages + 4;  // [1] correction accumulator complete (= every MMA retired)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kEgStages + 5);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m0 = blockIdx.y * kEgBM, n0 = blockIdx.x * BN;
+  const int m0 = blockIdx.y * kEgBM, n0 = blockIdx.x * kEgBN;
   const int nkb = K / kEgBK;
   const int nchunks = nkb / kEgChunkKB;        // K % 128 == 0 (checked on the host)
 
@@ -477,7 +474,7 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;       // columns [0,BN): corrections, [BN,2BN) / [2BN,3BN): hi*hi chunks
+  const uint32_t tmem_base = *tmem_slot;       // columns [0,BN): corrections, [BN,2BN) / [2BN,3BN): hi*hi chunks (BN = kEgBN)
 
   if (warp == 0) {
     if (lane == 0) {
@@ -489,12 +486,12 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
       uint32_t phase = 0;
       for (int kb = 0; kb < nkb; ++kb) {
         mbar_wait(&empty[stage], phase ^ 1u);
-        mbar_arrive_expect_tx(&full[stage], kStageBytes);
-        unsigned char* st = smem + stage * kStageBytes;
+        mbar_arrive_expect_tx(&full[stage], kEgStageBytes);
+        unsigned char* st = smem + stage * kEgStageBytes;
         eg_tma_load_2d(st, &tmap_a_hi, kb * kEgBK, m0, &full[stage]);            // rows past M are zero-filled
         eg_tma_load_2d(st + kEgBox, &tmap_a_lo, kb * kEgBK, m0, &full[stage]);
         eg_tma_load_2d(st + 2 * kEgBox, &tmap_w_hi, kb * kEgBK, n0, &full[stage]);
-        eg_tma_load_2d(st + 2 * kEgBox + kWBox, &tmap_w_lo, kb * kEgBK, n0, &full[stage]);
+        eg_tma_load_2d(st + 2 * kEgBox + kEgWBox, &tmap_w_lo, kb * kEgBK, n0, &full[stage]);
         if (++stage == kEgStages) { stage = 0; phase ^= 1u; }
       }
     }
@@ -507,19 +504,19 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
         const uint32_t buf = c & 1, use = c >> 1;
         mbar_wait(&cempty[buf], (use & 1u) ^ 1u);               // the epilogue has read this chunk buffer's last sums
         tc_fence_after();
-        const uint32_t d_main = tmem_base + static_cast<uint32_t>(BN) * (1u + buf);
+        const uint32_t d_main = tmem_base + static_cast<uint32_t>(kEgBN) * (1u + buf);
         for (int kc = 0; kc < kEgChunkKB; ++kc) {
           mbar_wait(&full[stage], phase);
           tc_fence_after();
-          const uint32_t st = base + stage * kStageBytes;
+          const uint32_t st = base + stage * kEgStageBytes;
           const uint64_t a_hi = tc_smem_desc(st), a_lo = tc_smem_desc(st + kEgBox);
-          const uint64_t w_hi = tc_smem_desc(st + 2 * kEgBox), w_lo = tc_smem_desc(st + 2 * kEgBox + kWBox);
+          const uint64_t w_hi = tc_smem_desc(st + 2 * kEgBox), w_lo = tc_smem_desc(st + 2 * kEgBox + kEgWBox);
 #pragma unroll
           for (int k = 0; k < kEgBK / 8; ++k) {
             const uint64_t o = static_cast<uint64_t>(2 * k);    // 8 tf32 = 32 B inside the swizzle atom
-            eg_mma_tf32(tmem_base, a_lo + o, w_hi + o, kIdesc, (c | kc | k) != 0 ? 1u : 0u);
-            eg_mma_tf32(tmem_base, a_hi + o, w_lo + o, kIdesc, 1u);
-            eg_mma_tf32(d_main, a_hi + o, w_hi + o, kIdesc, (kc | k) != 0 ? 1u : 0u);
+            eg_mma_tf32(tmem_base, a_lo + o, w_hi + o, kEgIdesc, (c | kc | k) != 0 ? 1u : 0u);
+            eg_mma_tf32(tmem_base, a_hi + o, w_lo + o, kEgIdesc, 1u);
+            eg_mma_tf32(d_main, a_hi + o, w_hi + o, kEgIdesc, (kc | k) != 0 ? 1u : 0u);
           }
           eg_commit(&empty[stage]);
           if (++stage == kEgStages) { stage = 0; phase ^= 1u; }
@@ -533,17 +530,17 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
     const int quarter = warp & 3;                               // TMEM lanes [32*quarter, +32) belong to this warp
     const int row = m0 + quarter * 32 + lane;
     const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
-    float acc[BN];
+    float acc[kEgBN];
 #pragma unroll
-    for (int j = 0; j < BN; ++j) acc[j] = 0.0f;
+    for (int j = 0; j < kEgBN; ++j) acc[j] = 0.0f;
     for (int c = 0; c < nchunks; ++c) {
       const uint32_t buf = c & 1, use = c >> 1;
       mbar_wait(&cfull[buf], use & 1u);
       tc_fence_after();
 #pragma unroll
-      for (int c0 = 0; c0 < BN; c0 += 32) {
+      for (int c0 = 0; c0 < kEgBN; c0 += 32) {
         uint32_t v[32];
-        tc_ld32(lane_addr + static_cast<uint32_t>(BN) * (1u + buf) + static_cast<uint32_t>(c0), v);
+        tc_ld32(lane_addr + static_cast<uint32_t>(kEgBN) * (1u + buf) + static_cast<uint32_t>(c0), v);
 #pragma unroll
         for (int j = 0; j < 32; ++j) acc[c0 + j] += __uint_as_float(v[j]);      // fp32 add, round to nearest
       }
@@ -554,7 +551,7 @@ enc_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a_hi, const __grid_c
     mbar_wait(sfull, 0u);
     tc_fence_after();
 #pragma unroll
-    for (int c0 = 0; c0 < BN; c0 += 32) {
+    for (int c0 = 0; c0 < kEgBN; c0 += 32) {
       uint32_t v[32];
       tc_ld32(lane_addr + static_cast<uint32_t>(c0), v);
       if (row < M) {

@@ -97,8 +97,6 @@ struct rse_index {
   struct Stash { DevBuf q_dev, b_tokptr, b_terms, b_idf; int nq = 0; } stash[RSE_MAX_STASH];
   // K4 tensor-core path
   int tc_mode = 0;                 // 0 auto, 1 off (exact scan only), 2 force on
-  bool second_chance = true;       // RSE_NO_SECOND_CHANCE=1 switches the second filter pass off (diagnostics)
-  int enc_bn_override = 0;         // RSE_ENC_BN=64|128 forces the encoder GEMM tile width (diagnostics)
   int survivor_div = 5;            // probe sample density: expected first-pass survivors ~ cap / survivor_div (RSE_TC_SURVIVOR_DIV).
                                    // r02 sweep, ms per 256-query step, isotropic / clustered / dense-clustered S-600k:
                                    // 3: 1.155 / 1.460 / 2.336   5: 1.146 / 1.223 / 1.785   8: 1.174 / 1.240 / 1.454
@@ -155,13 +153,6 @@ struct rse_index {
   bool bm25_overlap_pending = false;
   int ov_nq = 0, ov_limit = 0;
   double ov_k1 = 0.0, ov_b = 0.0;
-  bool wide_scan = true;           // RSE_WIDE_SCAN=0: the r01 chunk-loop kernel for widths other than 384
-  bool overlap_enabled = true;
-  bool bm25_qfast = true;          // RSE_BM25_QFAST=0: group-major CTA order (r01)
-  int bm25_pad = 0;                // RSE_BM25_PAD: extra dynamic shared memory per BM25 CTA (occupancy experiments)
-  int bm25_wide_pct = 100;         // RSE_BM25_WIDE_PCT: share of the range groups launched in the wide shape (r02: 25 / 40 /
-                                   // 60 / 100 % -> 1.064 / 1.071 / 1.087 / 1.050 ms per step: a second launch waits for the first)
-  bool bm25_wide = true;           // RSE_BM25_WIDE=0: the 512-thread BM25 CTA underneath the filter as well
   // RSE_TIMELINE=1: timed events at the stage boundaries of a hybrid step on both streams, printed (ms since the
   // step's first event) to stderr by rse_hybrid_fetch — a development aid, off by default
   bool timeline = false;
@@ -174,10 +165,9 @@ struct rse_index {
   // the probe's stratified row sample (knn_tc3.cuh tc3_sample_kernel): one row of every sample_stride, own small shadow
   DevBuf tc_sample;
   CUtensorMap tmap_s16{};
-  int64_t sample_tiles = 0;        // 0 = no sample (small corpus, RSE_TC_SAMPLE=0): the probe strides over the main shadow
+  int64_t sample_tiles = 0;        // 0 = no sample (small corpus): the probe strides over the main shadow
   int sample_stride = 64;          // RSE_TC_SAMPLE_STRIDE (r02 sweep on S-600k: 16 -> 1.137, 32 -> 1.106, 64 -> 1.091 ms per step)
   int probe_rank = 0;              // RSE_TC_PROBE_RANK: force the probe's order statistic j (tests: 1 = always too tight)
-  bool use_sample = true;          // RSE_TC_SAMPLE=0 switches the sample path off
   int sample_min_tiles = 16;       // RSE_TC_SAMPLE_MIN_TILES: 262 k rows at stride 64 (tests lower it for small corpora)
   int shadow_state = 0;            // 0 = not built, 1 = usable, -1 = corpus has non-finite norms: exact scan only
   CUtensorMap tmap_a16{};          // [n_rows][384] f16, box {64, 128}, SWIZZLE_128B
@@ -211,11 +201,7 @@ struct rse_index {
   double* normk = nullptr;
   double normk_k1 = NAN, normk_b = NAN;
   Post16* post16 = nullptr;        // {doc, tf, w}: postings with the (k1, b)-dependent weight precomputed (bm25_stream_kernel)
-  uint2* post8 = nullptr;          // {doc, round(w * wq_scale)}: the 8-byte stream of bm25_fx_kernel (padded by one pair)
-  double wq_scale = 0.0;
-  uint32_t* post4 = nullptr;       // (doc % range) | round(w * wq4_scale) << 13: the 4-byte stream (padded by one quad)
-  double wq4_scale = 0.0;
-  bool bm25_p4 = true;             // RSE_BM25_P4=0: bm25_fx_kernel reads the 8-byte stream (r02 first half)
+  uint32_t* post4 = nullptr;       // (doc % range) | round(w * wq4_scale) << 13: the stream of bm25_fx_kernel (padded by one quad)
   double w_k1 = NAN, w_b = NAN;
   DevBuf b_shi, b_slo, b_scnt, b_status, b_flagged;
   int bm25_mode = 0;               // 0 = fixed-point streaming kernel (default), 1 = exact-order streaming kernel, 2 = general kernel only
@@ -308,7 +294,7 @@ void release_embeddings(rse_index* h) {
 }
 
 void release_bm25(rse_index* h) {
-  free_ptr(h->indptr); free_ptr(h->post); free_ptr(h->dl); free_ptr(h->roff); free_ptr(h->normk); free_ptr(h->post16); free_ptr(h->post8); free_ptr(h->post4);
+  free_ptr(h->indptr); free_ptr(h->post); free_ptr(h->dl); free_ptr(h->roff); free_ptr(h->normk); free_ptr(h->post16); free_ptr(h->post4);
   h->w_k1 = NAN; h->w_b = NAN;
   h->df_host.clear();
   h->n_terms = h->n_postings = h->n_docs = h->n_movies = 0;
@@ -387,7 +373,7 @@ int launch_scan(rse_index* h, const float* q, const double* sb, int nq, float* d
     return launch_scan384<16, FMA>(h, q, sb, nq, dist);
   }
   // any width that keeps the rows 16-byte aligned: the staged kernel (queries must fit beside the stages)
-  if (h->dim % 4 == 0 && h->wide_scan && wide_smem_bytes(16, h->dim) <= 200 * 1024) {
+  if (h->dim % 4 == 0 && wide_smem_bytes(16, h->dim) <= 200 * 1024) {
     if (nq <= 1) return launch_scan_wide<1, FMA>(h, q, sb, nq, dist);
     if (nq <= 2) return launch_scan_wide<2, FMA>(h, q, sb, nq, dist);
     if (nq <= 4) return launch_scan_wide<4, FMA>(h, q, sb, nq, dist);
@@ -576,7 +562,7 @@ int ensure_shadow(rse_index* h) {
   // threshold); smaller corpora keep the strided-tile probe over the main shadow
   h->sample_tiles = 0;
   const int64_t n_sample = (h->n_rows + h->sample_stride - 1) / h->sample_stride;
-  if (h->use_sample && n_sample >= static_cast<int64_t>(h->sample_min_tiles) * kT3TileRows) {
+  if (n_sample >= static_cast<int64_t>(h->sample_min_tiles) * kT3TileRows) {
     const int64_t s_pad = (n_sample + kT3TileRows - 1) / kT3TileRows * kT3TileRows;
     const size_t s_bytes = sizeof(__half) * static_cast<size_t>(s_pad) * kScanD;
     ENSURE(h->tc_sample, s_bytes);
@@ -686,10 +672,10 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
   // Sample path (r02): the probe runs over the stratified row sample instead of a strided subset of tiles, and the
   // threshold is the sample's j-th best value, j = sample_probe_rank << K' — a few hundred survivors per query
   // instead of K' * tile_stride; the refine kernel verifies the bound and re-arms the second chance when it was too
-  // tight (1e-7 per query by construction), so it needs the second chance enabled.
+  // tight (1e-7 per query by construction).
   int kth = kprime;
   bool sampled = false;
-  if (h->sample_tiles > 0 && h->second_chance && kprime <= 256) {
+  if (h->sample_tiles > 0 && kprime <= 256) {
     const int clusters_s = static_cast<int>(std::min<int64_t>(max_clusters, h->sample_tiles));
     const int j = h->probe_rank > 0 ? std::min(h->probe_rank, kprime) : sample_probe_rank(kprime, h->sample_stride);
     if (static_cast<int64_t>(clusters_s) * 2 * kT3ProbeTop >= 8ll * j &&
@@ -800,12 +786,10 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
   float* thr2 = thr + nq_pad;
   unsigned int* gate = static_cast<unsigned int*>(h->tc_cnt.p) + nq_pad;
   {
-    int rc = knn_tc_refine(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, nullptr, nullptr,
-                           h->second_chance ? thr2 : nullptr, h->second_chance ? gate : nullptr,
+    int rc = knn_tc_refine(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, nullptr, nullptr, thr2, gate,
                            sampled ? thr + 2 * nq_pad : nullptr);
     if (rc != RSE_OK) return rc;
   }
-  if (!h->second_chance) return RSE_OK;
   // 5. second chance: one more filter pass + refine for the armed queries only (blocks without one are skipped).
   //    Enqueued unconditionally, gated on the device: two near-empty launches when no query needs it.
   knn_tc3_kernel<1><<<grid_f, kT3Threads, kT3SmemBytes, h->stream>>>(
@@ -1001,18 +985,7 @@ int rse_create(int32_t device, rse_index** out) {
     cudaMemset(h->dev_counters, 0, sizeof(unsigned long long) * 8);
   else
     h->dev_counters = nullptr;
-  // diagnostics: RSE_NO_OVERLAP=1 keeps the hybrid step's BM25 on the caller's stream (no second stream)
-  if (const char* ev = std::getenv("RSE_BM25_P4")) h->bm25_p4 = !(ev[0] == '0');
-  if (const char* ev = std::getenv("RSE_BM25_QFAST")) h->bm25_qfast = !(ev[0] == '0');
-  if (const char* ev = std::getenv("RSE_BM25_PAD")) h->bm25_pad = std::max(0, std::atoi(ev));
-  if (const char* ev = std::getenv("RSE_BM25_WIDE_PCT")) { const int v = std::atoi(ev); if (v >= 0 && v <= 100) h->bm25_wide_pct = v; }
-  if (const char* ev = std::getenv("RSE_BM25_WIDE")) h->bm25_wide = !(ev[0] == '0');
-  if (const char* ev = std::getenv("RSE_WIDE_SCAN")) h->wide_scan = !(ev[0] == '0');
-  if (const char* ev = std::getenv("RSE_NO_OVERLAP")) h->overlap_enabled = !(ev[0] == '1');
   if (const char* ev = std::getenv("RSE_TIMELINE")) h->timeline = ev[0] == '1';
-  if (const char* ev = std::getenv("RSE_NO_SECOND_CHANCE")) h->second_chance = !(ev[0] == '1');
-  if (const char* ev = std::getenv("RSE_ENC_BN")) { const int v = std::atoi(ev); if (v == 64 || v == 128) h->enc_bn_override = v; }
-  if (const char* ev = std::getenv("RSE_TC_SAMPLE")) h->use_sample = !(ev[0] == '0');
   if (const char* ev = std::getenv("RSE_TC_SAMPLE_STRIDE")) { const int v = std::atoi(ev); if (v >= 2 && v <= 256) h->sample_stride = v; }
   if (const char* ev = std::getenv("RSE_TC_SAMPLE_MIN_TILES")) { const int v = std::atoi(ev); if (v >= 1) h->sample_min_tiles = v; }
   if (const char* ev = std::getenv("RSE_TC_PROBE_RANK")) { const int v = std::atoi(ev); if (v >= 1) h->probe_rank = v; }
@@ -1448,14 +1421,10 @@ int rse_load_bm25(rse_index* h, const int64_t* indptr, const uint32_t* doc_idx, 
   if (!(h->attr_mask & (1u << 14))) {
     CK(cudaFuncSetAttribute(bm25_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBmRange * 9));
     CK(cudaFuncSetAttribute(bm25_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bs_smem_bytes()));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg) + h->bm25_pad));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg)));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg) + h->bm25_pad));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg)));
-    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg)));
+    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg)));
+    CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsWideThreads>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     h->attr_mask |= 1u << 14;
   }
   return RSE_OK;
@@ -1542,10 +1511,19 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
 
   // streaming path (bm25_stream_kernel): k <= 32; needs the weighted postings of this (k1, b)
   const bool stream = k <= 32 && h->n_postings > 0 && h->bm25_mode != 2;
+  // the 4-byte posting stream of the fixed-point kernel: wq4_scale = largest power of two with
+  // (k1 + 1) * wq4_scale <= 2^19; 0 = no stream (0 < w <= k1 + 1 needs normk >= 0)
+  double wq4_scale = 0.0;
+  if (k1 >= 0.0 && b >= 0.0 && b <= 1.0 && k1p1 < 1048576.0) {
+    int e = 0;
+    const double m = std::frexp(k1p1, &e);                 // k1p1 = m * 2^e, 0.5 <= m < 1
+    wq4_scale = std::ldexp(1.0, m == 0.5 ? 20 - e : 19 - e);
+  }
   // fixed-point sums must stay below 2^31: idf <= log(N + 2), w < k1 + 1, <= 16 tokens; the scale is the largest
-  // power of two that allows (2^21 for the default k1), and the path needs at least 2^12
+  // power of two that allows (2^21 for the default k1), and the path needs at least 2^12 and the 4-byte stream (a
+  // scale of 2^12 bounds k1 + 1 below 2^15 / ln 2 < 2^20, so the stream always exists when the scale does)
   double fx_scale = 0.0;
-  if (stream && h->bm25_mode == 0 && k1 >= 0.0 && b >= 0.0 && b <= 1.0) {      // 0 < w <= k1 + 1 needs normk >= 0
+  if (stream && h->bm25_mode == 0 && wq4_scale > 0.0) {
     const double max_sum = (k1 + 1.0) * std::log(static_cast<double>(h->n_movies) + 2.0) * 16.0 + 1.0;
     int e = 0;
     std::frexp(max_sum, &e);                               // max_sum < 2^e
@@ -1556,23 +1534,10 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
   if (stream) {
     if (!(h->w_k1 == k1 && h->w_b == b)) {
       if (!h->post16) CK(cudaMalloc(&h->post16, sizeof(Post16) * static_cast<size_t>(h->n_postings)));
-      // compact stream of the fixed-point kernel: wq_scale = largest power of two with (k1 + 1) * wq_scale <= 2^31
-      h->wq_scale = 0.0;
-      if (k1 >= 0.0 && b >= 0.0 && b <= 1.0 && k1p1 < 1048576.0) {
-        int e = 0;
-        const double m = std::frexp(k1p1, &e);                 // k1p1 = m * 2^e, 0.5 <= m < 1
-        h->wq_scale = std::ldexp(1.0, m == 0.5 ? 32 - e : 31 - e);
-        if (!h->post8) CK(cudaMalloc(&h->post8, sizeof(uint2) * (static_cast<size_t>(h->n_postings) + 2)));
-        h->wq4_scale = 0.0;
-        if (h->bm25_p4) {                                      // largest power of two with (k1 + 1) * wq4_scale <= 2^19
-          h->wq4_scale = std::ldexp(1.0, m == 0.5 ? 20 - e : 19 - e);
-          if (!h->post4) CK(cudaMalloc(&h->post4, sizeof(uint32_t) * (static_cast<size_t>(h->n_postings) + 8)));
-        }
-      }
+      if (wq4_scale > 0.0 && !h->post4) CK(cudaMalloc(&h->post4, sizeof(uint32_t) * (static_cast<size_t>(h->n_postings) + 8)));
       const int threads = 256;
       bm25_weight_kernel<<<static_cast<unsigned int>((h->n_postings + threads - 1) / threads), threads, 0, h->stream>>>(
-          h->post, h->normk, h->n_postings, k1p1, h->post16, h->wq_scale > 0.0 ? h->post8 : nullptr, h->wq_scale,
-          h->wq4_scale > 0.0 ? h->post4 : nullptr, h->wq4_scale);
+          h->post, h->normk, h->n_postings, k1p1, h->post16, wq4_scale > 0.0 ? h->post4 : nullptr, wq4_scale);
       LAUNCHED(h);
       h->w_k1 = k1; h->w_b = b;
     }
@@ -1618,38 +1583,24 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
       uint2* fin = static_cast<uint2*>(h->b_shi.p) - static_cast<int64_t>(q0) * ng * kFxFinalCap;
       int* fcnt = static_cast<int*>(h->b_scnt.p) - static_cast<int64_t>(q0) * ng;
       status = static_cast<int*>(h->b_status.p);
-      const int rpg_arg = h->bm25_qfast ? -rpg : rpg;
+      const double idfx_scale = fx_scale / wq4_scale;
       // underneath the tensor-core filter (hybrid step, second stream): wide CTAs (bm25.cuh: 28 warps beside the
-      // filter's CTA).  Alone the 512-thread shape is the faster one (4 CTAs per SM: 284 against 318 us), so the
-      // groups CAN be split between the two shapes — measured, the split loses (see bm25_wide_pct)
-      const bool under_filter = h->bm25_wide && h->bm25_qfast && h->stream_b && h->stream == h->stream_b;
-      const int g_wide = under_filter ? std::min(ng, std::max(1, (ng * h->bm25_wide_pct + 50) / 100)) : 0;
-      const bool p4 = h->bm25_p4 && h->wq4_scale > 0.0 && h->post4;
-      const uint2* stream8 = p4 ? reinterpret_cast<const uint2*>(h->post4) : h->post8;   // P4 reads it as uint32
-      const double idfx_scale = fx_scale / (p4 ? h->wq4_scale : h->wq_scale);
-      auto launch_fx = [&](auto kernel, dim3 grid, int threads, size_t smem, int g0) {
-        kernel<<<grid, threads, smem, h->stream>>>(
-            h->indptr, stream8, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
-            static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), idfx_scale, q0, k,
-            rpg_arg, ng, g0, fin, fcnt, status);
-      };
-      if (g_wide > 0) {
-        if (p4) launch_fx(bm25_fx_kernel<kBsWideThreads, true>, dim3(nc, g_wide), kBsWideThreads, fx_smem_bytes(rpg), 0);
-        else launch_fx(bm25_fx_kernel<kBsWideThreads, false>, dim3(nc, g_wide), kBsWideThreads, fx_smem_bytes(rpg), 0);
-        LAUNCHED(h);
-      }
-      if (g_wide < ng) {
-        const int g_rest = ng - g_wide;
-        const dim3 grid = h->bm25_qfast ? dim3(nc, g_rest) : dim3(ng, nc);
-        if (p4) launch_fx(bm25_fx_kernel<kBsThreads, true>, grid, kBsThreads, fx_smem_bytes(rpg) + h->bm25_pad, g_wide);
-        else launch_fx(bm25_fx_kernel<kBsThreads, false>, grid, kBsThreads, fx_smem_bytes(rpg) + h->bm25_pad, g_wide);
-        LAUNCHED(h);
-      }
+      // filter's CTA).  Alone the 512-thread shape is the faster one (4 CTAs per SM: 284 against 318 us).  Splitting
+      // the groups between the two shapes loses (r02, 25 / 40 / 60 / 100 % wide -> 1.064 / 1.071 / 1.087 / 1.050 ms
+      // per step): a second launch waits for the first.
+      const bool under_filter = h->stream_b && h->stream == h->stream_b;
+      const int threads = under_filter ? kBsWideThreads : kBsThreads;
+      const auto kernel = under_filter ? bm25_fx_kernel<kBsWideThreads> : bm25_fx_kernel<kBsThreads>;
+      kernel<<<dim3(nc, ng), threads, fx_smem_bytes(rpg), h->stream>>>(
+          h->indptr, h->post4, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
+          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), idfx_scale, q0, k, rpg,
+          ng, fin, fcnt, status);
+      LAUNCHED(h);
       bm25_fx_finish_kernel<<<nc, kBmThreads, 0, h->stream>>>(
           fin, fcnt, ng, status, h->indptr, h->post16, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
           static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k,
           static_cast<double*>(h->b_score.p), static_cast<int*>(h->b_doc.p), static_cast<int*>(h->b_count.p),
-          h->dev_counters, p4 ? idfx_scale : 0.0);
+          h->dev_counters, idfx_scale);
       LAUNCHED(h);
     } else if (stream) {
       const size_t per_qs = static_cast<size_t>(ng) * std::max(k, 2 * kFxFinalCap);
@@ -1895,11 +1846,11 @@ int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limi
     // kernel keeps one 178 KB CTA per SM busy on the tensor pipe at ~20 % issue utilisation, and one BM25 CTA
     // (38 KB, 512 threads) fits beside it.
     tl_mark(h, kTlStart, h->stream);
-    h->bm25_overlap_pending = h->overlap_enabled;
+    h->bm25_overlap_pending = true;
     h->ov_nq = nq; h->ov_limit = limit; h->ov_k1 = k1; h->ov_b = b;
     rc = knn_local_begin(h, static_cast<const float*>(h->q_dev.p), nq, kprime, static_cast<long long*>(h->cand.p));
     if (rc != RSE_OK) { h->bm25_overlap_pending = false; return rc; }
-    const bool overlapped = h->overlap_enabled && !h->bm25_overlap_pending;   // the filter launch consumed the request
+    const bool overlapped = !h->bm25_overlap_pending;         // the filter launch consumed the request
     h->bm25_overlap_pending = false;
     if (!overlapped) {
       tl_mark(h, kTlBm25Start, h->stream);
@@ -2177,31 +2128,23 @@ template <int EPI>
 int enc_gemm_tc(rse_index* h, const float* A_hi, const float* A_lo, const float* W_hi, const float* W_lo, const float* bias,
                 float* C, float* C_lo, int M, int N, int K) {
   if (!(h->attr_mask & (1u << 17))) {
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<0, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(128)));
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<1, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(128)));
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<0, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<2, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(128)));
-    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, eg_smem_bytes(64)));
+    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEgSmemBytes));
+    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEgSmemBytes));
+    CK(cudaFuncSetAttribute(enc_gemm_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEgSmemBytes));
     h->attr_mask |= 1u << 17;
   }
   // 64-wide tiles, two CTAs per SM (r02, 256 queries / 2.5 k tokens, ms per host-buffer encode call: 64-wide
   // everywhere 1.35, 128-wide everywhere 1.46, 128-wide unless that leaves SMs idle 1.49): the kernel is bound by
   // the latency of its operand ring and by wave quantisation, so more, smaller tiles in flight win
   const int m_tiles = (M + kEgBM - 1) / kEgBM;
-  int bn = (N % 64 == 0) ? 64 : 128;
-  if (h->enc_bn_override == 128) bn = 128;
   CUtensorMap ta_h, ta_l, tw_h, tw_l;
   int rc = make_tmap_f32(h, &ta_h, A_hi, M, K, kEgBM);
   if (rc == RSE_OK) rc = make_tmap_f32(h, &ta_l, A_lo, M, K, kEgBM);
-  if (rc == RSE_OK) rc = make_tmap_f32(h, &tw_h, W_hi, N, K, bn);
-  if (rc == RSE_OK) rc = make_tmap_f32(h, &tw_l, W_lo, N, K, bn);
+  if (rc == RSE_OK) rc = make_tmap_f32(h, &tw_h, W_hi, N, K, kEgBN);
+  if (rc == RSE_OK) rc = make_tmap_f32(h, &tw_l, W_lo, N, K, kEgBN);
   if (rc != RSE_OK) return rc;
-  dim3 grid((N + bn - 1) / bn, m_tiles);
-  if (bn == 128)
-    enc_gemm_tc_kernel<EPI, 128><<<grid, kEgThreads, eg_smem_bytes(128), h->stream>>>(ta_h, ta_l, tw_h, tw_l, bias, C, C_lo, M, N, K);
-  else
-    enc_gemm_tc_kernel<EPI, 64><<<grid, kEgThreads, eg_smem_bytes(64), h->stream>>>(ta_h, ta_l, tw_h, tw_l, bias, C, C_lo, M, N, K);
+  dim3 grid((N + kEgBN - 1) / kEgBN, m_tiles);
+  enc_gemm_tc_kernel<EPI><<<grid, kEgThreads, kEgSmemBytes, h->stream>>>(ta_h, ta_l, tw_h, tw_l, bias, C, C_lo, M, N, K);
   LAUNCHED(h);
   return RSE_OK;
 }
@@ -2943,13 +2886,13 @@ int sharded_knn_exchange(rse_index* h, const float* q_all_dev, int nq_all, int k
   ENSURE(h->sh_mine, sizeof(long long) * static_cast<size_t>(R) * std::max(ns, 1) * per);
   *bm25_overlapped = false;
   if (with_bm25 && ns > 0) {
-    h->bm25_overlap_pending = h->overlap_enabled;
+    h->bm25_overlap_pending = true;
     h->ov_nq = ns; h->ov_limit = limit; h->ov_k1 = k1; h->ov_b = b;
   }
   int rc = knn_local_begin(h, q_all_dev, nq_all, kprime, static_cast<long long*>(h->sh_cand.p));
   if (rc != RSE_OK) { h->bm25_overlap_pending = false; return rc; }
   if (with_bm25 && ns > 0) {
-    *bm25_overlapped = h->overlap_enabled && !h->bm25_overlap_pending;     // the filter launch consumed the request
+    *bm25_overlapped = !h->bm25_overlap_pending;              // the filter launch consumed the request
     h->bm25_overlap_pending = false;
     if (!*bm25_overlapped) {
       rc = bm25_run(h, ns, limit, k1, b);
