@@ -313,6 +313,50 @@ int rse_encode_images_dev(rse_index *h, int32_t slot, const float *pixels_dev, i
 int rse_hybrid_stage_dev(rse_index *h, int32_t nq, const float *q_dev, const int32_t *tok_indptr,
                          const int32_t *term_rows);
 
+/* ------------------------------------------------------------------ cross-encoder rerank of a fused batch
+ * HybridSearch.rrf_search(..., rerank_method="cross_encoder") (hybrid_search.py:279-312) for a whole staged batch, on
+ * the device (csrc/rerank.cuh): RRF over the WHOLE union of the two hit lists (up to 2 * limit ids per query), one
+ * (query, document) pair per union member scored by the cross-encoder of an encoder slot, a stable descending sort on
+ * (cross_encoder_score, rrf_score), the first `limit`.
+ *   rse_rerank_docs_load : the document-token store.  ids[n_docs] strictly ascending (the movies.id universe);
+ *                          tok_indptr[n_docs + 1] (from 0, non-decreasing) / tokens = the cross-encoder tokenizer's
+ *                          ids of each document's text f"{title} - {description}" WITHOUT special tokens.  4 B per
+ *                          token in HBM.  A new load replaces the store.
+ *   rse_hybrid_rerank_run: on the batch staged by rse_hybrid_stage / rse_hybrid_stage_dev.  q_tok_indptr[nq + 1] /
+ *                          q_tok_ids = the cross-encoder tokenizer's ids of each query (no special tokens); cls_id /
+ *                          sep_id its [CLS] / [SEP].  A pair is [CLS] q[:a] [SEP] d[:b] [SEP] with token types 0 for
+ *                          the first a + 2 tokens and 1 for the rest, (a, b) by the HF fast tokenizers' longest_first
+ *                          truncation to max_length (rse_pair_truncate).  activation 0 = the classifier logit, 1 =
+ *                          float32(1 / (1 + exp(-logit))) in fp64.  Synchronises ONCE, after the pairs are assembled,
+ *                          to cut them into encoder slices (rse_set_rerank_token_budget) — besides the wait for the
+ *                          tensor-core KNN's overflow flags that every hybrid step has.  The plain hybrid results of
+ *                          the staged batch (rse_hybrid_fetch) are not touched.
+ *                          RSE_ERR_STATE: no store, nothing staged, submit tickets in flight, or a fused id missing
+ *                          from the store (the message names the first).  RSE_ERR_INVALID: the slot is not a finalized
+ *                          head-1 BERT, activation not 0 / 1, a query / store / cls / sep token >= vocab_size.
+ *                          RSE_ERR_UNSUPPORTED: limit outside [1, 128], max_length < 4 or > max_positions.
+ *   rse_hybrid_rerank_fetch: [nq, limit] id, rrf score, bm25_rank / sem_rank (0-based, -1 = None), rrf_rank (1-based
+ *                          fused position), cross-encoder score; count[nq].  Synchronises.
+ *   rse_set_rerank_token_budget: most tokens per encoder slice (default 131072: the TinyBERT encoder's scratch is
+ *                          ~9 KB per token); a pair longer than the budget is a slice of its own.  Results do not
+ *                          depend on it.
+ *   rse_hybrid_rerank_timing: with rse_set_timing on, device ms of the last run's hybrid / assembly / encoder / order
+ *                          stages (out_ms[4]).  Synchronises.
+ *   rse_pair_truncate    : the truncation rule alone (host arithmetic, no handle): n1 query and n2 document tokens
+ *                          -> the (a, b) kept for max_length (>= 4). */
+int rse_rerank_docs_load(rse_index *h, const int64_t *ids, int64_t n_docs, const int64_t *tok_indptr,
+                         const int32_t *tokens);
+int rse_hybrid_rerank_run(rse_index *h, int32_t slot, double k, int32_t tie_mode, int32_t limit,
+                          int32_t knn_multiplier, double k1, double b, const int32_t *q_tok_indptr,
+                          const int32_t *q_tok_ids, int32_t cls_id, int32_t sep_id, int32_t max_length,
+                          int32_t activation);
+int rse_hybrid_rerank_fetch(rse_index *h, int32_t limit, int64_t *out_id, double *out_score,
+                            int32_t *out_bm25_rank, int32_t *out_sem_rank, int32_t *out_rrf_rank,
+                            float *out_ce_score, int32_t *out_count);
+int rse_set_rerank_token_budget(rse_index *h, int64_t tokens);
+int rse_hybrid_rerank_timing(rse_index *h, float *out_ms);
+int rse_pair_truncate(int32_t n1, int32_t n2, int32_t max_length, int32_t *a, int32_t *b);
+
 /* ------------------------------------------------------------------ multi-GPU: row shards over one box (SURVEY §8e)
  * One process per GPU, one handle per process; the HANDLE owns the NCCL communicator (NCCL is bound at run time:
  * libnccl.so.2, or $RSE_NCCL_LIB).  The chunk-embedding matrix is cut by row into contiguous shards aligned to

@@ -138,6 +138,14 @@ _SIGNATURES = {
     "rse_encode_images": (ctypes.c_int, [c_void_p, c_int32, POINTER(c_float), c_int32, POINTER(c_float)]),
     "rse_encode_images_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
     "rse_hybrid_stage_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
+    "rse_rerank_docs_load": (ctypes.c_int, [c_void_p, POINTER(c_int64), c_int64, POINTER(c_int64), POINTER(c_int32)]),
+    "rse_hybrid_rerank_run": (ctypes.c_int, [c_void_p, c_int32, c_double, c_int32, c_int32, c_int32, c_double, c_double,
+                                             POINTER(c_int32), POINTER(c_int32), c_int32, c_int32, c_int32, c_int32]),
+    "rse_hybrid_rerank_fetch": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               c_void_p, c_void_p]),
+    "rse_set_rerank_token_budget": (ctypes.c_int, [c_void_p, c_int64]),
+    "rse_hybrid_rerank_timing": (ctypes.c_int, [c_void_p, POINTER(c_float)]),
+    "rse_pair_truncate": (ctypes.c_int, [c_int32, c_int32, c_int32, POINTER(c_int32), POINTER(c_int32)]),
     "rse_comm_unique_id": (ctypes.c_int, [c_void_p]),
     "rse_comm_init": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32]),
     "rse_comm_destroy": (ctypes.c_int, [c_void_p]),
@@ -174,6 +182,16 @@ def load_library() -> ctypes.CDLL:
             fn.argtypes = args
         _lib = L
     return _lib
+
+
+def pair_truncate(n1: int, n2: int, max_length: int):
+    """(a, b): how many of n1 query and n2 document tokens a cross-encoder pair of max_length keeps (rse_pair_truncate,
+    the HF fast tokenizers' longest_first rule)."""
+    a, b = c_int32(0), c_int32(0)
+    rc = load_library().rse_pair_truncate(int(n1), int(n2), int(max_length), ctypes.byref(a), ctypes.byref(b))
+    if rc != RSE_OK:
+        raise RseError(rc, "rse_pair_truncate: n1, n2 >= 0 and max_length >= 4")
+    return int(a.value), int(b.value)
 
 
 def _ptr(a, ty):
@@ -576,6 +594,63 @@ class Index:
         self._check(self._L.rse_hybrid_stage_dev(self._h, int(nq), c_void_p(q_ptr), c_void_p(tok_indptr.ctypes.data),
                                                  c_void_p(term_rows.ctypes.data)))
         self._staged_nq = int(nq)
+
+    # ------------------------------------------------------------------ cross-encoder rerank of a fused batch
+    def rerank_docs_load(self, ids, tok_indptr, tokens):
+        """The document-token store: ids strictly ascending, CSR token ids (no special tokens) per document."""
+        ids = _c(ids, np.int64)
+        tok_indptr = _c(tok_indptr, np.int64)
+        tokens = _c(tokens, np.int32)
+        if len(tok_indptr) != len(ids) + 1:
+            raise ValueError("tok_indptr must have len(ids) + 1 entries")
+        if tokens.size == 0:
+            tokens = np.zeros(1, np.int32)
+        self._check(self._L.rse_rerank_docs_load(self._h, _ptr(ids, c_int64), len(ids), _ptr(tok_indptr, c_int64),
+                                                 _ptr(tokens, c_int32)))
+
+    def set_rerank_token_budget(self, tokens: int):
+        self._check(self._L.rse_set_rerank_token_budget(self._h, int(tokens)))
+
+    def hybrid_rerank_run(self, slot: int, k: float, limit: int, q_tok_indptr, q_tok_ids, *, cls_id: int, sep_id: int,
+                          max_length: int, activation: int = 0, knn_multiplier: int = 10, k1: float = 1.5,
+                          b: float = 0.75, tie_mode: int = TIE_REFERENCE):
+        """RRF over the whole union + cross-encoder rerank of the staged batch (include/rse.h); the query token ids
+        come without special tokens."""
+        q_tok_indptr = _c(q_tok_indptr, np.int32)
+        q_tok_ids = _c(q_tok_ids, np.int32)
+        nq = getattr(self, "_staged_nq", 0)
+        if nq and len(q_tok_indptr) != nq + 1:               # (nothing staged: the library reports the state)
+            raise ValueError("q_tok_indptr must have (staged queries) + 1 entries")
+        if q_tok_ids.size == 0:
+            q_tok_ids = np.zeros(1, np.int32)
+        self._check(self._L.rse_hybrid_rerank_run(self._h, int(slot), float(k), int(tie_mode), int(limit),
+                                                  int(knn_multiplier), float(k1), float(b), _ptr(q_tok_indptr, c_int32),
+                                                  _ptr(q_tok_ids, c_int32), int(cls_id), int(sep_id), int(max_length),
+                                                  int(activation)))
+        self._rerank_nq = self._staged_nq
+
+    def hybrid_rerank_fetch(self, limit: int):
+        """-> (id int64, rrf score float64, bm25_rank, sem_rank (-1 = None), rrf_rank int32, each [nq, limit];
+        cross-encoder score float32 [nq, limit]; count int32 [nq])."""
+        nq = getattr(self, "_rerank_nq", 0)
+        oid = np.zeros((nq, limit), np.int64)
+        osc = np.zeros((nq, limit), np.float64)
+        orb = np.zeros((nq, limit), np.int32)
+        ors = np.zeros((nq, limit), np.int32)
+        orr = np.zeros((nq, limit), np.int32)
+        oce = np.zeros((nq, limit), np.float32)
+        oc = np.zeros(nq, np.int32)
+        self._check(self._L.rse_hybrid_rerank_fetch(self._h, int(limit), c_void_p(oid.ctypes.data),
+                                                    c_void_p(osc.ctypes.data), c_void_p(orb.ctypes.data),
+                                                    c_void_p(ors.ctypes.data), c_void_p(orr.ctypes.data),
+                                                    c_void_p(oce.ctypes.data), c_void_p(oc.ctypes.data)))
+        return oid, osc, orb, ors, orr, oce, oc
+
+    def hybrid_rerank_timing(self):
+        """Device ms of the last timed rerank run: (hybrid, assembly, encoder, order)."""
+        out = (c_float * 4)()
+        self._check(self._L.rse_hybrid_rerank_timing(self._h, out))
+        return tuple(float(x) for x in out)
 
     # ------------------------------------------------------------------ multi-GPU (library-owned NCCL communicator)
     @staticmethod

@@ -38,10 +38,11 @@ struct FuseIn {
 };
 
 // mode 0 = rrf (param = k), mode 1 = weighted (param = alpha)
-// outputs [nq][limit]: id, score, a, b  (rrf: a/b = bm25_rank/sem_rank as double, -1 = None;
-//                                        weighted: a/b = bm25_norm/sem_norm)
+// inputs [nq][limit]; outputs [nq][out_w] (limit <= out_w <= 2 * limit): id, score, a, b  (rrf: a/b =
+// bm25_rank/sem_rank as double, -1 = None; weighted: a/b = bm25_norm/sem_norm).  out_w = limit is the reference's
+// [:limit]; out_w = 2 * limit keeps the whole union in fused order (what the cross-encoder rerank scores).
 __global__ void __launch_bounds__(32)
-fuse_kernel(FuseIn in, int nq, int limit, int mode, double param, int tie_mode, long long* __restrict__ out_id,
+fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int tie_mode, long long* __restrict__ out_id,
             double* __restrict__ out_score, double* __restrict__ out_a, double* __restrict__ out_b,
             int* __restrict__ out_count) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -153,8 +154,8 @@ fuse_kernel(FuseIn in, int nq, int limit, int mode, double param, int tie_mode, 
   }
   __syncwarp();
 
-  // ---- stable descending sort by rank counting, then [:limit] ---------------
-  const int n_out = n < limit ? n : limit;
+  // ---- stable descending sort by rank counting, then [:out_w] ---------------
+  const int n_out = n < out_w ? n : out_w;
   for (int i = lane; i < n; i += 32) {
     const double si = score[i];
     int rank = 0;
@@ -162,13 +163,13 @@ fuse_kernel(FuseIn in, int nq, int limit, int mode, double param, int tie_mode, 
       const double sj = score[j];
       rank += (sj > si) || (sj == si && j < i);
     }
-    if (rank < limit) {
-      const int64_t o = static_cast<int64_t>(q) * limit + rank;
+    if (rank < out_w) {
+      const int64_t o = static_cast<int64_t>(q) * out_w + rank;
       out_id[o] = order[i]; out_score[o] = si; out_a[o] = va[i]; out_b[o] = vb[i];
     }
   }
-  for (int i = n_out + lane; i < limit; i += 32) {
-    const int64_t o = static_cast<int64_t>(q) * limit + i;
+  for (int i = n_out + lane; i < out_w; i += 32) {
+    const int64_t o = static_cast<int64_t>(q) * out_w + i;
     out_id[o] = -1; out_score[o] = 0.0; out_a[o] = -1.0; out_b[o] = -1.0;
   }
   if (lane == 0) out_count[q] = n_out;

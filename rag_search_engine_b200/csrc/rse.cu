@@ -23,6 +23,7 @@
 #include "knn_scan.cuh"
 #include "select.cuh"
 #include "knn_tc3.cuh"
+#include "rerank.cuh"
 
 using namespace rse;
 
@@ -214,6 +215,25 @@ struct rse_index {
   int64_t n_doc_ids = 0;
   long long* movie_ids = nullptr;
   int64_t n_movie_ids = 0;
+
+  // ---- cross-encoder rerank of a fused batch (rerank.cuh): the document-token store (CSR over ascending ids) ...
+  long long* rr_doc_ids = nullptr;
+  long long* rr_doc_indptr = nullptr;
+  int32_t* rr_doc_tok = nullptr;
+  int64_t rr_n_docs = 0;
+  int32_t rr_max_tok = -1;
+  int64_t rr_max_doc_len = 0;      // longest document: bounds a pair's length together with the queries and max_length
+  int64_t rr_budget = 1 << 17;     // tokens per encoder slice: the encoder's scratch is ~9 KB per TinyBERT token
+  // ... the whole fused union [nq, 2 * limit], the packed pairs, and the [nq, limit] results back to back
+  DevBuf rr_fid, rr_fsc, rr_fa, rr_fb, rr_fcnt, rr_row, rr_ab, rr_qnp, rr_qnt, rr_qpb, rr_qtb, rr_meta, rr_qptr, rr_qtok;
+  DevBuf rr_ids, rr_types, rr_cus, rr_logit, rr_pack;
+  int* rr_pin_meta = nullptr;
+  size_t rr_pin_meta_n = 0;
+  char* rr_pin_out = nullptr;
+  size_t rr_pin_out_bytes = 0;
+  int rr_nq = 0, rr_limit = 0;
+  cudaEvent_t rr_ev[5] = {};       // rse_set_timing: hybrid | assembly | encoder | order boundaries of the last run
+  bool rr_timed = false;
 
   // cudaFuncSetAttribute is per device: remember per HANDLE which kernels were configured (a process-wide static
   // flag would leave the second device of a multi-GPU process unconfigured)
@@ -1033,6 +1053,14 @@ void rse_destroy(rse_index* h) {
   if (h->stream_b) cudaStreamDestroy(h->stream_b);
   free_ptr(h->doc_ids);
   free_ptr(h->movie_ids);
+  free_ptr(h->rr_doc_ids); free_ptr(h->rr_doc_indptr); free_ptr(h->rr_doc_tok);
+  for (DevBuf* b : {&h->rr_fid, &h->rr_fsc, &h->rr_fa, &h->rr_fb, &h->rr_fcnt, &h->rr_row, &h->rr_ab, &h->rr_qnp,
+                    &h->rr_qnt, &h->rr_qpb, &h->rr_qtb, &h->rr_meta, &h->rr_qptr, &h->rr_qtok, &h->rr_ids, &h->rr_types,
+                    &h->rr_cus, &h->rr_logit, &h->rr_pack})
+    free_buf(*b);
+  if (h->rr_pin_meta) cudaFreeHost(h->rr_pin_meta);
+  if (h->rr_pin_out) cudaFreeHost(h->rr_pin_out);
+  for (cudaEvent_t e : h->rr_ev) if (e) cudaEventDestroy(e);
   for (auto& e : h->enc) enc_release(e);
   free_ptr(h->dev_counters);
   if (h->comm) { if (NcclApi* n = nccl_api()) n->CommDestroy(h->comm); h->comm = nullptr; }
@@ -1680,7 +1708,8 @@ int rse_bm25(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows, 
 // ------------------------------------------------------------------ fusion
 namespace {
 
-int fuse_launch(rse_index* h, int mode, double param, int tie_mode, int nq, int limit, const FuseIn& in,
+// inputs [nq, limit]; outputs [nq, out_w] (fuse_kernel: limit <= out_w <= 2 * limit)
+int fuse_launch(rse_index* h, int mode, double param, int tie_mode, int nq, int limit, int out_w, const FuseIn& in,
                 long long* o_id, double* o_sc, double* o_a, double* o_b, int* o_cnt) {
   if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "fusion: limit must be in [1, 128]");
   if (tie_mode != RSE_TIE_REFERENCE && tie_mode != RSE_TIE_BY_ID) return fail(h, RSE_ERR_INVALID, "fusion: bad tie_mode");
@@ -1690,7 +1719,7 @@ int fuse_launch(rse_index* h, int mode, double param, int tie_mode, int nq, int 
                             static_cast<int>(fuse_smem_bytes(RSE_MAX_FUSE_LIMIT))));
     h->attr_mask |= 1u << 15;
   }
-  fuse_kernel<<<nq, 32, smem, h->stream>>>(in, nq, limit, mode, param, tie_mode, o_id, o_sc, o_a, o_b, o_cnt);
+  fuse_kernel<<<nq, 32, smem, h->stream>>>(in, nq, limit, out_w, mode, param, tie_mode, o_id, o_sc, o_a, o_b, o_cnt);
   LAUNCHED(h);
   return RSE_OK;
 }
@@ -1721,7 +1750,7 @@ int fuse_host(rse_index* h, int mode, double param, int tie_mode, int nq, int li
             static_cast<const int*>(h->f_bcnt.p),      static_cast<const long long*>(h->f_sid.p),
             nullptr,                                   static_cast<const int*>(h->f_scnt.p),
             static_cast<const double*>(h->f_sds.p)};
-  int rc = fuse_launch(h, mode, param, tie_mode, nq, limit, in, static_cast<long long*>(h->f_oid.p),
+  int rc = fuse_launch(h, mode, param, tie_mode, nq, limit, limit, in, static_cast<long long*>(h->f_oid.p),
                        static_cast<double*>(h->f_osc.p), static_cast<double*>(h->f_oa.p),
                        static_cast<double*>(h->f_ob.p), static_cast<int*>(h->f_ocnt.p));
   if (rc != RSE_OK) return rc;
@@ -1807,10 +1836,11 @@ int rse_hybrid_stage(rse_index* h, int32_t nq, const float* q_host, const int32_
 namespace {
 
 // BM25 + (local KNN | merge of gathered shard candidates) + aggregation + fusion on the staged batch.
-// Outputs go to the given device buffers ([nq, limit]).
+// Outputs go to the given device buffers ([nq, out_w]: out_w = limit is the reference's [:limit], 2 * limit the
+// whole fused union the cross-encoder rerank scores).
 int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limit, int knn_multiplier, double k1,
                     double b, const long long* gathered, int n_lists, long long* o_id, double* o_sc, double* o_a,
-                    double* o_b, int* o_cnt) {
+                    double* o_b, int* o_cnt, int out_w) {
   const int nq = h->staged_nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
   if (mode != 0 && mode != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid: mode must be 0 (rrf) or 1 (weighted)");
@@ -1879,7 +1909,7 @@ int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limi
             static_cast<const float*>(h->o_dist.p), static_cast<const int*>(h->o_count.p), nullptr};
   in.bm25_idx = static_cast<const int*>(h->b_doc.p); in.bm25_table = h->doc_ids; in.bm25_table_n = h->n_doc_ids;
   in.sem_idx = static_cast<const int*>(h->o_movie.p); in.sem_table = h->movie_ids; in.sem_table_n = h->n_movie_ids;
-  rc = fuse_launch(h, mode, param, tie_mode, nq, limit, in, o_id, o_sc, o_a, o_b, o_cnt);
+  rc = fuse_launch(h, mode, param, tie_mode, nq, limit, out_w, in, o_id, o_sc, o_a, o_b, o_cnt);
   tl_mark(h, kTlStepEnd, h->stream);
   return rc;
 }
@@ -1901,7 +1931,7 @@ int rse_hybrid_run(rse_index* h, int32_t mode, double param, int32_t tie_mode, i
   return hybrid_run_impl(h, mode, param, tie_mode, limit, knn_multiplier, k1, b, nullptr, 0,
                          reinterpret_cast<long long*>(pk), reinterpret_cast<double*>(pk + 8 * n),
                          reinterpret_cast<double*>(pk + 16 * n), reinterpret_cast<double*>(pk + 24 * n),
-                         reinterpret_cast<int*>(pk + 32 * n));
+                         reinterpret_cast<int*>(pk + 32 * n), limit);
 }
 
 int rse_hybrid_run_merged_dev(rse_index* h, int32_t mode, double param, int32_t tie_mode, int32_t limit,
@@ -1913,7 +1943,8 @@ int rse_hybrid_run_merged_dev(rse_index* h, int32_t mode, double param, int32_t 
     return fail(h, RSE_ERR_INVALID, "rse_hybrid_run_merged_dev: bad arguments");
   return hybrid_run_impl(h, mode, param, tie_mode, limit, knn_multiplier, k1, b,
                          reinterpret_cast<const long long*>(gathered_dev), n_lists,
-                         reinterpret_cast<long long*>(out_id_dev), out_score_dev, out_a_dev, out_b_dev, out_count_dev);
+                         reinterpret_cast<long long*>(out_id_dev), out_score_dev, out_a_dev, out_b_dev, out_count_dev,
+                         limit);
 }
 
 int rse_hybrid_fetch(rse_index* h, int32_t limit, int64_t* out_id, double* out_score, double* out_a, double* out_b,
@@ -2150,9 +2181,13 @@ int enc_gemm_tc(rse_index* h, const float* A_hi, const float* A_lo, const float*
 }
 }
 
-// ids / type_ids / cu_seqlens are on the device already; x <- encoder output [T, hidden]; out <- head output
-int enc_forward(rse_index* h, Encoder& e, int n_seq, int T, bool has_types, float* out_dev) {
+// A BERT slot on device inputs: ids / type_ids (NULL = all 0) [T] and cu_seqlens [n_seq + 1] (starting at 0) are on the
+// handle's device, max_len is the longest sequence; x <- encoder output [T, hidden]; out <- head output.  The host
+// entry points (enc_run) and the batched rerank (rse_hybrid_rerank_run) both end here.
+int enc_forward(rse_index* h, Encoder& e, const int32_t* ids, const int32_t* type_ids, const int32_t* cu, int n_seq,
+                int T, int max_len, float* out_dev) {
   const rse_encoder_config& c = e.cfg;
+  e.max_len = max_len;
   const int H = c.hidden, I = c.intermediate;
   const bool tc = e.mode == 0 && e.tc_ok;
   ENSURE(e.posidx, sizeof(int32_t) * T);
@@ -2176,12 +2211,11 @@ int enc_forward(rse_index* h, Encoder& e, int n_seq, int T, bool has_types, floa
   float* x_l = tc ? static_cast<float*>(e.x_l.p) : nullptr;
   float* ctx_l = tc ? static_cast<float*>(e.ctx_l.p) : nullptr;
   float* ff_l = tc ? static_cast<float*>(e.ff_l.p) : nullptr;
-  const int32_t* cu = static_cast<const int32_t*>(e.cu.p);
   enc_positions_kernel<<<(T + 255) / 256, 256, 0, h->stream>>>(cu, n_seq, T, static_cast<int32_t*>(e.posidx.p));
   LAUNCHED(h);
   const int tok_grid = (T + 3) / 4;
   enc_embed_ln_kernel<<<tok_grid, 128, 0, h->stream>>>(
-      static_cast<const int32_t*>(e.ids.p), has_types ? static_cast<const int32_t*>(e.type_ids.p) : nullptr,
+      ids, type_ids,
       static_cast<const int32_t*>(e.posidx.p), T, H, c.vocab_size, c.max_positions, c.type_vocab, e.word, e.pos, e.type,
       e.elng, e.elnb, c.ln_eps, x, x_h, x_l);
   LAUNCHED(h);
@@ -2407,9 +2441,13 @@ int enc_run(rse_index* h, int32_t slot, const int32_t* ids, const int32_t* type_
   CK(cudaMemcpyAsync(e.cu.p, pin + 2 * static_cast<size_t>(T), sizeof(int32_t) * (n_seq + 1), cudaMemcpyHostToDevice, h->stream));
   CK(cudaEventRecord(e.pin_ev[pb], h->stream));
   h->stats.h2d_bytes += static_cast<int64_t>(sizeof(int32_t)) * (static_cast<int64_t>(T) * (type_ids ? 2 : 1) + n_seq + 1);
-  e.max_len = max_len;
-  if (e.clip) return clip_text_forward(h, e, n_seq, T, out_dev);
-  return enc_forward(h, e, n_seq, T, type_ids != nullptr, out_dev);
+  if (e.clip) {
+    e.max_len = max_len;
+    return clip_text_forward(h, e, n_seq, T, out_dev);
+  }
+  return enc_forward(h, e, static_cast<const int32_t*>(e.ids.p),
+                     type_ids ? static_cast<const int32_t*>(e.type_ids.p) : nullptr, static_cast<const int32_t*>(e.cu.p),
+                     n_seq, T, max_len, out_dev);
 }
 
 }  // namespace
@@ -2777,6 +2815,252 @@ int rse_hybrid_stage_dev(rse_index* h, int32_t nq, const float* q_dev, const int
   return RSE_OK;
 }
 
+// ------------------------------------------------------------------ cross-encoder rerank of a fused batch (rerank.cuh)
+int rse_rerank_docs_load(rse_index* h, const int64_t* ids, int64_t n_docs, const int64_t* tok_indptr,
+                         const int32_t* tokens) {
+  if (!h) return RSE_ERR_INVALID;
+  if (n_docs < 1 || !ids || !tok_indptr) return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: bad arguments");
+  if (tok_indptr[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: tok_indptr must start at 0");
+  for (int64_t i = 0; i < n_docs; ++i) {
+    if (i > 0 && ids[i] <= ids[i - 1])
+      return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: ids must be strictly ascending (at " + std::to_string(i) + ")");
+    if (tok_indptr[i + 1] < tok_indptr[i])
+      return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: tok_indptr must not decrease (at " + std::to_string(i) + ")");
+  }
+  const int64_t n_tok = tok_indptr[n_docs];
+  if (n_tok > 0 && !tokens) return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: tokens is NULL");
+  int32_t max_tok = -1;
+  int64_t max_len = 0;
+  for (int64_t i = 0; i < n_docs; ++i) max_len = std::max(max_len, tok_indptr[i + 1] - tok_indptr[i]);
+  for (int64_t i = 0; i < n_tok; ++i) {
+    if (tokens[i] < 0) return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load: negative token id");
+    max_tok = std::max(max_tok, tokens[i]);
+  }
+  CK(cudaSetDevice(h->device));
+  CK(cudaStreamSynchronize(h->stream));                       // a rerank run may still read the old store
+  free_ptr(h->rr_doc_ids); free_ptr(h->rr_doc_indptr); free_ptr(h->rr_doc_tok);
+  h->rr_n_docs = 0; h->rr_max_tok = -1;
+  CK(cudaMalloc(&h->rr_doc_ids, 8 * n_docs));
+  CK(cudaMalloc(&h->rr_doc_indptr, 8 * (n_docs + 1)));
+  CK(cudaMalloc(&h->rr_doc_tok, 4 * std::max<int64_t>(n_tok, 1)));
+  CK(cudaMemcpy(h->rr_doc_ids, ids, 8 * n_docs, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(h->rr_doc_indptr, tok_indptr, 8 * (n_docs + 1), cudaMemcpyHostToDevice));
+  if (n_tok > 0) CK(cudaMemcpy(h->rr_doc_tok, tokens, 4 * n_tok, cudaMemcpyHostToDevice));
+  h->rr_n_docs = n_docs; h->rr_max_tok = max_tok; h->rr_max_doc_len = max_len;
+  return RSE_OK;
+}
+
+int rse_set_rerank_token_budget(rse_index* h, int64_t tokens) {
+  if (!h) return RSE_ERR_INVALID;
+  if (tokens < 1 || tokens > INT_MAX) return fail(h, RSE_ERR_INVALID, "rse_set_rerank_token_budget: tokens must be in [1, 2^31)");
+  h->rr_budget = tokens;
+  return RSE_OK;
+}
+
+int rse_pair_truncate(int32_t n1, int32_t n2, int32_t max_length, int32_t* a, int32_t* b) {
+  if (n1 < 0 || n2 < 0 || max_length < 4 || !a || !b) return RSE_ERR_INVALID;
+  int x = 0, y = 0;
+  pair_truncate(n1, n2, max_length - 3, &x, &y);
+  *a = x; *b = y;
+  return RSE_OK;
+}
+
+namespace {
+void rr_mark(rse_index* h, int i) {
+  if (h->timing && h->rr_ev[i]) cudaEventRecord(h->rr_ev[i], h->stream);
+}
+}  // namespace
+
+int rse_hybrid_rerank_run(rse_index* h, int32_t slot, double k, int32_t tie_mode, int32_t limit,
+                          int32_t knn_multiplier, double k1, double b, const int32_t* q_tok_indptr,
+                          const int32_t* q_tok_ids, int32_t cls_id, int32_t sep_id, int32_t max_length,
+                          int32_t activation) {
+  if (!h) return RSE_ERR_INVALID;
+  h->rr_nq = 0;
+  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: limit must be in [1, 128]");
+  if (activation != 0 && activation != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: activation must be 0 (logit) or 1 (sigmoid)");
+  if (h->rr_n_docs < 1) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: no document store (rse_rerank_docs_load)");
+  const int nq = h->staged_nq;
+  if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: nothing staged");
+  if (h->next_ticket != h->next_collect)
+    return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: rse_hybrid_submit tickets are in flight (collect or drain them)");
+  if (slot < 0 || slot >= RSE_MAX_ENCODERS) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: slot out of range");
+  Encoder& e = h->enc[slot];
+  if (!e.created || !e.finalized || e.clip || e.cfg.head != 1)
+    return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: the slot does not hold a finalized head-1 (cross-encoder) BERT");
+  if (max_length < 4 || max_length > e.cfg.max_positions)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: max_length must be in [4, max_positions]");
+  const int vocab = e.cfg.vocab_size;
+  if (!q_tok_indptr || q_tok_indptr[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: q_tok_indptr must start at 0");
+  for (int q = 0; q < nq; ++q)
+    if (q_tok_indptr[q + 1] < q_tok_indptr[q]) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: q_tok_indptr must not decrease");
+  const int n_qtok = q_tok_indptr[nq];
+  if (n_qtok > 0 && !q_tok_ids) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: q_tok_ids is NULL");
+  int max_q = 0;
+  for (int q = 0; q < nq; ++q) max_q = std::max(max_q, q_tok_indptr[q + 1] - q_tok_indptr[q]);
+  for (int i = 0; i < n_qtok; ++i)
+    if (q_tok_ids[i] < 0 || q_tok_ids[i] >= vocab)
+      return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: query token id " + std::to_string(q_tok_ids[i]) + " outside the vocabulary");
+  if (cls_id < 0 || cls_id >= vocab || sep_id < 0 || sep_id >= vocab)
+    return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: cls_id / sep_id outside the vocabulary");
+  if (h->rr_max_tok >= vocab)
+    return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: the document store holds token id " + std::to_string(h->rr_max_tok) +
+                                        " >= the encoder's vocab_size " + std::to_string(vocab));
+  const int W = 2 * limit;
+  const int64_t P = static_cast<int64_t>(nq) * W;
+  if (P * max_length > INT_MAX) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: nq * 2 * limit * max_length exceeds 2^31 tokens (split the batch)");
+  CK(cudaSetDevice(h->device));
+  if (h->timing)
+    for (cudaEvent_t& ev : h->rr_ev) if (!ev) CK(cudaEventCreate(&ev));
+  h->rr_timed = h->timing;
+  ENSURE(h->rr_fid, 8 * P); ENSURE(h->rr_fsc, 8 * P); ENSURE(h->rr_fa, 8 * P); ENSURE(h->rr_fb, 8 * P);
+  ENSURE(h->rr_fcnt, 4 * static_cast<size_t>(nq));
+  ENSURE(h->rr_row, 4 * P); ENSURE(h->rr_ab, 8 * P);
+  ENSURE(h->rr_qnp, 4 * static_cast<size_t>(nq)); ENSURE(h->rr_qnt, 4 * static_cast<size_t>(nq));
+  ENSURE(h->rr_qpb, 4 * static_cast<size_t>(nq + 1)); ENSURE(h->rr_qtb, 4 * static_cast<size_t>(nq + 1));
+  const size_t meta_n = kRrMetaHead + static_cast<size_t>(P) + 1;
+  ENSURE(h->rr_meta, 4 * meta_n);
+  ENSURE(h->rr_qptr, 4 * static_cast<size_t>(nq + 1)); ENSURE(h->rr_qtok, 4 * static_cast<size_t>(std::max(n_qtok, 1)));
+  if (h->rr_pin_meta_n < meta_n) {
+    if (h->rr_pin_meta) CK(cudaFreeHost(h->rr_pin_meta));
+    h->rr_pin_meta = nullptr; h->rr_pin_meta_n = 0;
+    CK(cudaMallocHost(reinterpret_cast<void**>(&h->rr_pin_meta), 4 * (meta_n + meta_n / 2)));
+    h->rr_pin_meta_n = meta_n + meta_n / 2;
+  }
+  CK(cudaMemcpyAsync(h->rr_qptr.p, q_tok_indptr, 4 * static_cast<size_t>(nq + 1), cudaMemcpyHostToDevice, h->stream));
+  if (n_qtok > 0) CK(cudaMemcpyAsync(h->rr_qtok.p, q_tok_ids, 4 * static_cast<size_t>(n_qtok), cudaMemcpyHostToDevice, h->stream));
+  h->stats.h2d_bytes += 4 * static_cast<int64_t>(nq + 1 + n_qtok);
+  int* meta = static_cast<int*>(h->rr_meta.p);
+  CK(cudaMemsetAsync(meta, 0, 4, h->stream));
+  CK(cudaMemsetAsync(meta + 1, 0xFF, 4, h->stream));
+
+  // 1. the hybrid step, with the whole union (2 * limit) in fused order into the rerank's own buffers
+  rr_mark(h, 0);
+  long long* fid = static_cast<long long*>(h->rr_fid.p);
+  double* fsc = static_cast<double*>(h->rr_fsc.p);
+  double* fa = static_cast<double*>(h->rr_fa.p);
+  double* fb = static_cast<double*>(h->rr_fb.p);
+  int* fcnt = static_cast<int*>(h->rr_fcnt.p);
+  int rc = hybrid_run_impl(h, 0, k, tie_mode, limit, knn_multiplier, k1, b, nullptr, 0, fid, fsc, fa, fb, fcnt, W);
+  if (rc != RSE_OK) return rc;
+  rr_mark(h, 1);
+
+  // 2. pair assembly
+  const int* qptr = static_cast<const int*>(h->rr_qptr.p);
+  int* row = static_cast<int*>(h->rr_row.p);
+  int2* ab = static_cast<int2*>(h->rr_ab.p);
+  int* qpb = static_cast<int*>(h->rr_qpb.p);
+  int* qtb = static_cast<int*>(h->rr_qtb.p);
+  rerank_len_kernel<<<nq, kRrThreads, 0, h->stream>>>(fid, fcnt, W, h->rr_doc_ids, h->rr_n_docs, h->rr_doc_indptr, qptr,
+                                                      max_length - 3, row, ab, static_cast<int*>(h->rr_qnp.p),
+                                                      static_cast<int*>(h->rr_qnt.p), meta);
+  LAUNCHED(h);
+  rerank_scan_kernel<<<1, kRrScanThreads, 0, h->stream>>>(static_cast<const int*>(h->rr_qnp.p),
+                                                          static_cast<const int*>(h->rr_qnt.p), nq, qpb, qtb, meta);
+  LAUNCHED(h);
+  // ids / type_ids are sized for the worst case of the batch (every union full, every pair as long as the longest
+  // query and the longest document allow): their size is known before the step's one host round trip
+  const size_t t_cap = static_cast<size_t>(P) * std::min<int64_t>(max_length, max_q + h->rr_max_doc_len + 3);
+  ENSURE(h->rr_ids, 4 * t_cap); ENSURE(h->rr_types, 4 * t_cap);
+  int* cu = meta + kRrMetaHead;
+  int* ids = static_cast<int*>(h->rr_ids.p);
+  int* types = static_cast<int*>(h->rr_types.p);
+  rerank_pack_kernel<<<nq, kRrThreads, 0, h->stream>>>(fcnt, W, row, ab, qpb, qtb, qptr,
+                                                       static_cast<const int*>(h->rr_qtok.p), h->rr_doc_indptr,
+                                                       h->rr_doc_tok, cls_id, sep_id, cu, ids, types);
+  LAUNCHED(h);
+  rr_mark(h, 2);
+  // THE host round trip of the step: the pair count, the missing-id flag and cu_seqlens, which the host needs to cut
+  // the pairs into encoder slices of at most rr_budget tokens
+  CK(cudaMemcpyAsync(h->rr_pin_meta, meta, 4 * meta_n, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(4 * meta_n);
+  CK(cudaStreamSynchronize(h->stream));
+  const int* hm = h->rr_pin_meta;
+  if (hm[0] != 0) {
+    const unsigned first = static_cast<unsigned>(hm[1]);
+    long long id = -1;
+    CK(cudaMemcpy(&id, fid + first, 8, cudaMemcpyDeviceToHost));
+    return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: " + std::to_string(hm[0]) + " fused id(s) not in the document store, first " +
+                                      std::to_string(id) + " (query " + std::to_string(first / W) + ")");
+  }
+  const int n_pairs = hm[2];
+  const int* hcu = hm + kRrMetaHead;
+
+  // 3. the cross-encoder, in slices of the token budget
+  ENSURE(h->rr_logit, 4 * static_cast<size_t>(std::max(n_pairs, 1)));
+  ENSURE(h->rr_cus, 4 * (static_cast<size_t>(n_pairs) + 1));
+  float* logit = static_cast<float*>(h->rr_logit.p);
+  int* cus = static_cast<int*>(h->rr_cus.p);
+  for (int p0 = 0; p0 < n_pairs;) {
+    int p1 = p0 + 1, max_len = hcu[p0 + 1] - hcu[p0];
+    while (p1 < n_pairs && hcu[p1 + 1] - hcu[p0] <= h->rr_budget) {
+      max_len = std::max(max_len, hcu[p1 + 1] - hcu[p1]);
+      ++p1;
+    }
+    const int n = p1 - p0, T = hcu[p1] - hcu[p0];
+    rerank_rebase_kernel<<<(n + 256) / 256, 256, 0, h->stream>>>(cu, p0, n, cus);
+    LAUNCHED(h);
+    rc = enc_forward(h, e, ids + hcu[p0], types + hcu[p0], cus, n, T, max_len, logit + p0);
+    if (rc != RSE_OK) return rc;
+    p0 = p1;
+  }
+  rr_mark(h, 3);
+
+  // 4. the reference's reorder, [:limit], into one buffer for a single copy back
+  const size_t n = static_cast<size_t>(nq) * limit;
+  ENSURE(h->rr_pack, 32 * n + 4 * static_cast<size_t>(nq));
+  char* pk = static_cast<char*>(h->rr_pack.p);
+  rerank_order_kernel<<<nq, kRrThreads, 0, h->stream>>>(
+      fid, fsc, fa, fb, fcnt, W, qpb, logit, activation, limit, reinterpret_cast<long long*>(pk),
+      reinterpret_cast<double*>(pk + 8 * n), reinterpret_cast<float*>(pk + 16 * n), reinterpret_cast<int*>(pk + 20 * n),
+      reinterpret_cast<int*>(pk + 24 * n), reinterpret_cast<int*>(pk + 28 * n), reinterpret_cast<int*>(pk + 32 * n));
+  LAUNCHED(h);
+  rr_mark(h, 4);
+  h->rr_nq = nq; h->rr_limit = limit;
+  return RSE_OK;
+}
+
+int rse_hybrid_rerank_fetch(rse_index* h, int32_t limit, int64_t* out_id, double* out_score, int32_t* out_bm25_rank,
+                            int32_t* out_sem_rank, int32_t* out_rrf_rank, float* out_ce_score, int32_t* out_count) {
+  if (!h) return RSE_ERR_INVALID;
+  const int nq = h->rr_nq;
+  if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_fetch: no rerank run to fetch");
+  if (limit != h->rr_limit) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_fetch: limit differs from the last rse_hybrid_rerank_run");
+  if (!out_id || !out_score || !out_bm25_rank || !out_sem_rank || !out_rrf_rank || !out_ce_score || !out_count)
+    return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_fetch: bad arguments");
+  const size_t n = static_cast<size_t>(nq) * limit;
+  const size_t bytes = 32 * n + 4 * static_cast<size_t>(nq);
+  CK(cudaSetDevice(h->device));
+  if (h->rr_pin_out_bytes < bytes) {
+    if (h->rr_pin_out) CK(cudaFreeHost(h->rr_pin_out));
+    h->rr_pin_out = nullptr; h->rr_pin_out_bytes = 0;
+    CK(cudaMallocHost(reinterpret_cast<void**>(&h->rr_pin_out), bytes + bytes / 2));
+    h->rr_pin_out_bytes = bytes + bytes / 2;
+  }
+  CK(cudaMemcpyAsync(h->rr_pin_out, h->rr_pack.p, bytes, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(bytes);
+  CK(cudaStreamSynchronize(h->stream));
+  const char* p = h->rr_pin_out;
+  std::memcpy(out_id, p, 8 * n);
+  std::memcpy(out_score, p + 8 * n, 8 * n);
+  std::memcpy(out_ce_score, p + 16 * n, 4 * n);
+  std::memcpy(out_bm25_rank, p + 20 * n, 4 * n);
+  std::memcpy(out_sem_rank, p + 24 * n, 4 * n);
+  std::memcpy(out_rrf_rank, p + 28 * n, 4 * n);
+  std::memcpy(out_count, p + 32 * n, 4 * static_cast<size_t>(nq));
+  return RSE_OK;
+}
+
+int rse_hybrid_rerank_timing(rse_index* h, float* out_ms) {
+  if (!h) return RSE_ERR_INVALID;
+  if (!out_ms) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_timing: bad arguments");
+  if (!h->rr_timed || h->rr_nq <= 0)
+    return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_timing: the last rerank run was not timed (rse_set_timing)");
+  CK(cudaEventSynchronize(h->rr_ev[4]));
+  for (int i = 0; i < 4; ++i) CK(cudaEventElapsedTime(&out_ms[i], h->rr_ev[i], h->rr_ev[i + 1]));
+  return RSE_OK;
+}
+
 // ------------------------------------------------------------------ multi-GPU (library-owned NCCL communicator)
 #define NCK(call)                                                                                     \
   do {                                                                                                \
@@ -2976,7 +3260,7 @@ int rse_hybrid_sharded_run_dev(rse_index* h, int32_t mode, double param, int32_t
             static_cast<const float*>(h->o_dist.p), static_cast<const int*>(h->o_count.p), nullptr};
   in.bm25_idx = static_cast<const int*>(h->b_doc.p); in.bm25_table = h->doc_ids; in.bm25_table_n = h->n_doc_ids;
   in.sem_idx = static_cast<const int*>(h->o_movie.p); in.sem_table = h->movie_ids; in.sem_table_n = h->n_movie_ids;
-  return fuse_launch(h, mode, param, tie_mode, ns, limit, in, reinterpret_cast<long long*>(out_id_dev), out_score_dev,
+  return fuse_launch(h, mode, param, tie_mode, ns, limit, limit, in, reinterpret_cast<long long*>(out_id_dev), out_score_dev,
                      out_a_dev, out_b_dev, out_count_dev);
 }
 

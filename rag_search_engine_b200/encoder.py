@@ -94,6 +94,12 @@ def pack(id_lists: Sequence[Sequence[int]], type_lists: Optional[Sequence[Sequen
     return ids, tt, cu
 
 
+def hf_text_tokenizer(hf_tok) -> Callable[[List[str]], List[List[int]]]:
+    """A HuggingFace tokenizer as the single-text tokenizer of the batched rerank: ids without special tokens.  With a
+    fast tokenizer these are exactly the segments its pair encoding (truncation=True) is built from."""
+    return lambda texts: hf_tok(list(texts), add_special_tokens=False)["input_ids"]
+
+
 class GpuSentenceEncoder:
     """``encode(texts) -> float32[n, hidden]`` like SentenceTransformer.encode (normalised mean-pooled BERT)."""
 
@@ -154,13 +160,21 @@ class GpuCrossEncoder:
     """``predict(pairs) -> float32[n]`` like sentence_transformers.CrossEncoder.predict for a 1-label model.
     Returns the classifier LOGITS (``activation="sigmoid"`` applies the logistic function, which some
     sentence-transformers versions do by default for num_labels = 1; the reference only sorts by the score,
-    hybrid_search.py:304-309, and the order is the same either way)."""
+    hybrid_search.py:304-309, and the order is the same either way).
+
+    The batched rerank of ``HybridSearch.rrf_search_batch(..., rerank_method="cross_encoder")`` builds the pairs on
+    the device from single-text token ids: ``tokenizer`` (texts -> token-id lists WITHOUT special tokens) and the
+    ``cls_id`` / ``sep_id`` it wraps them in."""
 
     def __init__(self, index, state_dict, config: dict = TINYBERT_L2_CONFIG,
                  pair_tokenizer: Optional[Callable[[List[Sequence[str]]], tuple]] = None, *, slot: int = 1,
-                 max_length: int = 512, activation: Optional[str] = None):
+                 max_length: int = 512, activation: Optional[str] = None,
+                 tokenizer: Optional[Callable[[List[str]], List[List[int]]]] = None, cls_id: int = 101,
+                 sep_id: int = 102):
         self.index, self.slot, self.config = index, slot, dict(config)
         self.pair_tokenizer = pair_tokenizer
+        self.tokenizer = tokenizer
+        self.cls_id, self.sep_id = int(cls_id), int(sep_id)
         self.max_length = min(int(max_length), int(config["max_positions"]))
         self.activation = activation
         _load(index, slot, self.config, 1, state_dict)
@@ -175,7 +189,15 @@ class GpuCrossEncoder:
             enc = hf_tok([p[0] for p in pairs], [p[1] for p in pairs], truncation=True, max_length=ml)
             return enc["input_ids"], enc["token_type_ids"]
         sd = {k: v for k, v in model.state_dict().items()}
-        return cls(index, sd, config_from_hf(model.config), tok, slot=slot, max_length=ml)
+        return cls(index, sd, config_from_hf(model.config), tok, slot=slot, max_length=ml,
+                   tokenizer=hf_text_tokenizer(hf_tok), cls_id=hf_tok.cls_token_id, sep_id=hf_tok.sep_token_id)
+
+    def tokenize(self, texts) -> List[List[int]]:
+        """Single texts -> token ids without special tokens (the pieces the device assembles into pairs)."""
+        if self.tokenizer is None:
+            raise RuntimeError("GpuCrossEncoder has no single-text tokenizer: pass tokenizer=<texts -> token-id lists "
+                               "without special tokens> (e.g. hf_text_tokenizer(hf_tokenizer))")
+        return self.tokenizer(list(texts))
 
     def predict_ids(self, id_lists, type_lists) -> np.ndarray:
         ml = self.max_length                                   # (copy only what has to be cut)

@@ -12,6 +12,7 @@ CPython-set tie order reproduced on the device).  When both retrievers are the G
 """
 from __future__ import annotations
 
+import itertools
 import logging
 import time
 from pathlib import Path
@@ -51,7 +52,7 @@ class HybridSearch:
 
     @classmethod
     def from_loaded(cls, index: "_lib.Index", term_row: Dict[str, int], doc_ids, movie_ids, *, registry_key,
-                    device: int = 0, tie_mode: str = "reference") -> "HybridSearch":
+                    device: int = 0, tie_mode: str = "reference", cross_encoder=None) -> "HybridSearch":
         """The batch / stream entry points over a handle whose indexes are ALREADY in HBM (rse_load_bm25 +
         rse_load_embeddings / rse_attach_embeddings_dev done by the caller): for corpora that never lived in a
         SQLite file — synthetic benchmarks, a shard of a larger service.  The single-query text methods, which
@@ -70,7 +71,7 @@ class HybridSearch:
                                    emb=np.zeros((int(index.n_rows), 0), np.float32))
         sem._closed = True
         self.keyword, self.semantic, self._index = kw, sem, index
-        self.cross_encoder = None
+        self.cross_encoder = cross_encoder
         runtime.adopt(self.db_path, device, index)
         self._closed = False
         return self
@@ -239,10 +240,32 @@ class HybridSearch:
         return [flat[q * L:q * L + cnt[q]] for q in range(nq)]
 
     def rrf_search_batch(self, token_lists, query_vecs, k=60, limit: int = 10, knn_multiplier: int = 10,
-                         k1: float = 1.5, b: float = 0.75, as_arrays: bool = False):
+                         k1: float = 1.5, b: float = 0.75, as_arrays: bool = False, rerank_method: str | None = None,
+                         rerank_query_ids=None):
         """[{id, score, bm25_rank, sem_rank}] per query; BM25 + KNN + aggregation + RRF in one device call.
         ``as_arrays=True`` returns the packed result instead — (id int64, score, bm25_rank, sem_rank as float64
-        with -1 = None, each [nq, limit]; count int32[nq]) — for callers that do not want Python objects."""
+        with -1 = None, each [nq, limit]; count int32[nq]) — for callers that do not want Python objects.
+
+        ``rerank_method="cross_encoder"`` ranks like ``rrf_search(q, rerank_method="cross_encoder")`` for the whole
+        batch on the device (``self.cross_encoder``, a ``GpuCrossEncoder`` on this object's handle, after
+        ``load_rerank_documents``): ``rerank_query_ids`` are the cross-encoder tokenizer's ids of each query without
+        special tokens (``cross_encoder.tokenize(texts)``).  Hits are {id, score, bm25_rank, sem_rank, rrf_rank,
+        cross_encoder_score}; ``as_arrays=True`` gives (id, score, bm25_rank, sem_rank, rrf_rank, cross_encoder_score,
+        count) with int32 ranks (-1 = None)."""
+        if rerank_method is not None:
+            ce = self._rerank_encoder(rerank_method)
+            if not self._gpu_retrievers():
+                raise RuntimeError("*_batch needs the GPU KeywordSearch and SemanticSearch of this package")
+            self._ensure_id_tables()
+            tok_indptr, rows = self.keyword._term_rows(token_lists)
+            if len(tok_indptr) == 1:
+                if not as_arrays:
+                    return []
+                z = [np.zeros((0, limit), t) for t in (np.int64, np.float64, np.int32, np.int32, np.int32, np.float32)]
+                return (*z, np.zeros(0, np.int32))
+            self._index.hybrid_stage(query_vecs, tok_indptr, rows)
+            return self._rerank_staged(ce, len(tok_indptr) - 1, rerank_query_ids, k, limit, knn_multiplier, k1, b,
+                                       as_arrays)
         res = self._hybrid_batch(0, float(k), token_lists, query_vecs, limit, knn_multiplier, k1, b)
         return res if as_arrays else self._unpack_rrf(res, len(res[4]))
 
@@ -253,12 +276,15 @@ class HybridSearch:
                   "score": float(osc[q, j])} for j in range(oc[q])] for q in range(len(oc))]
 
     def rrf_search_texts(self, token_lists, encoder_ids, encoder, k=60, limit: int = 10, knn_multiplier: int = 10,
-                         k1: float = 1.5, b: float = 0.75, as_arrays: bool = False):
+                         k1: float = 1.5, b: float = 0.75, as_arrays: bool = False, rerank_method: str | None = None,
+                         rerank_query_ids=None):
         """Text in: the query vectors are produced by ``encoder`` (encoder.GpuSentenceEncoder) ON THE DEVICE and
         handed to the hybrid step there (``rse_encode_dev`` -> ``rse_hybrid_stage_dev``): no host hop for the
         vectors.  ``token_lists`` are the BM25 tokens of the queries (the reference's ``preprocess`` output),
-        ``encoder_ids`` the encoder's token ids ([CLS] ... [SEP]) of the same queries."""
+        ``encoder_ids`` the encoder's token ids ([CLS] ... [SEP]) of the same queries.  ``rerank_method`` /
+        ``rerank_query_ids`` as in ``rrf_search_batch``."""
         import torch
+        ce = self._rerank_encoder(rerank_method) if rerank_method is not None else None
         if not self._gpu_retrievers():
             raise RuntimeError("rrf_search_texts needs the GPU KeywordSearch and SemanticSearch of this package")
         self._ensure_id_tables()
@@ -272,9 +298,84 @@ class HybridSearch:
         if n != nq:
             raise ValueError("token_lists and encoder_ids describe different numbers of queries")
         self._index.hybrid_stage_dev(nq, buf.data_ptr(), tok_indptr, rows)
+        if ce is not None:
+            return self._rerank_staged(ce, nq, rerank_query_ids, k, limit, knn_multiplier, k1, b, as_arrays)
         self._index.hybrid_run(0, float(k), limit, knn_multiplier=knn_multiplier, k1=k1, b=b, tie_mode=self.tie_mode)
         res = self._index.hybrid_fetch(limit)
         return res if as_arrays else self._unpack_rrf(res, nq)
+
+    # ---------------- cross-encoder rerank of a batch (hybrid_search.py:279-312) on the device ---------------- #
+    def load_rerank_documents(self, ids=None, token_lists=None) -> int:
+        """Upload the cross-encoder's token ids of every document text, ``f"{title} - {description}"``, the strings
+        ``rrf_search`` pairs with the query (an id without a ``movies`` row is ``"<missing> - "``, what
+        ``KeywordSearch.search`` reports for it).  Without arguments the texts are read from this object's SQLite
+        database for every id the two retrievers can return and tokenised with ``self.cross_encoder.tokenize``;
+        ``ids`` + ``token_lists`` (ids without special tokens, per id) upload a ready store instead — the only form
+        an object made by ``from_loaded`` has.  Returns the number of documents."""
+        if ids is None:
+            ce = self._rerank_encoder("cross_encoder")
+            universe = np.union1d(np.asarray(self.keyword._arr.doc_ids, np.int64),
+                                  np.asarray(self.semantic._arr.movie_ids, np.int64))
+            import sqlite3
+            conn = sqlite3.connect(self.db_path)
+            try:
+                rows = {int(i): (t, d) for i, t, d in conn.execute("SELECT id, title, description FROM movies")}
+            finally:
+                conn.close()
+            texts = []
+            for i in universe.tolist():
+                title, desc = rows.get(i, ("<missing>", ""))
+                texts.append(f"{title} - {desc or ''}")
+            ids, token_lists = universe, ce.tokenize(texts)
+        ids = np.asarray(ids, np.int64)
+        if len(token_lists) != len(ids):
+            raise ValueError("ids and token_lists differ in length")
+        order = np.argsort(ids, kind="stable")
+        lens = np.fromiter((len(token_lists[i]) for i in order.tolist()), np.int64, count=len(ids))
+        indptr = np.zeros(len(ids) + 1, np.int64)
+        np.cumsum(lens, out=indptr[1:])
+        tokens = np.fromiter(itertools.chain.from_iterable(token_lists[i] for i in order.tolist()), np.int32,
+                             count=int(indptr[-1]))
+        self._index.rerank_docs_load(ids[order], indptr, tokens)
+        return len(ids)
+
+    def _rerank_encoder(self, rerank_method):
+        if rerank_method != "cross_encoder":
+            raise ValueError(f"rerank_method must be None or 'cross_encoder' for a batch, not {rerank_method!r}")
+        ce = getattr(self, "cross_encoder", None)
+        if ce is None or not hasattr(ce, "index") or not hasattr(ce, "cls_id"):
+            raise RuntimeError("the batched rerank needs HybridSearch(cross_encoder=GpuCrossEncoder(...))")
+        if ce.index is not self._index:
+            raise ValueError("the cross-encoder lives on another handle than the hybrid index: create it on "
+                             "runtime.acquire(db_path, device) (or the index given to from_loaded)")
+        if ce.activation not in (None, "sigmoid"):
+            raise ValueError(f"unsupported cross-encoder activation {ce.activation!r}")
+        return ce
+
+    def _rerank_staged(self, ce, nq, rerank_query_ids, k, limit, knn_multiplier, k1, b, as_arrays):
+        if rerank_query_ids is None or len(rerank_query_ids) != nq:
+            raise ValueError("rerank_query_ids must hold the cross-encoder token ids of every query")
+        q_ptr = np.zeros(nq + 1, np.int32)
+        np.cumsum([len(x) for x in rerank_query_ids], out=q_ptr[1:])
+        q_ids = np.fromiter(itertools.chain.from_iterable(rerank_query_ids), np.int32, count=int(q_ptr[-1]))
+        self._index.hybrid_rerank_run(ce.slot, float(k), limit, q_ptr, q_ids, cls_id=ce.cls_id, sep_id=ce.sep_id,
+                                      max_length=ce.max_length, activation=int(ce.activation == "sigmoid"),
+                                      knn_multiplier=knn_multiplier, k1=k1, b=b, tie_mode=self.tie_mode)
+        res = self._index.hybrid_rerank_fetch(limit)
+        return res if as_arrays else self._unpack_rerank(res, nq)
+
+    @staticmethod
+    def _unpack_rerank(res, nq):
+        """[{id, score, bm25_rank, sem_rank, rrf_rank, cross_encoder_score}] per query (as _unpack_rrf)."""
+        oid, osc, orb, ors, orr, oce, oc = res
+        ra = orb.astype(object); ra[orb < 0] = None
+        rb = ors.astype(object); rb[ors < 0] = None
+        flat = [{"id": i, "score": s, "bm25_rank": a, "sem_rank": b_, "rrf_rank": r, "cross_encoder_score": c}
+                for i, s, a, b_, r, c in zip(oid.ravel().tolist(), osc.ravel().tolist(), ra.ravel().tolist(),
+                                             rb.ravel().tolist(), orr.ravel().tolist(), oce.ravel().tolist())]
+        L = oid.shape[1] if oid.ndim == 2 else 0
+        cnt = oc.tolist()
+        return [flat[q * L:q * L + cnt[q]] for q in range(nq)]
 
     def rrf_search_stream(self, batches, k=60, limit: int = 10, knn_multiplier: int = 10, k1: float = 1.5,
                           b: float = 0.75, as_arrays: bool = False):
