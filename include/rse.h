@@ -90,13 +90,16 @@ int rse_attach_embeddings_dev(rse_index *h, const float *emb_dev, int64_t n_rows
                               const int32_t *movie_idx_dev, int64_t pos_base);
 int rse_set_fma(rse_index *h, int32_t use_fma);
 /* K4, the tcgen05 path for query batches (probe -> filter -> EXACT re-score, results identical to the
- * streaming scan): 0 = auto (batches of >= RSE_TC_MIN_BATCH queries on >= 256 k rows, dim 384), 1 = never,
- * 2 = whenever the shape allows it.  The probe/filter GEMM runs over an fp16 normalised shadow of the corpus
- * (knn_tc3.cuh; built once at the first batch that needs it, +768 B per row of device memory).  Measured on
+ * streaming scan): 0 = auto (batches of >= RSE_TC_MIN_BATCH queries on >= 256 k rows), 1 = never,
+ * 2 = whenever the shape allows it.  K4 serves embedding widths dim = 64 KB, KB = 1..8 (64..512, e.g. 384 for
+ * MiniLM, 512 for CLIP); any other width always takes the exact scan.  The probe/filter GEMM runs over an fp16
+ * normalised shadow of the corpus (knn_tc3.cuh; built once at the first batch that needs it, +2 * dim B per row
+ * of device memory: 768 B at 384).  Measured on
  * S-600k (bench.py knn_small_batches, r02): the K4 chain costs 0.75-0.82 ms per call for 1..64 queries, the exact
  * scan 1.21 / 1.41 / 1.65 / 1.72 / 2.32 / 3.98 ms for 1 / 2 / 3 / 4 / 8 / 16 — K4 wins from the first query on.  A
  * single query takes the exact streaming scan (north_star: batch-1 = the HBM-bound kernel; no shadow needed) until
- * a batch has built the shadow, and K4 from then on; mode 2 sends it through K4 from the start. */
+ * a batch has built the shadow, and K4 from then on at dim 384 (the width that was measured; at any other width a
+ * single query stays on the exact scan in auto mode); mode 2 sends it through K4 from the start. */
 #define RSE_TC_MIN_BATCH 2
 int rse_set_tc_mode(rse_index *h, int32_t mode);
 

@@ -69,11 +69,11 @@ static_assert(kTcCandCap * 8 <= kRefineStagingBytes, "the survivor pairs must fi
 // 42 of the kernel's 64 us on the isotropic corpus — 39 k random rows per launch at 1.4 TB/s; staged: 13 us with two
 // stages).  Lane l then walks ITS row in order from shared memory (the reference's sequential sum); float4 j of row r
 // sits at slot j ^ (r & 7), so the 8 lanes of a quarter-warp hit 8 different 16-byte bank groups.  STAGES - 1 lines
-// are in flight while one is summed.
-template <bool FMA, int STAGES>
+// are in flight while one is summed.  D = the row width, a multiple of 64.
+template <bool FMA, int STAGES, int D>
 __device__ __forceinline__ float staged_row_dot(const float* __restrict__ emb, uint32_t myrow, const float* s_q,
                                                 unsigned char* wbuf, int lane) {
-  constexpr int kChunks = kScanD / kRefineChunkFloats;                     // 12
+  constexpr int kChunks = D / kRefineChunkFloats;                          // 384 wide: 12
   const uint32_t wbuf_s = smem_u32(wbuf);
   auto issue = [&](int k) {
     if (k < kChunks) {
@@ -82,7 +82,7 @@ __device__ __forceinline__ float staged_row_dot(const float* __restrict__ emb, u
         const int r = 4 * it + (lane >> 3);
         const uint32_t row = __shfl_sync(0xFFFFFFFFu, myrow, r);
         cp_async16_cg(wbuf_s + (k % STAGES) * kRefineStageBytes + r * 128 + (((lane & 7) ^ (r & 7)) << 4),
-                      emb + static_cast<int64_t>(row) * kScanD + k * kRefineChunkFloats + (lane & 7) * 4);
+                      emb + static_cast<int64_t>(row) * D + k * kRefineChunkFloats + (lane & 7) * 4);
       }
     }
     cp_async_commit();                                                     // (an empty group past the last line)
@@ -120,7 +120,8 @@ __device__ unsigned long long g_refine_ns[8 * 4096];
 #define RT_SYNC()
 #endif
 
-template <bool FMA>
+// KB = D / 64 (the row width of knn_tc3_kernel<MODE, KB>); the exact re-score is the sequential sum over all D.
+template <bool FMA, int KB>
 __global__ void __launch_bounds__(kSelThreads, 2)
 knn_refine_kernel(const float* __restrict__ emb, const float* __restrict__ amag, const float* __restrict__ q,
                   const double* __restrict__ sb, const uint2* __restrict__ cand_pairs,
@@ -130,9 +131,10 @@ knn_refine_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
                   const float* __restrict__ thr2, const unsigned int* __restrict__ gate,
                   unsigned long long* __restrict__ counters, float* __restrict__ thr2_out,
                   unsigned int* __restrict__ gate_out, const float* __restrict__ tverify) {
+  constexpr int D = KB * 64;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   uint2* pairs = reinterpret_cast<uint2*>(smem_raw);                       // [cap]
-  __shared__ float s_q[kScanD];
+  __shared__ float s_q[D];
   __shared__ unsigned int s_hist[256];
   __shared__ unsigned int s_prefix, s_need, s_m, s_digit, s_before;
   __shared__ unsigned int s_warp[8];
@@ -178,7 +180,7 @@ knn_refine_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
         k_and &= key; k_or |= key;
       }
   }
-  for (int i = threadIdx.x; i < kScanD; i += blockDim.x) s_q[i] = q[static_cast<int64_t>(qi) * kScanD + i];
+  for (int i = threadIdx.x; i < D; i += blockDim.x) s_q[i] = q[static_cast<int64_t>(qi) * D + i];
   k_and = __reduce_and_sync(0xFFFFFFFFu, k_and);
   k_or = __reduce_or_sync(0xFFFFFFFFu, k_or);
   if ((threadIdx.x & 31) == 0) { s_and[threadIdx.x >> 5] = k_and; s_or[threadIdx.x >> 5] = k_or; }
@@ -298,9 +300,9 @@ knn_refine_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
       const int i = base + lane;
       const uint32_t myrow = s_rows[i < static_cast<int>(m) ? i : static_cast<int>(m) - 1];
       float acc;
-      if (stages == 4) acc = staged_row_dot<FMA, 4>(emb, myrow, s_q, wbuf, lane);
-      else if (stages == 3) acc = staged_row_dot<FMA, 3>(emb, myrow, s_q, wbuf, lane);
-      else acc = staged_row_dot<FMA, 2>(emb, myrow, s_q, wbuf, lane);
+      if (stages == 4) acc = staged_row_dot<FMA, 4, D>(emb, myrow, s_q, wbuf, lane);
+      else if (stages == 3) acc = staged_row_dot<FMA, 3, D>(emb, myrow, s_q, wbuf, lane);
+      else acc = staged_row_dot<FMA, 2, D>(emb, myrow, s_q, wbuf, lane);
       if (i < static_cast<int>(m)) {
         const float d = cosine_tail(acc, sqrt(static_cast<double>(__ldg(amag + myrow))), sbq);
         keys[i] = knn_key(f32_orderable(__float_as_uint(d)), pos_base + static_cast<uint64_t>(myrow));
@@ -311,15 +313,20 @@ knn_refine_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
       unsigned long long key = ~0ull;
       if (i < static_cast<int>(m)) {
         const uint32_t row = s_rows[i];
-        const float4* rp = reinterpret_cast<const float4*>(emb + static_cast<int64_t>(row) * kScanD);
+        const float4* rp = reinterpret_cast<const float4*>(emb + static_cast<int64_t>(row) * D);
         float acc = 0.0f;
+        // 24 float4 in flight per step; when D / 4 is not a multiple of 24 (every width but 192 and 384) the last
+        // step is a partial one, still summed in index order
+        constexpr bool kTail = (D / 4) % 24 != 0;
 #pragma unroll 1
-        for (int c0 = 0; c0 < kScanD / 4; c0 += 24) {
+        for (int c0 = 0; c0 < D / 4; c0 += 24) {
           float4 a[24];
 #pragma unroll
-          for (int c = 0; c < 24; ++c) a[c] = __ldg(rp + c0 + c);
+          for (int c = 0; c < 24; ++c)
+            if (!kTail || c0 + c < D / 4) a[c] = __ldg(rp + c0 + c);
 #pragma unroll
           for (int c = 0; c < 24; ++c) {
+            if (kTail && c0 + c >= D / 4) break;
             acc = mac<FMA>(acc, a[c].x, s_q[4 * (c0 + c) + 0]);
             acc = mac<FMA>(acc, a[c].y, s_q[4 * (c0 + c) + 1]);
             acc = mac<FMA>(acc, a[c].z, s_q[4 * (c0 + c) + 2]);

@@ -15,11 +15,21 @@
 // and the 256 queries (196 KB) now FIT in the shared memory of a CTA pair (98 KB each, the A operand
 // of a cta_group::2 UMMA) so they are loaded once per launch.  The accumulator is cos~ directly.
 //
-// Error bound (eps = kTcEps = 2.5e-3 is kept; the fp16 shadow is TIGHTER than TF32 truncation):
+// Widths: every kernel here is instantiated for KB = D / 64 = 1..8 k-blocks of 64 halves (D = 64..512; the
+// sentence-transformers 384 is KB = 6, CLIP's 512 is KB = 8).  Only the k-loops, the resident-query block (16 KB per
+// k-block per CTA: 128 KB at KB = 8, 210,224 B of shared memory in all) and the shadow layout depend on KB; tile,
+// UMMA shape, ring, epilogue, probe and survivor queues do not.  768 wide would need 192 KB of resident queries plus
+// the ring: more than a CTA may have (a 64-query tile is the way there).
+//
+// Error bound (eps = kTcEps = 2.5e-3 is kept; the fp16 shadow is TIGHTER than TF32 truncation), for a row width
+// D = 64 KB <= 512:
 //   |a^_i| <= 1, so fp16_rn has relative error <= 2^-11 above 2^-14 and absolute error <= 2^-25 below;
-//   |cos~ - cos| <= (2^-10 + 2^-22) * sum|a^_i q^_i| + 2^-25 * (sum|a^_i| + sum|q^_i|) + accumulation
-//                <= 9.8e-4 + 1.2e-6 + 4.6e-5 (384 fp32 adds, truncating)  <  1.1e-3,
-//   plus ~2.3e-5 for the reference's own fp32 rounding of dot — less than half of eps.
+//   |cos~ - cos| <= (2^-10 + 2^-22) * sum|a^_i q^_i| + 2^-25 * (sum|a^_i| + sum|q^_i|) + D * 2^-23 (truncating adds)
+//     sum|a^_i q^_i| <= 1 (Cauchy-Schwarz, unit vectors): 9.77e-4 at every D;
+//     sum|a^_i| <= sqrt(D) for a unit vector: 2^-25 * 2 sqrt(D) = 2^-24 sqrt(D) <= 1.35e-6 (384: 1.17e-6);
+//     D fp32 adds, truncating: D * 2^-23 <= 6.10e-5 (384: 4.58e-5);
+//   together <= 1.04e-3 at D = 512 (1.02e-3 at 384), plus D * 2^-24 <= 3.05e-5 (384: 2.29e-5) for the reference's
+//   own fp32 rounding of dot: <= 1.07e-3, less than half of eps at every width K4 serves.
 //
 // Mapping: cluster of 2 CTAs (one TPC) x 74, persistent over 256-row tiles.
 //   UMMA 256x256x16 kind::f16 cta_group::2:  A = the queries (M = 256: 128 per CTA, resident),
@@ -48,7 +58,7 @@ namespace rse {
 constexpr int kT3TileRows = 256;                          // UMMA M (CTA pair)
 constexpr int kT3HalfRows = 128;                          // rows each CTA streams per tile = queries each CTA holds
 constexpr int kT3BK = 64;                                 // halves per k-block: one 128-byte swizzle atom
-constexpr int kT3KBlocks = kScanD / kT3BK;                // 6
+constexpr int kT3MaxKBlocks = 8;                          // KB = D / 64 k-blocks per row, 1..8 (D = 64..512; 384: KB = 6)
 constexpr int kT3StageBytes = kT3HalfRows * kT3BK * 2;    // 16,384
 constexpr int kT3Stages = 4;                              // 64 KB of rows in flight per SM.  3..7 stages measure the same
                                                           // (0.81-0.85 ms, r01): the pass is not fill-bound, and the
@@ -60,12 +70,14 @@ constexpr int kT3Stages = 4;                              // 64 KB of rows in fl
 constexpr int kT3ProbeTop = 8;                            // MODE 2: sample values kept per thread
 constexpr int kT3QueueCap = 128;                          // per-warp survivor queue (entries of 12 B)
 constexpr int kT3QueueFlush = 32;                         // flushed to global memory once this full
-constexpr int kT3QBytes = kT3KBlocks * kT3StageBytes;     // 98,304: this CTA's 128 queries
 constexpr int kT3EpiWarps = 8;                            // two per TMEM lane quarter
 constexpr int kT3Threads = 64 + 32 * kT3EpiWarps;         // 320
-constexpr int kT3SmemBytes = kT3QBytes + kT3Stages * kT3StageBytes + kT3EpiWarps * (kT3QueueCap * 12 + 4) +
-                             32 * 8 + 16 + 1024;
-static_assert(kT3SmemBytes <= 232448, "knn_tc3: shared memory budget");
+// this CTA's 128 resident queries: KB k-blocks of 16 KB (384 wide: 98,304)
+__host__ __device__ constexpr int t3_qbytes(int kb) { return kb * kT3StageBytes; }
+// 384 wide: 177,456 B; 512 wide (KB = 8): 210,224 B of the 232,448 a CTA may have
+__host__ __device__ constexpr int t3_smem_bytes(int kb) {
+  return t3_qbytes(kb) + kT3Stages * kT3StageBytes + kT3EpiWarps * (kT3QueueCap * 12 + 4) + 32 * 8 + 16 + 1024;
+}
 // kind::f16: D = f32 (bit 4), A = B = f16 (format 0), both K-major, N = 256 rows, M = 256 queries (pair)
 constexpr uint32_t kT3Idesc = (1u << 4) | ((kT3TileRows >> 3) << 17) | ((kTcBN >> 4) << 24);
 
@@ -321,37 +333,50 @@ __device__ __forceinline__ void tc_ld128(uint32_t taddr, uint32_t (&v)[128]) {
 // keeps the whole index on the exact scan (MiniLM embeddings are unit-norm; this is a guard).
 //
 // Layout: the shadow is private to the probe/filter GEMM, so it is stored the way the GEMM consumes it —
-// [row / 128][k-block 0..5][row % 128][64 halves]: every pipeline stage (128 rows x one 128-byte k-block)
+// [row / 128][k-block 0..KB-1][row % 128][64 halves]: every pipeline stage (128 rows x one 128-byte k-block)
 // is ONE contiguous 16 KB block of HBM.  (A row-major shadow made each stage 128 separate 128-byte
 // pieces 768 B apart; the filter pass then stalled on TMA data at 4.5 TB/s, r01 ncu.)  The buffer is
 // padded with zero rows to a multiple of 256 rows.
+// A warp converts 128 floats (32 float4) per step; at D = 64, 192, 320 and 448 (KB odd) the last step is a half
+// step: lanes 0..15 hold its 16 float4.
+template <int KB>
 __device__ __forceinline__ int64_t t3_shadow_offset(int64_t row, int kb) {      // in halves
-  return (((row >> 7) * kT3KBlocks + kb) * kT3HalfRows + (row & 127)) * kT3BK;
+  return (((row >> 7) * KB + kb) * kT3HalfRows + (row & 127)) * kT3BK;
 }
+template <int KB>
+__device__ __forceinline__ void t3_shadow_row(const float* __restrict__ emb, const float* __restrict__ amag, int64_t r,
+                                              int lane, __half* __restrict__ shadow, unsigned int* __restrict__ bad) {
+  const float am = __ldg(amag + r);
+  float inv = 0.0f;
+  if (am > 0.0f && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
+  else if (!(am < 0.0f) && lane == 0) atomicAdd(bad, 1u);              // 0, +inf or NaN
+  const float4* src = reinterpret_cast<const float4*>(emb + r * (KB * kT3BK));
+#pragma unroll
+  for (int j = 0; j < (KB + 1) / 2; ++j) {
+    if (KB % 2 != 0 && j == KB / 2 && lane >= 16) break;                // the half step
+    const int f4 = j * 32 + lane;                                       // float4 index inside the row: 0..16 KB - 1
+    const float4 f = __ldg(src + f4);
+    const __half2 lo = __floats2half2_rn(__fmul_rn(f.x, inv), __fmul_rn(f.y, inv));
+    const __half2 hi = __floats2half2_rn(__fmul_rn(f.z, inv), __fmul_rn(f.w, inv));
+    uint2 o;
+    o.x = *reinterpret_cast<const uint32_t*>(&lo);
+    o.y = *reinterpret_cast<const uint32_t*>(&hi);
+    const int kb = f4 >> 4, within = f4 & 15;                           // 16 float4 (= 64 halves) per k-block
+    reinterpret_cast<uint2*>(shadow + t3_shadow_offset<KB>(r, kb))[within] = o;
+  }
+}
+template <int KB>
 __global__ void __launch_bounds__(256)
 tc3_shadow_kernel(const float* __restrict__ emb, const float* __restrict__ amag, int64_t n_rows,
                   __half* __restrict__ shadow, unsigned int* __restrict__ bad) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
-  for (int64_t r = warp0; r < n_rows; r += n_warps) {
-    const float am = __ldg(amag + r);
-    float inv = 0.0f;
-    if (am > 0.0f && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
-    else if (!(am < 0.0f) && lane == 0) atomicAdd(bad, 1u);            // 0, +inf or NaN
-    const float4* src = reinterpret_cast<const float4*>(emb + r * kScanD);
-#pragma unroll
-    for (int j = 0; j < kScanD / 128; ++j) {
-      const int f4 = j * 32 + lane;                                     // float4 index inside the row: 0..95
-      const float4 f = __ldg(src + f4);
-      const __half2 lo = __floats2half2_rn(__fmul_rn(f.x, inv), __fmul_rn(f.y, inv));
-      const __half2 hi = __floats2half2_rn(__fmul_rn(f.z, inv), __fmul_rn(f.w, inv));
-      uint2 o;
-      o.x = *reinterpret_cast<const uint32_t*>(&lo);
-      o.y = *reinterpret_cast<const uint32_t*>(&hi);
-      const int kb = f4 >> 4, within = f4 & 15;                         // 16 float4 (= 64 halves) per k-block
-      reinterpret_cast<uint2*>(shadow + t3_shadow_offset(r, kb))[within] = o;
-    }
+  if (KB == 2) {
+#pragma unroll 1                                                        // (unrolled, this loop spills at KB = 2)
+    for (int64_t r = warp0; r < n_rows; r += n_warps) t3_shadow_row<KB>(emb, amag, r, lane, shadow, bad);
+  } else {
+    for (int64_t r = warp0; r < n_rows; r += n_warps) t3_shadow_row<KB>(emb, amag, r, lane, shadow, bad);
   }
 }
 
@@ -369,6 +394,7 @@ __device__ __forceinline__ int64_t t3_sample_source(int64_t i, int stride, int64
   const int64_t gs = n_rows - g < stride ? n_rows - g : stride;
   return g + static_cast<int64_t>(x % static_cast<uint32_t>(gs));
 }
+template <int KB>
 __global__ void __launch_bounds__(256)
 tc3_sample_kernel(const float* __restrict__ emb, const float* __restrict__ amag, int64_t n_rows, int stride,
                   int64_t n_sample, __half* __restrict__ sample) {
@@ -380,9 +406,10 @@ tc3_sample_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
     const float am = __ldg(amag + r);
     float inv = 0.0f;                                                    // empty slots stay zero rows
     if (am > 0.0f && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
-    const float4* src = reinterpret_cast<const float4*>(emb + r * kScanD);
+    const float4* src = reinterpret_cast<const float4*>(emb + r * (KB * kT3BK));
 #pragma unroll
-    for (int j = 0; j < kScanD / 128; ++j) {
+    for (int j = 0; j < (KB + 1) / 2; ++j) {
+      if (KB % 2 != 0 && j == KB / 2 && lane >= 16) break;              // the half step
       const int f4 = j * 32 + lane;
       const float4 f = __ldg(src + f4);
       const __half2 lo = __floats2half2_rn(__fmul_rn(f.x, inv), __fmul_rn(f.y, inv));
@@ -391,14 +418,16 @@ tc3_sample_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
       o.x = *reinterpret_cast<const uint32_t*>(&lo);
       o.y = *reinterpret_cast<const uint32_t*>(&hi);
       const int kb = f4 >> 4, within = f4 & 15;
-      reinterpret_cast<uint2*>(sample + t3_shadow_offset(i, kb))[within] = o;
+      reinterpret_cast<uint2*>(sample + t3_shadow_offset<KB>(i, kb))[within] = o;
     }
   }
 }
 
 // q16[q] = fp16_rn(q / ||q||) for q < nq (||q|| = sb[q], the K1 factor), zero rows for the padding and
-// for queries whose norm is zero / non-finite (those get thr = +inf and are re-run exactly).
-__global__ void __launch_bounds__(96)
+// for queries whose norm is zero / non-finite (those get thr = +inf and are re-run exactly).  One thread per float4:
+// 16 KB threads per query (384 wide: 96).
+template <int KB>
+__global__ void __launch_bounds__(16 * KB)
 tc3_query_prep_kernel(const float* __restrict__ q, const double* __restrict__ sb, int nq, __half* __restrict__ q16) {
   const int qi = blockIdx.x;
   float inv = 0.0f;
@@ -407,13 +436,13 @@ tc3_query_prep_kernel(const float* __restrict__ q, const double* __restrict__ sb
     if (s > 0.0 && s < 1e300) inv = static_cast<float>(1.0 / s);
   }
   float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (qi < nq) f = __ldg(reinterpret_cast<const float4*>(q + static_cast<int64_t>(qi) * kScanD) + threadIdx.x);
+  if (qi < nq) f = __ldg(reinterpret_cast<const float4*>(q + static_cast<int64_t>(qi) * (KB * kT3BK)) + threadIdx.x);
   const __half2 lo = __floats2half2_rn(__fmul_rn(f.x, inv), __fmul_rn(f.y, inv));
   const __half2 hi = __floats2half2_rn(__fmul_rn(f.z, inv), __fmul_rn(f.w, inv));
   uint2 o;
   o.x = *reinterpret_cast<const uint32_t*>(&lo);
   o.y = *reinterpret_cast<const uint32_t*>(&hi);
-  reinterpret_cast<uint2*>(q16 + static_cast<int64_t>(qi) * kScanD)[threadIdx.x] = o;
+  reinterpret_cast<uint2*>(q16 + static_cast<int64_t>(qi) * (KB * kT3BK))[threadIdx.x] = o;
 }
 
 // thr[q] = 1 - tau_s - 2 eps (compared against cos~); +inf — nothing survives, the refine step then hands
@@ -517,13 +546,18 @@ tc3_probe_threshold_kernel(const uint32_t* __restrict__ dist, int64_t ld, int nq
 //                  fill of a 0.1 ms pass.)  MODE 0 is only used with one block.
 // gate (MODE 1, second-chance pass): gate[qb] == 0 -> block qb is skipped by every role; all zero -> the kernel
 //                  returns before any barrier / TMEM allocation (enqueued unconditionally, rse.cu).
+// KB = D / 64: k-blocks per row and per resident query (every k-loop, the resident-query block and the shadow layout).
 // grid = 2 * n_clusters (<= 148), cluster = 2.
-template <int MODE>
+template <int MODE, int KB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1)
 knn_tc3_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_constant__ CUtensorMap tmap_q,
                int64_t n_tiles, int64_t tile_stride, int nq, int n_qblocks, const float* __restrict__ thr,
                uint32_t* __restrict__ dist, int64_t ld, uint2* __restrict__ cand_pairs,
                unsigned int* __restrict__ cand_count, int cap, const unsigned int* __restrict__ gate) {
+  static_assert(KB >= 1 && KB <= kT3MaxKBlocks, "knn_tc3: 64 to 512 halves per row");
+  static_assert(t3_smem_bytes(KB) <= 232448, "knn_tc3: shared memory budget");
+  constexpr int kT3KBlocks = KB;
+  constexpr int kT3QBytes = t3_qbytes(KB);
   if (gate != nullptr) {
     bool any = false;
     for (int b = 0; b < n_qblocks; ++b) any |= gate[b] != 0u;

@@ -171,10 +171,11 @@ struct rse_index {
   int probe_rank = 0;              // RSE_TC_PROBE_RANK: force the probe's order statistic j (tests: 1 = always too tight)
   int sample_min_tiles = 16;       // RSE_TC_SAMPLE_MIN_TILES: 262 k rows at stride 64 (tests lower it for small corpora)
   int shadow_state = 0;            // 0 = not built, 1 = usable, -1 = corpus has non-finite norms: exact scan only
-  CUtensorMap tmap_a16{};          // [n_rows][384] f16, box {64, 128}, SWIZZLE_128B
-  CUtensorMap tmap_q16{};          // [256][384] f16, box {64, 128}
+  CUtensorMap tmap_a16{};          // the tiled shadow as [n_pad * KB][64] f16 lines, box {64, 128}, SWIZZLE_128B
+  CUtensorMap tmap_q16{};          // [nq_pad][dim] f16, box {64, 128}
   bool tmap_q16_ok = false;
   int tmap_q16_rows = 0;
+  int tmap_q16_dim = 0;            // the map is [nq_pad][dim]: a reload at another width needs a new one
   const void* tmap_q16_base = nullptr;
 
   // ---- a1: embeddings (vec0 physical layout)
@@ -246,6 +247,7 @@ struct rse_index {
 
   uint32_t attr_mask = 0;
   uint32_t attr_mask_wide = 0;     // knn_scan_wide_kernel instantiations
+  uint32_t attr_mask_tc = 0;       // bit KB-1: knn_tc3_kernel<*, KB>; bit 8 + KB-1: knn_refine_kernel<*, KB>
   rse_stats stats{};
   // device-side counters read back by rse_get_stats: [0] BM25 queries handed to the general kernel, [1] BM25
   // finalists re-scored exactly, [2] BM25 candidates merged by the finish kernel
@@ -468,8 +470,9 @@ typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuin
                                         const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                         CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// [rows][384] row-major matrix of f32 (elem_bytes 4) or f16 (2); box = one 128-byte swizzle atom x box_rows
-int make_tmap_any(rse_index* h, CUtensorMap* out, const void* base, int64_t rows, int box_rows, int elem_bytes) {
+// [rows][cols] row-major matrix of f32 (elem_bytes 4) or f16 (2); box = one 128-byte swizzle atom x box_rows
+int make_tmap_any(rse_index* h, CUtensorMap* out, const void* base, int64_t rows, int64_t cols, int box_rows,
+                  int elem_bytes) {
   static PFN_tmapEncodeTiled fn = nullptr;
   if (!fn) {
     void* p = nullptr;
@@ -478,8 +481,8 @@ int make_tmap_any(rse_index* h, CUtensorMap* out, const void* base, int64_t rows
     if (!p || qres != cudaDriverEntryPointSuccess) return fail(h, RSE_ERR_CUDA, "cuTensorMapEncodeTiled unavailable");
     fn = reinterpret_cast<PFN_tmapEncodeTiled>(p);
   }
-  const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(kScanD), static_cast<cuuint64_t>(rows)};
-  const cuuint64_t gstr[1] = {static_cast<cuuint64_t>(kScanD) * elem_bytes};
+  const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
+  const cuuint64_t gstr[1] = {static_cast<cuuint64_t>(cols) * elem_bytes};
   const cuuint32_t box[2] = {static_cast<cuuint32_t>(128 / elem_bytes), static_cast<cuuint32_t>(box_rows)};
   const cuuint32_t estr[2] = {1, 1};
   CUresult r = fn(out, elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2,
@@ -513,21 +516,22 @@ int make_tmap_lines(rse_index* h, CUtensorMap* out, const void* base, int64_t li
 
 // refine + exact re-score + emit for one block of queries whose survivors are in tc_rows / tc_cnt.
 // thr2 / gate != NULL: the second-chance pass (only the queries tc3_second_threshold_kernel re-armed).
+template <int KB>
 int knn_tc_refine(rse_index* h, const float* q_dev, const double* sb, int nqb, int kprime, long long* cand_dev,
                   int* status_dev, const float* thr2, const unsigned int* gate, float* thr2_out, unsigned int* gate_out,
                   const float* tverify) {
-  if (!(h->attr_mask & (1u << 10))) {
-    CK(cudaFuncSetAttribute(knn_refine_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRefineSmemBytes));
-    CK(cudaFuncSetAttribute(knn_refine_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRefineSmemBytes));
-    h->attr_mask |= 1u << 10;
+  if (!(h->attr_mask_tc & (1u << (8 + KB - 1)))) {
+    CK(cudaFuncSetAttribute(knn_refine_kernel<false, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRefineSmemBytes));
+    CK(cudaFuncSetAttribute(knn_refine_kernel<true, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRefineSmemBytes));
+    h->attr_mask_tc |= 1u << (8 + KB - 1);
   }
   if (h->fma)
-    knn_refine_kernel<true><<<nqb, kSelThreads, kRefineSmemBytes, h->stream>>>(
+    knn_refine_kernel<true, KB><<<nqb, kSelThreads, kRefineSmemBytes, h->stream>>>(
         h->emb, h->amag, q_dev, sb, static_cast<const uint2*>(h->tc_rows.p),
         static_cast<unsigned int*>(h->tc_cnt.p), kTcCandCap, kprime, h->pos_base, h->rowid, h->movie_idx,
         cand_dev, status_dev, 1, thr2, gate, h->dev_counters, thr2_out, gate_out, tverify);
   else
-    knn_refine_kernel<false><<<nqb, kSelThreads, kRefineSmemBytes, h->stream>>>(
+    knn_refine_kernel<false, KB><<<nqb, kSelThreads, kRefineSmemBytes, h->stream>>>(
         h->emb, h->amag, q_dev, sb, static_cast<const uint2*>(h->tc_rows.p),
         static_cast<unsigned int*>(h->tc_cnt.p), kTcCandCap, kprime, h->pos_base, h->rowid, h->movie_idx,
         cand_dev, status_dev, 1, thr2, gate, h->dev_counters, thr2_out, gate_out, tverify);
@@ -551,21 +555,23 @@ int scan_event(rse_index* h, cudaEvent_t* out) {
 
 // Build the fp16 normalised shadow (knn_tc3.cuh) once per corpus.  Returns RSE_OK with shadow_state = -1
 // when the corpus holds rows whose squared norm is not finite (the error bound needs a finite norm).
+// KB = dim / 64.
+template <int KB>
 int ensure_shadow(rse_index* h) {
   if (h->shadow_state != 0) return RSE_OK;
   const int64_t n_pad = (h->n_rows + kT3TileRows - 1) / kT3TileRows * kT3TileRows;     // zero rows up to a whole tile
-  const size_t shadow_bytes = sizeof(__half) * static_cast<size_t>(n_pad) * kScanD;
+  const size_t shadow_bytes = sizeof(__half) * static_cast<size_t>(n_pad) * h->dim;
   ENSURE(h->tc_shadow, shadow_bytes);
   ENSURE(h->tc_cnt, sizeof(unsigned int) * kTcBN);
   {
     // the last (partial) tile pair: zero it before the rows that exist are written
-    const size_t tail0 = sizeof(__half) * static_cast<size_t>(n_pad - kT3TileRows) * kScanD;
+    const size_t tail0 = sizeof(__half) * static_cast<size_t>(n_pad - kT3TileRows) * h->dim;
     CK(cudaMemsetAsync(static_cast<char*>(h->tc_shadow.p) + tail0, 0, shadow_bytes - tail0, h->stream));
   }
   unsigned int* bad = static_cast<unsigned int*>(h->tc_cnt.p);
   CK(cudaMemsetAsync(bad, 0, sizeof(unsigned int), h->stream));
   const int grid = h->sm_count * 8;
-  tc3_shadow_kernel<<<grid, 256, 0, h->stream>>>(h->emb, h->amag, h->n_rows, static_cast<__half*>(h->tc_shadow.p), bad);
+  tc3_shadow_kernel<KB><<<grid, 256, 0, h->stream>>>(h->emb, h->amag, h->n_rows, static_cast<__half*>(h->tc_shadow.p), bad);
   LAUNCHED(h);
   unsigned int nbad = 0;
   CK(cudaMemcpyAsync(&nbad, bad, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
@@ -575,8 +581,8 @@ int ensure_shadow(rse_index* h) {
     h->shadow_state = -1;
     return RSE_OK;
   }
-  // the tiled shadow as a 2-D array of 128-byte lines: [n_pad * 6 lines][64 halves], box = 128 lines = one stage
-  int rc = make_tmap_lines(h, &h->tmap_a16, h->tc_shadow.p, n_pad * kT3KBlocks, kT3HalfRows);
+  // the tiled shadow as a 2-D array of 128-byte lines: [n_pad * KB lines][64 halves], box = 128 lines = one stage
+  int rc = make_tmap_lines(h, &h->tmap_a16, h->tc_shadow.p, n_pad * KB, kT3HalfRows);
   if (rc != RSE_OK) return rc;
   // the probe's sample: its own small matrix from sample_min_tiles tiles on (262 k corpus rows, the automatic K4
   // threshold); smaller corpora keep the strided-tile probe over the main shadow
@@ -584,14 +590,14 @@ int ensure_shadow(rse_index* h) {
   const int64_t n_sample = (h->n_rows + h->sample_stride - 1) / h->sample_stride;
   if (n_sample >= static_cast<int64_t>(h->sample_min_tiles) * kT3TileRows) {
     const int64_t s_pad = (n_sample + kT3TileRows - 1) / kT3TileRows * kT3TileRows;
-    const size_t s_bytes = sizeof(__half) * static_cast<size_t>(s_pad) * kScanD;
+    const size_t s_bytes = sizeof(__half) * static_cast<size_t>(s_pad) * h->dim;
     ENSURE(h->tc_sample, s_bytes);
-    const size_t s_tail0 = sizeof(__half) * static_cast<size_t>(s_pad - kT3TileRows) * kScanD;
+    const size_t s_tail0 = sizeof(__half) * static_cast<size_t>(s_pad - kT3TileRows) * h->dim;
     CK(cudaMemsetAsync(static_cast<char*>(h->tc_sample.p) + s_tail0, 0, s_bytes - s_tail0, h->stream));
-    tc3_sample_kernel<<<grid, 256, 0, h->stream>>>(h->emb, h->amag, h->n_rows, h->sample_stride, n_sample,
+    tc3_sample_kernel<KB><<<grid, 256, 0, h->stream>>>(h->emb, h->amag, h->n_rows, h->sample_stride, n_sample,
                                                    static_cast<__half*>(h->tc_sample.p));
     LAUNCHED(h);
-    rc = make_tmap_lines(h, &h->tmap_s16, h->tc_sample.p, s_pad * kT3KBlocks, kT3HalfRows);
+    rc = make_tmap_lines(h, &h->tmap_s16, h->tc_sample.p, s_pad * KB, kT3HalfRows);
     if (rc != RSE_OK) return rc;
     h->sample_tiles = s_pad / kT3TileRows;
   }
@@ -667,19 +673,22 @@ int enqueue_bm25_overlapped(rse_index* h, cudaEvent_t after) {
 
 // ---- K4 over the fp16 shadow (knn_tc3.cuh) for a GROUP of up to kTcGroupBlocks blocks of 256 queries: one launch
 // per stage (query prep, probe, thresholds, filter, refine, gated second filter + refine) whatever the number of
-// blocks — r01 ran the whole chain once per block from a host loop.
+// blocks — r01 ran the whole chain once per block from a host loop.  KB = dim / 64 selects the instantiation.
 constexpr int kTcGroupBlocks = 8;                 // 2048 queries per group: 134 MB of survivor lists
 
+template <int KB>
 int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, int kprime, long long* cand_dev,
                   int* status_dev) {
-  if (!(h->attr_mask & (1u << 11))) {
-    CK(cudaFuncSetAttribute(knn_tc3_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
-    CK(cudaFuncSetAttribute(knn_tc3_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
-    CK(cudaFuncSetAttribute(knn_tc3_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
+  constexpr int kT3SmemBytes = t3_smem_bytes(KB);
+  if (!(h->attr_mask_tc & (1u << (KB - 1)))) {
+    CK(cudaFuncSetAttribute(knn_tc3_kernel<0, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
+    CK(cudaFuncSetAttribute(knn_tc3_kernel<1, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
+    CK(cudaFuncSetAttribute(knn_tc3_kernel<2, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
     // the filter shares its SMs with BM25 CTAs (hybrid step): ask for the full shared-memory carve-out, otherwise the
     // driver picks the smallest configuration that fits the filter alone and nothing else can become resident
-    CK(cudaFuncSetAttribute(knn_tc3_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    h->attr_mask |= 1u << 11;
+    // (at KB = 8 the filter's 210 KB leave no room for a BM25 CTA of the hybrid step: BM25 then runs after it)
+    CK(cudaFuncSetAttribute(knn_tc3_kernel<1, KB>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    h->attr_mask_tc |= 1u << (KB - 1);
   }
   const int64_t n_tiles = (h->n_rows + kT3TileRows - 1) / kT3TileRows;
   const int max_clusters = std::max(1, h->sm_count / 2);
@@ -713,19 +722,19 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
   if (!sparse_probe && nqg > kTcBN) {
     for (int b0 = 0; b0 < nqg; b0 += kTcBN) {
       const int nqb = std::min(kTcBN, nqg - b0);
-      int rc = knn_tc3_group(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqb, kprime,
-                             cand_dev + static_cast<int64_t>(b0) * kprime * 3, status_dev + b0);
+      int rc = knn_tc3_group<KB>(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqb, kprime,
+                                 cand_dev + static_cast<int64_t>(b0) * kprime * 3, status_dev + b0);
       if (rc != RSE_OK) return rc;
     }
     return RSE_OK;
   }
   const int nblk = (nqg + kTcBN - 1) / kTcBN;
   const int nq_pad = nblk * kTcBN;
-  ENSURE(h->tc_q16, sizeof(__half) * static_cast<size_t>(nq_pad) * kScanD);
-  if (!h->tmap_q16_ok || h->tmap_q16_rows != nq_pad || h->tmap_q16_base != h->tc_q16.p) {
-    int rc = make_tmap_any(h, &h->tmap_q16, h->tc_q16.p, nq_pad, kT3HalfRows, 2);
+  ENSURE(h->tc_q16, sizeof(__half) * static_cast<size_t>(nq_pad) * h->dim);
+  if (!h->tmap_q16_ok || h->tmap_q16_rows != nq_pad || h->tmap_q16_base != h->tc_q16.p || h->tmap_q16_dim != h->dim) {
+    int rc = make_tmap_any(h, &h->tmap_q16, h->tc_q16.p, nq_pad, h->dim, kT3HalfRows, 2);
     if (rc != RSE_OK) return rc;
-    h->tmap_q16_ok = true; h->tmap_q16_rows = nq_pad; h->tmap_q16_base = h->tc_q16.p;
+    h->tmap_q16_ok = true; h->tmap_q16_rows = nq_pad; h->tmap_q16_base = h->tc_q16.p; h->tmap_q16_dim = h->dim;
   }
   ENSURE(h->tc_thr, sizeof(float) * 3 * nq_pad);              // first-pass cuts, the second chance's, the bounds to verify
   ENSURE(h->tc_rows, sizeof(uint2) * static_cast<size_t>(nq_pad) * kTcCandCap);
@@ -740,12 +749,12 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
   __half* q16 = static_cast<__half*>(h->tc_q16.p);
   float* thr = static_cast<float*>(h->tc_thr.p);
 
-  tc3_query_prep_kernel<<<nq_pad, kScanD / 4, 0, h->stream>>>(q_dev, sb, nqg, q16);
+  tc3_query_prep_kernel<KB><<<nq_pad, 16 * KB, 0, h->stream>>>(q_dev, sb, nqg, q16);
   LAUNCHED(h);
 
   // 1. probe: approximate distances of a strided sample of tiles → K'-th smallest per query
   if (sparse_probe) {
-    knn_tc3_kernel<2><<<grid_p, kT3Threads, kT3SmemBytes, h->stream>>>(
+    knn_tc3_kernel<2, KB><<<grid_p, kT3Threads, kT3SmemBytes, h->stream>>>(
         sampled ? h->tmap_s16 : h->tmap_a16, h->tmap_q16, n_probe, tile_stride, nqg, nblk, nullptr, dist, ld_sel, nullptr,
         nullptr, 0, nullptr);
     LAUNCHED(h);
@@ -753,7 +762,7 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
                                                               sampled ? thr + 2 * nq_pad : nullptr);
     LAUNCHED(h);
   } else {
-    knn_tc3_kernel<0><<<grid_p, kT3Threads, kT3SmemBytes, h->stream>>>(
+    knn_tc3_kernel<0, KB><<<grid_p, kT3Threads, kT3SmemBytes, h->stream>>>(
         h->tmap_a16, h->tmap_q16, n_probe, tile_stride, nqg, 1, nullptr, dist, ld_probe, nullptr, nullptr, 0, nullptr);
     LAUNCHED(h);
     select_init_kernel<<<(nqg + 127) / 128, 128, 0, h->stream>>>(sel, nqg, static_cast<unsigned int>(kprime));
@@ -784,7 +793,7 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
     CK(cudaEventRecord(h->ev_prefilter, h->stream));
   }
   tl_mark(h, kTlPrefilter, h->stream);
-  knn_tc3_kernel<1><<<grid_f, kT3Threads, kT3SmemBytes, h->stream>>>(
+  knn_tc3_kernel<1, KB><<<grid_f, kT3Threads, kT3SmemBytes, h->stream>>>(
       h->tmap_a16, h->tmap_q16, n_tiles, 1, nqg, nblk, thr, nullptr, 0, static_cast<uint2*>(h->tc_rows.p),
       static_cast<unsigned int*>(h->tc_cnt.p), kTcCandCap, nullptr);
   LAUNCHED(h);
@@ -806,27 +815,47 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
   float* thr2 = thr + nq_pad;
   unsigned int* gate = static_cast<unsigned int*>(h->tc_cnt.p) + nq_pad;
   {
-    int rc = knn_tc_refine(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, nullptr, nullptr, thr2, gate,
+    int rc = knn_tc_refine<KB>(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, nullptr, nullptr, thr2, gate,
                            sampled ? thr + 2 * nq_pad : nullptr);
     if (rc != RSE_OK) return rc;
   }
   // 5. second chance: one more filter pass + refine for the armed queries only (blocks without one are skipped).
   //    Enqueued unconditionally, gated on the device: two near-empty launches when no query needs it.
-  knn_tc3_kernel<1><<<grid_f, kT3Threads, kT3SmemBytes, h->stream>>>(
+  knn_tc3_kernel<1, KB><<<grid_f, kT3Threads, kT3SmemBytes, h->stream>>>(
       h->tmap_a16, h->tmap_q16, n_tiles, 1, nqg, nblk, thr2, nullptr, 0, static_cast<uint2*>(h->tc_rows.p),
       static_cast<unsigned int*>(h->tc_cnt.p), kTcCandCap, gate);
   LAUNCHED(h);
-  return knn_tc_refine(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, thr2, gate, nullptr, nullptr, nullptr);
+  return knn_tc_refine<KB>(h, q_dev, sb, nqg, kprime, cand_dev, status_dev, thr2, gate, nullptr, nullptr, nullptr);
 }
 
+// K4 serves every width D = 64 KB, KB = 1..8 (knn_tc3_kernel<MODE, KB>); any other width keeps the exact scan
+bool tc_width_ok(int dim) { return dim % kT3BK == 0 && dim >= kT3BK && dim <= kT3MaxKBlocks * kT3BK; }
+
 bool tc_eligible(const rse_index* h, int nq, int kprime) {
-  if (h->tc_mode == 1 || h->dim != kScanD) return false;
+  if (h->tc_mode == 1 || !tc_width_ok(h->dim)) return false;
   if (((h->n_rows + 127) / 128) * 128 < 8ll * kprime || h->n_rows < 1024) return false;   // the probe needs a usable sample
   if (kprime * 4 > kTcCandCap || kprime * 2 > kTcRefineCap) return false;
   if (h->tc_mode == 2) return true;
   // a single query joins the batches once the shadow exists (K4 reads 768 B per row instead of 1536: 0.76 against
-  // 1.18 ms per call on S-600k) — but it never makes the library build the shadow
-  return (nq >= RSE_TC_MIN_BATCH || h->shadow_state == 1) && h->n_rows >= 262144;
+  // 1.18 ms per call on S-600k) — but it never makes the library build the shadow.  That was measured at 384 only:
+  // at any other width a single query keeps the exact scan.
+  return (nq >= RSE_TC_MIN_BATCH || (h->shadow_state == 1 && h->dim == kScanD)) && h->n_rows >= 262144;
+}
+
+// the shadow (built once) and every group of up to kTcGroupBlocks x 256 queries; leaves shadow_state = -1 and enqueues
+// nothing when the corpus cannot use K4
+template <int KB>
+int knn_tc3_run(rse_index* h, const float* q_dev, const double* sb, int nq, int kprime, long long* cand_dev,
+                int* status) {
+  int rc = ensure_shadow<KB>(h);
+  if (rc != RSE_OK || h->shadow_state < 0) return rc;
+  for (int b0 = 0; b0 < nq; b0 += kTcGroupBlocks * kTcBN) {
+    const int nqg = std::min(kTcGroupBlocks * kTcBN, nq - b0);
+    rc = knn_tc3_group<KB>(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqg, kprime,
+                           cand_dev + static_cast<int64_t>(b0) * kprime * 3, status + b0);
+    if (rc != RSE_OK) return rc;
+  }
+  return RSE_OK;
 }
 
 // Local top-kprime for nq device-resident queries → packed candidates (device), in two halves: _begin enqueues
@@ -855,15 +884,20 @@ int knn_local_begin(rse_index* h, const float* q_dev, int nq, int kprime, long l
   ENSURE(h->tc_status, sizeof(int) * nq);
   int* status = static_cast<int*>(h->tc_status.p);
   {
-    int rc = ensure_shadow(h);
+    int rc = RSE_OK;
+    switch (h->dim / kT3BK) {                      // tc_eligible: dim = 64 KB, KB = 1..8
+      case 1: rc = knn_tc3_run<1>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 2: rc = knn_tc3_run<2>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 3: rc = knn_tc3_run<3>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 4: rc = knn_tc3_run<4>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 5: rc = knn_tc3_run<5>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 6: rc = knn_tc3_run<6>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 7: rc = knn_tc3_run<7>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 8: rc = knn_tc3_run<8>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      default: return fail(h, RSE_ERR_STATE, "rse_knn: no tensor-core instantiation for this width");
+    }
     if (rc != RSE_OK) return rc;
     if (h->shadow_state < 0) return knn_exact_groups(h, q_dev, sb, nq, kprime, cand_dev);
-  }
-  for (int b0 = 0; b0 < nq; b0 += kTcGroupBlocks * kTcBN) {
-    const int nqg = std::min(kTcGroupBlocks * kTcBN, nq - b0);
-    int rc = knn_tc3_group(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqg, kprime,
-                           cand_dev + static_cast<int64_t>(b0) * kprime * 3, status + b0);
-    if (rc != RSE_OK) return rc;
   }
   h->stats.tc_queries += nq;
   if (h->pin_status_n < static_cast<size_t>(nq)) {
