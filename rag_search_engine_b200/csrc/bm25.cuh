@@ -432,6 +432,7 @@ __global__ void bm25_weight_kernel(const uint2* __restrict__ post, const double*
   if (out4) {
     unsigned int wq = __double2uint_rn(__dmul_rn(o.w, wq4_scale));
     if (wq > 0x7FFFFu) wq = 0x7FFFFu;                      // (k1+1) * wq4_scale <= 2^19: only a weight at the very top clamps
+    if (wq == 0u && o.w > 0.0) wq = 1u;                    // a weight word of 0 adds nothing: a posting that counts must not round to it
     out4[i] = (e.x % static_cast<uint32_t>(kBmRange)) | (wq << 13);
   }
 }
@@ -681,11 +682,15 @@ bm25_stream_kernel(const int64_t* __restrict__ indptr, const Post16* __restrict_
 // 4.8e-7).  The kernel is HBM-bound on the posting stream (in a hybrid step it shares the HBM with the tensor-core
 // filter), so it reads a 4-BYTE posting instead of the 16-byte {doc, tf, double w}: 13 bits of document offset
 // inside its range (the range is known from the slice being read) and a 19-bit weight, wq = round(w * wq4_scale)
-// with wq4_scale the largest power of two keeping (k1+1) * wq4_scale <= 2^19.  A weight is known to +-1 unit of wq
-// (0.5 from its rounding, the clamp at the top), i.e. +-idfx units of the sum (idfx = idf * scale / wq4_scale), and
-// each term adds <= 0.5 unit of its own rounding.  The sum is exact in that format and independent of the order, so
-// all the token slices of a range are cut into 128-posting items (a lane loads one aligned 16-byte QUAD) that the
-// warps take round robin with NO barrier between tokens.  Everything decided on these sums carries a margin of
+// with wq4_scale the largest power of two keeping (k1+1) * wq4_scale <= 2^19.  0 is a sentinel twice over — a weight
+// word of 0 adds nothing, a sum of 0 is an untouched document — so a posting with w > 0 is stored as wq >= 1, and a
+// contribution is ROUNDED UP, ceil(idfx * wq) >= 1: every document a query touches keeps a non-zero sum.  A weight is
+// known to +-1 unit of wq (0.5 from its rounding, the clamp at the top, the raise from 0 to 1), i.e. +-idfx units of
+// the sum (idfx = idf * scale / wq4_scale), and rounding up adds [0, 1) unit: a document's sum lies within
+// [-idfx_t, idfx_t + 1) per term of its exact value, so the sums of two documents disagree with their exact order by
+// less than sum_t (2 * idfx_t + 1).  The sum is exact in that format and independent of the order, so all the token
+// slices of a range are cut into 128-posting items (a lane loads one aligned 16-byte QUAD) that the warps take round
+// robin with NO barrier between tokens.  Everything decided on these sums compares two of them with a margin of
 // 2 * sum_t (idfx_t + 0.5) + 8 units PER QUERY, at least kFxMargin (~1e-3 in score units for a 16-token query with
 // the default k1); the finalists (k plus whatever lies within the margin of the k-th) are RE-SCORED in
 // bm25_fx_finish_kernel with the reference's own expression in query-token order — one thread per (document, token)
@@ -858,11 +863,12 @@ bm25_fx_body(const int64_t* __restrict__ indptr, const uint32_t* __restrict__ po
       }
     };
     auto item_apply = [&](const uint4& e, double idfx) {
-      // sums only grow and nothing reads them before the barrier: plain reductions, no returned value to wait for
+      // sums only grow and nothing reads them before the barrier: plain reductions, no returned value to wait for.
+      // Rounded UP, a contribution of a non-zero word is at least 1: a sum of 0 means "untouched" to the scan.
       const uint32_t w4[4] = {e.x, e.y, e.z, e.w};
 #pragma unroll
       for (int u = 0; u < 4; ++u)
-        if (w4[u] >> 13) atomicAdd(&acc[w4[u] & 0x1FFFu], __double2uint_rn(__dmul_rn(idfx, __uint2double_rn(w4[u] >> 13))));
+        if (w4[u] >> 13) atomicAdd(&acc[w4[u] & 0x1FFFu], __double2uint_ru(__dmul_rn(idfx, __uint2double_rn(w4[u] >> 13))));
     };
     {
       // DEPTH loads in flight per lane (a ring of named buffers: every index below is a compile-time constant)
@@ -1091,7 +1097,7 @@ bm25_merge_kernel(const unsigned long long* __restrict__ cand_hi, const unsigned
   }
   // per-thread heads (a thread may own several ranges when nr > blockDim; it keeps
   // the best head among them and re-scans its ranges after winning)
-  constexpr int kMaxOwn = 8;                 // nr <= 2048 ranges = 16.7 M docs
+  constexpr int kMaxOwn = 8;                 // nr <= 2048 ranges = 14,680,064 docs
   int head[kMaxOwn];
 #pragma unroll
   for (int i = 0; i < kMaxOwn; ++i) head[i] = 0;

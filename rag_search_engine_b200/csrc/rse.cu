@@ -1450,7 +1450,7 @@ int rse_load_bm25(rse_index* h, const int64_t* indptr, const uint32_t* doc_idx, 
   h->n_terms = n_terms; h->n_postings = n_postings; h->n_docs = n_docs; h->n_movies = n_movies; h->avgdl = avgdl;
   h->nr = static_cast<int>((n_docs + kBmRange - 1) / kBmRange);
   if (h->nr < 1) h->nr = 1;
-  if (h->nr > 2048) return fail(h, RSE_ERR_UNSUPPORTED, "rse_load_bm25: more than 16.7M documents");
+  if (h->nr > 2048) return fail(h, RSE_ERR_UNSUPPORTED, "rse_load_bm25: more than 14,680,064 documents (2048 ranges of 7168)");
   h->df_host.assign(df, df + n_terms);
 
   CK(cudaMalloc(&h->indptr, sizeof(int64_t) * (n_terms + 1)));
@@ -1665,7 +1665,9 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
           h->dev_counters, idfx_scale);
       LAUNCHED(h);
     } else if (stream) {
-      const size_t per_qs = static_cast<size_t>(ng) * std::max(k, 2 * kFxFinalCap);
+      // bm25_stream_kernel and bm25_merge_kernel index these lists as [q][ng][k]: offset by that stride (the buffers
+      // are sized for the larger fixed-point lists)
+      const int64_t per_qs = static_cast<int64_t>(ng) * k;
       shi = static_cast<unsigned long long*>(h->b_shi.p) - static_cast<int64_t>(q0) * per_qs;
       slo = static_cast<unsigned long long*>(h->b_slo.p) - static_cast<int64_t>(q0) * per_qs;
       scnt = static_cast<int*>(h->b_scnt.p) - static_cast<int64_t>(q0) * ng;
