@@ -41,8 +41,10 @@ extern "C" {
 /* Limits (documented in DESIGN.md §limits) */
 #define RSE_VEC0_BLOCK 1024     /* sqlite-vec default chunk_size (semantic_search.py:96-99 passes none) */
 #define RSE_MAX_KPRIME 4096     /* sqlite-vec caps k at 4096 */
-#define RSE_MAX_BM25_K 256
-#define RSE_MAX_FUSE_LIMIT 128
+#define RSE_MAX_BM25_K 512      /* rse_bm25 k; covers the k = 409 of a hybrid call at limit 409 */
+#define RSE_MAX_FUSE_LIMIT 1024 /* rse_fuse_weighted / rse_fuse_rrf: a padded union of two 409-deep lists has 818 ids */
+#define RSE_MAX_HYBRID_LIMIT 512 /* rse_hybrid*: also limit * knn_multiplier <= RSE_MAX_KPRIME (409 at multiplier 10) */
+#define RSE_MAX_RERANK_LIMIT 128 /* rse_hybrid_rerank_run */
 #define RSE_MAX_QUERY_TOKENS 255
 #define RSE_RRF_NOT_FOUND 99999 /* hybrid_search.py:247 */
 #define RSE_MAX_STASH 16        /* staged batches that can be parked in HBM (rse_hybrid_stash) */
@@ -165,7 +167,8 @@ int rse_load_bm25(rse_index *h, const int64_t *indptr, const uint32_t *doc_idx, 
  * duplicates kept, -1 = unknown term, skipped: keyword_search.py:205-210).
  * Outputs [nq, k]: scores (fp64, bit-exact reference arithmetic :224,:241-244),
  * dense doc indices, and per-query counts.  Order = sorted(..., reverse=True)
- * with dict-insertion tie order (:250). */
+ * with dict-insertion tie order (:250).  1 <= k <= RSE_MAX_BM25_K (512); above 256 the
+ * candidate lists of one call are held to 256 MB by scoring the batch in query chunks. */
 int rse_bm25(rse_index *h, const int32_t *tok_indptr, const int32_t *term_rows, int32_t nq,
              int32_t k, double k1, double b, double *out_score, int32_t *out_doc_idx,
              int32_t *out_count);
@@ -179,7 +182,8 @@ int rse_bm25(rse_index *h, const int32_t *tok_indptr, const int32_t *term_rows, 
  * weighted: hybrid_search.py:117-180 (min_max_norm utils.py:182-191,
  *           alpha*b + (1-alpha)*s :163).
  * rrf:      hybrid_search.py:217-272,379 (0-based ranks, NOT_FOUND=99999 :247,
- *           1/(k+r_b) + 1/(k+r_s) :255); out ranks are -1 for None. */
+ *           1/(k+r_b) + 1/(k+r_s) :255); out ranks are -1 for None.
+ * 1 <= limit <= RSE_MAX_FUSE_LIMIT (1024). */
 int rse_fuse_weighted(rse_index *h, int32_t nq, int32_t limit, double alpha, int32_t tie_mode,
                       const int64_t *bm25_id, const double *bm25_score, const int32_t *bm25_count,
                       const int64_t *sem_id, const double *sem_dist, const int32_t *sem_count,
@@ -198,7 +202,9 @@ int rse_fuse_rrf(rse_index *h, int32_t nq, int32_t limit, double k, int32_t tie_
  * doc_ids[n_docs] / movie_ids[n_movies_uni] map dense indices to movies.id (set with
  * rse_set_id_tables).  mode: 0 = rrf (param = k), 1 = weighted (param = alpha).
  * Outputs [nq, limit]; out_a/out_b = (bm25_rank, sem_rank) as doubles for rrf
- * (-1 = None) or (bm25_norm, sem_norm) for weighted. */
+ * (-1 = None) or (bm25_norm, sem_norm) for weighted.  Every hybrid entry point takes
+ * 1 <= limit <= RSE_MAX_HYBRID_LIMIT (512) with max(limit * knn_multiplier, limit) <= RSE_MAX_KPRIME:
+ * the reference's own ceiling at its multiplier 10 is limit 409 (sqlite-vec refuses k > 4096). */
 int rse_set_id_tables(rse_index *h, const int64_t *doc_ids, int64_t n_docs, const int64_t *movie_ids,
                       int64_t n_movie_ids);
 int rse_hybrid(rse_index *h, int32_t mode, double param, int32_t tie_mode, int32_t limit,

@@ -17,8 +17,10 @@ LIB_PATH = _HERE / "csrc" / "librse.so"
 
 RSE_OK = 0
 RSE_MAX_KPRIME = 4096
-RSE_MAX_BM25_K = 256
-RSE_MAX_FUSE_LIMIT = 128
+RSE_MAX_BM25_K = 512
+RSE_MAX_FUSE_LIMIT = 1024
+RSE_MAX_HYBRID_LIMIT = 512
+RSE_MAX_RERANK_LIMIT = 128
 RSE_MAX_QUERY_TOKENS = 255
 TIE_REFERENCE = 0
 TIE_BY_ID = 1

@@ -34,6 +34,8 @@ constexpr int kBmThreads = 256;
 constexpr int kBmMaxTokens = 255;
 constexpr int kBmDocsPerThread = kBmRange / kBmThreads;   // 32
 constexpr unsigned int kBmCandCap = 192;                    // survivors of the threshold pass kept in smem
+constexpr int kBmGeneralMaxK = 256;                         // bm25_score_kernel; bm25_deep_score_kernel above it
+constexpr int kBmDeepMaxK = 512;                            // = RSE_MAX_BM25_K
 
 struct Key128 {
   unsigned long long hi;   // ~orderable(score): ascending hi == descending score
@@ -112,6 +114,8 @@ __device__ __forceinline__ Key128 block_argmin(Key128 mine, Key128* s_k, int* s_
 
 // K6: one CTA per (range, query).
 //   cand_hi/lo: [nq][nr][k]; cand_cnt: [nq][nr]
+// kDeep (k > kBmGeneralMaxK): the range's k best are found by a radix selection instead of k barrier rounds.
+template <bool kDeep>
 __device__ __forceinline__ void
 bm25_score_one(const int64_t* __restrict__ indptr, const uint2* __restrict__ post,
                const uint32_t* __restrict__ roff, const double* __restrict__ normk, int nr,
@@ -124,7 +128,8 @@ bm25_score_one(const int64_t* __restrict__ indptr, const uint2* __restrict__ pos
   unsigned char* first = reinterpret_cast<unsigned char*>(acc + kBmRange); // [kBmRange]
   // token tables (scoring phase) and selection scratch (afterwards) share one buffer
   constexpr int kTokBytes = (kBmMaxTokens + 1) * (8 + 8 + 4);
-  constexpr int kSelBytes = (256 + static_cast<int>(kBmCandCap)) * static_cast<int>(sizeof(Key128));
+  constexpr int kSelBytes = kDeep ? 256 * 4 + kBmDeepMaxK * static_cast<int>(sizeof(Key128))
+                                  : (256 + static_cast<int>(kBmCandCap)) * static_cast<int>(sizeof(Key128));
   __shared__ __align__(16) unsigned char s_cand_mem[kTokBytes > kSelBytes ? kTokBytes : kSelBytes];
   long long* s_lo = reinterpret_cast<long long*>(s_cand_mem);
   double* s_idf = reinterpret_cast<double*>(s_cand_mem + (kBmMaxTokens + 1) * 8);
@@ -214,6 +219,73 @@ bm25_score_one(const int64_t* __restrict__ indptr, const uint2* __restrict__ pos
     kk.lo = (static_cast<unsigned long long>(first[l]) << 32) | (doc_base + static_cast<uint32_t>(l));
     return kk;
   };
+  if constexpr (kDeep) {
+    // Radix selection over the key (score desc, first token asc, doc asc), one byte per pass: the 8 bytes of the
+    // orderable score, the first token, then the document's offset in the range (13 bits: two passes).  Thread t
+    // owns documents t + 256 i: bit i of `live` (still tied with the threshold prefix) and of `taken` (strictly
+    // better than it).  The keys are distinct, so exactly min(k, touched) documents end up taken; they are
+    // collected and ordered by rank counting.
+    unsigned int* s_hist = reinterpret_cast<unsigned int*>(s_cand_mem);              // [256]
+    Key128* s_sel = reinterpret_cast<Key128*>(s_cand_mem + 256 * 4);                // [kBmDeepMaxK]
+    __shared__ unsigned int s_warp[kBmThreads / 32], s_digit, s_before, s_touched;
+    auto digit = [&](int pass, int l) -> unsigned int {
+      if (pass < 8) {
+        const uint64_t hi = ~f64_orderable(static_cast<uint64_t>(__double_as_longlong(acc[l])));
+        return static_cast<unsigned int>(hi >> (56 - 8 * pass)) & 0xFFu;
+      }
+      if (pass == 8) return first[l];
+      return pass == 9 ? static_cast<unsigned int>(l) >> 8 : static_cast<unsigned int>(l) & 0xFFu;
+    };
+    uint32_t live = 0u, taken = 0u;
+#pragma unroll 4
+    for (int i = 0; i < kBmDocsPerThread; ++i)
+      if (first[threadIdx.x + i * kBmThreads] != 0xFF) live |= 1u << i;
+    if (threadIdx.x == 0) s_touched = 0u;
+    __syncthreads();
+    if (live) atomicAdd(&s_touched, static_cast<unsigned int>(__popc(live)));
+    __syncthreads();
+    unsigned int need = static_cast<unsigned int>(k);
+    if (s_touched <= need) {
+      taken = live;
+    } else {
+      for (int pass = 0; pass < 11; ++pass) {
+        s_hist[threadIdx.x] = 0u;
+        __syncthreads();
+        for (uint32_t m = live; m; m &= m - 1u)
+          atomicAdd(&s_hist[digit(pass, threadIdx.x + (__ffs(m) - 1) * kBmThreads)], 1u);
+        __syncthreads();
+        block_pick_digit(s_hist, need, s_warp, &s_digit, &s_before);
+        const unsigned int d = s_digit, in_bin = s_hist[d];
+        need -= s_before;
+        for (uint32_t m = live; m; m &= m - 1u) {
+          const int i = __ffs(m) - 1;
+          const unsigned int g = digit(pass, threadIdx.x + i * kBmThreads);
+          if (g < d) taken |= 1u << i;
+          if (g != d) live &= ~(1u << i);
+        }
+        if (in_bin == need) { taken |= live; break; }                 // the whole bin is in: uniform
+        __syncthreads();                                              // s_hist / s_digit are read before the reset
+      }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) s_touched = 0u;
+    __syncthreads();
+    for (uint32_t m = taken; m; m &= m - 1u) {
+      const int l = threadIdx.x + (__ffs(m) - 1) * kBmThreads;
+      s_sel[atomicAdd(&s_touched, 1u)] = make_key(l);
+    }
+    __syncthreads();
+    const int nc = static_cast<int>(s_touched);
+    for (int i = threadIdx.x; i < nc; i += kBmThreads) {
+      const Key128 me = s_sel[i];
+      int rank = 0;
+      for (int j = 0; j < nc; ++j) rank += key_less(s_sel[j], me) ? 1 : 0;
+      cand_hi[cbase * k + rank] = me.hi;
+      cand_lo[cbase * k + rank] = me.lo;
+    }
+    if (threadIdx.x == 0) cand_cnt[cbase] = nc;
+    return;
+  }
   if (k <= 32) {
     // Fast path.  (1) every thread finds the best of its 32 documents; (2) each warp sorts its 32
     // thread-bests with shuffles; (3) warp 0 merges the 8 sorted lists to the k-th best overall — a
@@ -348,14 +420,26 @@ bm25_score_kernel(const int64_t* __restrict__ indptr, const uint2* __restrict__ 
                   unsigned long long* __restrict__ cand_hi, unsigned long long* __restrict__ cand_lo,
                   int* __restrict__ cand_cnt, const int* __restrict__ flagged) {
   if (!flagged) {
-    bm25_score_one(indptr, post, roff, normk, nr, n_docs, tok_indptr, term_rows, tok_idf, q0 + blockIdx.y, k, k1p1, cand_hi,
+    bm25_score_one<false>(indptr, post, roff, normk, nr, n_docs, tok_indptr, term_rows, tok_idf, q0 + blockIdx.y, k, k1p1, cand_hi,
                    cand_lo, cand_cnt);
     return;
   }
   const int n = flagged[0];
   for (int j = blockIdx.y; j < n; j += gridDim.y)
-    bm25_score_one(indptr, post, roff, normk, nr, n_docs, tok_indptr, term_rows, tok_idf, flagged[1 + j], k, k1p1, cand_hi,
+    bm25_score_one<false>(indptr, post, roff, normk, nr, n_docs, tok_indptr, term_rows, tok_idf, flagged[1 + j], k, k1p1, cand_hi,
                    cand_lo, cand_cnt);
+}
+
+// k > kBmGeneralMaxK: grid (nr, nq), CTA (r, j) scores query q0 + j; the per-range lists go through bm25_merge_kernel.
+__global__ void __launch_bounds__(kBmThreads)
+bm25_deep_score_kernel(const int64_t* __restrict__ indptr, const uint2* __restrict__ post,
+                       const uint32_t* __restrict__ roff, const double* __restrict__ normk, int nr,
+                       int64_t n_docs, const int32_t* __restrict__ tok_indptr, const int32_t* __restrict__ term_rows,
+                       const double* __restrict__ tok_idf, int q0, int k, double k1p1,
+                       unsigned long long* __restrict__ cand_hi, unsigned long long* __restrict__ cand_lo,
+                       int* __restrict__ cand_cnt) {
+  bm25_score_one<true>(indptr, post, roff, normk, nr, n_docs, tok_indptr, term_rows, tok_idf, q0 + blockIdx.y, k, k1p1,
+                       cand_hi, cand_lo, cand_cnt);
 }
 
 // flagged[0] = number of queries in [q0, q0 + nc) with status != 0, flagged[1..] = those queries (ascending)

@@ -59,4 +59,28 @@ __host__ __device__ __forceinline__ int next_pow2(int x) {
   return p;
 }
 
+// 256 threads, 256 histogram bins (one per thread): the digit d with  sum(hist[0..d-1]) < need <= sum(hist[0..d]).
+// The thread that owns d writes *out_digit = d and *out_before = sum(hist[0..d-1]); *out_digit stays 256 when
+// the histogram holds fewer than `need` entries.  s_warp: 8 words of scratch.  Ends with a barrier.
+__device__ __forceinline__ void block_pick_digit(const unsigned int* s_hist, unsigned int need, unsigned int* s_warp,
+                                                 unsigned int* out_digit, unsigned int* out_before) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned int c = s_hist[threadIdx.x];
+  unsigned int incl = c;
+#pragma unroll
+  for (int off = 1; off < 32; off <<= 1) {
+    const unsigned int o = __shfl_up_sync(0xFFFFFFFFu, incl, off);
+    if (lane >= off) incl += o;
+  }
+  if (lane == 31) s_warp[warp] = incl;
+  if (threadIdx.x == 0) *out_digit = 256u;
+  __syncthreads();
+  unsigned int base = 0u;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) base += (w < warp) ? s_warp[w] : 0u;
+  incl += base;
+  if (incl >= need && incl - c < need) { *out_digit = threadIdx.x; *out_before = incl - c; }
+  __syncthreads();
+}
+
 }  // namespace rse

@@ -9,8 +9,12 @@
 // or ascending id in RSE_TIE_BY_ID mode; the stable descending sort is done by
 // rank counting (rank = #greater + #equal-before).
 //
-// Latency-bound, ≤ 2*limit items per query: one warp per query, lane 0 runs the
-// serial set emulation in shared memory, all lanes do the scoring / ranking.
+// Latency-bound, ≤ 2*limit items per query.  Up to kFuseMaxLimit (every hybrid call of the serving loop, the
+// fusion entry points and the cross-encoder rerank): one warp per query, lane 0 runs the serial set emulation in
+// shared memory with the keys in the table slots, all lanes do the scoring / ranking.  Above it, up to
+// kFuseDeepLimit (deep result lists for a reranker): one CTA of 256 threads per query; the sets hold 16-bit indices
+// into the staged ids (8-byte slots for a 2048-id union would need 384 KB of shared memory, more than a block may
+// have), and the ascending-id union, the scoring and the rank counting are spread over all eight warps.
 #pragma once
 #include "common.cuh"
 #include "pyset.h"
@@ -18,6 +22,8 @@
 namespace rse {
 
 constexpr int kFuseMaxLimit = 128;
+constexpr int kFuseDeepLimit = 1024;
+constexpr int kFuseDeepThreads = 256;
 
 __host__ __device__ inline int fuse_cap_side(int limit) { return pyset_capacity_for(limit); }
 __host__ __device__ inline int fuse_cap_union(int limit) { return pyset_capacity_for(2 * limit); }
@@ -25,6 +31,17 @@ __host__ __device__ inline int fuse_cap_union(int limit) { return pyset_capacity
 __host__ __device__ inline size_t fuse_smem_bytes(int limit) {
   size_t tables = static_cast<size_t>(2 * fuse_cap_side(limit) + 2 * fuse_cap_union(limit)) * 8;
   return tables + static_cast<size_t>(2 * limit) * 8 * 4 + 64;
+}
+// deep kernel: order / score / a / b [2L] and the staged ids, scores, distances [L] x 2 (8 B each), then the four
+// tables of 16-bit slots — 192 KB at limit 1024
+__host__ __device__ inline size_t fuse_deep_smem_bytes(int limit) {
+  size_t tables = static_cast<size_t>(2 * fuse_cap_side(limit) + 2 * fuse_cap_union(limit)) * 2;
+  return static_cast<size_t>(2 * limit) * 8 * 6 + tables + 64;
+}
+
+template <int kThreads>
+__device__ __forceinline__ void fuse_sync() {
+  if constexpr (kThreads == 32) __syncwarp(); else __syncthreads();
 }
 
 struct FuseIn {
@@ -41,32 +58,55 @@ struct FuseIn {
 // inputs [nq][limit]; outputs [nq][out_w] (limit <= out_w <= 2 * limit): id, score, a, b  (rrf: a/b =
 // bm25_rank/sem_rank as double, -1 = None; weighted: a/b = bm25_norm/sem_norm).  out_w = limit is the reference's
 // [:limit]; out_w = 2 * limit keeps the whole union in fused order (what the cross-encoder rerank scores).
-__global__ void __launch_bounds__(32)
+// The deep kernel's shared memory allows one CTA per SM anyway; saying so (min blocks 1) keeps ptxas from spilling
+// the set emulation's loop state at 48 registers.
+template <int kMaxLimit>
+__global__ void __launch_bounds__(kMaxLimit > kFuseMaxLimit ? kFuseDeepThreads : 32, kMaxLimit > kFuseMaxLimit ? 1 : 0)
 fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int tie_mode, long long* __restrict__ out_id,
             double* __restrict__ out_score, double* __restrict__ out_a, double* __restrict__ out_b,
             int* __restrict__ out_count) {
+  constexpr bool kDeep = kMaxLimit > kFuseMaxLimit;
+  constexpr int kThreads = kDeep ? kFuseDeepThreads : 32;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int q = blockIdx.x;
   if (q >= nq) return;
   const int lane = threadIdx.x;
   const int cs = fuse_cap_side(limit), cu = fuse_cap_union(limit);
-  int64_t* ta = reinterpret_cast<int64_t*>(smem_raw);
-  int64_t* tb = ta + cs;
-  int64_t* tr = tb + cs;
-  int64_t* sc = tr + cu;
-  int64_t* order = sc + cu;                                  // [2*limit]
-  double* score = reinterpret_cast<double*>(order + 2 * limit);
-  double* va = score + 2 * limit;
-  double* vb = va + 2 * limit;
+  int64_t *ta, *tb, *tr, *sc, *order;
+  double *score, *va, *vb;
+  long long *s_bid, *s_sid;
+  double *s_bsc, *s_sds;
+  uint16_t* t16 = nullptr;
   __shared__ int s_n;
-
-  // the two hit lists are staged in shared memory by the whole warp first: the set emulation below is a serial
-  // walk by one lane, and every global load in it was a ~500-cycle round trip (23 us per 256-query batch)
-  __shared__ long long s_bid[kFuseMaxLimit], s_sid[kFuseMaxLimit];
-  __shared__ double s_bsc[kFuseMaxLimit], s_sds[kFuseMaxLimit];
+  if constexpr (kDeep) {
+    order = reinterpret_cast<int64_t*>(smem_raw);                 // [2*limit]
+    score = reinterpret_cast<double*>(order + 2 * limit);
+    va = score + 2 * limit;
+    vb = va + 2 * limit;
+    s_bid = reinterpret_cast<long long*>(vb + 2 * limit);         // [limit], s_sid right behind: the key array of
+    s_sid = s_bid + limit;                                        // the index-slot sets (b's slots start at limit)
+    s_bsc = reinterpret_cast<double*>(s_sid + limit);
+    s_sds = s_bsc + limit;
+    t16 = reinterpret_cast<uint16_t*>(s_sds + limit);             // ta, tb [cs], tr, scratch [cu]
+    if (lane == 0) s_n = 0;
+  } else {
+    ta = reinterpret_cast<int64_t*>(smem_raw);
+    tb = ta + cs;
+    tr = tb + cs;
+    sc = tr + cu;
+    order = sc + cu;                                              // [2*limit]
+    score = reinterpret_cast<double*>(order + 2 * limit);
+    va = score + 2 * limit;
+    vb = va + 2 * limit;
+    // the two hit lists are staged in shared memory by the whole warp first: the set emulation below is a serial
+    // walk by one lane, and every global load in it was a ~500-cycle round trip (23 us per 256-query batch)
+    __shared__ long long s_bid_w[kFuseMaxLimit], s_sid_w[kFuseMaxLimit];
+    __shared__ double s_bsc_w[kFuseMaxLimit], s_sds_w[kFuseMaxLimit];
+    s_bid = s_bid_w; s_sid = s_sid_w; s_bsc = s_bsc_w; s_sds = s_sds_w;
+  }
   int nb = in.bm25_count[q]; if (nb > limit) nb = limit; if (nb < 0) nb = 0;
   int ns = in.sem_count[q];  if (ns > limit) ns = limit; if (ns < 0) ns = 0;
-  for (int i = lane; i < limit; i += 32) {
+  for (int i = lane; i < limit; i += kThreads) {
     const int64_t o = static_cast<int64_t>(q) * limit + i;
     long long b_id = -1ll, s_id = -1ll;
     if (i < nb) {
@@ -82,13 +122,42 @@ fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int
     s_sid[i] = s_id;
     s_sds[i] = i < ns ? (in.sem_dist64 ? in.sem_dist64[o] : static_cast<double>(in.sem_dist[o])) : 0.0;   // float(hit["distance"])
   }
-  __syncwarp();
+  fuse_sync<kThreads>();
   const long long* bid = s_bid;
   const double* bsc = s_bsc;
   const long long* sid = s_sid;
   auto sem_d = [&](int i) -> double { return s_sds[i]; };
 
-  if (lane == 0) {
+  if constexpr (kDeep) {
+    if (tie_mode == 0) {
+      if (lane == 0)
+        s_n = pyset_union_order(PySetIndexedKeys{reinterpret_cast<const int64_t*>(bid), limit}, nb, ns, t16, cs,
+                                t16 + cs, cs, t16 + 2 * cs, cu, t16 + 2 * cs + cu, cu, order);
+    } else {
+      // ascending-id union: member e of bid[0..nb) ++ sid[0..ns) is kept when no earlier member has its id, and
+      // lands at the number of kept members with a smaller id
+      unsigned char* kept = reinterpret_cast<unsigned char*>(t16);
+      const int m = nb + ns;
+      auto member = [&](int e) -> int64_t { return e < nb ? bid[e] : sid[e - nb]; };
+      for (int e = lane; e < m; e += kThreads) {
+        const int64_t v = member(e);
+        bool first = true;
+        for (int j = 0; j < e && first; ++j) first = member(j) != v;
+        kept[e] = first;
+      }
+      __syncthreads();
+      int mine = 0;
+      for (int e = lane; e < m; e += kThreads) {
+        if (!kept[e]) continue;
+        const int64_t v = member(e);
+        int pos = 0;
+        for (int j = 0; j < m; ++j) pos += kept[j] && member(j) < v;
+        order[pos] = v;
+        ++mine;
+      }
+      if (mine) atomicAdd(&s_n, mine);
+    }
+  } else if (lane == 0) {
     int n;
     if (tie_mode == 0) {
       n = pyset_union_order(reinterpret_cast<const int64_t*>(bid), nb, reinterpret_cast<const int64_t*>(sid), ns,
@@ -111,9 +180,9 @@ fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int
     }
     s_n = n;
   }
-  __syncwarp();
+  fuse_sync<kThreads>();
   const int n = s_n;
-  if (n < 0) {   // cannot happen within kFuseMaxLimit; keep the failure visible
+  if (n < 0) {   // cannot happen within kMaxLimit; keep the failure visible
     if (lane == 0) out_count[q] = -1;
     return;
   }
@@ -129,7 +198,7 @@ fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int
   }
 
   // ---- score every union member -------------------------------------------
-  for (int i = lane; i < n; i += 32) {
+  for (int i = lane; i < n; i += kThreads) {
     const int64_t id = order[i];
     int rb = -1, rs = -1;
     for (int j = 0; j < nb; ++j) if (bid[j] == id) rb = j;      // dict: last assignment wins
@@ -152,11 +221,11 @@ fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int
     }
     score[i] = s; va[i] = a; vb[i] = b;
   }
-  __syncwarp();
+  fuse_sync<kThreads>();
 
   // ---- stable descending sort by rank counting, then [:out_w] ---------------
   const int n_out = n < out_w ? n : out_w;
-  for (int i = lane; i < n; i += 32) {
+  for (int i = lane; i < n; i += kThreads) {
     const double si = score[i];
     int rank = 0;
     for (int j = 0; j < n; ++j) {
@@ -168,7 +237,7 @@ fuse_kernel(FuseIn in, int nq, int limit, int out_w, int mode, double param, int
       out_id[o] = order[i]; out_score[o] = si; out_a[o] = va[i]; out_b[o] = vb[i];
     }
   }
-  for (int i = n_out + lane; i < out_w; i += 32) {
+  for (int i = n_out + lane; i < out_w; i += kThreads) {
     const int64_t o = static_cast<int64_t>(q) * out_w + i;
     out_id[o] = -1; out_score[o] = 0.0; out_a[o] = -1.0; out_b[o] = -1.0;
   }

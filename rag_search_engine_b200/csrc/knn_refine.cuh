@@ -23,31 +23,6 @@ namespace rse {
 // (knn_tc3, unit-norm operands) instead of dot~/|a| (knn_tc / knn_tc2), so the band is not scaled by |q|.
 // smem: kRefineSmemBytes = 80 KB (the pairs, cap * 8 <= 64 KB; later the row staging area, or the keys of the slow
 // path) + 8 KB (keys of the fast path).
-// 256 threads, 256 histogram bins (one per thread): the digit d with  sum(hist[0..d-1]) < need <= sum(hist[0..d]).
-// The thread that owns d writes *out_digit = d and *out_before = sum(hist[0..d-1]); *out_digit stays 256 when
-// the histogram holds fewer than `need` entries.  s_warp: 8 words of scratch.  Ends with a barrier.
-__device__ __forceinline__ void block_pick_digit(const unsigned int* s_hist, unsigned int need, unsigned int* s_warp,
-                                                 unsigned int* out_digit, unsigned int* out_before) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const unsigned int c = s_hist[threadIdx.x];
-  unsigned int incl = c;
-#pragma unroll
-  for (int off = 1; off < 32; off <<= 1) {
-    const unsigned int o = __shfl_up_sync(0xFFFFFFFFu, incl, off);
-    if (lane >= off) incl += o;
-  }
-  if (lane == 31) s_warp[warp] = incl;
-  if (threadIdx.x == 0) *out_digit = 256u;
-  __syncthreads();
-  unsigned int base = 0u;
-#pragma unroll
-  for (int w = 0; w < 8; ++w) base += (w < warp) ? s_warp[w] : 0u;
-  incl += base;
-  if (incl >= need && incl - c < need) { *out_digit = threadIdx.x; *out_before = incl - c; }
-  __syncthreads();
-}
-
-
 // 16-byte asynchronous copy global -> shared, L2 only (the staged rows are read once)
 __device__ __forceinline__ void cp_async16_cg(uint32_t smem_dst, const void* gmem_src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gmem_src) : "memory");

@@ -1482,6 +1482,7 @@ int rse_load_bm25(rse_index* h, const int64_t* indptr, const uint32_t* doc_idx, 
   h->stats.bm25_docs = n_docs;
   if (!(h->attr_mask & (1u << 14))) {
     CK(cudaFuncSetAttribute(bm25_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBmRange * 9));
+    CK(cudaFuncSetAttribute(bm25_deep_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBmRange * 9));
     CK(cudaFuncSetAttribute(bm25_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bs_smem_bytes()));
     CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, fx_smem_bytes(kBsMaxRpg)));
     CK(cudaFuncSetAttribute(bm25_fx_kernel<kBsThreads>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -1553,7 +1554,7 @@ int bm25_stage(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows
 // h->b_score / b_doc / b_count ([nq][k]).
 int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
   if (!h->indptr) return fail(h, RSE_ERR_STATE, "rse_bm25: no BM25 index loaded");
-  if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 256]");
+  if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 512]");
   ENSURE(h->b_score, sizeof(double) * static_cast<size_t>(nq) * k);
   ENSURE(h->b_doc, sizeof(int) * static_cast<size_t>(nq) * k);
   ENSURE(h->b_count, sizeof(int) * nq);
@@ -1564,7 +1565,14 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
     LAUNCHED(h);
     h->normk_k1 = k1; h->normk_b = b;
   }
-  const int chunk = 4096;
+  // Queries per launch.  Above kBmGeneralMaxK the per-range candidate lists (16 B per candidate, nr * k per query:
+  // 688 KB at k = 512 over the 84 ranges of 600 k documents, 16 MB over 2048 ranges) are held within 256 MB by
+  // scoring the batch in chunks: 390 queries at k = 512 on 600 k documents, so a 256-query batch is one launch.
+  constexpr size_t kDeepCandBudget = size_t(256) << 20;
+  const bool deep = k > kBmGeneralMaxK;
+  const int chunk = deep ? static_cast<int>(std::max<size_t>(1, std::min<size_t>(4096, kDeepCandBudget /
+                                                             (static_cast<size_t>(h->nr) * k * 16))))
+                         : 4096;
   const size_t per_q = static_cast<size_t>(h->nr) * k;
   ENSURE(h->b_chi, sizeof(unsigned long long) * per_q * std::min(nq, chunk));
   ENSURE(h->b_clo, sizeof(unsigned long long) * per_q * std::min(nq, chunk));
@@ -1688,9 +1696,14 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
       LAUNCHED(h);
     }
     dim3 grid(h->nr, stream ? std::min(nc, 16) : nc);
-    bm25_score_kernel<<<grid, kBmThreads, kBmRange * 9, h->stream>>>(
-        h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, static_cast<const int32_t*>(h->b_tokptr.p),
-        static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, k1p1, chi, clo, ccnt, flagged);
+    if (deep)
+      bm25_deep_score_kernel<<<grid, kBmThreads, kBmRange * 9, h->stream>>>(
+          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, static_cast<const int32_t*>(h->b_tokptr.p),
+          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, k1p1, chi, clo, ccnt);
+    else
+      bm25_score_kernel<<<grid, kBmThreads, kBmRange * 9, h->stream>>>(
+          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, static_cast<const int32_t*>(h->b_tokptr.p),
+          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, k1p1, chi, clo, ccnt, flagged);
     LAUNCHED(h);
     bm25_merge_kernel<<<nc, kBmThreads, 0, h->stream>>>(chi, clo, ccnt, h->nr, q0, k, static_cast<double*>(h->b_score.p),
                                                         static_cast<int*>(h->b_doc.p), static_cast<int*>(h->b_count.p),
@@ -1701,7 +1714,7 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
 }
 
 int bm25_device(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows, int nq, int k, double k1, double b) {
-  if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 256]");
+  if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 512]");
   int rc = bm25_stage(h, tok_indptr, term_rows, nq);
   if (rc != RSE_OK) return rc;
   return bm25_run(h, nq, k, k1, b);
@@ -1747,15 +1760,27 @@ namespace {
 // inputs [nq, limit]; outputs [nq, out_w] (fuse_kernel: limit <= out_w <= 2 * limit)
 int fuse_launch(rse_index* h, int mode, double param, int tie_mode, int nq, int limit, int out_w, const FuseIn& in,
                 long long* o_id, double* o_sc, double* o_a, double* o_b, int* o_cnt) {
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "fusion: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "fusion: limit must be in [1, 1024]");
   if (tie_mode != RSE_TIE_REFERENCE && tie_mode != RSE_TIE_BY_ID) return fail(h, RSE_ERR_INVALID, "fusion: bad tie_mode");
+  if (limit > kFuseMaxLimit) {
+    if (!(h->attr_mask & (1u << 16))) {
+      CK(cudaFuncSetAttribute(fuse_kernel<kFuseDeepLimit>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              static_cast<int>(fuse_deep_smem_bytes(kFuseDeepLimit))));
+      h->attr_mask |= 1u << 16;
+    }
+    fuse_kernel<kFuseDeepLimit><<<nq, kFuseDeepThreads, fuse_deep_smem_bytes(limit), h->stream>>>(
+        in, nq, limit, out_w, mode, param, tie_mode, o_id, o_sc, o_a, o_b, o_cnt);
+    LAUNCHED(h);
+    return RSE_OK;
+  }
   const size_t smem = fuse_smem_bytes(limit);
   if (smem > 48 * 1024 && !(h->attr_mask & (1u << 15))) {     // per handle: the attribute is per device (ADVICE r01)
-    CK(cudaFuncSetAttribute(fuse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            static_cast<int>(fuse_smem_bytes(RSE_MAX_FUSE_LIMIT))));
+    CK(cudaFuncSetAttribute(fuse_kernel<kFuseMaxLimit>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            static_cast<int>(fuse_smem_bytes(kFuseMaxLimit))));
     h->attr_mask |= 1u << 15;
   }
-  fuse_kernel<<<nq, 32, smem, h->stream>>>(in, nq, limit, out_w, mode, param, tie_mode, o_id, o_sc, o_a, o_b, o_cnt);
+  fuse_kernel<kFuseMaxLimit><<<nq, 32, smem, h->stream>>>(in, nq, limit, out_w, mode, param, tie_mode, o_id, o_sc, o_a,
+                                                          o_b, o_cnt);
   LAUNCHED(h);
   return RSE_OK;
 }
@@ -1768,7 +1793,7 @@ int fuse_host(rse_index* h, int mode, double param, int tie_mode, int nq, int li
                             !out_score || !out_a || !out_b || !out_count)))
     return fail(h, RSE_ERR_INVALID, "fusion: bad arguments");
   if (nq == 0) return RSE_OK;
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "fusion: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "fusion: limit must be in [1, 1024]");
   CK(cudaSetDevice(h->device));
   const size_t n = static_cast<size_t>(nq) * limit;
   ENSURE(h->f_bid, 8 * n); ENSURE(h->f_bsc, 8 * n); ENSURE(h->f_bcnt, 4 * static_cast<size_t>(nq));
@@ -1880,7 +1905,7 @@ int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limi
   const int nq = h->staged_nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
   if (mode != 0 && mode != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid: mode must be 0 (rrf) or 1 (weighted)");
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
   if (knn_multiplier < 0) return fail(h, RSE_ERR_INVALID, "rse_hybrid: knn_multiplier < 0");
   CK(cudaSetDevice(h->device));
   const int kprime = std::max(limit * knn_multiplier, limit);   // semantic_search.py:251
@@ -1957,7 +1982,7 @@ int rse_hybrid_run(rse_index* h, int32_t mode, double param, int32_t tie_mode, i
   if (!h) return RSE_ERR_INVALID;
   const int nq = h->staged_nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
   const size_t n = static_cast<size_t>(nq) * limit;
   // the five result arrays live back to back in one buffer, so rse_hybrid_fetch is ONE device-to-host copy into
   // pinned memory (five copies into pageable caller buffers were five synchronous staging round trips)
@@ -2029,7 +2054,7 @@ int rse_hybrid_submit(rse_index* h, int32_t mode, double param, int32_t tie_mode
                       double b, int64_t* ticket) {
   if (!h) return RSE_ERR_INVALID;
   if (!ticket || nq < 1 || !q_host || !tok_indptr) return fail(h, RSE_ERR_INVALID, "rse_hybrid_submit: bad arguments");
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
   if (h->next_ticket - h->next_collect >= 2)
     return fail(h, RSE_ERR_STATE, "rse_hybrid_submit: two batches already in flight, collect one first");
   CK(cudaSetDevice(h->device));
@@ -2913,7 +2938,7 @@ int rse_hybrid_rerank_run(rse_index* h, int32_t slot, double k, int32_t tie_mode
                           int32_t activation) {
   if (!h) return RSE_ERR_INVALID;
   h->rr_nq = 0;
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_RERANK_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: limit must be in [1, 128]");
   if (activation != 0 && activation != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: activation must be 0 (logit) or 1 (sigmoid)");
   if (h->rr_n_docs < 1) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: no document store (rse_rerank_docs_load)");
   const int nq = h->staged_nq;
@@ -3258,7 +3283,7 @@ int rse_hybrid_sharded_run_dev(rse_index* h, int32_t mode, double param, int32_t
   if (!q_all_dev || nq_all < 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid_sharded_run_dev: bad arguments");
   if (!h->comm) return fail(h, RSE_ERR_STATE, "no communicator: call rse_comm_init first");
   if (mode != 0 && mode != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid: mode must be 0 (rrf) or 1 (weighted)");
-  if (limit < 1 || limit > RSE_MAX_FUSE_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 128]");
+  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
   if (knn_multiplier < 0) return fail(h, RSE_ERR_INVALID, "rse_hybrid: knn_multiplier < 0");
   if (!h->emb || !h->movie_idx || !h->indptr || !h->doc_ids || !h->movie_ids)
     return fail(h, RSE_ERR_STATE, "rse_hybrid: needs embeddings (with movie_idx), a BM25 index and id tables");

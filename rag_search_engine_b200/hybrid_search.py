@@ -85,14 +85,14 @@ class HybridSearch:
 
     # ---------------- fusion on the device ---------------- #
     def _fuse_inputs(self, bm25_hits, sem_hits, limit):
-        L = max(1, min(limit, _lib.RSE_MAX_FUSE_LIMIT))
-        if limit > _lib.RSE_MAX_FUSE_LIMIT:
-            raise ValueError(f"limit {limit} exceeds the fusion kernel's limit of {_lib.RSE_MAX_FUSE_LIMIT}")
+        L = max(1, min(limit, _lib.RSE_MAX_HYBRID_LIMIT))
+        if limit > _lib.RSE_MAX_HYBRID_LIMIT:
+            raise ValueError(f"limit {limit} exceeds the hybrid limit of {_lib.RSE_MAX_HYBRID_LIMIT}")
         # the retrievers are asked for k=limit; a plugged-in retriever may return more — the reference
         # would fuse all of them, so size the device call to what actually came back
         L = max(L, len(bm25_hits), len(sem_hits))
         if L > _lib.RSE_MAX_FUSE_LIMIT:
-            raise ValueError("retriever returned more hits than the fusion kernel supports (128)")
+            raise ValueError(f"retriever returned more hits than the fusion kernel supports ({_lib.RSE_MAX_FUSE_LIMIT})")
         bid = np.full((1, L), -1, np.int64); bsc = np.zeros((1, L)); sid = np.full((1, L), -1, np.int64)
         sds = np.zeros((1, L))
         for j, h in enumerate(bm25_hits):
@@ -136,7 +136,7 @@ class HybridSearch:
                 pad = lambda a, fill: np.concatenate([a, np.full((1, Lout - L), fill, a.dtype)], 1)  # noqa: E731
                 bid, bsc, sid, sds = pad(bid, -1), pad(bsc, 0.0), pad(sid, -1), pad(sds, 0.0)
             if n_union > _lib.RSE_MAX_FUSE_LIMIT:
-                raise ValueError("union of retriever hits exceeds the fusion kernel's limit (128)")
+                raise ValueError(f"union of retriever hits exceeds the fusion kernel's limit ({_lib.RSE_MAX_FUSE_LIMIT})")
             oid, osc, orb, ors, oc = self._index.fuse_rrf(Lout, k, bid, bsc, bc, sid, sds, sc, tie_mode=self.tie_mode)
             bm25_meta = {int(h["id"]): h for h in bm25_hits}
             sem_meta = {int(h["movie_id"]): h for h in sem_hits}
