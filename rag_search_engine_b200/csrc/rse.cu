@@ -36,6 +36,29 @@ struct DevBuf {
   size_t bytes = 0;
 };
 
+// the device inputs of one hybrid batch: query vectors and the BM25 tokens bm25_stage derives (token pointer, term
+// rows, idf)
+struct Batch {
+  DevBuf q, tokptr, terms, idf;
+  int nq = 0;
+};
+
+// pinned host landing buffer of the tensor-core path's per-query overflow flags
+struct PinnedFlags {
+  int* p = nullptr;
+  size_t n = 0;
+};
+
+// what knn_local_begin leaves for knn_local_finish.  flags != nullptr: the tensor-core path ran, its per-query
+// overflow flags are in tc_status and on their way into pinned memory (ready at ev)
+struct PendingKnn {
+  const float* q = nullptr;
+  int nq = 0, kprime = 0;
+  long long* cand = nullptr;
+  const int* flags = nullptr;
+  cudaEvent_t ev = nullptr;
+};
+
 // ---- §8(f2)/(f3): a BERT-family encoder resident next to the index (encoder.cuh)
 struct EncLayer {
   float *wqkv = nullptr, *bqkv = nullptr, *wo = nullptr, *bo = nullptr, *ln1g = nullptr, *ln1b = nullptr;
@@ -92,24 +115,19 @@ struct rse_index {
   std::vector<cudaEvent_t> scan_ev;   // 2 per timed launch
   size_t scan_ev_used = 0;
   std::vector<int> scan_ev_passes;    // K4: how many 256-query passes each timed filter launch covered (else 1)
-  // staged hybrid query batch (rse_hybrid_stage)
-  int staged_nq = 0;
+  // staged hybrid query batch (rse_hybrid_stage); rse_knn and rse_bm25 upload their inputs into its buffers too
+  Batch staged;
   // rse_hybrid_stash: staged batches parked in HBM (a bench / server rotating over several resident batches)
-  struct Stash { DevBuf q_dev, b_tokptr, b_terms, b_idf; int nq = 0; } stash[RSE_MAX_STASH];
+  Batch stash[RSE_MAX_STASH];
   // K4 tensor-core path
   int tc_mode = 0;                 // 0 auto, 1 off (exact scan only), 2 force on
   int survivor_div = 5;            // probe sample density: expected first-pass survivors ~ cap / survivor_div (RSE_TC_SURVIVOR_DIV).
                                    // r02 sweep, ms per 256-query step, isotropic / clustered / dense-clustered S-600k:
                                    // 3: 1.155 / 1.460 / 2.336   5: 1.146 / 1.223 / 1.785   8: 1.174 / 1.240 / 1.454
-  // pending tensor-core batch (knn_local_begin / knn_local_finish)
-  bool knn_pending = false;
   // rse_set_defer_flags: rse_knn_local_dev does not wait for the tensor-core path's overflow flags; they stay on
   // the device (tc_status) and rse_knn_flags_dev adds their count into a caller-owned device counter
   bool defer_flags_dev = false;
   int last_flags_n = 0;
-  const float* pend_q = nullptr;
-  int pend_nq = 0, pend_kprime = 0;
-  long long* pend_cand = nullptr;
   DevBuf f_pack;                   // rse_hybrid_run results: id | score | a | b | count, back to back
   size_t pack_n = 0;
   int pack_nq = 0;
@@ -122,20 +140,19 @@ struct rse_index {
     char* pin = nullptr; size_t bytes = 0; cudaEvent_t ev = nullptr;
     size_t n = 0; int nq = 0; long long ticket = -1;
     // the tensor-core path's per-query overflow flags are NOT waited for by submit (that wait is what would keep
-    // the host one KNN stage behind the device): they land here and collect checks them; a batch with a flagged
-    // query (rare: a mass tie at the K'-th distance) is re-run through the blocking call from the copies below
-    int* pin_status = nullptr; size_t pin_status_n = 0; bool deferred = false;
+    // the host one KNN stage behind the device): they land in `flags` and `knn` keeps them for collect; a batch with
+    // a flagged query (rare: a mass tie at the K'-th distance) is re-run through the blocking call from the copies below
+    PinnedFlags flags;
+    PendingKnn knn;
     std::vector<int32_t> tok_indptr, term_rows;
     int mode = 0, tie_mode = 0, limit = 0, knn_multiplier = 0; double param = 0.0, k1 = 0.0, b = 0.0;
-    // the slot's own device copies of the staged inputs and of the packed results, swapped into the handle around
-    // stage + run: batch i+1's uploads (copy stream) overlap batch i's kernels, batch i's result copy (third
-    // stream) overlaps batch i+1's first kernels — the main stream carries kernels only
-    DevBuf q_dev, b_tokptr, b_terms, b_idf, f_pack;
+    // the slot's own device inputs and packed results: batch i+1's uploads (copy stream) overlap batch i's kernels,
+    // batch i's result copy (third stream) overlaps batch i+1's first kernels — the main stream carries kernels only
+    Batch in;
+    DevBuf f_pack;
   } out_slot[2];
   cudaStream_t stream_h2d = nullptr, stream_d2h = nullptr;
   cudaEvent_t ev_fused = nullptr;
-  bool defer_status = false;       // set around the run of a submit
-  bool run_deferred = false;       // ... and whether that run left its flags unchecked
   long long pipeline_reruns = 0;
   long long next_ticket = 0, next_collect = 0;
   float* pin_q[2] = {nullptr, nullptr};   // pinned staging of the query vectors, alternating with the tickets
@@ -143,17 +160,13 @@ struct rse_index {
   cudaEvent_t ev_q[2] = {nullptr, nullptr};
   char* pin_stage = nullptr;       // pinned staging for the token / idf upload of a hybrid or BM25 batch
   size_t pin_stage_bytes = 0;
-  int* pin_status = nullptr;       // pinned host copy of the per-query overflow flags
-  size_t pin_status_n = 0;
+  PinnedFlags pin_status;          // pinned host copy of the per-query overflow flags
   cudaEvent_t ev_status = nullptr;
   cudaEvent_t ev_stage = nullptr;  // the uploads out of pin_stage have completed
   // hybrid step: BM25 runs on a second, lowest-priority stream UNDER the tensor-core filter pass (one BM25 CTA fits
-  // next to the filter's CTA on every SM); see hybrid_run_impl / knn_tc3_block
+  // next to the filter's CTA on every SM); see hybrid_local / knn_tc3_group
   cudaStream_t stream_b = nullptr;
   cudaEvent_t ev_prefilter = nullptr, ev_bm25_done = nullptr;
-  bool bm25_overlap_pending = false;
-  int ov_nq = 0, ov_limit = 0;
-  double ov_k1 = 0.0, ov_b = 0.0;
   // RSE_TIMELINE=1: timed events at the stage boundaries of a hybrid step on both streams, printed (ms since the
   // step's first event) to stderr by rse_hybrid_fetch — a development aid, off by default
   bool timeline = false;
@@ -189,7 +202,7 @@ struct rse_index {
   int32_t* movie_idx = nullptr;
 
   // ---- knn scratch (grow-only)
-  DevBuf q_dev, sb, sel, hist, selkeys, cand, dist, o_dist, o_pos, o_rowid, o_movie, o_count;
+  DevBuf sb, sel, hist, selkeys, cand, dist, o_dist, o_pos, o_rowid, o_movie, o_count;
   int64_t dist_ld = 0;
 
   // ---- a6: BM25
@@ -208,7 +221,7 @@ struct rse_index {
   DevBuf b_shi, b_slo, b_scnt, b_status, b_flagged;
   int bm25_mode = 0;               // 0 = fixed-point streaming kernel (default), 1 = exact-order streaming kernel, 2 = general kernel only
   std::vector<int64_t> df_host;
-  DevBuf b_tokptr, b_terms, b_idf, b_chi, b_clo, b_ccnt, b_score, b_doc, b_count;
+  DevBuf b_chi, b_clo, b_ccnt, b_score, b_doc, b_count;
 
   // ---- fusion scratch + id tables
   DevBuf f_bid, f_bsc, f_bcnt, f_sid, f_sds, f_scnt, f_oid, f_osc, f_oa, f_ob, f_ocnt;
@@ -300,6 +313,11 @@ template <typename T>
 void free_ptr(T*& p) {
   if (p) cudaFree(p);
   p = nullptr;
+}
+
+void free_batch(Batch& b) {
+  for (DevBuf* d : {&b.q, &b.tokptr, &b.terms, &b.idf}) free_buf(*d);
+  b.nq = 0;
 }
 
 void release_embeddings(rse_index* h) {
@@ -622,7 +640,18 @@ int sample_probe_rank(int kprime, int stride) {
   return kprime;
 }
 
-extern "C" int bm25_run_fwd(rse_index* h, int nq, int k, double k1, double b);   // = bm25_run (defined further down)
+// defined with the BM25 entry points further down, inside the ABI's extern "C" block
+extern "C" int bm25_run(rse_index* h, const Batch& in, int nq, int k, double k1, double b, cudaStream_t s,
+                        bool under_filter);
+
+// the BM25 batch a hybrid step hands to the KNN, to be enqueued underneath the tensor-core filter pass; `enqueued`
+// reports whether that happened (the exact path has no filter pass: the caller then runs it itself)
+struct Bm25Job {
+  const Batch* in;
+  int k;
+  double k1, b;
+  bool enqueued = false;
+};
 
 enum { kTlStart = 0, kTlPrefilter, kTlFilterEnd, kTlKnnEnd, kTlBm25Start, kTlBm25End, kTlStepEnd, kTlCount };
 
@@ -647,12 +676,11 @@ void tl_print(rse_index* h) {
   h->tl_set[kTlStart] = false;
 }
 
-// Enqueue the pending BM25 batch of a hybrid step on the second stream, ordered behind `after` (an event on the main
-// stream).  Called right after the filter kernel has been launched, so the filter's CTAs are placed first and BM25
-// fills what is left of every SM.
-int enqueue_bm25_overlapped(rse_index* h, cudaEvent_t after) {
-  if (!h->bm25_overlap_pending) return RSE_OK;
-  h->bm25_overlap_pending = false;
+// Enqueue the BM25 batch of a hybrid step on the second stream, ordered behind `after` (an event on the main stream).
+// Called right after the filter kernel has been launched, so the filter's CTAs are placed first and BM25 fills what
+// is left of every SM.
+int enqueue_bm25_overlapped(rse_index* h, Bm25Job& job, cudaEvent_t after) {
+  job.enqueued = true;
   if (!h->stream_b) {
     int lo = 0, hi = 0;
     CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));          // lo = numerically largest = lowest priority
@@ -661,10 +689,7 @@ int enqueue_bm25_overlapped(rse_index* h, cudaEvent_t after) {
   }
   CK(cudaStreamWaitEvent(h->stream_b, after, 0));
   tl_mark(h, kTlBm25Start, h->stream_b);
-  cudaStream_t main_stream = h->stream;
-  h->stream = h->stream_b;
-  const int rc = bm25_run_fwd(h, h->ov_nq, h->ov_limit, h->ov_k1, h->ov_b);
-  h->stream = main_stream;
+  const int rc = bm25_run(h, *job.in, job.in->nq, job.k, job.k1, job.b, h->stream_b, true);
   if (rc != RSE_OK) return rc;
   tl_mark(h, kTlBm25End, h->stream_b);
   CK(cudaEventRecord(h->ev_bm25_done, h->stream_b));
@@ -678,7 +703,7 @@ constexpr int kTcGroupBlocks = 8;                 // 2048 queries per group: 134
 
 template <int KB>
 int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, int kprime, long long* cand_dev,
-                  int* status_dev) {
+                  int* status_dev, Bm25Job* bm25) {
   constexpr int kT3SmemBytes = t3_smem_bytes(KB);
   if (!(h->attr_mask_tc & (1u << (KB - 1)))) {
     CK(cudaFuncSetAttribute(knn_tc3_kernel<0, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, kT3SmemBytes));
@@ -723,7 +748,7 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
     for (int b0 = 0; b0 < nqg; b0 += kTcBN) {
       const int nqb = std::min(kTcBN, nqg - b0);
       int rc = knn_tc3_group<KB>(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqb, kprime,
-                                 cand_dev + static_cast<int64_t>(b0) * kprime * 3, status_dev + b0);
+                                 cand_dev + static_cast<int64_t>(b0) * kprime * 3, status_dev + b0, bm25);
       if (rc != RSE_OK) return rc;
     }
     return RSE_OK;
@@ -788,7 +813,8 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
     int rc = scan_event(h, &e0);
     if (rc != RSE_OK) return rc;
   }
-  if (h->bm25_overlap_pending) {
+  const bool overlap = bm25 && !bm25->enqueued;
+  if (overlap) {
     if (!h->ev_prefilter) CK(cudaEventCreateWithFlags(&h->ev_prefilter, cudaEventDisableTiming));
     CK(cudaEventRecord(h->ev_prefilter, h->stream));
   }
@@ -798,8 +824,8 @@ int knn_tc3_group(rse_index* h, const float* q_dev, const double* sb, int nqg, i
       static_cast<unsigned int*>(h->tc_cnt.p), kTcCandCap, nullptr);
   LAUNCHED(h);
   tl_mark(h, kTlFilterEnd, h->stream);
-  {
-    int rc = enqueue_bm25_overlapped(h, h->ev_prefilter);     // no-op unless a hybrid step asked for it
+  if (overlap) {
+    int rc = enqueue_bm25_overlapped(h, *bm25, h->ev_prefilter);
     if (rc != RSE_OK) return rc;
   }
   if (e0) {
@@ -846,13 +872,13 @@ bool tc_eligible(const rse_index* h, int nq, int kprime) {
 // nothing when the corpus cannot use K4
 template <int KB>
 int knn_tc3_run(rse_index* h, const float* q_dev, const double* sb, int nq, int kprime, long long* cand_dev,
-                int* status) {
+                int* status, Bm25Job* bm25) {
   int rc = ensure_shadow<KB>(h);
   if (rc != RSE_OK || h->shadow_state < 0) return rc;
   for (int b0 = 0; b0 < nq; b0 += kTcGroupBlocks * kTcBN) {
     const int nqg = std::min(kTcGroupBlocks * kTcBN, nq - b0);
     rc = knn_tc3_group<KB>(h, q_dev + static_cast<int64_t>(b0) * h->dim, sb + b0, nqg, kprime,
-                           cand_dev + static_cast<int64_t>(b0) * kprime * 3, status + b0);
+                           cand_dev + static_cast<int64_t>(b0) * kprime * 3, status + b0, bm25);
     if (rc != RSE_OK) return rc;
   }
   return RSE_OK;
@@ -861,9 +887,11 @@ int knn_tc3_run(rse_index* h, const float* q_dev, const double* sb, int nq, int 
 // Local top-kprime for nq device-resident queries → packed candidates (device), in two halves: _begin enqueues
 // everything and, on the tensor-core path, an asynchronous read-back of the per-query overflow flags; _finish
 // waits for that read-back only (an event, not the stream) and re-runs flagged queries through the exact scan.
-// The hybrid step enqueues its BM25 kernels between the two, so the device never idles on the host round trip.
-int knn_local_begin(rse_index* h, const float* q_dev, int nq, int kprime, long long* cand_dev) {
-  h->knn_pending = false;
+// The hybrid step enqueues its BM25 kernels between the two, so the device never idles on the host round trip, and
+// hands `bm25` down to be enqueued underneath the filter pass when the tensor-core path runs.  The flags land in `pin`.
+int knn_local_begin(rse_index* h, const float* q_dev, int nq, int kprime, long long* cand_dev, PinnedFlags& pin,
+                    Bm25Job* bm25, PendingKnn& pend) {
+  pend = PendingKnn{};
   if (!h->emb) return fail(h, RSE_ERR_STATE, "rse_knn: no embeddings loaded");
   if (nq <= 0) return RSE_OK;
   if (kprime < 1 || kprime > RSE_MAX_KPRIME)
@@ -886,46 +914,41 @@ int knn_local_begin(rse_index* h, const float* q_dev, int nq, int kprime, long l
   {
     int rc = RSE_OK;
     switch (h->dim / kT3BK) {                      // tc_eligible: dim = 64 KB, KB = 1..8
-      case 1: rc = knn_tc3_run<1>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 2: rc = knn_tc3_run<2>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 3: rc = knn_tc3_run<3>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 4: rc = knn_tc3_run<4>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 5: rc = knn_tc3_run<5>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 6: rc = knn_tc3_run<6>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 7: rc = knn_tc3_run<7>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
-      case 8: rc = knn_tc3_run<8>(h, q_dev, sb, nq, kprime, cand_dev, status); break;
+      case 1: rc = knn_tc3_run<1>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 2: rc = knn_tc3_run<2>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 3: rc = knn_tc3_run<3>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 4: rc = knn_tc3_run<4>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 5: rc = knn_tc3_run<5>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 6: rc = knn_tc3_run<6>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 7: rc = knn_tc3_run<7>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
+      case 8: rc = knn_tc3_run<8>(h, q_dev, sb, nq, kprime, cand_dev, status, bm25); break;
       default: return fail(h, RSE_ERR_STATE, "rse_knn: no tensor-core instantiation for this width");
     }
     if (rc != RSE_OK) return rc;
     if (h->shadow_state < 0) return knn_exact_groups(h, q_dev, sb, nq, kprime, cand_dev);
   }
   h->stats.tc_queries += nq;
-  if (h->pin_status_n < static_cast<size_t>(nq)) {
-    if (h->pin_status) CK(cudaFreeHost(h->pin_status));
-    h->pin_status = nullptr; h->pin_status_n = 0;
-    CK(cudaMallocHost(reinterpret_cast<void**>(&h->pin_status), sizeof(int) * (static_cast<size_t>(nq) + 256)));
-    h->pin_status_n = static_cast<size_t>(nq) + 256;
+  if (pin.n < static_cast<size_t>(nq)) {
+    if (pin.p) CK(cudaFreeHost(pin.p));
+    pin = PinnedFlags{};
+    CK(cudaMallocHost(reinterpret_cast<void**>(&pin.p), sizeof(int) * (static_cast<size_t>(nq) + 256)));
+    pin.n = static_cast<size_t>(nq) + 256;
   }
   if (!h->ev_status) CK(cudaEventCreateWithFlags(&h->ev_status, cudaEventDisableTiming));
-  CK(cudaMemcpyAsync(h->pin_status, status, sizeof(int) * nq, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(pin.p, status, sizeof(int) * nq, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaEventRecord(h->ev_status, h->stream));
-  h->knn_pending = true;
-  h->pend_q = q_dev; h->pend_nq = nq; h->pend_kprime = kprime; h->pend_cand = cand_dev;
+  pend = PendingKnn{q_dev, nq, kprime, cand_dev, pin.p, h->ev_status};
   return RSE_OK;
 }
 
-int knn_local_finish(rse_index* h) {
-  if (!h->knn_pending) return RSE_OK;
-  h->knn_pending = false;
-  CK(cudaEventSynchronize(h->ev_status));
-  const float* q_dev = h->pend_q;
-  const int nq = h->pend_nq, kprime = h->pend_kprime;
-  long long* cand_dev = h->pend_cand;
+int knn_local_finish(rse_index* h, const PendingKnn& pend) {
+  if (!pend.flags) return RSE_OK;
+  CK(cudaEventSynchronize(pend.ev));
+  const int kprime = pend.kprime;
   const double* sb = static_cast<const double*>(h->sb.p);
-  const int* st = h->pin_status;
   std::vector<int> flagged;
-  for (int q = 0; q < nq; ++q)
-    if (st[q]) flagged.push_back(q);
+  for (int q = 0; q < pend.nq; ++q)
+    if (pend.flags[q]) flagged.push_back(q);
   if (flagged.empty()) return RSE_OK;
   // the flagged queries (a mass tie at the K'-th distance; second chance already tried) go through the exact scan,
   // gathered into one contiguous group: one pass serves up to 16 of them wherever they sat in the batch
@@ -937,22 +960,23 @@ int knn_local_finish(rse_index* h) {
   ENSURE(h->fb_cand, sizeof(long long) * static_cast<size_t>(nf) * kprime * 3);
   CK(cudaMemcpyAsync(h->fb_list.p, flagged.data(), sizeof(int) * nf, cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));                      // `flagged` is a pageable temporary
-  knn_gather_queries_kernel<<<nf, 128, 0, h->stream>>>(q_dev, sb, static_cast<const int*>(h->fb_list.p), h->dim,
+  knn_gather_queries_kernel<<<nf, 128, 0, h->stream>>>(pend.q, sb, static_cast<const int*>(h->fb_list.p), h->dim,
                                                       static_cast<float*>(h->fb_q.p), static_cast<double*>(h->fb_sb.p));
   LAUNCHED(h);
   int rc = knn_exact_groups(h, static_cast<const float*>(h->fb_q.p), static_cast<const double*>(h->fb_sb.p), nf, kprime,
                             static_cast<long long*>(h->fb_cand.p));
   if (rc != RSE_OK) return rc;
   knn_scatter_cand_kernel<<<nf, 128, 0, h->stream>>>(static_cast<const long long*>(h->fb_cand.p),
-                                                    static_cast<const int*>(h->fb_list.p), kprime * 3, cand_dev);
+                                                    static_cast<const int*>(h->fb_list.p), kprime * 3, pend.cand);
   LAUNCHED(h);
   return RSE_OK;
 }
 
 int knn_local(rse_index* h, const float* q_dev, int nq, int kprime, long long* cand_dev) {
-  int rc = knn_local_begin(h, q_dev, nq, kprime, cand_dev);
+  PendingKnn pend;
+  int rc = knn_local_begin(h, q_dev, nq, kprime, cand_dev, h->pin_status, nullptr, pend);
   if (rc != RSE_OK) return rc;
-  return knn_local_finish(h);
+  return knn_local_finish(h, pend);
 }
 
 int aggregate(rse_index* h, const long long* cand, int nq, int k, int kprime, float* o_dist, long long* o_rowid,
@@ -963,9 +987,23 @@ int aggregate(rse_index* h, const long long* cand, int nq, int k, int kprime, fl
   return RSE_OK;
 }
 
+// the n_lists candidate lists of K' per query gathered from the shards of one corpus → one merged list in h->cand
+int merge_candidates(rse_index* h, const long long* gathered, int n_lists, int nq, int kprime) {
+  const int n2 = next_pow2(n_lists * kprime);
+  const size_t smem = static_cast<size_t>(n2) * 12;
+  if (smem > 200 * 1024)
+    return fail(h, RSE_ERR_UNSUPPORTED, "knn merge: n_lists*kprime too large for the merge kernel");
+  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(knn_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(nq) * kprime * 3);
+  knn_merge_kernel<<<nq, kSelThreads, smem, h->stream>>>(gathered, n_lists, nq, kprime, n2,
+                                                         static_cast<long long*>(h->cand.p));
+  LAUNCHED(h);
+  return RSE_OK;
+}
+
 int upload_queries(rse_index* h, const float* q_host, int nq) {
-  ENSURE(h->q_dev, sizeof(float) * static_cast<size_t>(nq) * h->dim);
-  CK(cudaMemcpyAsync(h->q_dev.p, q_host, sizeof(float) * static_cast<size_t>(nq) * h->dim, cudaMemcpyHostToDevice,
+  ENSURE(h->staged.q, sizeof(float) * static_cast<size_t>(nq) * h->dim);
+  CK(cudaMemcpyAsync(h->staged.q.p, q_host, sizeof(float) * static_cast<size_t>(nq) * h->dim, cudaMemcpyHostToDevice,
                      h->stream));
   h->stats.h2d_bytes += static_cast<int64_t>(sizeof(float)) * nq * h->dim;
   return RSE_OK;
@@ -1056,29 +1094,30 @@ void rse_destroy(rse_index* h) {
     if (st) cudaStreamSynchronize(st);
   release_embeddings(h);
   release_bm25(h);
-  for (DevBuf* b : {&h->q_dev, &h->sb, &h->sel, &h->hist, &h->selkeys, &h->cand, &h->dist, &h->o_dist, &h->o_pos,
-                    &h->o_rowid, &h->o_movie, &h->o_count, &h->b_tokptr, &h->b_terms, &h->b_idf, &h->b_chi, &h->b_clo,
-                    &h->b_ccnt, &h->b_score, &h->b_doc, &h->b_count, &h->f_bid, &h->f_bsc, &h->f_bcnt, &h->f_sid,
-                    &h->f_sds, &h->f_scnt, &h->f_oid, &h->f_osc, &h->f_oa, &h->f_ob, &h->f_ocnt, &h->tc_thr,
+  for (DevBuf* b : {&h->sb, &h->sel, &h->hist, &h->selkeys, &h->cand, &h->dist, &h->o_dist, &h->o_pos, &h->o_rowid,
+                    &h->o_movie, &h->o_count, &h->b_chi, &h->b_clo, &h->b_ccnt, &h->b_score, &h->b_doc, &h->b_count,
+                    &h->f_bid, &h->f_bsc, &h->f_bcnt, &h->f_sid, &h->f_sds, &h->f_scnt, &h->f_oid, &h->f_osc, &h->f_oa,
+                    &h->f_ob, &h->f_ocnt, &h->tc_thr,
                     &h->tc_rows, &h->tc_cnt, &h->tc_status, &h->fb_list, &h->fb_q, &h->fb_sb, &h->fb_cand, &h->tc_q16, &h->b_shi, &h->b_slo, &h->b_scnt,
                     &h->b_status, &h->b_flagged})
     free_buf(*b);
-  if (h->pin_status) cudaFreeHost(h->pin_status);
+  if (h->pin_status.p) cudaFreeHost(h->pin_status.p);
   if (h->pin_stage) cudaFreeHost(h->pin_stage);
   if (h->pin_out) cudaFreeHost(h->pin_out);
   for (auto& sl : h->out_slot) {
     if (sl.pin) cudaFreeHost(sl.pin);
-    if (sl.pin_status) cudaFreeHost(sl.pin_status);
+    if (sl.flags.p) cudaFreeHost(sl.flags.p);
     if (sl.ev) cudaEventDestroy(sl.ev);
-    for (DevBuf* d : {&sl.q_dev, &sl.b_tokptr, &sl.b_terms, &sl.b_idf, &sl.f_pack}) if (d->p) cudaFree(d->p);
+    free_batch(sl.in);
+    free_buf(sl.f_pack);
   }
   if (h->stream_h2d) cudaStreamDestroy(h->stream_h2d);
   if (h->stream_d2h) cudaStreamDestroy(h->stream_d2h);
   if (h->ev_fused) cudaEventDestroy(h->ev_fused);
   for (int i = 0; i < 2; ++i) { if (h->pin_q[i]) cudaFreeHost(h->pin_q[i]); if (h->ev_q[i]) cudaEventDestroy(h->ev_q[i]); }
   free_buf(h->f_pack);
-  for (auto& st : h->stash)
-    for (DevBuf* d : {&st.q_dev, &st.b_tokptr, &st.b_terms, &st.b_idf}) free_buf(*d);
+  free_batch(h->staged);
+  for (Batch& st : h->stash) free_batch(st);
   if (h->ev_status) cudaEventDestroy(h->ev_status);
   if (h->ev_stage) cudaEventDestroy(h->ev_stage);
   for (cudaEvent_t e : h->tl) if (e) cudaEventDestroy(e);
@@ -1306,12 +1345,10 @@ int rse_knn_local_dev(rse_index* h, const float* q_dev, int32_t nq, int32_t kpri
   CK(cudaSetDevice(h->device));
   h->last_flags_n = 0;
   if (!h->defer_flags_dev) return knn_local(h, q_dev, nq, kprime, reinterpret_cast<long long*>(cand_dev));
-  int rc = knn_local_begin(h, q_dev, nq, kprime, reinterpret_cast<long long*>(cand_dev));
+  PendingKnn pend;
+  int rc = knn_local_begin(h, q_dev, nq, kprime, reinterpret_cast<long long*>(cand_dev), h->pin_status, nullptr, pend);
   if (rc != RSE_OK) return rc;
-  if (h->knn_pending) {                  // tensor-core path: the flags are in tc_status; nobody waits for them here
-    h->knn_pending = false;
-    h->last_flags_n = nq;
-  }
+  if (pend.flags) h->last_flags_n = nq;  // tensor-core path: the flags are in tc_status; nobody waits for them here
   return RSE_OK;
 }
 
@@ -1349,7 +1386,7 @@ int rse_knn(rse_index* h, const float* q_host, int32_t nq, int32_t kprime, float
   ENSURE(h->o_rowid, sizeof(long long) * n);
   ENSURE(h->o_movie, sizeof(int) * n);
   ENSURE(h->o_count, sizeof(int) * nq);
-  rc = knn_local(h, static_cast<const float*>(h->q_dev.p), nq, kprime, static_cast<long long*>(h->cand.p));
+  rc = knn_local(h, static_cast<const float*>(h->staged.q.p), nq, kprime, static_cast<long long*>(h->cand.p));
   if (rc != RSE_OK) return rc;
   knn_unpack_kernel<<<nq, 128, 0, h->stream>>>(static_cast<const long long*>(h->cand.p), nq, kprime,
                                                static_cast<float*>(h->o_dist.p), static_cast<long long*>(h->o_pos.p),
@@ -1390,7 +1427,7 @@ int rse_knn_movies(rse_index* h, const float* q_host, int32_t nq, int32_t k, int
   ENSURE(h->o_rowid, sizeof(long long) * n);
   ENSURE(h->o_movie, sizeof(int) * n);
   ENSURE(h->o_count, sizeof(int) * nq);
-  rc = knn_local(h, static_cast<const float*>(h->q_dev.p), nq, kprime, static_cast<long long*>(h->cand.p));
+  rc = knn_local(h, static_cast<const float*>(h->staged.q.p), nq, kprime, static_cast<long long*>(h->cand.p));
   if (rc != RSE_OK) return rc;
   rc = aggregate(h, static_cast<const long long*>(h->cand.p), nq, k, kprime, static_cast<float*>(h->o_dist.p),
                  static_cast<long long*>(h->o_rowid.p), static_cast<int*>(h->o_movie.p),
@@ -1420,15 +1457,8 @@ int rse_knn_merge_movies_dev(rse_index* h, const int64_t* gathered_dev, int32_t 
     return fail(h, RSE_ERR_INVALID, "rse_knn_merge_movies_dev: bad arguments");
   if (nq == 0) return RSE_OK;
   CK(cudaSetDevice(h->device));
-  const int n2 = next_pow2(n_lists * kprime);
-  const size_t smem = static_cast<size_t>(n2) * 12;
-  if (smem > 200 * 1024)
-    return fail(h, RSE_ERR_UNSUPPORTED, "rse_knn_merge_movies_dev: n_lists*kprime too large for the merge kernel");
-  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(knn_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(nq) * kprime * 3);
-  knn_merge_kernel<<<nq, kSelThreads, smem, h->stream>>>(reinterpret_cast<const long long*>(gathered_dev), n_lists, nq,
-                                                         kprime, n2, static_cast<long long*>(h->cand.p));
-  LAUNCHED(h);
+  int rc = merge_candidates(h, reinterpret_cast<const long long*>(gathered_dev), n_lists, nq, kprime);
+  if (rc != RSE_OK) return rc;
   return aggregate(h, static_cast<const long long*>(h->cand.p), nq, k, kprime, out_dist_dev,
                    reinterpret_cast<long long*>(out_chunk_rowid_dev), out_movie_idx_dev, out_count_dev);
 }
@@ -1496,7 +1526,8 @@ int rse_load_bm25(rse_index* h, const int64_t* indptr, const uint32_t* doc_idx, 
 namespace {
 
 // tokens → device, with host-computed idf (keyword_search.py:224, same libm `log` as CPython).
-int bm25_stage(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows, int nq) {
+int bm25_stage(rse_index* h, Batch& in, const int32_t* tok_indptr, const int32_t* term_rows, int nq,
+               cudaStream_t s) {
   if (!h->indptr) return fail(h, RSE_ERR_STATE, "rse_bm25: no BM25 index loaded");
   const int64_t ntok = tok_indptr[nq];
   if (tok_indptr[0] != 0 || ntok < 0) return fail(h, RSE_ERR_INVALID, "rse_bm25: bad tok_indptr");
@@ -1510,7 +1541,7 @@ int bm25_stage(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows
   if (!h->ev_stage) CK(cudaEventCreateWithFlags(&h->ev_stage, cudaEventDisableTiming));
   else CK(cudaEventSynchronize(h->ev_stage));               // the previous batch's uploads are out of the buffer
   if (h->pin_stage_bytes < need) {
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaStreamSynchronize(s));
     if (h->pin_stage) CK(cudaFreeHost(h->pin_stage));
     h->pin_stage = nullptr; h->pin_stage_bytes = 0;
     CK(cudaMallocHost(reinterpret_cast<void**>(&h->pin_stage), need + need / 2 + 4096));
@@ -1537,22 +1568,22 @@ int bm25_stage(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows
     }
   }
   std::memcpy(ptr, tok_indptr, bytes_ptr);
-  ENSURE(h->b_tokptr, sizeof(int32_t) * (nq + 1));
-  ENSURE(h->b_terms, sizeof(int32_t) * std::max<int64_t>(ntok, 1));
-  ENSURE(h->b_idf, sizeof(double) * std::max<int64_t>(ntok, 1));
-  CK(cudaMemcpyAsync(h->b_tokptr.p, ptr, bytes_ptr, cudaMemcpyHostToDevice, h->stream));
+  ENSURE(in.tokptr, sizeof(int32_t) * (nq + 1));
+  ENSURE(in.terms, sizeof(int32_t) * std::max<int64_t>(ntok, 1));
+  ENSURE(in.idf, sizeof(double) * std::max<int64_t>(ntok, 1));
+  CK(cudaMemcpyAsync(in.tokptr.p, ptr, bytes_ptr, cudaMemcpyHostToDevice, s));
   if (ntok > 0) {
-    CK(cudaMemcpyAsync(h->b_terms.p, terms, sizeof(int32_t) * ntok, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(h->b_idf.p, idf, sizeof(double) * ntok, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(in.terms.p, terms, sizeof(int32_t) * ntok, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(in.idf.p, idf, sizeof(double) * ntok, cudaMemcpyHostToDevice, s));
   }
-  CK(cudaEventRecord(h->ev_stage, h->stream));
+  CK(cudaEventRecord(h->ev_stage, s));
   h->stats.h2d_bytes += static_cast<int64_t>(bytes_ptr) + (ntok > 0 ? static_cast<int64_t>(ntok) * 12 : 0);
   return RSE_OK;
 }
 
-// scoring + top-k on the staged tokens; results stay on the device in
-// h->b_score / b_doc / b_count ([nq][k]).
-int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
+// scoring + top-k on the first nq queries of the staged tokens, on stream s; results stay on the device in
+// h->b_score / b_doc / b_count ([nq][k]).  under_filter: the batch shares the SMs with the tensor-core filter pass.
+int bm25_run(rse_index* h, const Batch& in, int nq, int k, double k1, double b, cudaStream_t s, bool under_filter) {
   if (!h->indptr) return fail(h, RSE_ERR_STATE, "rse_bm25: no BM25 index loaded");
   if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 512]");
   ENSURE(h->b_score, sizeof(double) * static_cast<size_t>(nq) * k);
@@ -1560,7 +1591,7 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
   ENSURE(h->b_count, sizeof(int) * nq);
   if (!(h->normk_k1 == k1 && h->normk_b == b) && h->n_docs > 0) {
     const int threads = 256;
-    bm25_norm_kernel<<<static_cast<unsigned int>((h->n_docs + threads - 1) / threads), threads, 0, h->stream>>>(
+    bm25_norm_kernel<<<static_cast<unsigned int>((h->n_docs + threads - 1) / threads), threads, 0, s>>>(
         h->dl, h->n_docs, k1, b, h->avgdl, h->normk);
     LAUNCHED(h);
     h->normk_k1 = k1; h->normk_b = b;
@@ -1578,6 +1609,9 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
   ENSURE(h->b_clo, sizeof(unsigned long long) * per_q * std::min(nq, chunk));
   ENSURE(h->b_ccnt, sizeof(int) * static_cast<size_t>(h->nr) * std::min(nq, chunk));
   const double k1p1 = k1 + 1.0;
+  const int32_t* tokptr = static_cast<const int32_t*>(in.tokptr.p);
+  const int32_t* terms = static_cast<const int32_t*>(in.terms.p);
+  const double* idf = static_cast<const double*>(in.idf.p);
 
   // streaming path (bm25_stream_kernel): k <= 32; needs the weighted postings of this (k1, b)
   const bool stream = k <= 32 && h->n_postings > 0 && h->bm25_mode != 2;
@@ -1606,7 +1640,7 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
       if (!h->post16) CK(cudaMalloc(&h->post16, sizeof(Post16) * static_cast<size_t>(h->n_postings)));
       if (wq4_scale > 0.0 && !h->post4) CK(cudaMalloc(&h->post4, sizeof(uint32_t) * (static_cast<size_t>(h->n_postings) + 8)));
       const int threads = 256;
-      bm25_weight_kernel<<<static_cast<unsigned int>((h->n_postings + threads - 1) / threads), threads, 0, h->stream>>>(
+      bm25_weight_kernel<<<static_cast<unsigned int>((h->n_postings + threads - 1) / threads), threads, 0, s>>>(
           h->post, h->normk, h->n_postings, k1p1, h->post16, wq4_scale > 0.0 ? h->post4 : nullptr, wq4_scale);
       LAUNCHED(h);
       h->w_k1 = k1; h->w_b = b;
@@ -1636,7 +1670,7 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
     ENSURE(h->b_scnt, sizeof(int) * static_cast<size_t>(ng) * std::min(nq, chunk));
     ENSURE(h->b_status, sizeof(int) * nq);
     ENSURE(h->b_flagged, sizeof(int) * (std::min(nq, chunk) + 1));
-    CK(cudaMemsetAsync(h->b_status.p, 0, sizeof(int) * nq, h->stream));
+    CK(cudaMemsetAsync(h->b_status.p, 0, sizeof(int) * nq, s));
   }
   h->stats.bm25_queries += nq;
   for (int q0 = 0; q0 < nq; q0 += chunk) {
@@ -1658,17 +1692,13 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
       // filter's CTA).  Alone the 512-thread shape is the faster one (4 CTAs per SM: 284 against 318 us).  Splitting
       // the groups between the two shapes loses (r02, 25 / 40 / 60 / 100 % wide -> 1.064 / 1.071 / 1.087 / 1.050 ms
       // per step): a second launch waits for the first.
-      const bool under_filter = h->stream_b && h->stream == h->stream_b;
       const int threads = under_filter ? kBsWideThreads : kBsThreads;
       const auto kernel = under_filter ? bm25_fx_kernel<kBsWideThreads> : bm25_fx_kernel<kBsThreads>;
-      kernel<<<dim3(nc, ng), threads, fx_smem_bytes(rpg), h->stream>>>(
-          h->indptr, h->post4, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
-          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), idfx_scale, q0, k, rpg,
-          ng, fin, fcnt, status);
+      kernel<<<dim3(nc, ng), threads, fx_smem_bytes(rpg), s>>>(h->indptr, h->post4, h->roff, h->nr, tokptr, terms, idf,
+                                                               idfx_scale, q0, k, rpg, ng, fin, fcnt, status);
       LAUNCHED(h);
-      bm25_fx_finish_kernel<<<nc, kBmThreads, 0, h->stream>>>(
-          fin, fcnt, ng, status, h->indptr, h->post16, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
-          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k,
+      bm25_fx_finish_kernel<<<nc, kBmThreads, 0, s>>>(
+          fin, fcnt, ng, status, h->indptr, h->post16, h->roff, h->nr, tokptr, terms, idf, q0, k,
           static_cast<double*>(h->b_score.p), static_cast<int*>(h->b_doc.p), static_cast<int*>(h->b_count.p),
           h->dev_counters, idfx_scale);
       LAUNCHED(h);
@@ -1681,10 +1711,8 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
       scnt = static_cast<int*>(h->b_scnt.p) - static_cast<int64_t>(q0) * ng;
       status = static_cast<int*>(h->b_status.p);
       dim3 sgrid(ng, nc);
-      bm25_stream_kernel<<<sgrid, kBsThreads, bs_smem_bytes(), h->stream>>>(
-          h->indptr, h->post16, h->roff, h->nr, static_cast<const int32_t*>(h->b_tokptr.p),
-          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, rpg, ng, shi, slo, scnt,
-          status);
+      bm25_stream_kernel<<<sgrid, kBsThreads, bs_smem_bytes(), s>>>(h->indptr, h->post16, h->roff, h->nr, tokptr, terms,
+                                                                    idf, q0, k, rpg, ng, shi, slo, scnt, status);
       LAUNCHED(h);
     }
     // general kernel: every query when the streaming path does not apply, else only the flagged ones
@@ -1692,22 +1720,21 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
     int* flagged = nullptr;
     if (stream) {
       flagged = static_cast<int*>(h->b_flagged.p);
-      bm25_flag_compact_kernel<<<1, 256, 0, h->stream>>>(status, q0, nc, flagged, h->dev_counters);
+      bm25_flag_compact_kernel<<<1, 256, 0, s>>>(status, q0, nc, flagged, h->dev_counters);
       LAUNCHED(h);
     }
     dim3 grid(h->nr, stream ? std::min(nc, 16) : nc);
     if (deep)
-      bm25_deep_score_kernel<<<grid, kBmThreads, kBmRange * 9, h->stream>>>(
-          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, static_cast<const int32_t*>(h->b_tokptr.p),
-          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, k1p1, chi, clo, ccnt);
+      bm25_deep_score_kernel<<<grid, kBmThreads, kBmRange * 9, s>>>(
+          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, tokptr, terms, idf, q0, k, k1p1, chi, clo, ccnt);
     else
-      bm25_score_kernel<<<grid, kBmThreads, kBmRange * 9, h->stream>>>(
-          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, static_cast<const int32_t*>(h->b_tokptr.p),
-          static_cast<const int32_t*>(h->b_terms.p), static_cast<const double*>(h->b_idf.p), q0, k, k1p1, chi, clo, ccnt, flagged);
+      bm25_score_kernel<<<grid, kBmThreads, kBmRange * 9, s>>>(
+          h->indptr, h->post, h->roff, h->normk, h->nr, h->n_docs, tokptr, terms, idf, q0, k, k1p1, chi, clo, ccnt,
+          flagged);
     LAUNCHED(h);
-    bm25_merge_kernel<<<nc, kBmThreads, 0, h->stream>>>(chi, clo, ccnt, h->nr, q0, k, static_cast<double*>(h->b_score.p),
-                                                        static_cast<int*>(h->b_doc.p), static_cast<int*>(h->b_count.p),
-                                                        shi, slo, scnt, ng, status);
+    bm25_merge_kernel<<<nc, kBmThreads, 0, s>>>(chi, clo, ccnt, h->nr, q0, k, static_cast<double*>(h->b_score.p),
+                                                static_cast<int*>(h->b_doc.p), static_cast<int*>(h->b_count.p), shi, slo,
+                                                scnt, ng, status);
     LAUNCHED(h);
   }
   return RSE_OK;
@@ -1715,18 +1742,12 @@ int bm25_run(rse_index* h, int nq, int k, double k1, double b) {
 
 int bm25_device(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows, int nq, int k, double k1, double b) {
   if (k < 1 || k > RSE_MAX_BM25_K) return fail(h, RSE_ERR_UNSUPPORTED, "rse_bm25: k must be in [1, 512]");
-  int rc = bm25_stage(h, tok_indptr, term_rows, nq);
+  int rc = bm25_stage(h, h->staged, tok_indptr, term_rows, nq, h->stream);
   if (rc != RSE_OK) return rc;
-  return bm25_run(h, nq, k, k1, b);
+  return bm25_run(h, h->staged, nq, k, k1, b, h->stream, false);
 }
 
 }  // namespace
-
-// internal trampoline (not part of the ABI in include/rse.h): lets the KNN code above enqueue a BM25 batch
-__attribute__((visibility("hidden"))) int bm25_run_fwd(rse_index* h, int nq, int k, double k1, double b) {
-  return bm25_run(h, nq, k, k1, b);
-}
-
 
 int rse_bm25(rse_index* h, const int32_t* tok_indptr, const int32_t* term_rows, int32_t nq, int32_t k, double k1,
              double b, double* out_score, int32_t* out_doc_idx, int32_t* out_count) {
@@ -1876,90 +1897,78 @@ int rse_set_id_tables(rse_index* h, const int64_t* doc_ids, int64_t n_docs, cons
   return RSE_OK;
 }
 
-int rse_hybrid_stage(rse_index* h, int32_t nq, const float* q_host, const int32_t* tok_indptr,
-                     const int32_t* term_rows) {
-  if (!h) return RSE_ERR_INVALID;
-  if (nq < 0 || (nq > 0 && (!q_host || !tok_indptr))) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage: bad arguments");
-  if (!h->emb || !h->movie_idx || !h->indptr || !h->doc_ids || !h->movie_ids)
-    return fail(h, RSE_ERR_STATE, "rse_hybrid: needs embeddings (with movie_idx), a BM25 index and id tables");
-  h->staged_nq = 0;
-  if (nq == 0) return RSE_OK;
-  if (tok_indptr[nq] > 0 && !term_rows) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage: term_rows is NULL");
-  CK(cudaSetDevice(h->device));
-  int rc = bm25_stage(h, tok_indptr, term_rows, nq);
-  if (rc != RSE_OK) return rc;
-  rc = upload_queries(h, q_host, nq);
-  if (rc != RSE_OK) return rc;
-  h->staged_nq = nq;
-  return RSE_OK;                      // asynchronous: rse_hybrid_run / _fetch (or rse_synchronize) order behind it
-}
-
 namespace {
 
-// BM25 + (local KNN | merge of gathered shard candidates) + aggregation + fusion on the staged batch.
-// Outputs go to the given device buffers ([nq, out_w]: out_w = limit is the reference's [:limit], 2 * limit the
-// whole fused union the cross-encoder rerank scores).
-int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limit, int knn_multiplier, double k1,
-                    double b, const long long* gathered, int n_lists, long long* o_id, double* o_sc, double* o_a,
-                    double* o_b, int* o_cnt, int out_w) {
-  const int nq = h->staged_nq;
-  if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
+int check_hybrid_state(rse_index* h) {
+  if (!h->emb || !h->movie_idx || !h->indptr || !h->doc_ids || !h->movie_ids)
+    return fail(h, RSE_ERR_STATE, "rse_hybrid: needs embeddings (with movie_idx), a BM25 index and id tables");
+  return RSE_OK;
+}
+
+// the arguments every hybrid entry point shares, and the state a step needs → K' (semantic_search.py:251), or an error
+int hybrid_kprime(rse_index* h, int mode, int limit, int knn_multiplier) {
   if (mode != 0 && mode != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid: mode must be 0 (rrf) or 1 (weighted)");
   if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
   if (knn_multiplier < 0) return fail(h, RSE_ERR_INVALID, "rse_hybrid: knn_multiplier < 0");
-  CK(cudaSetDevice(h->device));
-  const int kprime = std::max(limit * knn_multiplier, limit);   // semantic_search.py:251
+  const int kprime = std::max(limit * knn_multiplier, limit);
   if (kprime > RSE_MAX_KPRIME) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit*knn_multiplier exceeds 4096");
-  int rc = RSE_OK;
-  bool join_bm25 = false;
+  const int rc = check_hybrid_state(h);
+  return rc != RSE_OK ? rc : kprime;
+}
+
+// The inputs of one hybrid batch → `in`, on stream s: the tokens through bm25_stage, then the query vectors (`kind`:
+// from host or device memory).  `in` holds no batch unless this succeeds.
+int stage_batch(rse_index* h, Batch& in, int nq, const float* q, cudaMemcpyKind kind, const int32_t* tok_indptr,
+                const int32_t* term_rows, cudaStream_t s) {
+  int rc = check_hybrid_state(h);
+  if (rc != RSE_OK) return rc;
+  in.nq = 0;
+  if (nq == 0) return RSE_OK;
+  if (tok_indptr[nq] > 0 && !term_rows) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage: term_rows is NULL");
+  CK(cudaSetDevice(h->device));
+  rc = bm25_stage(h, in, tok_indptr, term_rows, nq, s);
+  if (rc != RSE_OK) return rc;
+  const size_t bytes = sizeof(float) * static_cast<size_t>(nq) * h->dim;
+  ENSURE(in.q, bytes);
+  CK(cudaMemcpyAsync(in.q.p, q, bytes, kind, s));
+  if (kind == cudaMemcpyHostToDevice) h->stats.h2d_bytes += static_cast<int64_t>(bytes);
+  in.nq = nq;
+  return RSE_OK;
+}
+
+// Where a hybrid step writes its results: [nq, w] each (w = limit is the reference's [:limit], 2 * limit the whole
+// fused union the cross-encoder rerank scores).
+struct Fused {
+  long long* id;
+  double *score, *a, *b;
+  int* count;
+  int w;
+};
+
+// the five result arrays back to back in one buffer, so rse_hybrid_fetch / _collect is ONE device-to-host copy into
+// pinned memory (five copies into pageable caller buffers were five synchronous staging round trips)
+int packed_results(rse_index* h, DevBuf& pack, int nq, int limit, Fused* out) {
   const size_t n = static_cast<size_t>(nq) * limit;
-  ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(nq) * kprime * 3);
+  ENSURE(pack, 32 * n + 4 * static_cast<size_t>(nq));
+  char* pk = static_cast<char*>(pack.p);
+  *out = Fused{reinterpret_cast<long long*>(pk), reinterpret_cast<double*>(pk + 8 * n),
+               reinterpret_cast<double*>(pk + 16 * n), reinterpret_cast<double*>(pk + 24 * n),
+               reinterpret_cast<int*>(pk + 32 * n), limit};
+  return RSE_OK;
+}
+
+// The end of every hybrid step, for nq queries whose BM25 lists are in b_score / b_doc / b_count: [merge of the
+// n_lists gathered shard lists into h->cand →] per-movie aggregation of the KNN candidates in h->cand → join of BM25
+// on the second stream (join_bm25) → fusion.
+int hybrid_tail(rse_index* h, int mode, double param, int tie_mode, int nq, int limit, int kprime,
+                const long long* gathered, int n_lists, bool join_bm25, const Fused& out) {
+  const size_t n = static_cast<size_t>(nq) * limit;
   ENSURE(h->o_dist, sizeof(float) * n);
   ENSURE(h->o_rowid, sizeof(long long) * n);
   ENSURE(h->o_movie, sizeof(int) * n);
   ENSURE(h->o_count, sizeof(int) * nq);
-  if (gathered) {
-    const int n2 = next_pow2(n_lists * kprime);
-    const size_t smem = static_cast<size_t>(n2) * 12;
-    if (smem > 200 * 1024)
-      return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_run_merged_dev: n_lists*kprime too large for the merge kernel");
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(knn_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    // BM25 (k = limit, hybrid_search.py:70), then the merge of the gathered KNN candidates
-    rc = bm25_run(h, nq, limit, k1, b);
-    if (rc != RSE_OK) return rc;
-    knn_merge_kernel<<<nq, kSelThreads, smem, h->stream>>>(gathered, n_lists, nq, kprime, n2,
-                                                           static_cast<long long*>(h->cand.p));
-    LAUNCHED(h);
-  } else {
-    // KNN (k = limit, hybrid_search.py:88) is enqueued first; BM25 (hybrid_search.py:70) goes in behind it while
-    // the tensor-core path's overflow flags travel back, so the host round trip costs the device nothing
-    // ... and when the KNN takes the tensor-core path, on a second stream UNDERNEATH the filter pass: the filter
-    // kernel keeps one 178 KB CTA per SM busy on the tensor pipe at ~20 % issue utilisation, and one BM25 CTA
-    // (38 KB, 512 threads) fits beside it.
-    tl_mark(h, kTlStart, h->stream);
-    h->bm25_overlap_pending = true;
-    h->ov_nq = nq; h->ov_limit = limit; h->ov_k1 = k1; h->ov_b = b;
-    rc = knn_local_begin(h, static_cast<const float*>(h->q_dev.p), nq, kprime, static_cast<long long*>(h->cand.p));
-    if (rc != RSE_OK) { h->bm25_overlap_pending = false; return rc; }
-    const bool overlapped = !h->bm25_overlap_pending;         // the filter launch consumed the request
-    h->bm25_overlap_pending = false;
-    if (!overlapped) {
-      tl_mark(h, kTlBm25Start, h->stream);
-      rc = bm25_run(h, nq, limit, k1, b);
-      if (rc != RSE_OK) return rc;
-      tl_mark(h, kTlBm25End, h->stream);
-    }
-    h->run_deferred = false;
-    if (h->defer_status && h->knn_pending) {                  // rse_hybrid_submit: flags are checked by collect
-      h->knn_pending = false;
-      h->run_deferred = true;
-    } else {
-      rc = knn_local_finish(h);
-      if (rc != RSE_OK) return rc;
-    }
-    tl_mark(h, kTlKnnEnd, h->stream);
-    join_bm25 = overlapped;
-  }
+  int rc = gathered ? merge_candidates(h, gathered, n_lists, nq, kprime) : RSE_OK;
+  if (rc != RSE_OK) return rc;
   rc = aggregate(h, static_cast<const long long*>(h->cand.p), nq, limit, kprime, static_cast<float*>(h->o_dist.p),
                  static_cast<long long*>(h->o_rowid.p), static_cast<int*>(h->o_movie.p), static_cast<int*>(h->o_count.p));
   if (rc != RSE_OK) return rc;
@@ -1970,29 +1979,68 @@ int hybrid_run_impl(rse_index* h, int mode, double param, int tie_mode, int limi
             static_cast<const float*>(h->o_dist.p), static_cast<const int*>(h->o_count.p), nullptr};
   in.bm25_idx = static_cast<const int*>(h->b_doc.p); in.bm25_table = h->doc_ids; in.bm25_table_n = h->n_doc_ids;
   in.sem_idx = static_cast<const int*>(h->o_movie.p); in.sem_table = h->movie_ids; in.sem_table_n = h->n_movie_ids;
-  rc = fuse_launch(h, mode, param, tie_mode, nq, limit, out_w, in, o_id, o_sc, o_a, o_b, o_cnt);
+  rc = fuse_launch(h, mode, param, tie_mode, nq, limit, out.w, in, out.id, out.score, out.a, out.b, out.count);
   tl_mark(h, kTlStepEnd, h->stream);
   return rc;
 }
 
+// BM25 + local KNN + aggregation + fusion on the batch `in`.  The tensor-core path's overflow flags land in `pin`;
+// with `keep` the flagged queries are left to the caller (rse_hybrid_submit: collect checks them), else they are
+// re-run through the exact scan before the aggregation.
+int hybrid_local(rse_index* h, int mode, double param, int tie_mode, int limit, int kprime, double k1, double b,
+                 const Batch& in, PinnedFlags& pin, PendingKnn* keep, const Fused& out) {
+  const int nq = in.nq;
+  ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(nq) * kprime * 3);
+  // KNN (k = limit, hybrid_search.py:88) is enqueued first; BM25 (hybrid_search.py:70) goes in behind it while
+  // the tensor-core path's overflow flags travel back, so the host round trip costs the device nothing
+  // ... and when the KNN takes the tensor-core path, on a second stream UNDERNEATH the filter pass: the filter
+  // kernel keeps one 178 KB CTA per SM busy on the tensor pipe at ~20 % issue utilisation, and one BM25 CTA
+  // (38 KB, 512 threads) fits beside it.
+  tl_mark(h, kTlStart, h->stream);
+  Bm25Job bm25{&in, limit, k1, b};
+  PendingKnn pend;
+  int rc = knn_local_begin(h, static_cast<const float*>(in.q.p), nq, kprime, static_cast<long long*>(h->cand.p), pin,
+                           &bm25, pend);
+  if (rc != RSE_OK) return rc;
+  if (!bm25.enqueued) {
+    tl_mark(h, kTlBm25Start, h->stream);
+    rc = bm25_run(h, in, nq, limit, k1, b, h->stream, false);
+    if (rc != RSE_OK) return rc;
+    tl_mark(h, kTlBm25End, h->stream);
+  }
+  if (keep) {
+    *keep = pend;
+  } else {
+    rc = knn_local_finish(h, pend);
+    if (rc != RSE_OK) return rc;
+  }
+  tl_mark(h, kTlKnnEnd, h->stream);
+  return hybrid_tail(h, mode, param, tie_mode, nq, limit, kprime, nullptr, 0, bm25.enqueued, out);
+}
+
 }  // namespace
+
+int rse_hybrid_stage(rse_index* h, int32_t nq, const float* q_host, const int32_t* tok_indptr,
+                     const int32_t* term_rows) {
+  if (!h) return RSE_ERR_INVALID;
+  if (nq < 0 || (nq > 0 && (!q_host || !tok_indptr))) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage: bad arguments");
+  // asynchronous: rse_hybrid_run / _fetch (or rse_synchronize) order behind it
+  return stage_batch(h, h->staged, nq, q_host, cudaMemcpyHostToDevice, tok_indptr, term_rows, h->stream);
+}
 
 int rse_hybrid_run(rse_index* h, int32_t mode, double param, int32_t tie_mode, int32_t limit, int32_t knn_multiplier,
                    double k1, double b) {
   if (!h) return RSE_ERR_INVALID;
-  const int nq = h->staged_nq;
+  const int nq = h->staged.nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
-  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
-  const size_t n = static_cast<size_t>(nq) * limit;
-  // the five result arrays live back to back in one buffer, so rse_hybrid_fetch is ONE device-to-host copy into
-  // pinned memory (five copies into pageable caller buffers were five synchronous staging round trips)
-  ENSURE(h->f_pack, 32 * n + 4 * static_cast<size_t>(nq));
-  char* pk = static_cast<char*>(h->f_pack.p);
-  h->pack_n = n; h->pack_nq = nq;
-  return hybrid_run_impl(h, mode, param, tie_mode, limit, knn_multiplier, k1, b, nullptr, 0,
-                         reinterpret_cast<long long*>(pk), reinterpret_cast<double*>(pk + 8 * n),
-                         reinterpret_cast<double*>(pk + 16 * n), reinterpret_cast<double*>(pk + 24 * n),
-                         reinterpret_cast<int*>(pk + 32 * n), limit);
+  const int kprime = hybrid_kprime(h, mode, limit, knn_multiplier);
+  if (kprime < 0) return kprime;
+  CK(cudaSetDevice(h->device));
+  Fused out;
+  int rc = packed_results(h, h->f_pack, nq, limit, &out);
+  if (rc != RSE_OK) return rc;
+  h->pack_n = static_cast<size_t>(nq) * limit; h->pack_nq = nq;
+  return hybrid_local(h, mode, param, tie_mode, limit, kprime, k1, b, h->staged, h->pin_status, nullptr, out);
 }
 
 int rse_hybrid_run_merged_dev(rse_index* h, int32_t mode, double param, int32_t tie_mode, int32_t limit,
@@ -2002,16 +2050,24 @@ int rse_hybrid_run_merged_dev(rse_index* h, int32_t mode, double param, int32_t 
   if (!h) return RSE_ERR_INVALID;
   if (!gathered_dev || n_lists < 1 || !out_id_dev || !out_score_dev || !out_a_dev || !out_b_dev || !out_count_dev)
     return fail(h, RSE_ERR_INVALID, "rse_hybrid_run_merged_dev: bad arguments");
-  return hybrid_run_impl(h, mode, param, tie_mode, limit, knn_multiplier, k1, b,
-                         reinterpret_cast<const long long*>(gathered_dev), n_lists,
-                         reinterpret_cast<long long*>(out_id_dev), out_score_dev, out_a_dev, out_b_dev, out_count_dev,
-                         limit);
+  const int nq = h->staged.nq;
+  if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_run: nothing staged");
+  const int kprime = hybrid_kprime(h, mode, limit, knn_multiplier);
+  if (kprime < 0) return kprime;
+  CK(cudaSetDevice(h->device));
+  // BM25 (k = limit, hybrid_search.py:70), then the merge of the gathered KNN candidates
+  int rc = bm25_run(h, h->staged, nq, limit, k1, b, h->stream, false);
+  if (rc != RSE_OK) return rc;
+  return hybrid_tail(h, mode, param, tie_mode, nq, limit, kprime, reinterpret_cast<const long long*>(gathered_dev),
+                     n_lists, false,
+                     Fused{reinterpret_cast<long long*>(out_id_dev), out_score_dev, out_a_dev, out_b_dev, out_count_dev,
+                           limit});
 }
 
 int rse_hybrid_fetch(rse_index* h, int32_t limit, int64_t* out_id, double* out_score, double* out_a, double* out_b,
                      int32_t* out_count) {
   if (!h) return RSE_ERR_INVALID;
-  const int nq = h->staged_nq;
+  const int nq = h->staged.nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_fetch: nothing staged");
   if (!out_id || !out_score || !out_a || !out_b || !out_count) return fail(h, RSE_ERR_INVALID, "rse_hybrid_fetch: bad arguments");
   const size_t n = static_cast<size_t>(nq) * limit;
@@ -2054,7 +2110,8 @@ int rse_hybrid_submit(rse_index* h, int32_t mode, double param, int32_t tie_mode
                       double b, int64_t* ticket) {
   if (!h) return RSE_ERR_INVALID;
   if (!ticket || nq < 1 || !q_host || !tok_indptr) return fail(h, RSE_ERR_INVALID, "rse_hybrid_submit: bad arguments");
-  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
+  const int kprime = hybrid_kprime(h, mode, limit, knn_multiplier);
+  if (kprime < 0) return kprime;
   if (h->next_ticket - h->next_collect >= 2)
     return fail(h, RSE_ERR_STATE, "rse_hybrid_submit: two batches already in flight, collect one first");
   CK(cudaSetDevice(h->device));
@@ -2078,52 +2135,34 @@ int rse_hybrid_submit(rse_index* h, int32_t mode, double param, int32_t tie_mode
   }
   std::memcpy(h->pin_q[s], q_host, qbytes);
 
-  // the slot's device buffers and flag buffer stand in for the handle's while this batch is staged and enqueued
-  auto swap_in_out = [&]() {
-    std::swap(h->q_dev, sl.q_dev); std::swap(h->b_tokptr, sl.b_tokptr); std::swap(h->b_terms, sl.b_terms);
-    std::swap(h->b_idf, sl.b_idf); std::swap(h->f_pack, sl.f_pack);
-    std::swap(h->pin_status, sl.pin_status); std::swap(h->pin_status_n, sl.pin_status_n);
-  };
-  swap_in_out();
-  cudaStream_t main_stream = h->stream;
-  h->stream = h->stream_h2d;                                  // uploads on the copy stream
-  int rc = rse_hybrid_stage(h, nq, h->pin_q[s], tok_indptr, term_rows);
-  h->stream = main_stream;
-  cudaError_t ce = cudaSuccess;
-  if (rc == RSE_OK) {
-    ce = cudaEventRecord(h->ev_q[s], h->stream_h2d);
-    if (ce == cudaSuccess) ce = cudaStreamWaitEvent(h->stream, h->ev_q[s], 0);
-    if (ce == cudaSuccess) {
-      h->defer_status = true;
-      rc = rse_hybrid_run(h, mode, param, tie_mode, limit, knn_multiplier, k1, b);
-      h->defer_status = false;
-    }
-  }
+  // the batch is staged into the SLOT's buffers (uploads on the copy stream) and runs from there: whatever the handle
+  // had staged is given up, so a later rse_hybrid_run / _fetch without a fresh rse_hybrid_stage fails
+  h->staged.nq = 0; h->pack_n = 0; h->pack_nq = 0;
+  int rc = stage_batch(h, sl.in, nq, h->pin_q[s], cudaMemcpyHostToDevice, tok_indptr, term_rows, h->stream_h2d);
+  if (rc != RSE_OK) return rc;
+  CK(cudaEventRecord(h->ev_q[s], h->stream_h2d));
+  CK(cudaStreamWaitEvent(h->stream, h->ev_q[s], 0));
+  Fused out;
+  rc = packed_results(h, sl.f_pack, nq, limit, &out);
+  if (rc != RSE_OK) return rc;
+  rc = hybrid_local(h, mode, param, tie_mode, limit, kprime, k1, b, sl.in, sl.flags, &sl.knn, out);
+  if (rc != RSE_OK) return rc;
   const size_t n = static_cast<size_t>(nq) * limit;
   const size_t bytes = 32 * n + 4 * static_cast<size_t>(nq);
-  if (rc == RSE_OK && ce == cudaSuccess) {
-    if (sl.bytes < bytes) {                                   // the slot is free: its previous ticket was collected
-      if (sl.pin) cudaFreeHost(sl.pin);
-      sl.pin = nullptr; sl.bytes = 0;
-      ce = cudaMallocHost(reinterpret_cast<void**>(&sl.pin), bytes + bytes / 2);
-      if (ce == cudaSuccess) sl.bytes = bytes + bytes / 2;
-    }
-    if (ce == cudaSuccess && !sl.ev) ce = cudaEventCreateWithFlags(&sl.ev, cudaEventDisableTiming);
-    // results: third stream, behind the fusion kernel
-    if (ce == cudaSuccess) ce = cudaEventRecord(h->ev_fused, h->stream);
-    if (ce == cudaSuccess) ce = cudaStreamWaitEvent(h->stream_d2h, h->ev_fused, 0);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(sl.pin, h->f_pack.p, bytes, cudaMemcpyDeviceToHost, h->stream_d2h);
-    if (ce == cudaSuccess) ce = cudaEventRecord(sl.ev, h->stream_d2h);
-    if (ce == cudaSuccess) h->stats.d2h_bytes += static_cast<int64_t>(bytes);
+  if (sl.bytes < bytes) {                                     // the slot is free: its previous ticket was collected
+    if (sl.pin) CK(cudaFreeHost(sl.pin));
+    sl.pin = nullptr; sl.bytes = 0;
+    CK(cudaMallocHost(reinterpret_cast<void**>(&sl.pin), bytes + bytes / 2));
+    sl.bytes = bytes + bytes / 2;
   }
-  swap_in_out();
-  // the staged batch lives in the SLOT's buffers: nothing is staged in the handle's own any more, so a later
-  // rse_hybrid_run / _fetch without a fresh rse_hybrid_stage must fail instead of touching stale pointers
-  h->staged_nq = 0; h->pack_n = 0; h->pack_nq = 0;
-  if (rc != RSE_OK) return rc;
-  if (ce != cudaSuccess) return fail(h, RSE_ERR_CUDA, std::string("rse_hybrid_submit: ") + cudaGetErrorString(ce));
-  sl.deferred = h->run_deferred;
-  if (sl.deferred) {
+  if (!sl.ev) CK(cudaEventCreateWithFlags(&sl.ev, cudaEventDisableTiming));
+  // results: third stream, behind the fusion kernel
+  CK(cudaEventRecord(h->ev_fused, h->stream));
+  CK(cudaStreamWaitEvent(h->stream_d2h, h->ev_fused, 0));
+  CK(cudaMemcpyAsync(sl.pin, sl.f_pack.p, bytes, cudaMemcpyDeviceToHost, h->stream_d2h));
+  CK(cudaEventRecord(sl.ev, h->stream_d2h));
+  h->stats.d2h_bytes += static_cast<int64_t>(bytes);
+  if (sl.knn.flags) {
     sl.tok_indptr.assign(tok_indptr, tok_indptr + nq + 1);
     sl.term_rows.assign(term_rows, term_rows + (term_rows ? tok_indptr[nq] : 0));
     sl.mode = mode; sl.tie_mode = tie_mode; sl.limit = limit; sl.knn_multiplier = knn_multiplier;
@@ -2146,9 +2185,9 @@ int rse_hybrid_collect(rse_index* h, int64_t ticket, int32_t* out_nq, int32_t* o
   const size_t n = sl.n;
   if (out_nq) *out_nq = sl.nq;
   if (out_limit) *out_limit = sl.nq ? static_cast<int32_t>(n / sl.nq) : 0;
-  if (sl.deferred) {
+  if (sl.knn.flags) {
     bool flagged = false;
-    for (int q = 0; q < sl.nq && !flagged; ++q) flagged = sl.pin_status[q] != 0;
+    for (int q = 0; q < sl.nq && !flagged; ++q) flagged = sl.knn.flags[q] != 0;
     if (flagged) {
       // the query vectors are still in this ticket's pinned staging buffer (the next ticket uses the other one);
       // the blocking call handles the flagged queries through the exact scan.  The batch submitted after this one
@@ -2159,9 +2198,9 @@ int rse_hybrid_collect(rse_index* h, int64_t ticket, int32_t* out_nq, int32_t* o
       const int rc = rse_hybrid(h, sl.mode, sl.param, sl.tie_mode, sl.limit, sl.knn_multiplier, sl.nq, h->pin_q[ticket & 1],
                                 sl.tok_indptr.data(), sl.term_rows.empty() ? nullptr : sl.term_rows.data(), sl.k1, sl.b,
                                 out_id, out_score, out_a, out_b, out_count);
-      h->staged_nq = 0; h->pack_n = 0; h->pack_nq = 0;
+      h->staged.nq = 0; h->pack_n = 0; h->pack_nq = 0;
       if (rc != RSE_OK) return rc;
-      sl.deferred = false;
+      sl.knn = PendingKnn{};
       ++h->next_collect;
       return RSE_OK;
     }
@@ -2863,17 +2902,7 @@ int rse_encode_images(rse_index* h, int32_t slot, const float* pixels_host, int3
 int rse_hybrid_stage_dev(rse_index* h, int32_t nq, const float* q_dev, const int32_t* tok_indptr, const int32_t* term_rows) {
   if (!h) return RSE_ERR_INVALID;
   if (nq < 1 || !q_dev || !tok_indptr) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage_dev: bad arguments");
-  if (!h->emb || !h->movie_idx || !h->indptr || !h->doc_ids || !h->movie_ids)
-    return fail(h, RSE_ERR_STATE, "rse_hybrid: needs embeddings (with movie_idx), a BM25 index and id tables");
-  h->staged_nq = 0;
-  if (tok_indptr[nq] > 0 && !term_rows) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stage_dev: term_rows is NULL");
-  CK(cudaSetDevice(h->device));
-  int rc = bm25_stage(h, tok_indptr, term_rows, nq);
-  if (rc != RSE_OK) return rc;
-  ENSURE(h->q_dev, sizeof(float) * static_cast<size_t>(nq) * h->dim);
-  CK(cudaMemcpyAsync(h->q_dev.p, q_dev, sizeof(float) * static_cast<size_t>(nq) * h->dim, cudaMemcpyDeviceToDevice, h->stream));
-  h->staged_nq = nq;
-  return RSE_OK;
+  return stage_batch(h, h->staged, nq, q_dev, cudaMemcpyDeviceToDevice, tok_indptr, term_rows, h->stream);
 }
 
 // ------------------------------------------------------------------ cross-encoder rerank of a fused batch (rerank.cuh)
@@ -2941,10 +2970,12 @@ int rse_hybrid_rerank_run(rse_index* h, int32_t slot, double k, int32_t tie_mode
   if (limit < 1 || limit > RSE_MAX_RERANK_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_rerank_run: limit must be in [1, 128]");
   if (activation != 0 && activation != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: activation must be 0 (logit) or 1 (sigmoid)");
   if (h->rr_n_docs < 1) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: no document store (rse_rerank_docs_load)");
-  const int nq = h->staged_nq;
+  const int nq = h->staged.nq;
   if (nq <= 0) return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: nothing staged");
   if (h->next_ticket != h->next_collect)
     return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_run: rse_hybrid_submit tickets are in flight (collect or drain them)");
+  const int kprime = hybrid_kprime(h, 0, limit, knn_multiplier);
+  if (kprime < 0) return kprime;
   if (slot < 0 || slot >= RSE_MAX_ENCODERS) return fail(h, RSE_ERR_INVALID, "rse_hybrid_rerank_run: slot out of range");
   Encoder& e = h->enc[slot];
   if (!e.created || !e.finalized || e.clip || e.cfg.head != 1)
@@ -3002,7 +3033,8 @@ int rse_hybrid_rerank_run(rse_index* h, int32_t slot, double k, int32_t tie_mode
   double* fa = static_cast<double*>(h->rr_fa.p);
   double* fb = static_cast<double*>(h->rr_fb.p);
   int* fcnt = static_cast<int*>(h->rr_fcnt.p);
-  int rc = hybrid_run_impl(h, 0, k, tie_mode, limit, knn_multiplier, k1, b, nullptr, 0, fid, fsc, fa, fb, fcnt, W);
+  int rc = hybrid_local(h, 0, k, tie_mode, limit, kprime, k1, b, h->staged, h->pin_status, nullptr,
+                        Fused{fid, fsc, fa, fb, fcnt, W});
   if (rc != RSE_OK) return rc;
   rr_mark(h, 1);
 
@@ -3220,36 +3252,29 @@ int rse_comm_allgather_dev(rse_index* h, const void* send_dev, void* recv_dev, i
 namespace {
 
 // local top-K' of ALL queries on this shard (+ deferred flag count or blocking exact fallback) + exchange:
-// leaves [n_ranks, ns, kprime, 3] in h->sh_mine.  Optionally starts the slice's BM25 underneath the filter pass.
-int sharded_knn_exchange(rse_index* h, const float* q_all_dev, int nq_all, int kprime, int32_t* flagged_dev, bool with_bm25,
-                         int limit, double k1, double b, bool* bm25_overlapped) {
+// leaves [n_ranks, ns, kprime, 3] in h->sh_mine.  `bm25`: the slice's BM25, started underneath the filter pass when
+// the tensor-core path runs, else on the main stream behind the KNN.
+int sharded_knn_exchange(rse_index* h, const float* q_all_dev, int nq_all, int kprime, int32_t* flagged_dev,
+                         Bm25Job* bm25) {
   if (!h->comm) return fail(h, RSE_ERR_STATE, "no communicator: call rse_comm_init first");
   const int R = h->comm_ranks, me = h->comm_rank;
   const int ns = query_slice(nq_all, R, me + 1) - query_slice(nq_all, R, me);
   const size_t per = static_cast<size_t>(kprime) * 3;
   ENSURE(h->sh_cand, sizeof(long long) * static_cast<size_t>(nq_all) * per);
   ENSURE(h->sh_mine, sizeof(long long) * static_cast<size_t>(R) * std::max(ns, 1) * per);
-  *bm25_overlapped = false;
-  if (with_bm25 && ns > 0) {
-    h->bm25_overlap_pending = true;
-    h->ov_nq = ns; h->ov_limit = limit; h->ov_k1 = k1; h->ov_b = b;
+  PendingKnn pend;
+  int rc = knn_local_begin(h, q_all_dev, nq_all, kprime, static_cast<long long*>(h->sh_cand.p), h->pin_status, bm25,
+                           pend);
+  if (rc != RSE_OK) return rc;
+  if (bm25 && !bm25->enqueued) {
+    rc = bm25_run(h, *bm25->in, bm25->in->nq, bm25->k, bm25->k1, bm25->b, h->stream, false);
+    if (rc != RSE_OK) return rc;
   }
-  int rc = knn_local_begin(h, q_all_dev, nq_all, kprime, static_cast<long long*>(h->sh_cand.p));
-  if (rc != RSE_OK) { h->bm25_overlap_pending = false; return rc; }
-  if (with_bm25 && ns > 0) {
-    *bm25_overlapped = !h->bm25_overlap_pending;              // the filter launch consumed the request
-    h->bm25_overlap_pending = false;
-    if (!*bm25_overlapped) {
-      rc = bm25_run(h, ns, limit, k1, b);
-      if (rc != RSE_OK) return rc;
-    }
-  }
-  if (h->knn_pending && flagged_dev) {                       // no host round trip: count the unfinished queries
-    h->knn_pending = false;
-    knn_flag_count_kernel<<<1, 256, 0, h->stream>>>(static_cast<const int*>(h->tc_status.p), nq_all, flagged_dev);
+  if (pend.flags && flagged_dev) {                           // no host round trip: count the unfinished queries
+    knn_flag_count_kernel<<<1, 256, 0, h->stream>>>(static_cast<const int*>(h->tc_status.p), pend.nq, flagged_dev);
     LAUNCHED(h);
   } else {
-    rc = knn_local_finish(h);                                // blocking, exact (flagged queries -> exact scan)
+    rc = knn_local_finish(h, pend);                          // blocking, exact (flagged queries -> exact scan)
     if (rc != RSE_OK) return rc;
   }
   return comm_exchange(h, static_cast<const long long*>(h->sh_cand.p), nq_all, kprime, static_cast<long long*>(h->sh_mine.p));
@@ -3264,8 +3289,7 @@ int rse_knn_sharded_dev(rse_index* h, const float* q_all_dev, int32_t nq_all, in
   if (!q_all_dev || nq_all < 1 || k < 1 || kprime < 1) return fail(h, RSE_ERR_INVALID, "rse_knn_sharded_dev: bad arguments");
   if (!h->emb || !h->movie_idx) return fail(h, RSE_ERR_STATE, "rse_knn_sharded_dev: needs embeddings with movie_idx");
   CK(cudaSetDevice(h->device));
-  bool ov = false;
-  int rc = sharded_knn_exchange(h, q_all_dev, nq_all, kprime, flagged_dev, false, 0, 0.0, 0.0, &ov);
+  int rc = sharded_knn_exchange(h, q_all_dev, nq_all, kprime, flagged_dev, nullptr);
   if (rc != RSE_OK) return rc;
   const int ns = query_slice(nq_all, h->comm_ranks, h->comm_rank + 1) - query_slice(nq_all, h->comm_ranks, h->comm_rank);
   if (ns == 0) return RSE_OK;
@@ -3282,47 +3306,22 @@ int rse_hybrid_sharded_run_dev(rse_index* h, int32_t mode, double param, int32_t
   if (!h) return RSE_ERR_INVALID;
   if (!q_all_dev || nq_all < 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid_sharded_run_dev: bad arguments");
   if (!h->comm) return fail(h, RSE_ERR_STATE, "no communicator: call rse_comm_init first");
-  if (mode != 0 && mode != 1) return fail(h, RSE_ERR_INVALID, "rse_hybrid: mode must be 0 (rrf) or 1 (weighted)");
-  if (limit < 1 || limit > RSE_MAX_HYBRID_LIMIT) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit must be in [1, 512]");
-  if (knn_multiplier < 0) return fail(h, RSE_ERR_INVALID, "rse_hybrid: knn_multiplier < 0");
-  if (!h->emb || !h->movie_idx || !h->indptr || !h->doc_ids || !h->movie_ids)
-    return fail(h, RSE_ERR_STATE, "rse_hybrid: needs embeddings (with movie_idx), a BM25 index and id tables");
-  const int R = h->comm_ranks, me = h->comm_rank;
-  const int ns = query_slice(nq_all, R, me + 1) - query_slice(nq_all, R, me);
-  if (h->staged_nq != ns)
+  const int kprime = hybrid_kprime(h, mode, limit, knn_multiplier);
+  if (kprime < 0) return kprime;
+  const int ns = query_slice(nq_all, h->comm_ranks, h->comm_rank + 1) - query_slice(nq_all, h->comm_ranks, h->comm_rank);
+  if (h->staged.nq != ns)
     return fail(h, RSE_ERR_STATE, "rse_hybrid_sharded_run_dev: the staged batch must be this rank's query slice (tokens)");
-  const int kprime = std::max(limit * knn_multiplier, limit);
-  if (kprime > RSE_MAX_KPRIME) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid: limit*knn_multiplier exceeds 4096");
   CK(cudaSetDevice(h->device));
-  bool overlapped = false;
-  int rc = sharded_knn_exchange(h, q_all_dev, nq_all, kprime, flagged_dev, true, limit, k1, b, &overlapped);
+  Bm25Job bm25{&h->staged, limit, k1, b};
+  int rc = sharded_knn_exchange(h, q_all_dev, nq_all, kprime, flagged_dev, ns > 0 ? &bm25 : nullptr);
   if (rc != RSE_OK) return rc;
   if (ns == 0) return RSE_OK;
   if (!out_id_dev || !out_score_dev || !out_a_dev || !out_b_dev || !out_count_dev)
     return fail(h, RSE_ERR_INVALID, "rse_hybrid_sharded_run_dev: output buffers are NULL");
-  const int n2 = next_pow2(R * kprime);
-  const size_t smem = static_cast<size_t>(n2) * 12;
-  if (smem > 200 * 1024) return fail(h, RSE_ERR_UNSUPPORTED, "rse_hybrid_sharded_run_dev: n_ranks*kprime too large for the merge kernel");
-  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(knn_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  const size_t n = static_cast<size_t>(ns) * limit;
-  ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(ns) * kprime * 3);
-  ENSURE(h->o_dist, sizeof(float) * n);
-  ENSURE(h->o_rowid, sizeof(long long) * n);
-  ENSURE(h->o_movie, sizeof(int) * n);
-  ENSURE(h->o_count, sizeof(int) * ns);
-  knn_merge_kernel<<<ns, kSelThreads, smem, h->stream>>>(static_cast<const long long*>(h->sh_mine.p), R, ns, kprime, n2,
-                                                         static_cast<long long*>(h->cand.p));
-  LAUNCHED(h);
-  rc = aggregate(h, static_cast<const long long*>(h->cand.p), ns, limit, kprime, static_cast<float*>(h->o_dist.p),
-                 static_cast<long long*>(h->o_rowid.p), static_cast<int*>(h->o_movie.p), static_cast<int*>(h->o_count.p));
-  if (rc != RSE_OK) return rc;
-  if (overlapped) CK(cudaStreamWaitEvent(h->stream, h->ev_bm25_done, 0));
-  FuseIn in{nullptr, static_cast<const double*>(h->b_score.p), static_cast<const int*>(h->b_count.p), nullptr,
-            static_cast<const float*>(h->o_dist.p), static_cast<const int*>(h->o_count.p), nullptr};
-  in.bm25_idx = static_cast<const int*>(h->b_doc.p); in.bm25_table = h->doc_ids; in.bm25_table_n = h->n_doc_ids;
-  in.sem_idx = static_cast<const int*>(h->o_movie.p); in.sem_table = h->movie_ids; in.sem_table_n = h->n_movie_ids;
-  return fuse_launch(h, mode, param, tie_mode, ns, limit, limit, in, reinterpret_cast<long long*>(out_id_dev), out_score_dev,
-                     out_a_dev, out_b_dev, out_count_dev);
+  return hybrid_tail(h, mode, param, tie_mode, ns, limit, kprime, static_cast<const long long*>(h->sh_mine.p),
+                     h->comm_ranks, bm25.enqueued,
+                     Fused{reinterpret_cast<long long*>(out_id_dev), out_score_dev, out_a_dev, out_b_dev, out_count_dev,
+                           limit});
 }
 
 int rse_hybrid_stash(rse_index* h, int32_t slot) {
@@ -3330,9 +3329,7 @@ int rse_hybrid_stash(rse_index* h, int32_t slot) {
   if (slot < 0 || slot >= RSE_MAX_STASH) return fail(h, RSE_ERR_INVALID, "rse_hybrid_stash: slot out of range");
   if (h->next_collect < h->next_ticket)
     return fail(h, RSE_ERR_STATE, "rse_hybrid_stash: tickets in flight (collect or drain them first)");
-  rse_index::Stash& st = h->stash[slot];
-  std::swap(h->q_dev, st.q_dev); std::swap(h->b_tokptr, st.b_tokptr); std::swap(h->b_terms, st.b_terms);
-  std::swap(h->b_idf, st.b_idf); std::swap(h->staged_nq, st.nq);
+  std::swap(h->staged, h->stash[slot]);
   h->pack_n = 0; h->pack_nq = 0;
   return RSE_OK;
 }
@@ -3359,7 +3356,7 @@ int rse_hybrid_drain(rse_index* h, int32_t* out_dropped) {
   while (h->next_collect < h->next_ticket) {
     rse_index::OutSlot& sl = h->out_slot[h->next_collect & 1];
     if (sl.ev) CK(cudaEventSynchronize(sl.ev));
-    sl.deferred = false;
+    sl.knn = PendingKnn{};
     ++h->next_collect;
     ++dropped;
   }
