@@ -268,8 +268,9 @@ int rse_hybrid_drain(rse_index *h, int32_t *out_dropped);
  *            output [n_seq, hidden]
  *   head 1 : BertModel -> pooler (tanh(dense([CLS]))) -> classifier (num_labels = 1); output [n_seq] logits
  * Weights are handed over tensor by tensor under their HuggingFace state_dict names (any prefix such as "bert." or
- * "0.auto_model." is ignored); tokenisation stays on the host (out of scope, SURVEY §2 #5): the caller passes the
- * token ids of the batch PACKED — ids[T] (+ optional token_type_ids[T], NULL = all 0) and cu_seqlens[n_seq + 1]
+ * "0.auto_model." is ignored).  rse_encode takes token ids (any tokenizer, run by the caller) and rse_encode_texts
+ * takes the texts themselves (BERT WordPiece on the device, see "BERT WordPiece on the device" below).  The ids come
+ * PACKED — ids[T] (+ optional token_type_ids[T], NULL = all 0) and cu_seqlens[n_seq + 1]
  * (sequence s owns tokens cu[s] .. cu[s+1]; what attention_mask == 1 selects).  fp32 throughout.
  * rse_encode_dev leaves the result on the device (out_dev on the handle's device, asynchronous on its stream), so
  * rse_hybrid_stage_dev can take the query vectors from there: text in, no host hop for the vectors. */
@@ -365,6 +366,63 @@ int rse_hybrid_rerank_fetch(rse_index *h, int32_t limit, int64_t *out_id, double
 int rse_set_rerank_token_budget(rse_index *h, int64_t tokens);
 int rse_hybrid_rerank_timing(rse_index *h, float *out_ms);
 int rse_pair_truncate(int32_t n1, int32_t n2, int32_t max_length, int32_t *a, int32_t *b);
+
+/* ------------------------------------------------------------------ BERT WordPiece on the device
+ * The tokenizers of both reference models (all-MiniLM-L6-v2, ms-marco-TinyBERT-L2-v2: HF BertTokenizerFast, the
+ * uncased BERT WordPiece vocab) run on the device (csrc/wordpiece.cuh) with ids identical to the HF fast tokenizer:
+ * the special tokens split off the raw text (literal, leftmost-longest), BertNormalizer, BertPreTokenizer, greedy
+ * longest-match WordPiece, optional [CLS] ... [SEP] and truncation.  Texts are UTF-8, back to back in `text`;
+ * offsets[n + 1] (from 0, non-decreasing) delimit them in bytes.  They go up through a pinned buffer.
+ *   rse_tokenizer_load : a tokenizer into a slot (a new load replaces it).  The description is built from the HF object
+ *                        by rag_search_engine_b200/wordpiece.py: cp_map / cp_class for every code point (what the
+ *                        normaliser makes of it, how the pre-tokenizer classes it), the two tries of word-initial and
+ *                        "##" pieces, the special ids and the added-token strings.  Every index is checked here.
+ *   rse_tokenize       : tokenize n texts into the handle's buffers.  add_special 1 = [CLS] pieces[:max_length - 2]
+ *                        [SEP] (the sentence encoder's input), 0 = pieces[:max_length] (the cross-encoder's single
+ *                        texts); max_length <= 0 keeps every piece.  out_total / out_max_len (may be NULL): ids in all,
+ *                        the longest sequence.  Synchronises once, for those two numbers.
+ *   rse_tokens_fetch   : the last rse_tokenize's ids[total] and cu_seqlens[n + 1] to host memory (synchronises), or
+ *   rse_tokens_fetch_dev : to device memory (asynchronous on the handle's stream).
+ *   rse_encode_texts(_dev): tokenize with [CLS] / [SEP] at max_length (2 .. max_positions) and run the BERT slot
+ *                        enc_slot on the ids where they are: rse_encode's output without host id lists.  One small
+ *                        device-to-host copy per call (the token total and the longest sequence the encoder launch needs).
+ *   rse_rerank_docs_load_texts: the store rse_rerank_docs_load would hold for the same ids and the tokenizer's ids of
+ *                        each text (no special tokens, no cut), built on the device.  ids[n_docs] strictly ascending.
+ * Errors: an unloaded slot RSE_ERR_STATE; bad offsets and malformed UTF-8 (the message names the first text)
+ * RSE_ERR_INVALID.  NFD (accent stripping) reorders combining marks by canonical class; the tables map each code point
+ * on its own, so a text with two code points whose marks survive the stripping (spacing marks of a non-zero class:
+ * the Mc viramas of Javanese, Balinese, Sundanese, Batak, Tagalog, Grantha and a few other scripts, the musical
+ * symbol stems) is refused with RSE_ERR_UNSUPPORTED, never tokenized differently, even when a starter separates the
+ * two; the Python layer hands those texts to the host tokenizer.  Without accent stripping nothing is refused.  Limits: max_input_chars_per_word <= 256, <= 32 added tokens, < 2^31
+ * ids per call. */
+#define RSE_MAX_TOKENIZERS 2
+typedef struct rse_wordpiece_desc {
+  const uint32_t *cp_map;       /* [0x110000]: bits 0-20 code point or extra row, 21-22 count (0-3), 23 reorder flag */
+  const uint32_t *extra;        /* [n_extra][3] code points of the 2- and 3-code-point outputs */
+  int32_t n_extra;
+  const uint8_t *cp_class;      /* [0x110000]: 0 other, 1 whitespace, 2 punctuation */
+  const int32_t *node_first;    /* [n_nodes + 1]: node 0 = word-initial root, node 1 = continuation root */
+  const int32_t *node_id;       /* [n_nodes]: vocab id of the piece ending at the node, -1 none */
+  int32_t n_nodes;
+  const int32_t *edge_cp;       /* [node_first[n_nodes]], ascending within a node */
+  const int32_t *edge_child;
+  const char *added;            /* added-token strings (UTF-8) back to back */
+  const int32_t *added_offsets; /* [n_added + 1] */
+  const int32_t *added_ids;     /* [n_added] */
+  int32_t n_added;
+  int32_t unk_id, cls_id, sep_id, max_input_chars_per_word;
+} rse_wordpiece_desc;
+int rse_tokenizer_load(rse_index *h, int32_t slot, const rse_wordpiece_desc *desc);
+int rse_tokenize(rse_index *h, int32_t slot, const char *text, const int64_t *offsets, int32_t n, int32_t add_special,
+                 int32_t max_length, int64_t *out_total, int32_t *out_max_len);
+int rse_tokens_fetch(rse_index *h, int32_t *ids_host, int32_t *cu_seqlens_host);
+int rse_tokens_fetch_dev(rse_index *h, int32_t *ids_dev, int32_t *cu_seqlens_dev);
+int rse_encode_texts(rse_index *h, int32_t tok_slot, int32_t enc_slot, const char *text, const int64_t *offsets,
+                     int32_t n, int32_t max_length, float *out_host);
+int rse_encode_texts_dev(rse_index *h, int32_t tok_slot, int32_t enc_slot, const char *text, const int64_t *offsets,
+                         int32_t n, int32_t max_length, float *out_dev);
+int rse_rerank_docs_load_texts(rse_index *h, int32_t tok_slot, const int64_t *ids, int64_t n_docs, const char *text,
+                               const int64_t *offsets);
 
 /* ------------------------------------------------------------------ multi-GPU: row shards over one box (SURVEY §8e)
  * One process per GPU, one handle per process; the HANDLE owns the NCCL communicator (NCCL is bound at run time:

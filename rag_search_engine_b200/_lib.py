@@ -73,6 +73,15 @@ class RseClipConfig(ctypes.Structure):
                 ("eos_token_id", c_int32), ("ln_eps", c_float)]
 
 
+class RseWordpieceDesc(ctypes.Structure):
+    """include/rse.h rse_wordpiece_desc."""
+    _fields_ = [("cp_map", c_void_p), ("extra", c_void_p), ("n_extra", c_int32), ("cp_class", c_void_p),
+                ("node_first", c_void_p), ("node_id", c_void_p), ("n_nodes", c_int32), ("edge_cp", c_void_p),
+                ("edge_child", c_void_p), ("added", c_void_p), ("added_offsets", c_void_p), ("added_ids", c_void_p),
+                ("n_added", c_int32), ("unk_id", c_int32), ("cls_id", c_int32), ("sep_id", c_int32),
+                ("max_input_chars_per_word", c_int32)]
+
+
 _SIGNATURES = {
     "rse_abi_version": (ctypes.c_int, []),
     "rse_create": (ctypes.c_int, [c_int32, POINTER(c_void_p)]),
@@ -148,6 +157,15 @@ _SIGNATURES = {
     "rse_set_rerank_token_budget": (ctypes.c_int, [c_void_p, c_int64]),
     "rse_hybrid_rerank_timing": (ctypes.c_int, [c_void_p, POINTER(c_float)]),
     "rse_pair_truncate": (ctypes.c_int, [c_int32, c_int32, c_int32, POINTER(c_int32), POINTER(c_int32)]),
+    "rse_tokenizer_load": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseWordpieceDesc)]),
+    "rse_tokenize": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_int32, POINTER(c_int64),
+                                    POINTER(c_int32)]),
+    "rse_tokens_fetch": (ctypes.c_int, [c_void_p, c_void_p, c_void_p]),
+    "rse_tokens_fetch_dev": (ctypes.c_int, [c_void_p, c_void_p, c_void_p]),
+    "rse_encode_texts": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
+    "rse_encode_texts_dev": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32,
+                                            c_void_p]),
+    "rse_rerank_docs_load_texts": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_void_p]),
     "rse_comm_unique_id": (ctypes.c_int, [c_void_p]),
     "rse_comm_init": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32]),
     "rse_comm_destroy": (ctypes.c_int, [c_void_p]),
@@ -647,6 +665,75 @@ class Index:
                                                     c_void_p(ors.ctypes.data), c_void_p(orr.ctypes.data),
                                                     c_void_p(oce.ctypes.data), c_void_p(oc.ctypes.data)))
         return oid, osc, orb, ors, orr, oce, oc
+
+    # ------------------------------------------------------------------ BERT WordPiece on the device
+    def tokenizer_load(self, slot: int, tables):
+        """A ``wordpiece.WordPieceTables`` into a tokenizer slot."""
+        arrs = dict(cp_map=_c(tables.cp_map, np.uint32), extra=_c(tables.extra, np.uint32).reshape(-1),
+                    cp_class=_c(tables.cp_class, np.uint8), node_first=_c(tables.node_first, np.int32),
+                    node_id=_c(tables.node_id, np.int32), edge_cp=_c(tables.edge_cp, np.int32),
+                    edge_child=_c(tables.edge_child, np.int32))
+        raw = [c.encode() for c, _ in tables.added]
+        added = np.frombuffer(b"".join(raw) or b"\0", np.uint8)
+        aoff = np.zeros(len(raw) + 1, np.int32)
+        np.cumsum([len(r) for r in raw], out=aoff[1:])
+        aid = np.asarray([i for _, i in tables.added] or [0], np.int32)
+        d = RseWordpieceDesc(n_extra=arrs["extra"].size // 3, n_nodes=arrs["node_id"].size, n_added=len(raw),
+                             unk_id=tables.unk_id, cls_id=tables.cls_id, sep_id=tables.sep_id,
+                             max_input_chars_per_word=tables.max_input_chars_per_word,
+                             added=added.ctypes.data, added_offsets=aoff.ctypes.data, added_ids=aid.ctypes.data,
+                             **{k: v.ctypes.data for k, v in arrs.items()})
+        self._check(self._L.rse_tokenizer_load(self._h, int(slot), ctypes.byref(d)))
+
+    @staticmethod
+    def _texts(data: bytes, offsets):
+        offsets = _c(offsets, np.int64)
+        return c_char_p(data), offsets, len(offsets) - 1
+
+    def tokenize(self, slot: int, data: bytes, offsets, add_special: bool, max_length: int = 0):
+        """UTF-8 texts (``data`` delimited by ``offsets[n + 1]``) -> (ids int32[total], cu_seqlens int32[n + 1])."""
+        txt, offs, n = self._texts(data, offsets)
+        total, ml = c_int64(0), c_int32(0)
+        self._check(self._L.rse_tokenize(self._h, int(slot), txt, c_void_p(offs.ctypes.data), n, int(bool(add_special)),
+                                         int(max_length), ctypes.byref(total), ctypes.byref(ml)))
+        ids = np.empty(max(total.value, 1), np.int32)
+        cu = np.empty(n + 1, np.int32)
+        self._check(self._L.rse_tokens_fetch(self._h, c_void_p(ids.ctypes.data), c_void_p(cu.ctypes.data)))
+        return ids[:total.value], cu
+
+    def tokenize_dev(self, slot: int, data: bytes, offsets, add_special: bool, max_length: int = 0):
+        """Same, ids left in the handle's buffers: -> (total, longest); then ``tokens_fetch_dev``."""
+        txt, offs, n = self._texts(data, offsets)
+        total, ml = c_int64(0), c_int32(0)
+        self._check(self._L.rse_tokenize(self._h, int(slot), txt, c_void_p(offs.ctypes.data), n, int(bool(add_special)),
+                                         int(max_length), ctypes.byref(total), ctypes.byref(ml)))
+        return int(total.value), int(ml.value)
+
+    def tokens_fetch_dev(self, ids_ptr: int, cu_ptr: int):
+        self._check(self._L.rse_tokens_fetch_dev(self._h, c_void_p(ids_ptr), c_void_p(cu_ptr)))
+
+    def encode_texts(self, tok_slot: int, enc_slot: int, data: bytes, offsets, max_length: int):
+        """Texts -> [n, hidden] float32 (head 0) / [n] logits (head 1): tokenized and encoded on the device."""
+        txt, offs, n = self._texts(data, offsets)
+        cfg = self._enc_cfg[int(enc_slot)]
+        out = np.zeros((n, cfg.hidden) if cfg.head == 0 else (n,), np.float32)
+        self._check(self._L.rse_encode_texts(self._h, int(tok_slot), int(enc_slot), txt, c_void_p(offs.ctypes.data), n,
+                                             int(max_length), c_void_p(out.ctypes.data)))
+        return out
+
+    def encode_texts_dev(self, tok_slot: int, enc_slot: int, data: bytes, offsets, max_length: int, out_ptr: int):
+        txt, offs, n = self._texts(data, offsets)
+        self._check(self._L.rse_encode_texts_dev(self._h, int(tok_slot), int(enc_slot), txt, c_void_p(offs.ctypes.data),
+                                                 n, int(max_length), c_void_p(out_ptr)))
+
+    def rerank_docs_load_texts(self, tok_slot: int, ids, data: bytes, offsets):
+        """The rerank store from UTF-8 document texts, tokenized on the device (ids strictly ascending)."""
+        ids = _c(ids, np.int64)
+        txt, offs, n = self._texts(data, offsets)
+        if n != len(ids):
+            raise ValueError("offsets must have len(ids) + 1 entries")
+        self._check(self._L.rse_rerank_docs_load_texts(self._h, int(tok_slot), c_void_p(ids.ctypes.data), len(ids), txt,
+                                                       c_void_p(offs.ctypes.data)))
 
     def hybrid_rerank_timing(self):
         """Device ms of the last timed rerank run: (hybrid, assembly, encoder, order)."""

@@ -24,6 +24,7 @@
 #include "select.cuh"
 #include "knn_tc3.cuh"
 #include "rerank.cuh"
+#include "wordpiece.cuh"
 
 using namespace rse;
 
@@ -248,6 +249,20 @@ struct rse_index {
   int rr_nq = 0, rr_limit = 0;
   cudaEvent_t rr_ev[5] = {};       // rse_set_timing: hybrid | assembly | encoder | order boundaries of the last run
   bool rr_timed = false;
+
+  // ---- BERT WordPiece on the device (wordpiece.cuh): each tokenizer slot's tables in one allocation ...
+  struct TokSlot {
+    bool loaded = false;
+    void* blob = nullptr;
+    WpTables t{};
+  } tok[RSE_MAX_TOKENIZERS];
+  // ... and the last tokenisation: texts, offsets, per-text counts, cu_seqlens (int64 | int32), ids, meta (kWpMeta)
+  DevBuf tk_text, tk_offs, tk_count, tk_cu64, tk_cu32, tk_ids, tk_meta;
+  char* tk_pin = nullptr;          // pinned staging of texts | offsets
+  size_t tk_pin_bytes = 0;
+  unsigned long long* tk_pin_meta = nullptr;
+  int tk_n = 0;                    // texts of the last rse_tokenize (0: nothing to fetch)
+  int64_t tk_total = 0;
 
   // cudaFuncSetAttribute is per device: remember per HANDLE which kernels were configured (a process-wide static
   // flag would leave the second device of a multi-GPU process unconfigured)
@@ -1134,6 +1149,10 @@ void rse_destroy(rse_index* h) {
   if (h->rr_pin_meta) cudaFreeHost(h->rr_pin_meta);
   if (h->rr_pin_out) cudaFreeHost(h->rr_pin_out);
   for (cudaEvent_t e : h->rr_ev) if (e) cudaEventDestroy(e);
+  for (auto& t : h->tok) if (t.blob) cudaFree(t.blob);
+  for (DevBuf* b : {&h->tk_text, &h->tk_offs, &h->tk_count, &h->tk_cu64, &h->tk_cu32, &h->tk_ids, &h->tk_meta}) free_buf(*b);
+  if (h->tk_pin) cudaFreeHost(h->tk_pin);
+  if (h->tk_pin_meta) cudaFreeHost(h->tk_pin_meta);
   for (auto& e : h->enc) enc_release(e);
   free_ptr(h->dev_counters);
   if (h->comm) { if (NcclApi* n = nccl_api()) n->CommDestroy(h->comm); h->comm = nullptr; }
@@ -3151,6 +3170,291 @@ int rse_hybrid_rerank_timing(rse_index* h, float* out_ms) {
     return fail(h, RSE_ERR_STATE, "rse_hybrid_rerank_timing: the last rerank run was not timed (rse_set_timing)");
   CK(cudaEventSynchronize(h->rr_ev[4]));
   for (int i = 0; i < 4; ++i) CK(cudaEventElapsedTime(&out_ms[i], h->rr_ev[i], h->rr_ev[i + 1]));
+  return RSE_OK;
+}
+
+// ------------------------------------------------------------------ BERT WordPiece on the device (wordpiece.cuh)
+int rse_tokenizer_load(rse_index* h, int32_t slot, const rse_wordpiece_desc* d) {
+  if (!h) return RSE_ERR_INVALID;
+  if (slot < 0 || slot >= RSE_MAX_TOKENIZERS || !d) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: bad arguments");
+  const rse_wordpiece_desc& x = *d;
+  if (!x.cp_map || !x.cp_class || !x.extra || x.n_extra < 1 || !x.node_first || !x.node_id || x.n_nodes < 2 ||
+      x.n_added < 0 || (x.n_added > 0 && (!x.added || !x.added_offsets || !x.added_ids)))
+    return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: a table is missing");
+  if (x.n_added > kWpMaxAdded) return fail(h, RSE_ERR_UNSUPPORTED, "rse_tokenizer_load: more than 32 added tokens");
+  if (x.max_input_chars_per_word < 1 || x.max_input_chars_per_word > kWpMaxWordChars)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_tokenizer_load: max_input_chars_per_word must be in [1, 256]");
+  // every index the kernels follow is checked here, once
+  const int n_nodes = x.n_nodes;
+  if (x.node_first[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: node_first must start at 0");
+  for (int i = 0; i < n_nodes; ++i)
+    if (x.node_first[i + 1] < x.node_first[i]) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: node_first must not decrease");
+  const int n_edges = x.node_first[n_nodes];
+  if (n_edges > 0 && (!x.edge_cp || !x.edge_child)) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: edges missing");
+  for (int i = 0; i < n_nodes; ++i)
+    for (int j = x.node_first[i]; j < x.node_first[i + 1]; ++j)
+      if (x.edge_child[j] < 2 || x.edge_child[j] >= n_nodes || (j > x.node_first[i] && x.edge_cp[j] <= x.edge_cp[j - 1]))
+        return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: a trie edge is out of range or out of order");
+  if (std::min({x.unk_id, x.cls_id, x.sep_id}) < 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: negative special id");
+  for (int i = 0; i < n_nodes; ++i) {
+    if (x.node_id[i] < -1) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: node_id below -1");
+  }
+  for (int i = 0; i < kWpCodePoints; ++i) {
+    const uint32_t m = x.cp_map[i], c = (m >> 21) & 3, v = m & kWpCpMask;
+    if ((m >> 24) || (c == 1 && v >= static_cast<uint32_t>(kWpCodePoints)) || (c > 1 && v >= static_cast<uint32_t>(x.n_extra)) ||
+        x.cp_class[i] > kWpPunct)
+      return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: code point map entry " + std::to_string(i) + " is out of range");
+  }
+  for (int64_t i = 0; i < 3ll * x.n_extra; ++i)
+    if (x.extra[i] >= static_cast<uint32_t>(kWpCodePoints)) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: extra code point out of range");
+  uint32_t first[8] = {};
+  if (x.n_added > 0 && x.added_offsets[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: added_offsets must start at 0");
+  for (int a = 0; a < x.n_added; ++a) {
+    if (x.added_offsets[a + 1] <= x.added_offsets[a] || x.added_ids[a] < 0)
+      return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load: an added token is empty or has a negative id");
+    const uint8_t b = static_cast<uint8_t>(x.added[x.added_offsets[a]]);
+    first[b >> 5] |= 1u << (b & 31);
+  }
+  const int n_added_bytes = x.n_added > 0 ? x.added_offsets[x.n_added] : 0;
+  // one allocation: map | extra | cls | node_first | node_id | edge_cp | edge_child | added bytes | offsets | ids
+  size_t off[11], at = 0;
+  const size_t sz[10] = {4ull * kWpCodePoints, 12ull * x.n_extra, 1ull * kWpCodePoints, 4ull * (n_nodes + 1),
+                         4ull * n_nodes, 4ull * n_edges, 4ull * n_edges, 1ull * n_added_bytes,
+                         4ull * (x.n_added + 1), 4ull * x.n_added};
+  for (int i = 0; i < 10; ++i) { off[i] = at; at += (sz[i] + 255) / 256 * 256; }
+  off[10] = at;
+  std::vector<char> host(at);
+  const void* src[10] = {x.cp_map, x.extra, x.cp_class, x.node_first, x.node_id, x.edge_cp, x.edge_child, x.added,
+                         x.added_offsets, x.added_ids};
+  for (int i = 0; i < 10; ++i) if (sz[i] && src[i]) std::memcpy(host.data() + off[i], src[i], sz[i]);
+  CK(cudaSetDevice(h->device));
+  CK(cudaStreamSynchronize(h->stream));                       // a tokenisation may still read the old tables
+  auto& ts = h->tok[slot];
+  if (ts.blob) CK(cudaFree(ts.blob));
+  ts.blob = nullptr;
+  ts.loaded = false;
+  CK(cudaMalloc(&ts.blob, at));
+  CK(cudaMemcpy(ts.blob, host.data(), at, cudaMemcpyHostToDevice));
+  char* b = static_cast<char*>(ts.blob);
+  WpTables& t = ts.t;
+  t.map = reinterpret_cast<const uint32_t*>(b + off[0]);
+  t.extra = reinterpret_cast<const uint32_t*>(b + off[1]);
+  t.cls = reinterpret_cast<const uint8_t*>(b + off[2]);
+  t.node_first = reinterpret_cast<const int32_t*>(b + off[3]);
+  t.node_id = reinterpret_cast<const int32_t*>(b + off[4]);
+  t.edge_cp = reinterpret_cast<const int32_t*>(b + off[5]);
+  t.edge_child = reinterpret_cast<const int32_t*>(b + off[6]);
+  t.added_bytes = reinterpret_cast<const uint8_t*>(b + off[7]);
+  t.added_off = reinterpret_cast<const int32_t*>(b + off[8]);
+  t.added_id = reinterpret_cast<const int32_t*>(b + off[9]);
+  t.n_added = x.n_added;
+  std::memcpy(t.added_first, first, sizeof(first));
+  t.unk = x.unk_id; t.cls_id = x.cls_id; t.sep_id = x.sep_id; t.max_chars = x.max_input_chars_per_word;
+  ts.loaded = true;
+  return RSE_OK;
+}
+
+namespace {
+// texts -> pinned -> device, the count pass and the scan, then THE small copy back of the call (meta, synchronises).
+// Leaves the counts in tk_count and cu_seqlens in tk_cu64 / tk_cu32; *cap = pieces kept per text.
+int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs, int64_t n, int special, int max_length,
+              const char* who, unsigned long long* meta, int* cap) {
+  const std::string w(who);
+  if (slot < 0 || slot >= RSE_MAX_TOKENIZERS) return fail(h, RSE_ERR_INVALID, w + ": tokenizer slot out of range");
+  if (!h->tok[slot].loaded) return fail(h, RSE_ERR_STATE, w + ": no tokenizer in this slot (rse_tokenizer_load)");
+  if (n < 1 || n > INT_MAX || !offs) return fail(h, RSE_ERR_INVALID, w + ": bad arguments (n < 1 or offsets NULL)");
+  if (offs[0] != 0) return fail(h, RSE_ERR_INVALID, w + ": offsets must start at 0");
+  for (int64_t i = 0; i < n; ++i)
+    if (offs[i + 1] < offs[i]) return fail(h, RSE_ERR_INVALID, w + ": offsets must not decrease (at " + std::to_string(i) + ")");
+  const int64_t bytes = offs[n];
+  if (bytes > 0 && !text) return fail(h, RSE_ERR_INVALID, w + ": text is NULL");
+  if (special && max_length > 0 && max_length < 2)
+    return fail(h, RSE_ERR_UNSUPPORTED, w + ": max_length must be >= 2 with [CLS] / [SEP]");
+  *cap = max_length > 0 ? max_length - 2 * special : INT_MAX;
+  CK(cudaSetDevice(h->device));
+  // every call ends in a synchronise after its uploads, so the pinned buffer is free again here
+  const size_t ob = 8 * static_cast<size_t>(n + 1), need = ob + static_cast<size_t>(bytes);
+  if (h->tk_pin_bytes < need) {
+    if (h->tk_pin) CK(cudaFreeHost(h->tk_pin));
+    h->tk_pin = nullptr; h->tk_pin_bytes = 0;
+    CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin), need + need / 4 + 256));
+    h->tk_pin_bytes = need + need / 4 + 256;
+  }
+  if (!h->tk_pin_meta) CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin_meta), 8 * kWpMeta));
+  std::memcpy(h->tk_pin, offs, ob);
+  if (bytes > 0) std::memcpy(h->tk_pin + ob, text, bytes);
+  ENSURE(h->tk_offs, ob);
+  ENSURE(h->tk_text, std::max<size_t>(bytes, 1));
+  ENSURE(h->tk_count, 4 * static_cast<size_t>(n));
+  ENSURE(h->tk_cu64, ob);
+  ENSURE(h->tk_cu32, 4 * static_cast<size_t>(n + 1));
+  ENSURE(h->tk_meta, 8 * kWpMeta);
+  CK(cudaMemcpyAsync(h->tk_offs.p, h->tk_pin, ob, cudaMemcpyHostToDevice, h->stream));
+  if (bytes > 0) CK(cudaMemcpyAsync(h->tk_text.p, h->tk_pin + ob, bytes, cudaMemcpyHostToDevice, h->stream));
+  h->stats.h2d_bytes += static_cast<int64_t>(need);
+  auto* dm = static_cast<unsigned long long*>(h->tk_meta.p);
+  CK(cudaMemsetAsync(dm, 0, 8 * kWpMeta, h->stream));
+  CK(cudaMemsetAsync(dm + 1, 0xFF, 8, h->stream));
+  CK(cudaMemsetAsync(dm + 3, 0xFF, 8, h->stream));
+  const int ni = static_cast<int>(n);
+  wp_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+      h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni, special,
+      *cap, static_cast<int32_t*>(h->tk_count.p), dm);
+  LAUNCHED(h);
+  wp_scan_kernel<<<1, kWpScanThreads, 0, h->stream>>>(static_cast<const int32_t*>(h->tk_count.p), ni,
+                                                      static_cast<int64_t*>(h->tk_cu64.p),
+                                                      static_cast<int32_t*>(h->tk_cu32.p), dm);
+  LAUNCHED(h);
+  CK(cudaMemcpyAsync(h->tk_pin_meta, dm, 8 * kWpMeta, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += 8 * kWpMeta;
+  CK(cudaStreamSynchronize(h->stream));
+  std::memcpy(meta, h->tk_pin_meta, 8 * kWpMeta);
+  if (meta[0])
+    return fail(h, RSE_ERR_INVALID, w + ": text " + std::to_string(meta[1]) + " is not well-formed UTF-8 (" +
+                                        std::to_string(meta[0]) + " text(s))");
+  if (meta[2])
+    return fail(h, RSE_ERR_UNSUPPORTED, w + ": text " + std::to_string(meta[3]) + " holds combining marks of two code points "
+                                        "that NFD's canonical reordering could move (" + std::to_string(meta[2]) +
+                                        " text(s)); tokenize such texts on the host");
+  if (meta[4] > static_cast<unsigned long long>(INT_MAX))
+    return fail(h, RSE_ERR_UNSUPPORTED, w + ": more than 2^31 token ids in one call (split the batch)");
+  return RSE_OK;
+}
+
+// the write pass of the texts tok_count uploaded, into ids (device, tk_cu64 positions)
+int tok_write(rse_index* h, int32_t slot, int n, int special, int cap, int32_t* ids) {
+  wp_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+      h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n, special,
+      cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
+  LAUNCHED(h);
+  return RSE_OK;
+}
+
+// tokenize ([CLS] ... [SEP], cut at max_length) into tk_ids, then the BERT slot on them: out_dev [n, hidden] / [n]
+int enc_texts(rse_index* h, int32_t tok_slot, int32_t enc_slot, const char* text, const int64_t* offs, int32_t n,
+              int32_t max_length, float* out_dev) {
+  h->tk_n = 0;
+  int rc = enc_check(h, enc_slot, true);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[enc_slot];
+  if (e.clip) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: the slot holds a CLIP tower (its tokenizer is not WordPiece)");
+  if (!out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: out is NULL");
+  if (max_length < 2 || max_length > e.cfg.max_positions)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_encode_texts: max_length must be in [2, max_positions]");
+  unsigned long long m[kWpMeta];
+  int cap = 0;
+  rc = tok_count(h, tok_slot, text, offs, n, 1, max_length, "rse_encode_texts", m, &cap);
+  if (rc != RSE_OK) return rc;
+  if (m[6] >= static_cast<unsigned long long>(e.cfg.vocab_size))
+    return fail(h, RSE_ERR_INVALID, "rse_encode_texts: token id " + std::to_string(m[6]) + " >= the encoder's vocab_size " +
+                                        std::to_string(e.cfg.vocab_size));
+  const int T = static_cast<int>(m[4]);
+  ENSURE(h->tk_ids, 4 * static_cast<size_t>(T));
+  rc = tok_write(h, tok_slot, n, 1, cap, static_cast<int32_t*>(h->tk_ids.p));
+  if (rc != RSE_OK) return rc;
+  h->tk_n = n; h->tk_total = T;
+  return enc_forward(h, e, static_cast<const int32_t*>(h->tk_ids.p), nullptr, static_cast<const int32_t*>(h->tk_cu32.p), n,
+                     T, static_cast<int>(m[5]), out_dev);
+}
+}  // namespace
+
+int rse_tokenize(rse_index* h, int32_t slot, const char* text, const int64_t* offsets, int32_t n, int32_t add_special,
+                 int32_t max_length, int64_t* out_total, int32_t* out_max_len) {
+  if (!h) return RSE_ERR_INVALID;
+  h->tk_n = 0;
+  if (add_special != 0 && add_special != 1) return fail(h, RSE_ERR_INVALID, "rse_tokenize: add_special must be 0 or 1");
+  unsigned long long m[kWpMeta];
+  int cap = 0;
+  int rc = tok_count(h, slot, text, offsets, n, add_special, max_length, "rse_tokenize", m, &cap);
+  if (rc != RSE_OK) return rc;
+  ENSURE(h->tk_ids, 4 * std::max<size_t>(m[4], 1));
+  rc = tok_write(h, slot, n, add_special, cap, static_cast<int32_t*>(h->tk_ids.p));
+  if (rc != RSE_OK) return rc;
+  h->tk_n = n; h->tk_total = static_cast<int64_t>(m[4]);
+  if (out_total) *out_total = h->tk_total;
+  if (out_max_len) *out_max_len = static_cast<int32_t>(m[5]);
+  return RSE_OK;
+}
+
+int rse_tokens_fetch(rse_index* h, int32_t* ids_host, int32_t* cu_seqlens_host) {
+  if (!h) return RSE_ERR_INVALID;
+  if (h->tk_n < 1) return fail(h, RSE_ERR_STATE, "rse_tokens_fetch: nothing tokenized (rse_tokenize)");
+  if (!cu_seqlens_host || (h->tk_total > 0 && !ids_host)) return fail(h, RSE_ERR_INVALID, "rse_tokens_fetch: bad arguments");
+  CK(cudaSetDevice(h->device));
+  CK(cudaMemcpyAsync(cu_seqlens_host, h->tk_cu32.p, 4 * static_cast<size_t>(h->tk_n + 1), cudaMemcpyDeviceToHost, h->stream));
+  if (h->tk_total > 0)
+    CK(cudaMemcpyAsync(ids_host, h->tk_ids.p, 4 * static_cast<size_t>(h->tk_total), cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += 4 * static_cast<int64_t>(h->tk_n + 1 + h->tk_total);
+  CK(cudaStreamSynchronize(h->stream));
+  return RSE_OK;
+}
+
+int rse_tokens_fetch_dev(rse_index* h, int32_t* ids_dev, int32_t* cu_seqlens_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  if (h->tk_n < 1) return fail(h, RSE_ERR_STATE, "rse_tokens_fetch_dev: nothing tokenized (rse_tokenize)");
+  if (!cu_seqlens_dev || (h->tk_total > 0 && !ids_dev)) return fail(h, RSE_ERR_INVALID, "rse_tokens_fetch_dev: bad arguments");
+  CK(cudaSetDevice(h->device));
+  CK(cudaMemcpyAsync(cu_seqlens_dev, h->tk_cu32.p, 4 * static_cast<size_t>(h->tk_n + 1), cudaMemcpyDeviceToDevice, h->stream));
+  if (h->tk_total > 0)
+    CK(cudaMemcpyAsync(ids_dev, h->tk_ids.p, 4 * static_cast<size_t>(h->tk_total), cudaMemcpyDeviceToDevice, h->stream));
+  return RSE_OK;
+}
+
+int rse_encode_texts_dev(rse_index* h, int32_t tok_slot, int32_t enc_slot, const char* text, const int64_t* offsets,
+                         int32_t n, int32_t max_length, float* out_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  return enc_texts(h, tok_slot, enc_slot, text, offsets, n, max_length, out_dev);
+}
+
+int rse_encode_texts(rse_index* h, int32_t tok_slot, int32_t enc_slot, const char* text, const int64_t* offsets,
+                     int32_t n, int32_t max_length, float* out_host) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = enc_check(h, enc_slot, true);
+  if (rc != RSE_OK) return rc;
+  if (!out_host || n < 1) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: bad arguments");
+  Encoder& e = h->enc[enc_slot];
+  if (e.clip) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: the slot holds a CLIP tower (its tokenizer is not WordPiece)");
+  const size_t n_out = static_cast<size_t>(n) * (e.cfg.head == 0 ? e.cfg.hidden : 1);
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.out, sizeof(float) * n_out);
+  rc = enc_texts(h, tok_slot, enc_slot, text, offsets, n, max_length, static_cast<float*>(e.out.p));
+  if (rc != RSE_OK) return rc;
+  CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);
+  CK(cudaStreamSynchronize(h->stream));
+  return RSE_OK;
+}
+
+int rse_rerank_docs_load_texts(rse_index* h, int32_t tok_slot, const int64_t* ids, int64_t n_docs, const char* text,
+                               const int64_t* offsets) {
+  if (!h) return RSE_ERR_INVALID;
+  h->tk_n = 0;
+  if (n_docs < 1 || n_docs > INT_MAX || !ids) return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load_texts: bad arguments");
+  for (int64_t i = 1; i < n_docs; ++i)
+    if (ids[i] <= ids[i - 1])
+      return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load_texts: ids must be strictly ascending (at " + std::to_string(i) + ")");
+  unsigned long long m[kWpMeta];
+  int cap = 0;
+  int rc = tok_count(h, tok_slot, text, offsets, n_docs, 0, 0, "rse_rerank_docs_load_texts", m, &cap);
+  if (rc != RSE_OK) return rc;
+  const int64_t n_tok = static_cast<int64_t>(m[4]);
+  free_ptr(h->rr_doc_ids); free_ptr(h->rr_doc_indptr); free_ptr(h->rr_doc_tok);   // (tok_count synchronised)
+  h->rr_n_docs = 0; h->rr_max_tok = -1;
+  CK(cudaMalloc(&h->rr_doc_ids, 8 * n_docs));
+  CK(cudaMalloc(&h->rr_doc_indptr, 8 * (n_docs + 1)));
+  CK(cudaMalloc(&h->rr_doc_tok, 4 * std::max<int64_t>(n_tok, 1)));
+  CK(cudaMemcpy(h->rr_doc_ids, ids, 8 * n_docs, cudaMemcpyHostToDevice));
+  CK(cudaMemcpyAsync(h->rr_doc_indptr, h->tk_cu64.p, 8 * (n_docs + 1), cudaMemcpyDeviceToDevice, h->stream));
+  rc = tok_write(h, tok_slot, static_cast<int>(n_docs), 0, cap, h->rr_doc_tok);
+  if (rc != RSE_OK) return rc;
+  CK(cudaStreamSynchronize(h->stream));
+  h->rr_n_docs = n_docs; h->rr_max_tok = n_tok > 0 ? static_cast<int32_t>(m[6]) : -1;
+  h->rr_max_doc_len = static_cast<int64_t>(m[5]);
+  // a store load is a one-off bulk upload: give its staging back instead of keeping ~1 KB per document in HBM and
+  // pinned memory
+  for (DevBuf* b : {&h->tk_text, &h->tk_offs, &h->tk_count, &h->tk_cu64, &h->tk_cu32}) free_buf(*b);
+  if (h->tk_pin) CK(cudaFreeHost(h->tk_pin));
+  h->tk_pin = nullptr; h->tk_pin_bytes = 0;
   return RSE_OK;
 }
 

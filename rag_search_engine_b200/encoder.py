@@ -7,9 +7,11 @@
   (rag_search_engine/utils/hybrid_search.py:296-297): pass it as ``HybridSearch(cross_encoder=...)``.
 
 Both run csrc/encoder.cuh through the C-ABI (``rse_encoder_*``, ``rse_encode``): HuggingFace BERT weights handed
-over under their state_dict names, fp32 throughout.  Tokenisation stays on the host and is pluggable: a
-HuggingFace tokenizer when one is available (``from_sentence_transformer`` / ``from_cross_encoder`` take it from
-the loaded reference model), or any callable returning token-id lists.  No weights are bundled and nothing is
+over under their state_dict names, fp32 throughout.  The tokenizer is pluggable: ``DeviceWordPiece`` runs a BERT
+WordPiece tokenizer on the device (csrc/wordpiece.cuh, ids identical to the HF fast tokenizer), and any callable
+returning token-id lists runs on the host.  ``from_sentence_transformer`` / ``from_cross_encoder`` take the loaded
+reference model's tokenizer and put it on the device when its pipeline is BERT WordPiece
+(``wordpiece.build_tables`` decides from the tokenizer object).  No weights are bundled and nothing is
 downloaded: without ``sentence-transformers`` (and its checkpoints) on the machine the caller supplies a
 ``state_dict`` — the tests use a randomly initialised ``transformers.BertModel`` of the same architecture.
 """
@@ -94,6 +96,78 @@ def pack(id_lists: Sequence[Sequence[int]], type_lists: Optional[Sequence[Sequen
     return ids, tt, cu
 
 
+def _utf8(texts):
+    """Texts -> (UTF-8 bytes back to back, int64 byte offsets [n + 1])."""
+    raw = [t.encode("utf-8") for t in texts]
+    offs = np.zeros(len(raw) + 1, np.int64)
+    np.cumsum([len(r) for r in raw], out=offs[1:])
+    return b"".join(raw), offs
+
+
+from .wordpiece import host_ids, plain_backend  # noqa: E402
+
+
+class DeviceWordPiece:
+    """A BERT WordPiece tokenizer on the device (csrc/wordpiece.cuh) in a tokenizer slot of ``index``.
+
+    Called on texts it returns what ``hf_tok(texts, add_special_tokens=..., truncation=..., max_length=...)
+    ["input_ids"]`` returns, so it drops into every ``tokenizer=`` argument; ``add_special_tokens`` / ``max_length``
+    fix which call it stands for (``max_length=None``: no cut).  The encoders use its device paths instead, where
+    the ids never become Python lists.  A text NFD could reorder (two code points whose combining marks survive the
+    accent stripping, see include/rse.h) goes to ``hf_tok``'s own Rust tokenizer on the host and is counted in
+    ``host_texts``.  ``UnsupportedTokenizer`` when ``hf_tok`` is not BERT WordPiece; ``maybe`` returns None then."""
+
+    def __init__(self, index, hf_tok, *, slot: int = 0, add_special_tokens: bool = True,
+                 max_length: Optional[int] = None):
+        from .wordpiece import build_tables
+        self.tables = build_tables(hf_tok)
+        self.backend = plain_backend(hf_tok)
+        self.index, self.slot = index, int(slot)
+        self.add_special_tokens = bool(add_special_tokens)
+        self.max_length = None if max_length is None else int(max_length)
+        self.cls_id, self.sep_id = self.tables.cls_id, self.tables.sep_id
+        self.host_texts = 0
+        index.tokenizer_load(self.slot, self.tables)
+
+    @classmethod
+    def maybe(cls, index, hf_tok, **kw) -> Optional["DeviceWordPiece"]:
+        from .wordpiece import UnsupportedTokenizer
+        try:
+            return cls(index, hf_tok, **kw)
+        except UnsupportedTokenizer:
+            return None
+
+    def host_ids(self, texts, add_special: bool, max_length: Optional[int]) -> List[List[int]]:
+        """The host tokenizer's ids under the same rule (the route of the texts the device refuses)."""
+        self.host_texts += len(texts)
+        return host_ids(self.backend, texts, add_special, max_length, self.cls_id, self.sep_id)
+
+    def host_routed(self, texts) -> List[int]:
+        return [i for i, t in enumerate(texts) if self.tables.needs_host(t)]
+
+    def tokenize(self, texts, add_special: Optional[bool] = None, max_length: Optional[int] = -1):
+        """-> (ids int32[total], cu_seqlens int32[n + 1]) on the host; defaults are this object's call rule."""
+        sp = self.add_special_tokens if add_special is None else bool(add_special)
+        ml = self.max_length if max_length == -1 else max_length
+        texts = list(texts)
+        routed = self.host_routed(texts)
+        if routed:
+            got = {i: ids for i, ids in zip(routed, self.host_ids([texts[i] for i in routed], sp, ml))}
+            keep = [i for i in range(len(texts)) if i not in got]
+            dev = self.__call__([texts[i] for i in keep], sp, ml) if keep else []
+            got.update(zip(keep, dev))
+            return pack([got[i] for i in range(len(texts))])[::2]
+        if not texts:
+            return np.zeros(0, np.int32), np.zeros(1, np.int32)
+        data, offs = _utf8(texts)
+        return self.index.tokenize(self.slot, data, offs, sp, ml or 0)
+
+    def __call__(self, texts, add_special: Optional[bool] = None, max_length: Optional[int] = -1) -> List[List[int]]:
+        ids, cu = self.tokenize(texts, add_special, max_length)
+        ids = ids.tolist()
+        return [ids[a:b] for a, b in zip(cu[:-1].tolist(), cu[1:].tolist())]
+
+
 def hf_text_tokenizer(hf_tok) -> Callable[[List[str]], List[List[int]]]:
     """A HuggingFace tokenizer as the single-text tokenizer of the batched rerank: ids without special tokens.  With a
     fast tokenizer these are exactly the segments its pair encoding (truncation=True) is built from."""
@@ -118,7 +192,9 @@ class GpuSentenceEncoder:
         bert = st_model[0].auto_model
         hf_tok = st_model.tokenizer
         msl = int(getattr(st_model, "max_seq_length", 256) or 256)
-        tok = lambda texts: hf_tok(list(texts), truncation=True, max_length=msl)["input_ids"]   # noqa: E731
+        tok = DeviceWordPiece.maybe(index, hf_tok, slot=slot, max_length=msl)
+        if tok is None:
+            tok = lambda texts: hf_tok(list(texts), truncation=True, max_length=msl)["input_ids"]   # noqa: E731
         return cls(index, bert.state_dict(), config_from_hf(bert.config), tok, slot=slot, max_seq_length=msl)
 
     def get_sentence_embedding_dimension(self) -> int:
@@ -147,12 +223,49 @@ class GpuSentenceEncoder:
         self.index.encode_dev(self.slot, ids, cu, out_ptr)
         return len(id_lists)
 
-    def encode(self, texts, show_progress_bar: bool = False, **_kw) -> np.ndarray:
+    def encode_texts_dev(self, texts: Sequence[str], out_ptr: int) -> int:
+        """Texts -> [n, hidden] fp32 at ``out_ptr`` on the device; with a ``DeviceWordPiece`` the ids never leave
+        the device, otherwise the host tokenizer's ids go through ``encode_ids_dev``.  Returns n."""
+        texts = list(texts)
+        tok = self.tokenizer
+        if not isinstance(tok, DeviceWordPiece) or tok.host_routed(texts):
+            return self.encode_ids_dev(self._host_tokenize(texts), out_ptr)
+        data, offs = _utf8(texts)
+        self.index.encode_texts_dev(tok.slot, self.slot, data, offs, self.max_seq_length, out_ptr)
+        return len(texts)
+
+    def _host_tokenize(self, texts):
+        tok = self.tokenizer
+        if isinstance(tok, DeviceWordPiece):
+            return tok(texts, True, self.max_seq_length)
+        return tok(texts)
+
+    def encode(self, texts, show_progress_bar: bool = False, max_tokens_per_call: int = 1 << 16, **_kw) -> np.ndarray:
         if self.tokenizer is None:
             raise RuntimeError("GpuSentenceEncoder has no tokenizer: pass tokenizer=<texts -> token-id lists> "
                                "(e.g. the reference model's HuggingFace tokenizer) or call encode_ids")
         single = isinstance(texts, str)
-        out = self.encode_ids(self.tokenizer([texts] if single else list(texts)))
+        texts = [texts] if single else list(texts)
+        tok = self.tokenizer
+        if not texts or not isinstance(tok, DeviceWordPiece) or tok.host_routed(texts):
+            out = self.encode_ids(self._host_tokenize(texts), max_tokens_per_call)
+            return out[0] if single else out
+        data, offs = _utf8(texts)
+        msl = self.max_seq_length
+        if int(np.minimum(np.diff(offs) + 2, msl).sum()) <= max_tokens_per_call:
+            # a text has at most one id per UTF-8 byte plus [CLS] / [SEP]: the batch fits one call, and its ids
+            # stay on the device
+            out = self.index.encode_texts(tok.slot, self.slot, data, offs, msl)
+        else:
+            # a bulk embedding: ids tokenized on the device come back as arrays and are cut into slices of at most
+            # max_tokens_per_call by their real lengths (the byte bound is ~6x the token count of English text)
+            ids, cu = self.index.tokenize(tok.slot, data, offs, True, msl)
+            out = np.empty((len(texts), int(self.config["hidden"])), np.float32)
+            lo = 0
+            while lo < len(texts):
+                hi = max(lo + 1, int(np.searchsorted(cu, int(cu[lo]) + max_tokens_per_call, side="right")) - 1)
+                out[lo:hi] = self.index.encode(self.slot, ids[cu[lo]:cu[hi]], cu[lo:hi + 1] - cu[lo])
+                lo = hi
         return out[0] if single else out
 
 
@@ -189,8 +302,10 @@ class GpuCrossEncoder:
             enc = hf_tok([p[0] for p in pairs], [p[1] for p in pairs], truncation=True, max_length=ml)
             return enc["input_ids"], enc["token_type_ids"]
         sd = {k: v for k, v in model.state_dict().items()}
+        single = DeviceWordPiece.maybe(index, hf_tok, slot=slot, add_special_tokens=False)
         return cls(index, sd, config_from_hf(model.config), tok, slot=slot, max_length=ml,
-                   tokenizer=hf_text_tokenizer(hf_tok), cls_id=hf_tok.cls_token_id, sep_id=hf_tok.sep_token_id)
+                   tokenizer=single if single is not None else hf_text_tokenizer(hf_tok), cls_id=hf_tok.cls_token_id,
+                   sep_id=hf_tok.sep_token_id)
 
     def tokenize(self, texts) -> List[List[int]]:
         """Single texts -> token ids without special tokens (the pieces the device assembles into pairs)."""

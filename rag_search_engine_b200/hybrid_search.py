@@ -21,6 +21,7 @@ from typing import Any, Dict, List, Optional, Sequence
 import numpy as np
 
 from . import _lib, runtime
+from .encoder import DeviceWordPiece, _utf8
 from .keyword_search import DEFAULT_DB_PATH, KeywordSearch
 from .semantic_search import SemanticSearch
 
@@ -249,7 +250,8 @@ class HybridSearch:
         ``rerank_method="cross_encoder"`` ranks like ``rrf_search(q, rerank_method="cross_encoder")`` for the whole
         batch on the device (``self.cross_encoder``, a ``GpuCrossEncoder`` on this object's handle, after
         ``load_rerank_documents``): ``rerank_query_ids`` are the cross-encoder tokenizer's ids of each query without
-        special tokens (``cross_encoder.tokenize(texts)``).  Hits are {id, score, bm25_rank, sem_rank, rrf_rank,
+        special tokens (``cross_encoder.tokenize(texts)``), or the query strings, which that tokenizer then
+        tokenizes.  Hits are {id, score, bm25_rank, sem_rank, rrf_rank,
         cross_encoder_score}; ``as_arrays=True`` gives (id, score, bm25_rank, sem_rank, rrf_rank, cross_encoder_score,
         count) with int32 ranks (-1 = None)."""
         if rerank_method is not None:
@@ -281,8 +283,10 @@ class HybridSearch:
         """Text in: the query vectors are produced by ``encoder`` (encoder.GpuSentenceEncoder) ON THE DEVICE and
         handed to the hybrid step there (``rse_encode_dev`` -> ``rse_hybrid_stage_dev``): no host hop for the
         vectors.  ``token_lists`` are the BM25 tokens of the queries (the reference's ``preprocess`` output),
-        ``encoder_ids`` the encoder's token ids ([CLS] ... [SEP]) of the same queries.  ``rerank_method`` /
-        ``rerank_query_ids`` as in ``rrf_search_batch``."""
+        ``encoder_ids`` the encoder's token ids ([CLS] ... [SEP]) of the same queries, or the query strings
+        themselves (tokenized by the encoder's tokenizer; on the device with a ``DeviceWordPiece``).  ``rerank_method``
+        / ``rerank_query_ids`` as in ``rrf_search_batch``; given query strings, ``rerank_query_ids`` may be omitted
+        and the cross-encoder's tokenizer makes them from the strings."""
         import torch
         ce = self._rerank_encoder(rerank_method) if rerank_method is not None else None
         if not self._gpu_retrievers():
@@ -294,7 +298,13 @@ class HybridSearch:
         if buf is None or buf.shape[0] < nq:
             buf = self._qvec_dev = torch.empty((max(nq, 256), self._index.dim), dtype=torch.float32,
                                                device=torch.device("cuda", self.device))
-        n = encoder.encode_ids_dev(encoder_ids, buf.data_ptr())
+        texts = len(encoder_ids) > 0 and all(isinstance(x, str) for x in encoder_ids)
+        if texts:
+            n = encoder.encode_texts_dev(encoder_ids, buf.data_ptr())
+            if ce is not None and rerank_query_ids is None:
+                rerank_query_ids = list(encoder_ids)
+        else:
+            n = encoder.encode_ids_dev(encoder_ids, buf.data_ptr())
         if n != nq:
             raise ValueError("token_lists and encoder_ids describe different numbers of queries")
         self._index.hybrid_stage_dev(nq, buf.data_ptr(), tok_indptr, rows)
@@ -326,6 +336,12 @@ class HybridSearch:
             for i in universe.tolist():
                 title, desc = rows.get(i, ("<missing>", ""))
                 texts.append(f"{title} - {desc or ''}")
+            tok = ce.tokenizer
+            if isinstance(tok, DeviceWordPiece) and not tok.host_routed(texts):
+                # tokenized on the device straight into the store (universe is ascending): no host id lists
+                data, offs = _utf8(texts)
+                self._index.rerank_docs_load_texts(tok.slot, universe, data, offs)
+                return len(universe)
             ids, token_lists = universe, ce.tokenize(texts)
         ids = np.asarray(ids, np.int64)
         if len(token_lists) != len(ids):
@@ -355,6 +371,8 @@ class HybridSearch:
     def _rerank_staged(self, ce, nq, rerank_query_ids, k, limit, knn_multiplier, k1, b, as_arrays):
         if rerank_query_ids is None or len(rerank_query_ids) != nq:
             raise ValueError("rerank_query_ids must hold the cross-encoder token ids of every query")
+        if all(isinstance(x, str) for x in rerank_query_ids):
+            rerank_query_ids = ce.tokenize(rerank_query_ids)
         q_ptr = np.zeros(nq + 1, np.int32)
         np.cumsum([len(x) for x in rerank_query_ids], out=q_ptr[1:])
         q_ids = np.fromiter(itertools.chain.from_iterable(rerank_query_ids), np.int32, count=int(q_ptr[-1]))
