@@ -318,6 +318,44 @@ typedef struct rse_clip_config {
 int rse_clip_create(rse_index *h, int32_t slot, const rse_clip_config *cfg);
 int rse_encode_images(rse_index *h, int32_t slot, const float *pixels_host, int32_t n, float *out_host);
 int rse_encode_images_dev(rse_index *h, int32_t slot, const float *pixels_dev, int32_t n, float *out_dev);
+
+/* ------------------------------------------------------------------ CLIP image preprocessing on the device
+ * transformers' CLIPImageProcessor (backend 0: torchvision, aten's uint8 antialiased bicubic) or
+ * CLIPImageProcessorPil (backend 1: Pillow's bicubic) from decoded RGB pixels, bit for bit (csrc/imgproc.cuh):
+ * resize to shortest_edge, center crop, rescale / normalise, CHW.  rse_imgproc_set binds a configuration to a CLIP
+ * vision slot (a new one replaces it); it requires do_resize and do_center_crop, crop_height == crop_width == the
+ * tower's image_size <= shortest_edge (so the processor never pads), rescale_factor > 0 and std != 0.
+ * Images: n packed HWC uint8 RGB in host memory, image i at byte offsets[i] with height hw[2i], width hw[2i + 1]:
+ *   rse_image_preprocess(_dev)  -> pixel_values [n, 3, image_size, image_size] fp32, host or device memory;
+ *   rse_encode_images_u8(_dev)  -> the vision tower's [n, projection_dim], host or device memory.
+ * The pixels go up in chunks of at most RSE_IMGPROC_CHUNK_BYTES through pinned staging, the copy of one chunk
+ * overlapping the kernels of the previous.  Per image, outside these limits RSE_ERR_UNSUPPORTED (the message names
+ * the image): H * W <= RSE_IMGPROC_MAX_PIXELS, each resized side <= RSE_IMGPROC_MAX_EDGE, a downscale of at most
+ * RSE_IMGPROC_MAX_SCALE per axis, and (backend 1) not more than 100 times taller than wide while shrinking vertically
+ * (Pillow then runs the vertical pass first).  A slot that is not a CLIP vision tower: RSE_ERR_INVALID; one without
+ * a configuration: RSE_ERR_STATE. */
+#define RSE_IMGPROC_MAX_PIXELS (1 << 24)
+#define RSE_IMGPROC_MAX_EDGE 65536
+#define RSE_IMGPROC_MAX_SCALE 32
+#define RSE_IMGPROC_CHUNK_BYTES (64 << 20)
+typedef struct rse_imgproc_cfg {
+  int32_t backend;                   /* 0 = CLIPImageProcessor (torchvision), 1 = CLIPImageProcessorPil */
+  int32_t shortest_edge;
+  int32_t crop_height, crop_width;
+  int32_t do_resize, do_center_crop, do_rescale, do_normalize;
+  double rescale_factor;
+  double mean[3], std[3];
+} rse_imgproc_cfg;
+int rse_imgproc_set(rse_index *h, int32_t vision_slot, const rse_imgproc_cfg *cfg);
+int rse_image_preprocess(rse_index *h, int32_t slot, const uint8_t *pixels, const int64_t *offsets,
+                         const int32_t *hw, int32_t n, float *out_host);
+int rse_image_preprocess_dev(rse_index *h, int32_t slot, const uint8_t *pixels, const int64_t *offsets,
+                             const int32_t *hw, int32_t n, float *out_dev);
+int rse_encode_images_u8(rse_index *h, int32_t slot, const uint8_t *pixels, const int64_t *offsets,
+                         const int32_t *hw, int32_t n, float *out_host);
+int rse_encode_images_u8_dev(rse_index *h, int32_t slot, const uint8_t *pixels, const int64_t *offsets,
+                             const int32_t *hw, int32_t n, float *out_dev);
+
 /* rse_hybrid_stage with the query vectors already ON THE DEVICE ([nq, dim] fp32, e.g. rse_encode_dev's output);
  * tokens still come from the host.  Followed by rse_hybrid_run / rse_hybrid_fetch as usual. */
 int rse_hybrid_stage_dev(rse_index *h, int32_t nq, const float *q_dev, const int32_t *tok_indptr,

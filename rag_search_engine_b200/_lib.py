@@ -73,6 +73,14 @@ class RseClipConfig(ctypes.Structure):
                 ("eos_token_id", c_int32), ("ln_eps", c_float)]
 
 
+class RseImgprocCfg(ctypes.Structure):
+    """include/rse.h rse_imgproc_cfg."""
+    _fields_ = [("backend", c_int32), ("shortest_edge", c_int32), ("crop_height", c_int32), ("crop_width", c_int32),
+                ("do_resize", c_int32), ("do_center_crop", c_int32), ("do_rescale", c_int32),
+                ("do_normalize", c_int32), ("rescale_factor", c_double), ("mean", c_double * 3),
+                ("std", c_double * 3)]
+
+
 class RseWordpieceDesc(ctypes.Structure):
     """include/rse.h rse_wordpiece_desc."""
     _fields_ = [("cp_map", c_void_p), ("extra", c_void_p), ("n_extra", c_int32), ("cp_class", c_void_p),
@@ -148,6 +156,11 @@ _SIGNATURES = {
     "rse_clip_create": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseClipConfig)]),
     "rse_encode_images": (ctypes.c_int, [c_void_p, c_int32, POINTER(c_float), c_int32, POINTER(c_float)]),
     "rse_encode_images_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
+    "rse_imgproc_set": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseImgprocCfg)]),
+    "rse_image_preprocess": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    "rse_image_preprocess_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    "rse_encode_images_u8": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    "rse_encode_images_u8_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
     "rse_hybrid_stage_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "rse_rerank_docs_load": (ctypes.c_int, [c_void_p, POINTER(c_int64), c_int64, POINTER(c_int64), POINTER(c_int32)]),
     "rse_hybrid_rerank_run": (ctypes.c_int, [c_void_p, c_int32, c_double, c_int32, c_int32, c_int32, c_double, c_double,
@@ -563,6 +576,57 @@ class Index:
     def encode_images_dev(self, slot: int, pixels_ptr: int, n: int, out_ptr: int):
         """Same with the pixels on the device and the result left there (asynchronous on the handle's stream)."""
         self._check(self._L.rse_encode_images_dev(self._h, int(slot), c_void_p(pixels_ptr), int(n), c_void_p(out_ptr)))
+
+    def imgproc_set(self, slot: int, *, backend: int, shortest_edge: int, crop_height: int, crop_width: int,
+                    rescale_factor: float, mean, std, do_resize: bool = True, do_center_crop: bool = True,
+                    do_rescale: bool = True, do_normalize: bool = True):
+        """Bind a CLIP image-preprocessing configuration (0 = CLIPImageProcessor, 1 = CLIPImageProcessorPil numerics)
+        to the vision tower in ``slot`` (rse_imgproc_set)."""
+        cfg = RseImgprocCfg(int(backend), int(shortest_edge), int(crop_height), int(crop_width), int(bool(do_resize)),
+                            int(bool(do_center_crop)), int(bool(do_rescale)), int(bool(do_normalize)),
+                            float(rescale_factor), (c_double * 3)(*map(float, mean)), (c_double * 3)(*map(float, std)))
+        self._check(self._L.rse_imgproc_set(self._h, int(slot), ctypes.byref(cfg)))
+
+    @staticmethod
+    def _pack_images(images):
+        """[H, W, 3] uint8 arrays -> (packed bytes, int64 offsets [n], int32 hw [n, 2])."""
+        arrs = [np.ascontiguousarray(a, np.uint8) for a in images]
+        for a in arrs:
+            if a.ndim != 3 or a.shape[2] != 3:
+                raise ValueError("images must be [H, W, 3] uint8 (RGB)")
+        sizes = np.array([a.size for a in arrs], np.int64)
+        offs = np.zeros(len(arrs), np.int64)
+        np.cumsum(sizes[:-1], out=offs[1:])
+        packed = np.empty(int(sizes.sum()), np.uint8)
+        for a, o, n in zip(arrs, offs, sizes):
+            packed[o:o + n] = a.reshape(-1)
+        hw = np.array([a.shape[:2] for a in arrs], np.int32).reshape(-1, 2)
+        return packed, offs, hw
+
+    def image_preprocess(self, slot: int, images) -> np.ndarray:
+        """[H, W, 3] uint8 RGB images (any sizes) -> pixel_values [n, 3, S, S] float32 through the slot's
+        preprocessing configuration, on the device."""
+        packed, offs, hw = self._pack_images(images)
+        cfg = self._enc_cfg[int(slot)]
+        out = np.zeros((len(offs), 3, cfg.image_size, cfg.image_size), np.float32)
+        self._check(self._L.rse_image_preprocess(self._h, int(slot), packed.ctypes.data, offs.ctypes.data,
+                                                 hw.ctypes.data, len(offs), out.ctypes.data))
+        return out
+
+    def encode_images_u8(self, slot: int, images) -> np.ndarray:
+        """[H, W, 3] uint8 RGB images -> [n, projection_dim] float32: preprocessing and the vision tower on the device."""
+        packed, offs, hw = self._pack_images(images)
+        out = np.zeros((len(offs), self._enc_cfg[int(slot)].projection_dim), np.float32)
+        self._check(self._L.rse_encode_images_u8(self._h, int(slot), packed.ctypes.data, offs.ctypes.data,
+                                                 hw.ctypes.data, len(offs), out.ctypes.data))
+        return out
+
+    def encode_images_u8_dev(self, slot: int, images, out_ptr: int):
+        """Same with the embeddings left on the device at ``out_ptr`` (asynchronous on the handle's stream once the
+        pixels are staged)."""
+        packed, offs, hw = self._pack_images(images)
+        self._check(self._L.rse_encode_images_u8_dev(self._h, int(slot), packed.ctypes.data, offs.ctypes.data,
+                                                     hw.ctypes.data, len(offs), c_void_p(out_ptr)))
 
     def encoder_set_tensor(self, slot: int, name: str, data):
         a = _c(data, np.float32).reshape(-1)

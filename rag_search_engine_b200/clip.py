@@ -6,11 +6,12 @@
 (``rse_clip_create``, ``rse_encode`` for text, ``rse_encode_images`` for images) in fp32; the output is what
 sentence-transformers' CLIP ``encode`` returns: ``get_text_features`` / ``get_image_features``, not normalised.
 
-Tokenisation (BPE) and image decoding / resizing / cropping stay on the host: the tokenizer is any callable
-``texts -> token-id lists`` (or a HuggingFace tokenizer), the image processor any callable ``images ->
-pixel_values [n, 3, S, S]`` (or a HuggingFace image processor).  ``from_sentence_transformer`` takes the weights,
-the tokenizer and the image processor from a loaded reference model.  No weights are bundled and nothing is
-downloaded.
+Tokenisation (BPE) and image decoding stay on the host: the tokenizer is any callable ``texts -> token-id lists``
+(or a HuggingFace tokenizer), the image processor any callable ``images -> pixel_values [n, 3, S, S]`` (or a
+HuggingFace image processor).  ``from_sentence_transformer`` takes the weights, the tokenizer and the image processor
+from a loaded reference model; when the image processor is a CLIP one ``DeviceImageProcessor`` accepts, the resize,
+crop and normalisation run on the device (csrc/imgproc.cuh) from the decoded uint8 pixels, bit for bit what the
+processor returns.  No weights are bundled and nothing is downloaded.
 """
 from __future__ import annotations
 
@@ -72,6 +73,102 @@ def tower_tensors(state_dict, tower: int) -> Iterator[Tuple[str, np.ndarray]]:
         yield name, a.astype(np.float32, copy=False)
 
 
+# per-image limits of the device preprocessing (include/rse.h RSE_IMGPROC_*): beyond them an image takes the host
+# processor.  2^24 pixels (48 MB of RGB, e.g. 4096 x 4096) keeps every image inside one 64 MB staging chunk; a
+# downscale of at most 32 per axis bounds the taps per output (129) and so the coefficient table.
+MAX_PIXELS = 1 << 24
+MAX_EDGE = 65536
+MAX_SCALE = 32
+
+
+def resized_size(h: int, w: int, shortest_edge: int) -> Tuple[int, int]:
+    """transformers' ``get_resize_output_image_size(default_to_square=False)``: (new_h, new_w)."""
+    short, long = (w, h) if w <= h else (h, w)
+    new_short, new_long = shortest_edge, int(shortest_edge * long / short)
+    return (new_long, new_short) if w <= h else (new_short, new_long)
+
+
+def _size_dict(size) -> dict:
+    if size is None:
+        return {}
+    keys = ("height", "width", "shortest_edge", "longest_edge", "max_height", "max_width")
+    d = dict(size) if isinstance(size, dict) else {k: getattr(size, k, None) for k in keys}
+    return {k: v for k, v in d.items() if v is not None}
+
+
+class DeviceImageProcessor:
+    """CLIP's image processor on the device: ``CLIPImageProcessor`` (torchvision backend) or ``CLIPImageProcessorPil``
+    numerics, chosen from the processor object, bound to the vision tower in ``slot`` (``rse_imgproc_set``).
+
+    ``maybe`` returns None for any configuration the device does not implement: another resample filter than BICUBIC,
+    a size other than ``{"shortest_edge": n}``, no center crop, a crop other than the tower's square image_size or
+    larger than the resized image (the processor would pad), ``do_pad``.  Images whose size is outside the device's
+    limits (``device_ok``) go through the host processor and are counted in ``host_images``."""
+
+    def __init__(self, index, hf_image_processor, slot: int):
+        p = hf_image_processor
+        self.index, self.slot, self.hf = index, int(slot), p
+        self.backend = 1 if getattr(p, "backend", "torchvision") == "pil" else 0
+        self.shortest_edge = int(_size_dict(p.size)["shortest_edge"])
+        crop = _size_dict(p.crop_size)
+        self.crop = int(crop["height"])
+        self.do_convert_rgb = bool(getattr(p, "do_convert_rgb", True))
+        self.host_images = 0
+        index.imgproc_set(self.slot, backend=self.backend, shortest_edge=self.shortest_edge, crop_height=self.crop,
+                          crop_width=int(crop["width"]), rescale_factor=float(p.rescale_factor),
+                          mean=list(p.image_mean), std=list(p.image_std), do_resize=True, do_center_crop=True,
+                          do_rescale=bool(p.do_rescale), do_normalize=bool(p.do_normalize))
+
+    @classmethod
+    def supported(cls, hf_image_processor, image_size: int) -> bool:
+        try:
+            import transformers
+        except ImportError:
+            return False
+        p = hf_image_processor
+        kinds = tuple(getattr(transformers, n) for n in ("CLIPImageProcessor", "CLIPImageProcessorPil")
+                      if hasattr(transformers, n))
+        if not kinds or type(p) not in kinds:
+            return False
+        size, crop = _size_dict(getattr(p, "size", None)), _size_dict(getattr(p, "crop_size", None))
+        mean, std = getattr(p, "image_mean", None), getattr(p, "image_std", None)
+        return (int(getattr(p, "resample", -1)) == 3                                    # PILImageResampling.BICUBIC
+                and bool(getattr(p, "do_resize", False)) and bool(getattr(p, "do_center_crop", False))
+                and not getattr(p, "do_pad", False)
+                and set(size) == {"shortest_edge"} and set(crop) == {"height", "width"}
+                and crop["height"] == crop["width"] == int(image_size) <= int(size["shortest_edge"]) <= MAX_EDGE
+                and mean is not None and std is not None and len(mean) == 3 and len(std) == 3
+                and all(float(x) != 0.0 for x in std) and float(getattr(p, "rescale_factor", 0.0)) > 0.0)
+
+    @classmethod
+    def maybe(cls, index, hf_image_processor, slot: int, image_size: int) -> Optional["DeviceImageProcessor"]:
+        """A DeviceImageProcessor for ``hf_image_processor`` on the vision tower of ``image_size`` in ``slot``, or None
+        when the device does not implement its configuration."""
+        return cls(index, hf_image_processor, slot) if cls.supported(hf_image_processor, image_size) else None
+
+    def device_ok(self, h: int, w: int) -> bool:
+        """Whether an h x w image is within the device's limits (else the host processor takes it)."""
+        if h < 1 or w < 1 or h * w > MAX_PIXELS:
+            return False
+        nh, nw = resized_size(h, w, self.shortest_edge)
+        if max(nh, nw) > MAX_EDGE or h > MAX_SCALE * nh or w > MAX_SCALE * nw:
+            return False
+        return not (self.backend == 1 and h > 100 * w and nh < h)     # Pillow shrinks such an image vertically first
+
+    def array(self, image) -> Optional[np.ndarray]:
+        """A PIL image -> its [H, W, 3] uint8 pixels as the processor sees them (after its RGB conversion), or None
+        when the host processor must take it."""
+        if image.mode != "RGB":
+            if not self.do_convert_rgb:
+                return None
+            from transformers.image_transforms import convert_to_rgb
+            image = convert_to_rgb(image)
+        a = np.asarray(image)
+        if a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] != 3 or not self.device_ok(a.shape[0], a.shape[1]):
+            return None
+        return a
+
+
 def _is_image(x) -> bool:
     return not isinstance(x, (str, bytes)) and hasattr(x, "size") and hasattr(x, "mode")      # a PIL image
 
@@ -87,6 +184,7 @@ class GpuClipModel:
         self.index, self.vision_slot, self.text_slot = index, int(vision_slot), int(text_slot)
         self.vision_config, self.text_config = dict(vision_config, tower=0), dict(text_config, tower=1)
         self.tokenizer, self.image_processor = tokenizer, image_processor
+        self.device_image_processor: Optional[DeviceImageProcessor] = None
         self.max_positions = int(self.text_config["max_positions"])
         sd = dict(state_dict)
         for slot, cfg in ((self.vision_slot, self.vision_config), (self.text_slot, self.text_config)):
@@ -106,7 +204,10 @@ class GpuClipModel:
         ml = int(text["max_positions"])
         tok = lambda texts: proc.tokenizer(list(texts), truncation=True, max_length=ml)["input_ids"]   # noqa: E731
         img = lambda images: proc.image_processor(list(images), return_tensors="np")["pixel_values"]   # noqa: E731
-        return cls(index, model.state_dict(), vision, text, tok, img, **kw)
+        m = cls(index, model.state_dict(), vision, text, tok, img, **kw)
+        m.device_image_processor = DeviceImageProcessor.maybe(index, proc.image_processor, m.vision_slot,
+                                                              vision["image_size"])
+        return m
 
     def get_sentence_embedding_dimension(self) -> int:
         return int(self.text_config["projection_dim"])
@@ -136,6 +237,25 @@ class GpuClipModel:
             out[lo:lo + max_images_per_call] = self.index.encode_images(self.vision_slot, px[lo:lo + max_images_per_call])
         return out
 
+    def encode_images(self, images, max_images_per_call: int = 256) -> np.ndarray:
+        """PIL images -> image embeddings.  With a ``device_image_processor`` the uint8 pixels go to the device
+        (``rse_encode_images_u8``) and the float pixel_values never exist on the host; an image outside its limits,
+        and every image without one, goes through the host image processor and ``encode_pixels``."""
+        images = list(images)
+        out = np.empty((len(images), self.get_sentence_embedding_dimension()), np.float32)
+        dp = self.device_image_processor
+        arrays = [dp.array(im) for im in images] if dp is not None else [None] * len(images)
+        dev_at = [i for i, a in enumerate(arrays) if a is not None]
+        host_at = [i for i, a in enumerate(arrays) if a is None]
+        for lo in range(0, len(dev_at), max_images_per_call):
+            at = dev_at[lo:lo + max_images_per_call]
+            out[at] = self.index.encode_images_u8(self.vision_slot, [arrays[i] for i in at])
+        if host_at:
+            if dp is not None:
+                dp.host_images += len(host_at)
+            out[host_at] = self.encode_pixels(self._preprocess([images[i] for i in host_at]), max_images_per_call)
+        return out
+
     def _tokenize(self, texts):
         if self.tokenizer is None:
             raise RuntimeError("GpuClipModel has no tokenizer: pass tokenizer=<texts -> token-id lists> "
@@ -159,5 +279,5 @@ class GpuClipModel:
         if txt_at:
             out[txt_at] = self.encode_ids(self._tokenize([items[i] for i in txt_at]))
         if img_at:
-            out[img_at] = self.encode_pixels(self._preprocess([items[i] for i in img_at]))
+            out[img_at] = self.encode_images([items[i] for i in img_at])
         return out[0] if single else out

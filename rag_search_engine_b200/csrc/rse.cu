@@ -20,6 +20,7 @@
 #include "common.cuh"
 #include "encoder.cuh"
 #include "fusion.cuh"
+#include "imgproc.cuh"
 #include "knn_scan.cuh"
 #include "select.cuh"
 #include "knn_tc3.cuh"
@@ -98,6 +99,18 @@ struct Encoder {
   DevBuf y, pix, patch, patch_l;      // LayerNorm output (the GEMM operand), device pixels, patch rows (+ lo half)
   float* pin_px[2] = {nullptr, nullptr};
   size_t pin_px_n[2] = {0, 0};
+  // ---- the image preprocessing bound to this vision slot (rse_imgproc_set, imgproc.cuh).  A chunk's image table
+  // and pixels are staged into ip_pin[b] and go up on the copy stream into ip_in[b], b alternating per chunk:
+  // ip_ev_up[b] = that upload is done (pinned buffer free, kernels may start), ip_ev_read[b] = the kernels that
+  // read ip_in[b] are done (the buffer may be overwritten)
+  bool ip_set = false;
+  rse_imgproc_cfg ipcfg{};
+  IpNorm ipnorm{};
+  char* ip_pin[2] = {nullptr, nullptr};
+  size_t ip_pin_n[2] = {0, 0};
+  DevBuf ip_in[2], ip_axes, ip_span, ip_w, ip_mid;
+  cudaEvent_t ip_ev_up[2] = {nullptr, nullptr}, ip_ev_read[2] = {nullptr, nullptr};
+  cudaStream_t ip_copy = nullptr;
 };
 
 }  // namespace
@@ -373,7 +386,15 @@ void enc_release(Encoder& e) {
     e.pin_in[i] = nullptr; e.pin_in_n[i] = 0; e.pin_ev[i] = nullptr;
     if (e.pin_px[i]) cudaFreeHost(e.pin_px[i]);
     e.pin_px[i] = nullptr; e.pin_px_n[i] = 0;
+    if (e.ip_pin[i]) cudaFreeHost(e.ip_pin[i]);
+    e.ip_pin[i] = nullptr; e.ip_pin_n[i] = 0;
+    for (cudaEvent_t* ev : {&e.ip_ev_up[i], &e.ip_ev_read[i]}) { if (*ev) cudaEventDestroy(*ev); *ev = nullptr; }
+    free_buf(e.ip_in[i]);
   }
+  for (DevBuf* b : {&e.ip_axes, &e.ip_span, &e.ip_w, &e.ip_mid}) free_buf(*b);
+  if (e.ip_copy) { cudaStreamSynchronize(e.ip_copy); cudaStreamDestroy(e.ip_copy); }
+  e.ip_copy = nullptr;
+  e.ip_set = false;
   e.created = e.finalized = e.clip = false;
 }
 
@@ -2911,6 +2932,270 @@ int rse_encode_images(rse_index* h, int32_t slot, const float* pixels_host, int3
   CK(cudaSetDevice(h->device));
   ENSURE(e.out, sizeof(float) * n_out);
   rc = clip_images(h, slot, pixels_host, n, static_cast<float*>(e.out.p), true);
+  if (rc != RSE_OK) return rc;
+  CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);
+  CK(cudaStreamSynchronize(h->stream));
+  return RSE_OK;
+}
+
+// ------------------------------------------------------------------ CLIP image preprocessing (imgproc.cuh)
+int rse_imgproc_set(rse_index* h, int32_t slot, const rse_imgproc_cfg* cfg) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = enc_check(h, slot, false);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[slot];
+  if (!e.clip || e.ccfg.tower != 0) return fail(h, RSE_ERR_INVALID, "rse_imgproc_set: the slot does not hold a CLIP vision tower");
+  if (!cfg) return fail(h, RSE_ERR_INVALID, "rse_imgproc_set: cfg is NULL");
+  const rse_imgproc_cfg& c = *cfg;
+  if (c.backend != 0 && c.backend != 1) return fail(h, RSE_ERR_INVALID, "rse_imgproc_set: backend must be 0 or 1");
+  const int S = e.ccfg.image_size;
+  if (!c.do_resize || !c.do_center_crop || c.crop_height != S || c.crop_width != S || c.shortest_edge < S ||
+      c.shortest_edge > RSE_IMGPROC_MAX_EDGE)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_imgproc_set: needs do_resize, do_center_crop and crop_height == crop_width == "
+                                        "the tower's image_size (" + std::to_string(S) + ") <= shortest_edge");
+  if (c.do_rescale && !(c.rescale_factor > 0.0 && std::isfinite(c.rescale_factor)))
+    return fail(h, RSE_ERR_INVALID, "rse_imgproc_set: rescale_factor must be finite and > 0");
+  IpNorm nm{};
+  nm.normalize = c.do_normalize ? 1 : 0;
+  for (int i = 0; i < 3; ++i) {
+    if (c.do_normalize && static_cast<float>(c.std[i]) == 0.0f) return fail(h, RSE_ERR_INVALID, "rse_imgproc_set: std must not be 0");
+    nm.m[i] = static_cast<float>(c.mean[i]);
+    nm.s[i] = static_cast<float>(c.std[i]);
+  }
+  if (c.backend == 0) {
+    if (c.do_rescale && c.do_normalize) {           // the fused form: float32 mean / std times float32(1 / rescale)
+      const float inv = static_cast<float>(1.0 / c.rescale_factor);
+      for (int i = 0; i < 3; ++i) { nm.m[i] = nm.m[i] * inv; nm.s[i] = nm.s[i] * inv; }
+    } else if (c.do_rescale) {
+      nm.rescale_mode = 1;
+      nm.rf = static_cast<float>(c.rescale_factor);
+    }
+  } else if (c.do_rescale) {
+    nm.rescale_mode = 2;
+    nm.rd = c.rescale_factor;
+  }
+  e.ipcfg = c;
+  e.ipnorm = nm;
+  e.ip_set = true;
+  return RSE_OK;
+}
+
+namespace {
+constexpr size_t kIpTable = size_t(64) << 10;     // the image table in front of a chunk's pixels
+constexpr int kIpChunkImages = static_cast<int>(kIpTable / sizeof(IpImage));
+
+// first input index / end of the taps of output i of an axis n_in -> n_out (imgproc.cuh ip_taps, host side)
+void ip_bounds(int i, int n_in, int n_out, int& lo, int& hi) {
+  const double scale = static_cast<double>(n_in) / n_out;
+  const double support = 2.0 * (scale > 1.0 ? scale : 1.0);
+  const double center = (i + 0.5) * scale;
+  lo = std::max(static_cast<int>(center - support + 0.5), 0);
+  hi = std::min(static_cast<int>(center + support + 0.5), n_in);
+}
+
+int ip_taps_max(int n_in, int n_out) {
+  if (n_in == n_out) return 1;
+  const double scale = static_cast<double>(n_in) / n_out;
+  return static_cast<int>(std::ceil(2.0 * (scale > 1.0 ? scale : 1.0))) * 2 + 1;
+}
+
+// checks every image, then chunk by chunk: stage -> upload (copy stream) -> coefficients, horizontal pass, vertical
+// pass (handle's stream) into out_dev [n, 3, S, S]
+int ip_run(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw, int32_t n,
+           float* out_dev) {
+  int rc = enc_check(h, slot, false);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[slot];
+  if (!e.clip || e.ccfg.tower != 0) return fail(h, RSE_ERR_INVALID, "rse_image_preprocess: the slot does not hold a CLIP vision tower");
+  if (!e.ip_set) return fail(h, RSE_ERR_STATE, "rse_image_preprocess: no rse_imgproc_set configuration for this slot");
+  if (n < 1 || !px || !offs || !hw || !out_dev) return fail(h, RSE_ERR_INVALID, "rse_image_preprocess: bad arguments (n < 1 or NULL)");
+  const rse_imgproc_cfg& c = e.ipcfg;
+  const int S = e.ccfg.image_size, se = c.shortest_edge;
+  std::vector<IpImage> im(n);
+  std::vector<int> taps(n);
+  for (int i = 0; i < n; ++i) {
+    const int H = hw[2 * i], W = hw[2 * i + 1];
+    const std::string at = "rse_image_preprocess: image " + std::to_string(i);
+    if (H < 1 || W < 1 || offs[i] < 0) return fail(h, RSE_ERR_INVALID, at + ": bad size or offset");
+    if (static_cast<int64_t>(H) * W > RSE_IMGPROC_MAX_PIXELS)
+      return fail(h, RSE_ERR_UNSUPPORTED, at + ": more than RSE_IMGPROC_MAX_PIXELS pixels");
+    IpImage& m = im[i];
+    m.off = offs[i]; m.H = H; m.W = W; m.out = i;
+    // transformers' get_resize_output_image_size(default_to_square=False): int(size * long / short)
+    const int sh = std::min(H, W), lg = std::max(H, W);
+    const int64_t nl = static_cast<int64_t>(static_cast<double>(static_cast<int64_t>(se) * lg) / sh);
+    if (nl > RSE_IMGPROC_MAX_EDGE) return fail(h, RSE_ERR_UNSUPPORTED, at + ": a resized side above RSE_IMGPROC_MAX_EDGE");
+    if (W <= H) { m.nw = se; m.nh = static_cast<int>(nl); } else { m.nh = se; m.nw = static_cast<int>(nl); }
+    if (H > static_cast<int64_t>(RSE_IMGPROC_MAX_SCALE) * m.nh || W > static_cast<int64_t>(RSE_IMGPROC_MAX_SCALE) * m.nw)
+      return fail(h, RSE_ERR_UNSUPPORTED, at + ": a downscale above RSE_IMGPROC_MAX_SCALE");
+    if (c.backend == 1 && H > 100ll * W && m.nh < H)
+      return fail(h, RSE_ERR_UNSUPPORTED, at + ": Pillow shrinks an image over 100 times taller than wide vertically first");
+    m.top = (m.nh - S) / 2;
+    m.left = (m.nw - S) / 2;
+    if (m.nh == H) {
+      m.ylo = m.top; m.rows = S;
+    } else {                                        // one row of slack on each side: the device computes the taps
+      int lo0, hi0, lo1, hi1;
+      ip_bounds(m.top, H, m.nh, lo0, hi0);
+      ip_bounds(m.top + S - 1, H, m.nh, lo1, hi1);
+      m.ylo = std::max(lo0 - 1, 0);
+      m.rows = std::min(hi1 + 1, H) - m.ylo;
+    }
+    taps[i] = std::max(ip_taps_max(W, m.nw), ip_taps_max(H, m.nh));
+  }
+  // chunks: consecutive images up to RSE_IMGPROC_CHUNK_BYTES of pixels (one image is at most 3 * 2^24 bytes)
+  std::vector<int> starts{0};
+  {
+    size_t bytes = 0;
+    for (int i = 0; i < n; ++i) {
+      const size_t b = static_cast<size_t>(im[i].H) * im[i].W * 3;
+      if (i > starts.back() && (bytes + b > size_t(RSE_IMGPROC_CHUNK_BYTES) || i - starts.back() >= kIpChunkImages)) {
+        starts.push_back(i);
+        bytes = 0;
+      }
+      bytes += b;
+    }
+    starts.push_back(n);
+  }
+  // scratch for the largest chunk (shared by all chunks: they run in order on one stream)
+  size_t max_px = 0, max_mid = 0, max_w = 0;
+  int max_cnt = 0;
+  for (size_t ci = 0; ci + 1 < starts.size(); ++ci) {
+    size_t pxb = 0, mid = 0;
+    int K = 1;
+    for (int i = starts[ci]; i < starts[ci + 1]; ++i) {
+      im[i].mid_off = static_cast<long long>(mid);
+      pxb += static_cast<size_t>(im[i].H) * im[i].W * 3;
+      mid += static_cast<size_t>(im[i].rows) * S * 3;
+      K = std::max(K, taps[i]);
+    }
+    const int cnt = starts[ci + 1] - starts[ci];
+    max_px = std::max(max_px, pxb); max_mid = std::max(max_mid, mid); max_cnt = std::max(max_cnt, cnt);
+    max_w = std::max(max_w, static_cast<size_t>(cnt) * 2 * S * K);
+  }
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.ip_axes, sizeof(IpAxis) * 2 * max_cnt);
+  ENSURE(e.ip_span, sizeof(int2) * 2 * max_cnt * S);
+  ENSURE(e.ip_w, sizeof(int) * max_w);
+  ENSURE(e.ip_mid, std::max<size_t>(max_mid, 1));
+  if (!e.ip_copy) CK(cudaStreamCreateWithFlags(&e.ip_copy, cudaStreamNonBlocking));
+  const size_t need = kIpTable + max_px;
+  for (int b = 0; b < 2; ++b) {
+    if (!e.ip_ev_up[b]) CK(cudaEventCreateWithFlags(&e.ip_ev_up[b], cudaEventDisableTiming));
+    if (!e.ip_ev_read[b]) CK(cudaEventCreateWithFlags(&e.ip_ev_read[b], cudaEventDisableTiming));
+    if (e.ip_pin_n[b] < need) {
+      CK(cudaEventSynchronize(e.ip_ev_up[b]));
+      if (e.ip_pin[b]) CK(cudaFreeHost(e.ip_pin[b]));
+      e.ip_pin[b] = nullptr; e.ip_pin_n[b] = 0;
+      CK(cudaMallocHost(reinterpret_cast<void**>(&e.ip_pin[b]), need));
+      e.ip_pin_n[b] = need;
+    }
+    ENSURE(e.ip_in[b], need);
+  }
+  IpAxis* axes = static_cast<IpAxis*>(e.ip_axes.p);
+  int2* span = static_cast<int2*>(e.ip_span.p);
+  int* wq = static_cast<int*>(e.ip_w.p);
+  uint8_t* mid = static_cast<uint8_t*>(e.ip_mid.p);
+  for (size_t ci = 0; ci + 1 < starts.size(); ++ci) {
+    const int b = static_cast<int>(ci & 1), i0 = starts[ci], cnt = starts[ci + 1] - i0;
+    CK(cudaEventSynchronize(e.ip_ev_up[b]));        // the upload out of this pinned buffer (two chunks ago) is done
+    IpImage* tab = reinterpret_cast<IpImage*>(e.ip_pin[b]);
+    uint8_t* dst = reinterpret_cast<uint8_t*>(e.ip_pin[b] + kIpTable);
+    size_t pxb = 0;
+    int K = 1, rows_w = 0;
+    for (int j = 0; j < cnt; ++j) {
+      IpImage m = im[i0 + j];
+      const size_t bytes = static_cast<size_t>(m.H) * m.W * 3;
+      std::memcpy(dst + pxb, px + m.off, bytes);
+      m.off = static_cast<long long>(pxb);
+      tab[j] = m;
+      pxb += bytes;
+      K = std::max(K, taps[i0 + j]);
+      rows_w = std::max(rows_w, m.rows * S);
+    }
+    char* din = static_cast<char*>(e.ip_in[b].p);
+    CK(cudaStreamWaitEvent(e.ip_copy, e.ip_ev_read[b], 0));
+    CK(cudaMemcpyAsync(din, tab, sizeof(IpImage) * cnt, cudaMemcpyHostToDevice, e.ip_copy));
+    CK(cudaMemcpyAsync(din + kIpTable, dst, pxb, cudaMemcpyHostToDevice, e.ip_copy));
+    CK(cudaEventRecord(e.ip_ev_up[b], e.ip_copy));
+    h->stats.h2d_bytes += static_cast<int64_t>(sizeof(IpImage) * cnt + pxb);
+    CK(cudaStreamWaitEvent(h->stream, e.ip_ev_up[b], 0));
+    const IpImage* dtab = reinterpret_cast<const IpImage*>(din);
+    imgproc_bits_kernel<<<dim3(cnt, 2), kIpThreads, 0, h->stream>>>(dtab, c.backend, K, axes);
+    LAUNCHED(h);
+    imgproc_coeff_kernel<<<dim3(cnt, 2), kIpThreads, 0, h->stream>>>(dtab, c.backend, S, S, S, K, axes, span, wq);
+    LAUNCHED(h);
+    imgproc_hpass_kernel<<<dim3((rows_w + kIpThreads - 1) / kIpThreads, cnt), kIpThreads, 0, h->stream>>>(
+        dtab, reinterpret_cast<const uint8_t*>(din + kIpTable), S, S, K, axes, span, wq, mid);
+    LAUNCHED(h);
+    imgproc_vpass_kernel<<<dim3((S * S + kIpThreads - 1) / kIpThreads, cnt), kIpThreads, 0, h->stream>>>(
+        dtab, S, S, S, K, axes, span, wq, mid, e.ipnorm, out_dev);                  // IpImage::out is the call's index
+    LAUNCHED(h);
+    CK(cudaEventRecord(e.ip_ev_read[b], h->stream));
+  }
+  return RSE_OK;
+}
+
+// preprocess into the slot's pixel buffer, then the vision tower
+int ip_encode(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw, int32_t n,
+              float* out_dev) {
+  int rc = enc_check(h, slot, true);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[slot];
+  if (!e.clip || e.ccfg.tower != 0) return fail(h, RSE_ERR_INVALID, "rse_encode_images_u8: the slot does not hold a CLIP vision tower");
+  if (n < 1 || !out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode_images_u8: bad arguments (n < 1 or NULL)");
+  if (static_cast<int64_t>(n) * e.cfg.max_positions > (1ll << 24))
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_encode_images_u8: more than 2^24 tokens in one call (split the batch)");
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.pix, sizeof(float) * static_cast<size_t>(n) * 3 * e.ccfg.image_size * e.ccfg.image_size);
+  rc = ip_run(h, slot, px, offs, hw, n, static_cast<float*>(e.pix.p));
+  if (rc != RSE_OK) return rc;
+  return clip_vision_forward(h, e, n, static_cast<const float*>(e.pix.p), out_dev);
+}
+}  // namespace
+
+int rse_image_preprocess_dev(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw,
+                             int32_t n, float* out_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  return ip_run(h, slot, px, offs, hw, n, out_dev);
+}
+
+int rse_image_preprocess(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw,
+                         int32_t n, float* out_host) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = enc_check(h, slot, false);
+  if (rc != RSE_OK) return rc;
+  if (!out_host || n < 1) return fail(h, RSE_ERR_INVALID, "rse_image_preprocess: bad arguments (n < 1 or NULL)");
+  Encoder& e = h->enc[slot];
+  const size_t n_out = static_cast<size_t>(n) * 3 * e.ccfg.image_size * e.ccfg.image_size;
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.out, sizeof(float) * n_out);
+  rc = ip_run(h, slot, px, offs, hw, n, static_cast<float*>(e.out.p));
+  if (rc != RSE_OK) return rc;
+  CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);
+  CK(cudaStreamSynchronize(h->stream));
+  return RSE_OK;
+}
+
+int rse_encode_images_u8_dev(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw,
+                             int32_t n, float* out_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  return ip_encode(h, slot, px, offs, hw, n, out_dev);
+}
+
+int rse_encode_images_u8(rse_index* h, int32_t slot, const uint8_t* px, const int64_t* offs, const int32_t* hw,
+                         int32_t n, float* out_host) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = enc_check(h, slot, true);
+  if (rc != RSE_OK) return rc;
+  if (!out_host || n < 1) return fail(h, RSE_ERR_INVALID, "rse_encode_images_u8: bad arguments (n < 1 or NULL)");
+  Encoder& e = h->enc[slot];
+  const size_t n_out = static_cast<size_t>(n) * (e.clip ? e.ccfg.projection_dim : 1);
+  CK(cudaSetDevice(h->device));
+  ENSURE(e.out, sizeof(float) * n_out);
+  rc = ip_encode(h, slot, px, offs, hw, n, static_cast<float*>(e.out.p));
   if (rc != RSE_OK) return rc;
   CK(cudaMemcpyAsync(out_host, e.out.p, sizeof(float) * n_out, cudaMemcpyDeviceToHost, h->stream));
   h->stats.d2h_bytes += static_cast<int64_t>(sizeof(float) * n_out);

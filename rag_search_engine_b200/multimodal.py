@@ -18,6 +18,8 @@ either.
 """
 from __future__ import annotations
 
+import os
+from concurrent.futures import ThreadPoolExecutor
 from typing import Dict, List, Optional, Sequence
 
 import numpy as np
@@ -70,13 +72,23 @@ class MultimodalSearch:
 
     def search_with_images(self, image_paths: Sequence[str], top_k: int = 5) -> List[List[Dict[str, object]]]:
         """``search_with_image`` for a list of image files: every image is opened the way ``embed_image`` opens
-        it, the vision tower encodes them in one ``model.encode`` call and the batch is ranked in one device call."""
+        it (on a thread pool), the vision tower encodes them in one ``model.encode`` call and the batch is ranked in
+        one device call."""
         self._check_documents()
         paths = list(image_paths)
         if not paths:
             return []
         from PIL import Image  # type: ignore
-        images = [Image.open(p).convert("RGB") for p in paths]
+
+        def load(p):
+            return Image.open(p).convert("RGB")
+        # Pillow releases the GIL while it decodes: with the preprocessing on the device, decoding is the host's
+        # whole share of the call, so the files are decoded in parallel (map keeps the input order)
+        if len(paths) > 1:
+            with ThreadPoolExecutor(max_workers=min(len(paths), os.cpu_count() or 1, 16)) as pool:
+                images = list(pool.map(load, paths))
+        else:
+            images = [load(p) for p in paths]
         embs = np.asarray(self.model.encode(images, convert_to_numpy=True), np.float32)
         return self.search_with_vectors(embs, top_k=top_k)
 
