@@ -529,6 +529,11 @@ int rse_get_stats(rse_index *h, rse_stats *out);
 /* Survivor counts of the most recent K4 filter pass (one per query of its 256-query block; a count above the
  * survivor cap of 8192 means the query overflowed and was re-run).  Synchronises.  n <= 256. */
 int rse_tc_last_survivors(rse_index *h, int32_t *out_counts, int32_t n);
+/* The survivors of query `query` (an index into the most recent K4 group, 0 .. 2047) as the last filter pass left
+ * them: corpus row (local) and cos~, the tensor-core value the filter compared with its threshold.  Copies
+ * min(count, 8192, cap) pairs in the order they were appended; *out_n = the survivor count (above 8192: the list
+ * overflowed).  Read-only; synchronises. */
+int rse_tc_last_pairs(rse_index *h, int32_t query, int64_t *out_rows, float *out_cos, int32_t cap, int32_t *out_n);
 /* The order statistic j of the K4 probe's row sample (DESIGN.md §5 "The probe's sample"): the smallest j with
  * P(Binomial(kprime, 1 / stride) >= j) <= 1e-7, capped at kprime.  Pure host arithmetic — exported so that the claim
  * can be checked against an independent binomial tail (tests/test_host_cpu.py). */

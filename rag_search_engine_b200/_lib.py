@@ -144,6 +144,8 @@ _SIGNATURES = {
     "rse_hybrid_drain": (ctypes.c_int, [c_void_p, POINTER(c_int32)]),
     "rse_hybrid_stash": (ctypes.c_int, [c_void_p, c_int32]),
     "rse_tc_last_survivors": (ctypes.c_int, [c_void_p, POINTER(c_int32), c_int32]),
+    "rse_tc_last_pairs": (ctypes.c_int, [c_void_p, c_int32, POINTER(c_int64), POINTER(c_float), c_int32,
+                                         POINTER(c_int32)]),
     "rse_tc_probe_rank": (ctypes.c_int, [c_int32, c_int32]),
     "rse_encoder_create": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseEncoderConfig)]),
     "rse_encoder_set_tensor": (ctypes.c_int, [c_void_p, c_int32, c_char_p, POINTER(c_float), c_int64]),
@@ -533,6 +535,16 @@ class Index:
         out = np.zeros(int(n), np.int32)
         self._check(self._L.rse_tc_last_survivors(self._h, _ptr(out, c_int32), int(n)))
         return out
+
+    def tc_last_pairs(self, query: int, cap: int = 8192):
+        """(rows int64[m], cos~ float32[m], count) of one query's survivors in the last K4 filter pass."""
+        rows = np.zeros(int(cap), np.int64)
+        cos = np.zeros(int(cap), np.float32)
+        n = c_int32(0)
+        self._check(self._L.rse_tc_last_pairs(self._h, int(query), _ptr(rows, c_int64), _ptr(cos, c_float), int(cap),
+                                              ctypes.byref(n)))
+        m = min(n.value, int(cap), 8192)
+        return rows[:m], cos[:m], n.value
 
     def hybrid_drain(self) -> int:
         """Wait for and discard every ticket still in flight; the handle accepts submits again afterwards."""

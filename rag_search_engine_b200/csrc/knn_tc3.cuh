@@ -29,7 +29,14 @@
 //     sum|a^_i| <= sqrt(D) for a unit vector: 2^-25 * 2 sqrt(D) = 2^-24 sqrt(D) <= 1.35e-6 (384: 1.17e-6);
 //     D fp32 adds, truncating: D * 2^-23 <= 6.10e-5 (384: 4.58e-5);
 //   together <= 1.04e-3 at D = 512 (1.02e-3 at 384), plus D * 2^-24 <= 3.05e-5 (384: 2.29e-5) for the reference's
-//   own fp32 rounding of dot: <= 1.07e-3, less than half of eps at every width K4 serves.
+//   own fp32 rounding of dot, plus D * 2^-24 <= 3.05e-5 for squares of the norm sum that are subnormal or flush
+//   (amag >= FLT_MIN is required, kT3MinSq: each lost square is below 2^-149 against a sum of at least 2^-126):
+//   <= 1.10e-3, less than half of eps at every width K4 serves.
+//   The bound needs ||a^|| = ||q^|| = 1 (Cauchy-Schwarz above).  A row or query whose sum of squares is below FLT_MIN
+//   breaks that premise (squares lost to underflow: a 384-wide row of one 1.14e-22 and 383 x 2.6e-23 has amag 1.3e-44
+//   instead of 2.7e-43 and ||a^|| = 4.6), so it never reaches the shadow (kT3MinSq, kT3MinNorm).
+//   The accumulator term is measured on the B200, not only assumed: tests/test_gpu_knn_tc_bound.py reads every
+//   survivor's cos~ back (rse_tc_last_pairs) and holds it to tests/helpers/knn_tc_model.py.
 //
 // Mapping: cluster of 2 CTAs (one TPC) x 74, persistent over 256-row tiles.
 //   UMMA 256x256x16 kind::f16 cta_group::2:  A = the queries (M = 256: 128 per CTA, resident),
@@ -72,6 +79,12 @@ constexpr int kT3QueueCap = 128;                          // per-warp survivor q
 constexpr int kT3QueueFlush = 32;                         // flushed to global memory once this full
 constexpr int kT3EpiWarps = 8;                            // two per TMEM lane quarter
 constexpr int kT3Threads = 64 + 32 * kT3EpiWarps;         // 320
+// Smallest squared norm the shadow accepts (FLT_MIN = 2^-126) and its root, the smallest query norm (2^-63).  Below
+// FLT_MIN the reference's sequential fp32 sum of squares has lost squares to underflow: 1 / sqrt(amag) no longer
+// normalises the row, ||a^|| can be several times 1 and the error bound below does not hold.  Such rows keep the
+// whole corpus on the exact scan (like a zero norm), such queries get thr = +inf and are answered exactly.
+constexpr float kT3MinSq = 1.17549435e-38f;
+constexpr double kT3MinNorm = 1.0842021724855044e-19;     // 2^-63: sb = sqrt((double)m) >= 2^-63  <=>  m >= 2^-126
 // this CTA's 128 resident queries: KB k-blocks of 16 KB (384 wide: 98,304)
 __host__ __device__ constexpr int t3_qbytes(int kb) { return kb * kT3StageBytes; }
 // 384 wide: 177,456 B; 512 wide (KB = 8): 210,224 B of the 232,448 a CTA may have
@@ -348,8 +361,8 @@ __device__ __forceinline__ void t3_shadow_row(const float* __restrict__ emb, con
                                               int lane, __half* __restrict__ shadow, unsigned int* __restrict__ bad) {
   const float am = __ldg(amag + r);
   float inv = 0.0f;
-  if (am > 0.0f && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
-  else if (!(am < 0.0f) && lane == 0) atomicAdd(bad, 1u);              // 0, +inf or NaN
+  if (am >= kT3MinSq && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
+  else if (!(am < 0.0f) && lane == 0) atomicAdd(bad, 1u);              // 0, below FLT_MIN, +inf or NaN
   const float4* src = reinterpret_cast<const float4*>(emb + r * (KB * kT3BK));
 #pragma unroll
   for (int j = 0; j < (KB + 1) / 2; ++j) {
@@ -405,7 +418,7 @@ tc3_sample_kernel(const float* __restrict__ emb, const float* __restrict__ amag,
     const int64_t r = t3_sample_source(i, stride, n_rows);
     const float am = __ldg(amag + r);
     float inv = 0.0f;                                                    // empty slots stay zero rows
-    if (am > 0.0f && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
+    if (am >= kT3MinSq && am < __int_as_float(0x7F800000)) inv = static_cast<float>(1.0 / sqrt(static_cast<double>(am)));
     const float4* src = reinterpret_cast<const float4*>(emb + r * (KB * kT3BK));
 #pragma unroll
     for (int j = 0; j < (KB + 1) / 2; ++j) {
@@ -433,7 +446,7 @@ tc3_query_prep_kernel(const float* __restrict__ q, const double* __restrict__ sb
   float inv = 0.0f;
   if (qi < nq) {
     const double s = sb[qi];
-    if (s > 0.0 && s < 1e300) inv = static_cast<float>(1.0 / s);
+    if (s >= kT3MinNorm && s < 1e300) inv = static_cast<float>(1.0 / s);
   }
   float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
   if (qi < nq) f = __ldg(reinterpret_cast<const float4*>(q + static_cast<int64_t>(qi) * (KB * kT3BK)) + threadIdx.x);
@@ -454,7 +467,7 @@ __global__ void tc3_threshold_kernel(const SelState* __restrict__ st, const doub
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= kTcBN) return;
   float t = __int_as_float(0x7F800000);
-  if (q < nq && sb[q] > 0.0 && sb[q] < 1e300) {
+  if (q < nq && sb[q] >= kT3MinNorm && sb[q] < 1e300) {
     const SelState s = st[q];
     const unsigned long long hi_mask = s.mask >> 32, hi_pref = s.prefix >> 32;
     if (s.mask != 0ull) {
@@ -480,7 +493,7 @@ tc3_probe_threshold_kernel(const uint32_t* __restrict__ dist, int64_t ld, int nq
   __shared__ unsigned int s_warp[8];
   const int q = blockIdx.x;                        // grid = the padded query count (a multiple of 256)
   const float inf = __int_as_float(0x7F800000);
-  if (q >= nq || !(sb[q] > 0.0 && sb[q] < 1e300)) {
+  if (q >= nq || !(sb[q] >= kT3MinNorm && sb[q] < 1e300)) {
     if (threadIdx.x == 0) { thr[q] = inf; if (tver) tver[q] = inf; }
     return;
   }

@@ -3938,6 +3938,31 @@ int rse_tc_last_survivors(rse_index* h, int32_t* out_counts, int32_t n) {
   return RSE_OK;
 }
 
+int rse_tc_last_pairs(rse_index* h, int32_t query, int64_t* out_rows, float* out_cos, int32_t cap, int32_t* out_n) {
+  if (!h) return RSE_ERR_INVALID;
+  if (!out_rows || !out_cos || !out_n || cap < 0) return fail(h, RSE_ERR_INVALID, "rse_tc_last_pairs: bad arguments");
+  if (!h->tc_cnt.p || !h->tc_rows.p) return fail(h, RSE_ERR_STATE, "rse_tc_last_pairs: the tensor-core path has not run");
+  const int64_t n_lists = static_cast<int64_t>(h->tc_rows.bytes / (sizeof(uint2) * kTcCandCap));
+  if (query < 0 || query >= n_lists) return fail(h, RSE_ERR_INVALID, "rse_tc_last_pairs: query outside the last group");
+  CK(cudaSetDevice(h->device));
+  CK(cudaStreamSynchronize(h->stream));
+  unsigned int cnt = 0;
+  CK(cudaMemcpy(&cnt, static_cast<const unsigned int*>(h->tc_cnt.p) + query, sizeof(cnt), cudaMemcpyDeviceToHost));
+  // the list keeps the first kTcCandCap survivors; a larger count is an overflow (reported, not copied)
+  const int n = static_cast<int>(std::min<unsigned int>({cnt, static_cast<unsigned int>(kTcCandCap),
+                                                         static_cast<unsigned int>(cap)}));
+  std::vector<uint2> pairs(static_cast<size_t>(n));
+  if (n > 0)
+    CK(cudaMemcpy(pairs.data(), static_cast<const uint2*>(h->tc_rows.p) + static_cast<int64_t>(query) * kTcCandCap,
+                  sizeof(uint2) * n, cudaMemcpyDeviceToHost));
+  for (int i = 0; i < n; ++i) {
+    out_rows[i] = static_cast<int64_t>(pairs[i].x);
+    std::memcpy(&out_cos[i], &pairs[i].y, sizeof(float));
+  }
+  *out_n = static_cast<int32_t>(std::min<unsigned int>(cnt, 0x7FFFFFFFu));
+  return RSE_OK;
+}
+
 int rse_hybrid_drain(rse_index* h, int32_t* out_dropped) {
   if (!h) return RSE_ERR_INVALID;
   CK(cudaSetDevice(h->device));
