@@ -462,6 +462,43 @@ int rse_encode_texts_dev(rse_index *h, int32_t tok_slot, int32_t enc_slot, const
 int rse_rerank_docs_load_texts(rse_index *h, int32_t tok_slot, const int64_t *ids, int64_t n_docs, const char *text,
                                const int64_t *offsets);
 
+/* ------------------------------------------------------------------ CLIP byte-level BPE on the device
+ * The image search's CLIP tokenizer (clip-ViT-B-32's CLIPTokenizerFast: NFC / \s+ -> " " / lowercase, the CLIP split
+ * pattern, ByteLevel, BPE with the "</w>" suffix, <|startoftext|> ... <|endoftext|>) runs on the device
+ * (csrc/bpe.cuh) with ids identical to the HF fast tokenizer.  A tokenizer slot holds either kind; the last load
+ * decides.  rse_tokenize, rse_tokens_fetch(_dev) and rse_encode_texts(_dev) dispatch on it:
+ *   rse_tokenizer_load_bpe : the description built from the HF object by rag_search_engine_b200/bpe.py: cp_map /
+ *                        cp_class for every code point, the symbol of every byte (inside a piece and as its last byte),
+ *                        the merge table, the special ids and the added-token strings.  Every index is checked here.
+ *   rse_tokenize       : add_special 1 = <|startoftext|> ids[:max_length - 2] <|endoftext|>, 0 = ids[:max_length].
+ *                        A text stops at the cut; its tail is validated, never tokenized.
+ *   rse_encode_texts(_dev): enc_slot must hold a CLIP text tower (type ids none, max_length 2 .. max_positions); the
+ *                        tower runs on the ids where they are, in slices of at most 65536 tokens cut greedily in text
+ *                        order at their real lengths.  cu_seqlens (4 bytes a text) is the only copy to the host.
+ * Errors: an unloaded slot RSE_ERR_STATE; bad offsets and malformed UTF-8 RSE_ERR_INVALID (the message names the
+ * first text); a BPE slot with a BERT encoder or the rerank store, or a WordPiece slot with a CLIP tower,
+ * RSE_ERR_INVALID.  RSE_ERR_UNSUPPORTED refuses, never tokenizes differently, a text that holds a code point NFC
+ * could join or reorder with its neighbours (cp_map bit 23: non-zero combining class, a decomposition that starts
+ * with one, the starters a canonical composition can take as second member) or a piece longer than 256 bytes that
+ * is needed before the cut; the Python layer hands those texts to the host tokenizer.  Limits: <= 32 added tokens,
+ * < 2^31 ids per call. */
+typedef struct rse_bpe_desc {
+  const uint32_t *cp_map;       /* [0x110000]: bits 0-20 code point or extra row, 21-22 count (0-3), 23 host route */
+  const uint32_t *extra;        /* [n_extra][3] code points of the 2- and 3-code-point outputs */
+  int32_t n_extra;
+  const uint8_t *cp_class;      /* [0x110000]: 0 other, 1 whitespace, 2 letter (\p{L}), 3 number (\p{N}) */
+  const int32_t *byte_ids;      /* [512]: symbol of byte b inside a piece at [b], as its last byte at [256 + b] */
+  const int32_t *merges;        /* [merge_slots][4] {left, right, rank, merged}, left -1 = empty; linear probing from
+                                   the high 32 bits of ((uint64)left << 32 | right) * 0x9E3779B97F4A7C15, masked */
+  int32_t merge_slots;          /* a power of two, with at least one empty slot */
+  const char *added;            /* added-token strings (UTF-8) back to back */
+  const int32_t *added_offsets; /* [n_added + 1] */
+  const int32_t *added_ids;     /* [n_added] */
+  int32_t n_added;
+  int32_t bos_id, eos_id;
+} rse_bpe_desc;
+int rse_tokenizer_load_bpe(rse_index *h, int32_t slot, const rse_bpe_desc *desc);
+
 /* ------------------------------------------------------------------ multi-GPU: row shards over one box (SURVEY §8e)
  * One process per GPU, one handle per process; the HANDLE owns the NCCL communicator (NCCL is bound at run time:
  * libnccl.so.2, or $RSE_NCCL_LIB).  The chunk-embedding matrix is cut by row into contiguous shards aligned to

@@ -16,6 +16,7 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "csrc" / "librse.so"
 
 RSE_OK = 0
+RSE_ERR_UNSUPPORTED = -4
 RSE_MAX_KPRIME = 4096
 RSE_MAX_BM25_K = 512
 RSE_MAX_FUSE_LIMIT = 1024
@@ -88,6 +89,14 @@ class RseWordpieceDesc(ctypes.Structure):
                 ("edge_child", c_void_p), ("added", c_void_p), ("added_offsets", c_void_p), ("added_ids", c_void_p),
                 ("n_added", c_int32), ("unk_id", c_int32), ("cls_id", c_int32), ("sep_id", c_int32),
                 ("max_input_chars_per_word", c_int32)]
+
+
+class RseBpeDesc(ctypes.Structure):
+    """include/rse.h rse_bpe_desc."""
+    _fields_ = [("cp_map", c_void_p), ("extra", c_void_p), ("n_extra", c_int32), ("cp_class", c_void_p),
+                ("byte_ids", c_void_p), ("merges", c_void_p), ("merge_slots", c_int32), ("added", c_void_p),
+                ("added_offsets", c_void_p), ("added_ids", c_void_p), ("n_added", c_int32), ("bos_id", c_int32),
+                ("eos_id", c_int32)]
 
 
 _SIGNATURES = {
@@ -181,6 +190,7 @@ _SIGNATURES = {
     "rse_encode_texts_dev": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32,
                                             c_void_p]),
     "rse_rerank_docs_load_texts": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_void_p]),
+    "rse_tokenizer_load_bpe": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseBpeDesc)]),
     "rse_comm_unique_id": (ctypes.c_int, [c_void_p]),
     "rse_comm_init": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32]),
     "rse_comm_destroy": (ctypes.c_int, [c_void_p]),
@@ -762,6 +772,26 @@ class Index:
         self._check(self._L.rse_tokenizer_load(self._h, int(slot), ctypes.byref(d)))
 
     @staticmethod
+    def _added(added):
+        raw = [c.encode() for c, _ in added]
+        blob = np.frombuffer(b"".join(raw) or b"\0", np.uint8)
+        offs = np.zeros(len(raw) + 1, np.int32)
+        np.cumsum([len(r) for r in raw], out=offs[1:])
+        return blob, offs, np.asarray([i for _, i in added] or [0], np.int32)
+
+    def tokenizer_load_bpe(self, slot: int, tables):
+        """A ``bpe.BpeTables`` (CLIP's byte-level BPE) into a tokenizer slot."""
+        arrs = dict(cp_map=_c(tables.cp_map, np.uint32), extra=_c(tables.extra, np.uint32).reshape(-1),
+                    cp_class=_c(tables.cp_class, np.uint8), byte_ids=_c(tables.byte_ids, np.int32),
+                    merges=_c(tables.merges, np.int32).reshape(-1))
+        added, aoff, aid = self._added(tables.added)
+        d = RseBpeDesc(n_extra=arrs["extra"].size // 3, merge_slots=arrs["merges"].size // 4, n_added=len(tables.added),
+                       bos_id=tables.bos_id, eos_id=tables.eos_id, added=added.ctypes.data,
+                       added_offsets=aoff.ctypes.data, added_ids=aid.ctypes.data,
+                       **{k: v.ctypes.data for k, v in arrs.items()})
+        self._check(self._L.rse_tokenizer_load_bpe(self._h, int(slot), ctypes.byref(d)))
+
+    @staticmethod
     def _texts(data: bytes, offsets):
         offsets = _c(offsets, np.int64)
         return c_char_p(data), offsets, len(offsets) - 1
@@ -789,10 +819,12 @@ class Index:
         self._check(self._L.rse_tokens_fetch_dev(self._h, c_void_p(ids_ptr), c_void_p(cu_ptr)))
 
     def encode_texts(self, tok_slot: int, enc_slot: int, data: bytes, offsets, max_length: int):
-        """Texts -> [n, hidden] float32 (head 0) / [n] logits (head 1): tokenized and encoded on the device."""
+        """Texts -> [n, hidden] float32 (head 0) / [n] logits (head 1) / [n, projection_dim] (a CLIP text tower with a
+        BPE tokenizer): tokenized and encoded on the device."""
         txt, offs, n = self._texts(data, offsets)
         cfg = self._enc_cfg[int(enc_slot)]
-        out = np.zeros((n, cfg.hidden) if cfg.head == 0 else (n,), np.float32)
+        shape = (n, cfg.projection_dim) if isinstance(cfg, RseClipConfig) else (n, cfg.hidden) if cfg.head == 0 else (n,)
+        out = np.zeros(shape, np.float32)
         self._check(self._L.rse_encode_texts(self._h, int(tok_slot), int(enc_slot), txt, c_void_p(offs.ctypes.data), n,
                                              int(max_length), c_void_p(out.ctypes.data)))
         return out

@@ -6,20 +6,24 @@
 (``rse_clip_create``, ``rse_encode`` for text, ``rse_encode_images`` for images) in fp32; the output is what
 sentence-transformers' CLIP ``encode`` returns: ``get_text_features`` / ``get_image_features``, not normalised.
 
-Tokenisation (BPE) and image decoding stay on the host: the tokenizer is any callable ``texts -> token-id lists``
-(or a HuggingFace tokenizer), the image processor any callable ``images -> pixel_values [n, 3, S, S]`` (or a
-HuggingFace image processor).  ``from_sentence_transformer`` takes the weights, the tokenizer and the image processor
-from a loaded reference model; when the image processor is a CLIP one ``DeviceImageProcessor`` accepts, the resize,
-crop and normalisation run on the device (csrc/imgproc.cuh) from the decoded uint8 pixels, bit for bit what the
-processor returns.  No weights are bundled and nothing is downloaded.
+The tokenizer is pluggable: ``DeviceBPE`` runs CLIP's byte-level BPE on the device (csrc/bpe.cuh, ids identical to
+the HF fast tokenizer), and any callable ``texts -> token-id lists`` (or a HuggingFace tokenizer) runs on the host;
+the image processor is any callable ``images -> pixel_values [n, 3, S, S]`` (or a HuggingFace image processor).
+Image decoding stays on the host.  ``from_sentence_transformer`` takes the weights, the tokenizer and the image
+processor from a loaded reference model; its tokenizer goes on the device when ``bpe.build_bpe_tables`` accepts it,
+and when the image processor is a CLIP one ``DeviceImageProcessor`` accepts, the resize, crop and normalisation run
+on the device (csrc/imgproc.cuh) from the decoded uint8 pixels, bit for bit what the processor returns.  No weights
+are bundled and nothing is downloaded.
 """
 from __future__ import annotations
 
-from typing import Iterator, Optional, Sequence, Tuple
+import warnings
+from typing import Iterator, List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from .encoder import pack
+from ._lib import RSE_ERR_UNSUPPORTED, RseError
+from .encoder import DeviceTokenizer, _utf8, pack
 
 VISION_SLOT, TEXT_SLOT = 0, 1
 _TOWER_KEYS = {0: ("vision_model.", "visual_projection."), 1: ("text_model.", "text_projection.")}
@@ -169,6 +173,77 @@ class DeviceImageProcessor:
         return a
 
 
+class DeviceBPE(DeviceTokenizer):
+    """CLIP's byte-level BPE tokenizer on the device (csrc/bpe.cuh) in a tokenizer slot of ``index``.
+
+    Called on texts it returns what ``hf_tok(texts, add_special_tokens=..., truncation=..., max_length=...)
+    ["input_ids"]`` returns; ``add_special_tokens`` / ``max_length`` fix which call it stands for (``max_length=None``:
+    no cut).  ``GpuClipModel`` uses its device path instead, where the ids never become Python lists.  A text the
+    device refuses goes to ``hf_tok``'s own Rust tokenizer on the host and is counted in ``host_texts``: a text with a
+    code point NFC could join with its neighbours (``host_routed``, known up front), and, once the device reports one,
+    every text that could hold a piece longer than its word buffer.  ``UnsupportedTokenizer`` when ``hf_tok`` is not
+    the CLIP BPE pipeline; ``maybe`` returns None then."""
+
+    def __init__(self, index, hf_tok, *, slot: int = 0, add_special_tokens: bool = True,
+                 max_length: Optional[int] = None):
+        from .bpe import build_bpe_tables, plain_backend
+        self.tables = build_bpe_tables(hf_tok)
+        self.backend = plain_backend(hf_tok)
+        self.index, self.slot = index, int(slot)
+        self.add_special_tokens = bool(add_special_tokens)
+        self.max_length = None if max_length is None else int(max_length)
+        self.bos_id, self.eos_id = self.tables.bos_id, self.tables.eos_id
+        self.host_texts = 0
+        index.tokenizer_load_bpe(self.slot, self.tables)
+
+    def host_ids(self, texts, add_special: bool, max_length: Optional[int]) -> List[List[int]]:
+        """The host tokenizer's ids under the same rule (the route of the texts the device refuses)."""
+        from .bpe import host_ids
+        self.host_texts += len(texts)
+        return host_ids(self.backend, texts, add_special, max_length, self.bos_id, self.eos_id)
+
+    def host_routed(self, texts, long_pieces: bool = False) -> List[int]:
+        """The texts that go to the host: those with a code point NFC could join with its neighbours, and with
+        ``long_pieces`` also those that could hold a piece longer than the device's word buffer."""
+        t = self.tables
+        return [i for i, x in enumerate(texts) if t.needs_host(x) or (long_pieces and t.may_overflow(x))]
+
+    def run(self, texts, device, host):
+        """``device(texts)`` on the texts the device takes and ``host(texts)`` on the rest -> (the device's result or
+        None, the device's text indices, the host's result, the host's text indices)."""
+        routed = self.host_routed(texts)
+        for long_pieces in (False, True):
+            if long_pieces:
+                routed = self.host_routed(texts, True)
+            at = set(routed)
+            keep = [i for i in range(len(texts)) if i not in at]
+            try:
+                dev = device([texts[i] for i in keep]) if keep else None
+                break
+            except RseError as e:
+                if long_pieces or e.code != RSE_ERR_UNSUPPORTED:
+                    raise
+        return dev, keep, (host([texts[i] for i in routed]) if routed else []), routed
+
+    def tokenize(self, texts, add_special: Optional[bool] = None, max_length: Optional[int] = -1):
+        """-> (ids int32[total], cu_seqlens int32[n + 1]) on the host; defaults are this object's call rule."""
+        sp = self.add_special_tokens if add_special is None else bool(add_special)
+        ml = self.max_length if max_length == -1 else max_length
+        texts = list(texts)
+        if not texts:
+            return np.zeros(0, np.int32), np.zeros(1, np.int32)
+        dev, keep, hst, routed = self.run(texts, lambda x: self.index.tokenize(self.slot, *_utf8(x), sp, ml or 0),
+                                          lambda x: self.host_ids(x, sp, ml))
+        if not routed:
+            return dev
+        got = dict(zip(routed, hst))
+        if dev is not None:
+            ids, cu = dev
+            ids = ids.tolist()
+            got.update((i, ids[a:b]) for i, a, b in zip(keep, cu[:-1].tolist(), cu[1:].tolist()))
+        return pack([got[i] for i in range(len(texts))])[::2]
+
+
 def _is_image(x) -> bool:
     return not isinstance(x, (str, bytes)) and hasattr(x, "size") and hasattr(x, "mode")      # a PIL image
 
@@ -194,10 +269,11 @@ class GpuClipModel:
             index.encoder_finalize(slot)
 
     @classmethod
-    def from_sentence_transformer(cls, index, st_model, **kw) -> "GpuClipModel":
+    def from_sentence_transformer(cls, index, st_model, tok_slot: int = 0, **kw) -> "GpuClipModel":
         """From a loaded ``SentenceTransformer("clip-ViT-B-32")`` (llm/multimodal.py:28): its transformers
         ``CLIPModel`` weights, its processor's tokenizer (truncating to the text tower's length, as the
-        processor does) and its image processor."""
+        processor does; a ``DeviceBPE`` in tokenizer slot ``tok_slot`` of ``index`` when the device takes it, which
+        replaces whatever that slot held; a warning names the reason when it does not) and its image processor."""
         mod = st_model[0]
         model, proc = mod.model, mod.processor
         vision, text = clip_configs_from_hf(model.config)
@@ -205,6 +281,11 @@ class GpuClipModel:
         tok = lambda texts: proc.tokenizer(list(texts), truncation=True, max_length=ml)["input_ids"]   # noqa: E731
         img = lambda images: proc.image_processor(list(images), return_tensors="np")["pixel_values"]   # noqa: E731
         m = cls(index, model.state_dict(), vision, text, tok, img, **kw)
+        from .bpe import UnsupportedTokenizer
+        try:
+            m.tokenizer = DeviceBPE(index, proc.tokenizer, slot=tok_slot, max_length=ml)
+        except UnsupportedTokenizer as e:
+            warnings.warn(f"GpuClipModel: the CLIP tokenizer stays on the host ({e})")
         m.device_image_processor = DeviceImageProcessor.maybe(index, proc.image_processor, m.vision_slot,
                                                               vision["image_size"])
         return m
@@ -256,6 +337,27 @@ class GpuClipModel:
             out[host_at] = self.encode_pixels(self._preprocess([images[i] for i in host_at]), max_images_per_call)
         return out
 
+    def encode_texts(self, texts: Sequence[str]) -> np.ndarray:
+        """Texts -> text embeddings.  With a ``DeviceBPE`` the texts the device takes are tokenized and encoded on the
+        device (``rse_encode_texts``: their ids never leave it, the tower runs on slices of them cut at their real
+        lengths) and the texts it refuses go through the host tokenizer and ``encode_ids``; without one every text
+        takes the host path.  A text's embedding does not depend on the slice it is encoded in, so the result is the
+        same either way, bit for bit."""
+        texts = list(texts)
+        tok = self.tokenizer
+        if not texts or not isinstance(tok, DeviceBPE):
+            return self.encode_ids(self._tokenize(texts))
+        mp = self.max_positions
+        out = np.empty((len(texts), self.get_sentence_embedding_dimension()), np.float32)
+        dev, keep, hst, routed = tok.run(
+            texts, lambda x: self.index.encode_texts(tok.slot, self.text_slot, *_utf8(x), mp),
+            lambda x: self.encode_ids(tok.host_ids(x, True, mp)))
+        if dev is not None:
+            out[keep] = dev
+        if routed:
+            out[routed] = hst
+        return out
+
     def _tokenize(self, texts):
         if self.tokenizer is None:
             raise RuntimeError("GpuClipModel has no tokenizer: pass tokenizer=<texts -> token-id lists> "
@@ -277,7 +379,7 @@ class GpuClipModel:
         img_at = [i for i, x in enumerate(items) if _is_image(x)]
         txt_at = [i for i, x in enumerate(items) if not _is_image(x)]
         if txt_at:
-            out[txt_at] = self.encode_ids(self._tokenize([items[i] for i in txt_at]))
+            out[txt_at] = self.encode_texts([items[i] for i in txt_at])
         if img_at:
             out[img_at] = self.encode_images([items[i] for i in img_at])
         return out[0] if single else out

@@ -26,6 +26,7 @@
 #include "knn_tc3.cuh"
 #include "rerank.cuh"
 #include "wordpiece.cuh"
+#include "bpe.cuh"
 
 using namespace rse;
 
@@ -263,11 +264,14 @@ struct rse_index {
   cudaEvent_t rr_ev[5] = {};       // rse_set_timing: hybrid | assembly | encoder | order boundaries of the last run
   bool rr_timed = false;
 
-  // ---- BERT WordPiece on the device (wordpiece.cuh): each tokenizer slot's tables in one allocation ...
+  // ---- tokenizers on the device: each slot's tables in one allocation, BERT WordPiece (wordpiece.cuh) or CLIP's
+  // byte-level BPE (bpe.cuh) ...
   struct TokSlot {
     bool loaded = false;
+    bool bpe = false;
     void* blob = nullptr;
     WpTables t{};
+    BpeTables bt{};
   } tok[RSE_MAX_TOKENIZERS];
   // ... and the last tokenisation: texts, offsets, per-text counts, cu_seqlens (int64 | int32), ids, meta (kWpMeta)
   DevBuf tk_text, tk_offs, tk_count, tk_cu64, tk_cu32, tk_ids, tk_meta;
@@ -3535,6 +3539,83 @@ int rse_tokenizer_load(rse_index* h, int32_t slot, const rse_wordpiece_desc* d) 
   t.n_added = x.n_added;
   std::memcpy(t.added_first, first, sizeof(first));
   t.unk = x.unk_id; t.cls_id = x.cls_id; t.sep_id = x.sep_id; t.max_chars = x.max_input_chars_per_word;
+  ts.bpe = false;
+  ts.loaded = true;
+  return RSE_OK;
+}
+
+// ------------------------------------------------------------------ CLIP byte-level BPE on the device (bpe.cuh)
+int rse_tokenizer_load_bpe(rse_index* h, int32_t slot, const rse_bpe_desc* d) {
+  if (!h) return RSE_ERR_INVALID;
+  if (slot < 0 || slot >= RSE_MAX_TOKENIZERS || !d) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: bad arguments");
+  const rse_bpe_desc& x = *d;
+  if (!x.cp_map || !x.cp_class || !x.extra || x.n_extra < 1 || !x.byte_ids || !x.merges || x.n_added < 0 ||
+      (x.n_added > 0 && (!x.added || !x.added_offsets || !x.added_ids)))
+    return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: a table is missing");
+  if (x.n_added > kWpMaxAdded) return fail(h, RSE_ERR_UNSUPPORTED, "rse_tokenizer_load_bpe: more than 32 added tokens");
+  // every index the kernels follow is checked here, once
+  if (x.merge_slots < 2 || (x.merge_slots & (x.merge_slots - 1)))
+    return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: merge_slots must be a power of two >= 2");
+  if (std::min(x.bos_id, x.eos_id) < 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: negative special id");
+  for (int i = 0; i < 512; ++i)
+    if (x.byte_ids[i] < 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: negative byte symbol id");
+  int64_t empty = 0;
+  for (int64_t i = 0; i < x.merge_slots; ++i) {
+    const int32_t* m = x.merges + 4 * i;
+    if (m[0] < 0) { ++empty; continue; }
+    if (m[1] < 0 || m[2] < 0 || m[3] < 0)
+      return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: merge slot " + std::to_string(i) + " holds a negative id or rank");
+  }
+  if (empty == 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: the merge table has no empty slot");
+  for (int i = 0; i < kWpCodePoints; ++i) {
+    const uint32_t m = x.cp_map[i], c = (m >> 21) & 3, v = m & kWpCpMask;
+    if ((m >> 24) || (c == 1 && v >= static_cast<uint32_t>(kWpCodePoints)) || (c > 1 && v >= static_cast<uint32_t>(x.n_extra)) ||
+        x.cp_class[i] > kBpeNumber)
+      return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: code point map entry " + std::to_string(i) + " is out of range");
+  }
+  for (int64_t i = 0; i < 3ll * x.n_extra; ++i)
+    if (x.extra[i] >= static_cast<uint32_t>(kWpCodePoints)) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: extra code point out of range");
+  uint32_t first[8] = {};
+  if (x.n_added > 0 && x.added_offsets[0] != 0) return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: added_offsets must start at 0");
+  for (int a = 0; a < x.n_added; ++a) {
+    if (x.added_offsets[a + 1] <= x.added_offsets[a] || x.added_ids[a] < 0)
+      return fail(h, RSE_ERR_INVALID, "rse_tokenizer_load_bpe: an added token is empty or has a negative id");
+    const uint8_t b = static_cast<uint8_t>(x.added[x.added_offsets[a]]);
+    first[b >> 5] |= 1u << (b & 31);
+  }
+  const int n_added_bytes = x.n_added > 0 ? x.added_offsets[x.n_added] : 0;
+  // one allocation: map | extra | cls | byte ids | merges | added bytes | offsets | ids
+  size_t off[9], at = 0;
+  const size_t sz[8] = {4ull * kWpCodePoints, 12ull * x.n_extra, 1ull * kWpCodePoints, 4ull * 512,
+                        16ull * x.merge_slots, 1ull * n_added_bytes, 4ull * (x.n_added + 1), 4ull * x.n_added};
+  for (int i = 0; i < 8; ++i) { off[i] = at; at += (sz[i] + 255) / 256 * 256; }
+  off[8] = at;
+  std::vector<char> host(at);
+  const void* src[8] = {x.cp_map, x.extra, x.cp_class, x.byte_ids, x.merges, x.added, x.added_offsets, x.added_ids};
+  for (int i = 0; i < 8; ++i) if (sz[i] && src[i]) std::memcpy(host.data() + off[i], src[i], sz[i]);
+  CK(cudaSetDevice(h->device));
+  CK(cudaStreamSynchronize(h->stream));                       // a tokenisation may still read the old tables
+  auto& ts = h->tok[slot];
+  if (ts.blob) CK(cudaFree(ts.blob));
+  ts.blob = nullptr;
+  ts.loaded = false;
+  CK(cudaMalloc(&ts.blob, at));
+  CK(cudaMemcpy(ts.blob, host.data(), at, cudaMemcpyHostToDevice));
+  char* b = static_cast<char*>(ts.blob);
+  BpeTables& t = ts.bt;
+  t.map = reinterpret_cast<const uint32_t*>(b + off[0]);
+  t.extra = reinterpret_cast<const uint32_t*>(b + off[1]);
+  t.cls = reinterpret_cast<const uint8_t*>(b + off[2]);
+  t.byte_id = reinterpret_cast<const int32_t*>(b + off[3]);
+  t.merges = reinterpret_cast<const int4*>(b + off[4]);
+  t.merge_mask = static_cast<uint32_t>(x.merge_slots - 1);
+  t.added_bytes = reinterpret_cast<const uint8_t*>(b + off[5]);
+  t.added_off = reinterpret_cast<const int32_t*>(b + off[6]);
+  t.added_id = reinterpret_cast<const int32_t*>(b + off[7]);
+  t.n_added = x.n_added;
+  std::memcpy(t.added_first, first, sizeof(first));
+  t.bos_id = x.bos_id; t.eos_id = x.eos_id;
+  ts.bpe = true;
   ts.loaded = true;
   return RSE_OK;
 }
@@ -3582,9 +3663,15 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
   CK(cudaMemsetAsync(dm + 1, 0xFF, 8, h->stream));
   CK(cudaMemsetAsync(dm + 3, 0xFF, 8, h->stream));
   const int ni = static_cast<int>(n);
-  wp_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-      h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni, special,
-      *cap, static_cast<int32_t*>(h->tk_count.p), dm);
+  const bool bpe = h->tok[slot].bpe;
+  if (bpe)
+    bpe_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+        h->tok[slot].bt, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni,
+        special, *cap, static_cast<int32_t*>(h->tk_count.p), dm);
+  else
+    wp_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+        h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni, special,
+        *cap, static_cast<int32_t*>(h->tk_count.p), dm);
   LAUNCHED(h);
   wp_scan_kernel<<<1, kWpScanThreads, 0, h->stream>>>(static_cast<const int32_t*>(h->tk_count.p), ni,
                                                       static_cast<int64_t*>(h->tk_cu64.p),
@@ -3597,6 +3684,11 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
   if (meta[0])
     return fail(h, RSE_ERR_INVALID, w + ": text " + std::to_string(meta[1]) + " is not well-formed UTF-8 (" +
                                         std::to_string(meta[0]) + " text(s))");
+  if (meta[2] && bpe)
+    return fail(h, RSE_ERR_UNSUPPORTED, w + ": text " + std::to_string(meta[3]) + " needs the host tokenizer (a code point "
+                                        "NFC could join with its neighbours, or a piece longer than " +
+                                        std::to_string(kBpeMaxWord) + " bytes before the cut; " + std::to_string(meta[2]) +
+                                        " text(s))");
   if (meta[2])
     return fail(h, RSE_ERR_UNSUPPORTED, w + ": text " + std::to_string(meta[3]) + " holds combining marks of two code points "
                                         "that NFD's canonical reordering could move (" + std::to_string(meta[2]) +
@@ -3608,20 +3700,89 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
 
 // the write pass of the texts tok_count uploaded, into ids (device, tk_cu64 positions)
 int tok_write(rse_index* h, int32_t slot, int n, int special, int cap, int32_t* ids) {
-  wp_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-      h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n, special,
-      cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
+  if (h->tok[slot].bpe)
+    bpe_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+        h->tok[slot].bt, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n,
+        special, cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
+  else
+    wp_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
+        h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n, special,
+        cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
   LAUNCHED(h);
   return RSE_OK;
 }
 
 // tokenize ([CLS] ... [SEP], cut at max_length) into tk_ids, then the BERT slot on them: out_dev [n, hidden] / [n]
+bool tok_is_bpe(const rse_index* h, int32_t slot) {
+  return slot >= 0 && slot < RSE_MAX_TOKENIZERS && h->tok[slot].loaded && h->tok[slot].bpe;
+}
+
+// A CLIP text batch runs the tower in slices of at most this many tokens, greedy in text order (a text alone when it
+// is longer): the slices GpuClipModel.encode_ids cuts by default, so both paths make the same launches.
+constexpr int kClipTextTokensPerCall = 1 << 16;
+
+// tokenize (bos ... eos, cut at max_length) into tk_ids, then the CLIP text tower on them, slice by slice:
+// out_dev [n, projection_dim].  Only cu_seqlens comes to the host (the slices' bounds); the ids stay on the device.
+int clip_enc_texts(rse_index* h, int32_t tok_slot, Encoder& e, const char* text, const int64_t* offs, int32_t n,
+                   int32_t max_length, float* out_dev) {
+  if (!e.clip || e.ccfg.tower != 1)
+    return fail(h, RSE_ERR_INVALID, "rse_encode_texts: a BPE tokenizer feeds a CLIP text tower; the slot holds another encoder");
+  if (!out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: out is NULL");
+  if (max_length < 2 || max_length > e.ccfg.max_positions)
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_encode_texts: max_length must be in [2, max_positions]");
+  unsigned long long m[kWpMeta];
+  int cap = 0;
+  int rc = tok_count(h, tok_slot, text, offs, n, 1, max_length, "rse_encode_texts", m, &cap);
+  if (rc != RSE_OK) return rc;
+  if (m[6] >= static_cast<unsigned long long>(e.ccfg.vocab_size))
+    return fail(h, RSE_ERR_INVALID, "rse_encode_texts: token id " + std::to_string(m[6]) + " >= the encoder's vocab_size " +
+                                        std::to_string(e.ccfg.vocab_size));
+  const int T = static_cast<int>(m[4]);
+  std::vector<int32_t> cu(static_cast<size_t>(n) + 1);
+  CK(cudaMemcpy(cu.data(), h->tk_cu32.p, 4 * (static_cast<size_t>(n) + 1), cudaMemcpyDeviceToHost));   // (tok_count synchronised)
+  h->stats.d2h_bytes += 4 * (static_cast<int64_t>(n) + 1);
+  ENSURE(h->tk_ids, 4 * static_cast<size_t>(T));
+  rc = tok_write(h, tok_slot, n, 1, cap, static_cast<int32_t*>(h->tk_ids.p));
+  if (rc != RSE_OK) return rc;
+  h->tk_n = n; h->tk_total = T;
+  std::vector<int> bound{0};
+  int t_max = 0, n_max = 0;
+  for (int lo = 0; lo < n;) {
+    int hi = lo + 1;
+    while (hi < n && cu[hi + 1] - cu[lo] <= kClipTextTokensPerCall) ++hi;
+    bound.push_back(hi);
+    t_max = std::max(t_max, cu[hi] - cu[lo]);
+    n_max = std::max(n_max, hi - lo);
+    lo = hi;
+  }
+  rc = clip_buffers(h, e, t_max, e.mode == 0 && e.tc_ok);     // sized once for the largest slice
+  if (rc != RSE_OK) return rc;
+  ENSURE(e.ids, sizeof(int32_t) * t_max);
+  ENSURE(e.cu, sizeof(int32_t) * (n_max + 1));
+  const int proj = e.ccfg.projection_dim;
+  for (size_t k = 0; k + 1 < bound.size(); ++k) {
+    const int lo = bound[k], hi = bound[k + 1], ns = hi - lo, Ts = cu[hi] - cu[lo];
+    int max_len = 1;
+    for (int s = lo; s < hi; ++s) max_len = std::max(max_len, cu[s + 1] - cu[s]);
+    CK(cudaMemcpyAsync(e.ids.p, static_cast<const int32_t*>(h->tk_ids.p) + cu[lo], sizeof(int32_t) * Ts,
+                       cudaMemcpyDeviceToDevice, h->stream));
+    bpe_rebase_kernel<<<(ns + 256) / 256, 256, 0, h->stream>>>(static_cast<const int32_t*>(h->tk_cu32.p) + lo, ns,
+                                                               static_cast<int32_t*>(e.cu.p));
+    LAUNCHED(h);
+    e.max_len = max_len;
+    rc = clip_text_forward(h, e, ns, Ts, out_dev + static_cast<size_t>(lo) * proj);
+    if (rc != RSE_OK) return rc;
+  }
+  return RSE_OK;
+}
+
 int enc_texts(rse_index* h, int32_t tok_slot, int32_t enc_slot, const char* text, const int64_t* offs, int32_t n,
               int32_t max_length, float* out_dev) {
   h->tk_n = 0;
   int rc = enc_check(h, enc_slot, true);
   if (rc != RSE_OK) return rc;
   Encoder& e = h->enc[enc_slot];
+  if (tok_is_bpe(h, tok_slot)) return clip_enc_texts(h, tok_slot, e, text, offs, n, max_length, out_dev);
   if (e.clip) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: the slot holds a CLIP tower (its tokenizer is not WordPiece)");
   if (!out_dev) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: out is NULL");
   if (max_length < 2 || max_length > e.cfg.max_positions)
@@ -3698,8 +3859,11 @@ int rse_encode_texts(rse_index* h, int32_t tok_slot, int32_t enc_slot, const cha
   if (rc != RSE_OK) return rc;
   if (!out_host || n < 1) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: bad arguments");
   Encoder& e = h->enc[enc_slot];
-  if (e.clip) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: the slot holds a CLIP tower (its tokenizer is not WordPiece)");
-  const size_t n_out = static_cast<size_t>(n) * (e.cfg.head == 0 ? e.cfg.hidden : 1);
+  const bool bpe = tok_is_bpe(h, tok_slot);
+  if (bpe && (!e.clip || e.ccfg.tower != 1))
+    return fail(h, RSE_ERR_INVALID, "rse_encode_texts: a BPE tokenizer feeds a CLIP text tower; the slot holds another encoder");
+  if (!bpe && e.clip) return fail(h, RSE_ERR_INVALID, "rse_encode_texts: the slot holds a CLIP tower (its tokenizer is not WordPiece)");
+  const size_t n_out = static_cast<size_t>(n) * (bpe ? e.ccfg.projection_dim : e.cfg.head == 0 ? e.cfg.hidden : 1);
   CK(cudaSetDevice(h->device));
   ENSURE(e.out, sizeof(float) * n_out);
   rc = enc_texts(h, tok_slot, enc_slot, text, offsets, n, max_length, static_cast<float*>(e.out.p));
@@ -3718,6 +3882,8 @@ int rse_rerank_docs_load_texts(rse_index* h, int32_t tok_slot, const int64_t* id
   for (int64_t i = 1; i < n_docs; ++i)
     if (ids[i] <= ids[i - 1])
       return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load_texts: ids must be strictly ascending (at " + std::to_string(i) + ")");
+  if (tok_is_bpe(h, tok_slot))
+    return fail(h, RSE_ERR_INVALID, "rse_rerank_docs_load_texts: the slot holds a BPE tokenizer (the cross-encoder's is WordPiece)");
   unsigned long long m[kWpMeta];
   int cap = 0;
   int rc = tok_count(h, tok_slot, text, offsets, n_docs, 0, 0, "rse_rerank_docs_load_texts", m, &cap);

@@ -107,7 +107,26 @@ def _utf8(texts):
 from .wordpiece import host_ids, plain_backend  # noqa: E402
 
 
-class DeviceWordPiece:
+class DeviceTokenizer:
+    """What the device tokenizers (``DeviceWordPiece``, ``clip.DeviceBPE``) share: ``maybe`` and the
+    ``hf_tok(texts, ...)["input_ids"]``-shaped call over the subclass's ``tokenize``."""
+
+    @classmethod
+    def maybe(cls, index, hf_tok, **kw):
+        """An instance, or None when ``hf_tok`` is not the pipeline the device implements."""
+        from .wordpiece import UnsupportedTokenizer
+        try:
+            return cls(index, hf_tok, **kw)
+        except UnsupportedTokenizer:
+            return None
+
+    def __call__(self, texts, add_special: Optional[bool] = None, max_length: Optional[int] = -1) -> List[List[int]]:
+        ids, cu = self.tokenize(texts, add_special, max_length)
+        ids = ids.tolist()
+        return [ids[a:b] for a, b in zip(cu[:-1].tolist(), cu[1:].tolist())]
+
+
+class DeviceWordPiece(DeviceTokenizer):
     """A BERT WordPiece tokenizer on the device (csrc/wordpiece.cuh) in a tokenizer slot of ``index``.
 
     Called on texts it returns what ``hf_tok(texts, add_special_tokens=..., truncation=..., max_length=...)
@@ -128,14 +147,6 @@ class DeviceWordPiece:
         self.cls_id, self.sep_id = self.tables.cls_id, self.tables.sep_id
         self.host_texts = 0
         index.tokenizer_load(self.slot, self.tables)
-
-    @classmethod
-    def maybe(cls, index, hf_tok, **kw) -> Optional["DeviceWordPiece"]:
-        from .wordpiece import UnsupportedTokenizer
-        try:
-            return cls(index, hf_tok, **kw)
-        except UnsupportedTokenizer:
-            return None
 
     def host_ids(self, texts, add_special: bool, max_length: Optional[int]) -> List[List[int]]:
         """The host tokenizer's ids under the same rule (the route of the texts the device refuses)."""
@@ -161,11 +172,6 @@ class DeviceWordPiece:
             return np.zeros(0, np.int32), np.zeros(1, np.int32)
         data, offs = _utf8(texts)
         return self.index.tokenize(self.slot, data, offs, sp, ml or 0)
-
-    def __call__(self, texts, add_special: Optional[bool] = None, max_length: Optional[int] = -1) -> List[List[int]]:
-        ids, cu = self.tokenize(texts, add_special, max_length)
-        ids = ids.tolist()
-        return [ids[a:b] for a, b in zip(cu[:-1].tolist(), cu[1:].tolist())]
 
 
 def hf_text_tokenizer(hf_tok) -> Callable[[List[str]], List[List[int]]]:
