@@ -462,6 +462,41 @@ int rse_encode_texts_dev(rse_index *h, int32_t tok_slot, int32_t enc_slot, const
 int rse_rerank_docs_load_texts(rse_index *h, int32_t tok_slot, const int64_t *ids, int64_t n_docs, const char *text,
                                const int64_t *offsets);
 
+/* ------------------------------------------------------------------ the semantic index build on the device
+ * The chunk texts of SemanticSearch's build (semantic_search.py:164-188, store.plan_chunks) and their embeddings,
+ * without host strings (csrc/chunk.cuh).  Movie m of n_movies is two texts of the device buffer text_dev
+ * (text_bytes bytes, UTF-8): its title text_dev[offsets[2m], offsets[2m+1]) and its description
+ * text_dev[offsets[2m+1], offsets[2m+2]); offsets_dev[2 n_movies + 1] must lie in [0, text_bytes] and not decrease
+ * (checked on the device: RSE_ERR_INVALID names the first bad entry); they need not start at 0, so a slice of the
+ * offsets addresses a part of the movies in the same buffer.  Chunk 0 of a movie is its title,
+ * verbatim; chunk w + 1 is window w of the stripped description's sentences (Python's 29 whitespace code points; split
+ * at every whitespace run that follows '.', '!' or '?'; windows of max_chunk_size sentences, the next one carrying
+ * the last `overlap` of the previous when 0 < overlap < max_chunk_size) joined without a separator.
+ *   rse_chunk_count : chunk_cu_dev[n_movies + 1] / byte_cu_dev[n_movies + 1] (int64, device) = exclusive prefix
+ *                     sums of each movie's chunks and chunk-text bytes; out_n_chunks / out_n_bytes the totals.
+ *                     Synchronises once.  max_chunk_size < 1: RSE_ERR_INVALID.
+ *   rse_chunk_write : with the same movies and the scans rse_chunk_count wrote, every chunk text back to back at
+ *                     out_text_dev (out_n_bytes bytes), out_offsets_dev[n_chunks + 1] their byte offsets (from 0), out_movie_dev /
+ *                     out_index_dev[n_chunks] its movie row (movie_base + m) and chunk_index.  Asynchronous after the
+ *                     offsets check.
+ *   rse_tokenize_dev: rse_tokenize over n texts that are already on the device (text_dev / offsets_dev[n + 1] as
+ *                     above, e.g. rse_chunk_write's output), read in place; then rse_tokens_fetch(_dev) as usual.
+ *   rse_encode_tokens_dev: the sentence encoder (head 0) of enc_slot on the last rse_tokenize(_dev)'s ids where they
+ *                     are -> out_dev [n, hidden], in slices of at most max_tokens_per_call tokens cut greedily in text
+ *                     order at their real lengths (a longer text alone).  cu_seqlens (4 bytes a text) is the one copy
+ *                     to the host.  Every sequence needs 1 .. max_positions ids (tokenize with add_special 1 and
+ *                     max_length). */
+int rse_chunk_count(rse_index *h, const char *text_dev, int64_t text_bytes, const int64_t *offsets_dev, int32_t n_movies,
+                    int32_t max_chunk_size, int32_t overlap, int64_t *chunk_cu_dev, int64_t *byte_cu_dev,
+                    int64_t *out_n_chunks, int64_t *out_n_bytes);
+int rse_chunk_write(rse_index *h, const char *text_dev, int64_t text_bytes, const int64_t *offsets_dev, int32_t n_movies,
+                    int32_t max_chunk_size, int32_t overlap, const int64_t *chunk_cu_dev, const int64_t *byte_cu_dev,
+                    int32_t movie_base, char *out_text_dev, int64_t *out_offsets_dev, int32_t *out_movie_dev,
+                    int32_t *out_index_dev);
+int rse_tokenize_dev(rse_index *h, int32_t slot, const char *text_dev, int64_t text_bytes, const int64_t *offsets_dev,
+                     int32_t n, int32_t add_special, int32_t max_length, int64_t *out_total, int32_t *out_max_len);
+int rse_encode_tokens_dev(rse_index *h, int32_t enc_slot, int64_t max_tokens_per_call, float *out_dev);
+
 /* ------------------------------------------------------------------ CLIP byte-level BPE on the device
  * The image search's CLIP tokenizer (clip-ViT-B-32's CLIPTokenizerFast: NFC / \s+ -> " " / lowercase, the CLIP split
  * pattern, ByteLevel, BPE with the "</w>" suffix, <|startoftext|> ... <|endoftext|>) runs on the device

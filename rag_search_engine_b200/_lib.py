@@ -191,6 +191,13 @@ _SIGNATURES = {
                                             c_void_p]),
     "rse_rerank_docs_load_texts": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_void_p]),
     "rse_tokenizer_load_bpe": (ctypes.c_int, [c_void_p, c_int32, POINTER(RseBpeDesc)]),
+    "rse_chunk_count": (ctypes.c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p,
+                                       c_void_p, POINTER(c_int64), POINTER(c_int64)]),
+    "rse_chunk_write": (ctypes.c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p,
+                                       c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "rse_tokenize_dev": (ctypes.c_int, [c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32,
+                                        POINTER(c_int64), POINTER(c_int32)]),
+    "rse_encode_tokens_dev": (ctypes.c_int, [c_void_p, c_int32, c_int64, c_void_p]),
     "rse_comm_unique_id": (ctypes.c_int, [c_void_p]),
     "rse_comm_init": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32]),
     "rse_comm_destroy": (ctypes.c_int, [c_void_p]),
@@ -817,6 +824,38 @@ class Index:
 
     def tokens_fetch_dev(self, ids_ptr: int, cu_ptr: int):
         self._check(self._L.rse_tokens_fetch_dev(self._h, c_void_p(ids_ptr), c_void_p(cu_ptr)))
+
+    def tokenize_device_texts(self, slot: int, text_ptr: int, text_bytes: int, offsets_ptr: int, n: int,
+                              add_special: bool, max_length: int = 0):
+        """``tokenize_dev`` over n texts already in device memory (bytes at ``text_ptr``, int64 offsets[n + 1] at
+        ``offsets_ptr``), read in place: -> (total, longest); then ``tokens_fetch_dev`` / ``encode_tokens_dev``."""
+        total, ml = c_int64(0), c_int32(0)
+        self._check(self._L.rse_tokenize_dev(self._h, int(slot), c_void_p(text_ptr or 0), int(text_bytes),
+                                             c_void_p(offsets_ptr), int(n), int(bool(add_special)), int(max_length),
+                                             ctypes.byref(total), ctypes.byref(ml)))
+        return int(total.value), int(ml.value)
+
+    def encode_tokens_dev(self, enc_slot: int, max_tokens_per_call: int, out_ptr: int):
+        """The sentence encoder on the last tokenization's ids, on the device -> [n, hidden] fp32 at ``out_ptr``."""
+        self._check(self._L.rse_encode_tokens_dev(self._h, int(enc_slot), int(max_tokens_per_call), c_void_p(out_ptr)))
+
+    def chunk_count(self, text_ptr: int, text_bytes: int, offsets_ptr: int, n_movies: int, max_chunk_size: int,
+                    overlap: int, chunk_cu_ptr: int, byte_cu_ptr: int):
+        """Sentence chunking, count pass (device buffers): -> (chunks, chunk-text bytes) of the n_movies movies."""
+        nc, nb = c_int64(0), c_int64(0)
+        self._check(self._L.rse_chunk_count(self._h, c_void_p(text_ptr or 0), int(text_bytes), c_void_p(offsets_ptr),
+                                            int(n_movies), int(max_chunk_size), int(overlap), c_void_p(chunk_cu_ptr),
+                                            c_void_p(byte_cu_ptr), ctypes.byref(nc), ctypes.byref(nb)))
+        return int(nc.value), int(nb.value)
+
+    def chunk_write(self, text_ptr: int, text_bytes: int, offsets_ptr: int, n_movies: int, max_chunk_size: int,
+                    overlap: int, chunk_cu_ptr: int, byte_cu_ptr: int, movie_base: int, out_text_ptr: int,
+                    out_offsets_ptr: int, out_movie_ptr: int, out_index_ptr: int):
+        """Sentence chunking, write pass into the chunk CSR (device buffers; asynchronous)."""
+        self._check(self._L.rse_chunk_write(self._h, c_void_p(text_ptr or 0), int(text_bytes), c_void_p(offsets_ptr),
+                                            int(n_movies), int(max_chunk_size), int(overlap), c_void_p(chunk_cu_ptr),
+                                            c_void_p(byte_cu_ptr), int(movie_base), c_void_p(out_text_ptr),
+                                            c_void_p(out_offsets_ptr), c_void_p(out_movie_ptr), c_void_p(out_index_ptr)))
 
     def encode_texts(self, tok_slot: int, enc_slot: int, data: bytes, offsets, max_length: int):
         """Texts -> [n, hidden] float32 (head 0) / [n] logits (head 1) / [n, projection_dim] (a CLIP text tower with a

@@ -27,6 +27,7 @@
 #include "rerank.cuh"
 #include "wordpiece.cuh"
 #include "bpe.cuh"
+#include "chunk.cuh"
 
 using namespace rse;
 
@@ -280,6 +281,11 @@ struct rse_index {
   unsigned long long* tk_pin_meta = nullptr;
   int tk_n = 0;                    // texts of the last rse_tokenize (0: nothing to fetch)
   int64_t tk_total = 0;
+  unsigned long long tk_max_id = 0;  // the largest id of the last rse_tokenize(_dev)
+  const uint8_t* tk_src_text = nullptr;  // the texts the write pass reads: tk_text, or the caller's (rse_tokenize_dev)
+  const int64_t* tk_src_offs = nullptr;
+  // ---- sentence chunking (chunk.cuh): per-movie counts, the int32 scan output nobody reads, meta
+  DevBuf ck_chunks, ck_bytes, ck_cu32, ck_meta;
 
   // cudaFuncSetAttribute is per device: remember per HANDLE which kernels were configured (a process-wide static
   // flag would leave the second device of a multi-GPU process unconfigured)
@@ -1177,6 +1183,7 @@ void rse_destroy(rse_index* h) {
   for (auto& t : h->tok) if (t.blob) cudaFree(t.blob);
   for (DevBuf* b : {&h->tk_text, &h->tk_offs, &h->tk_count, &h->tk_cu64, &h->tk_cu32, &h->tk_ids, &h->tk_meta}) free_buf(*b);
   if (h->tk_pin) cudaFreeHost(h->tk_pin);
+  for (DevBuf* b : {&h->ck_chunks, &h->ck_bytes, &h->ck_cu32, &h->ck_meta}) free_buf(*b);
   if (h->tk_pin_meta) cudaFreeHost(h->tk_pin_meta);
   for (auto& e : h->enc) enc_release(e);
   free_ptr(h->dev_counters);
@@ -3623,6 +3630,9 @@ int rse_tokenizer_load_bpe(rse_index* h, int32_t slot, const rse_bpe_desc* d) {
 namespace {
 // texts -> pinned -> device, the count pass and the scan, then THE small copy back of the call (meta, synchronises).
 // Leaves the counts in tk_count and cu_seqlens in tk_cu64 / tk_cu32; *cap = pieces kept per text.
+int tok_count_dev(rse_index* h, int32_t slot, int64_t n, int special, int cap, const std::string& w,
+                  unsigned long long* meta);
+
 int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs, int64_t n, int special, int max_length,
               const char* who, unsigned long long* meta, int* cap) {
   const std::string w(who);
@@ -3646,18 +3656,27 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
     CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin), need + need / 4 + 256));
     h->tk_pin_bytes = need + need / 4 + 256;
   }
-  if (!h->tk_pin_meta) CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin_meta), 8 * kWpMeta));
   std::memcpy(h->tk_pin, offs, ob);
   if (bytes > 0) std::memcpy(h->tk_pin + ob, text, bytes);
   ENSURE(h->tk_offs, ob);
   ENSURE(h->tk_text, std::max<size_t>(bytes, 1));
-  ENSURE(h->tk_count, 4 * static_cast<size_t>(n));
-  ENSURE(h->tk_cu64, ob);
-  ENSURE(h->tk_cu32, 4 * static_cast<size_t>(n + 1));
-  ENSURE(h->tk_meta, 8 * kWpMeta);
   CK(cudaMemcpyAsync(h->tk_offs.p, h->tk_pin, ob, cudaMemcpyHostToDevice, h->stream));
   if (bytes > 0) CK(cudaMemcpyAsync(h->tk_text.p, h->tk_pin + ob, bytes, cudaMemcpyHostToDevice, h->stream));
   h->stats.h2d_bytes += static_cast<int64_t>(need);
+  h->tk_src_text = static_cast<const uint8_t*>(h->tk_text.p);
+  h->tk_src_offs = static_cast<const int64_t*>(h->tk_offs.p);
+  return tok_count_dev(h, slot, n, special, *cap, w, meta);
+}
+
+// the count pass and the scan over the texts at tk_src_text / tk_src_offs (device), then THE small copy back of the
+// call (meta, synchronises)
+int tok_count_dev(rse_index* h, int32_t slot, int64_t n, int special, int cap, const std::string& w,
+                  unsigned long long* meta) {
+  ENSURE(h->tk_count, 4 * static_cast<size_t>(n));
+  ENSURE(h->tk_cu64, 8 * static_cast<size_t>(n + 1));
+  ENSURE(h->tk_cu32, 4 * static_cast<size_t>(n + 1));
+  ENSURE(h->tk_meta, 8 * kWpMeta);
+  if (!h->tk_pin_meta) CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin_meta), 8 * (kWpMeta + 1)));
   auto* dm = static_cast<unsigned long long*>(h->tk_meta.p);
   CK(cudaMemsetAsync(dm, 0, 8 * kWpMeta, h->stream));
   CK(cudaMemsetAsync(dm + 1, 0xFF, 8, h->stream));
@@ -3666,12 +3685,10 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
   const bool bpe = h->tok[slot].bpe;
   if (bpe)
     bpe_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-        h->tok[slot].bt, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni,
-        special, *cap, static_cast<int32_t*>(h->tk_count.p), dm);
+        h->tok[slot].bt, h->tk_src_text, h->tk_src_offs, ni, special, cap, static_cast<int32_t*>(h->tk_count.p), dm);
   else
     wp_count_kernel<<<(ni + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-        h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), ni, special,
-        *cap, static_cast<int32_t*>(h->tk_count.p), dm);
+        h->tok[slot].t, h->tk_src_text, h->tk_src_offs, ni, special, cap, static_cast<int32_t*>(h->tk_count.p), dm);
   LAUNCHED(h);
   wp_scan_kernel<<<1, kWpScanThreads, 0, h->stream>>>(static_cast<const int32_t*>(h->tk_count.p), ni,
                                                       static_cast<int64_t*>(h->tk_cu64.p),
@@ -3695,6 +3712,7 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
                                         " text(s)); tokenize such texts on the host");
   if (meta[4] > static_cast<unsigned long long>(INT_MAX))
     return fail(h, RSE_ERR_UNSUPPORTED, w + ": more than 2^31 token ids in one call (split the batch)");
+  h->tk_max_id = meta[6];
   return RSE_OK;
 }
 
@@ -3702,12 +3720,10 @@ int tok_count(rse_index* h, int32_t slot, const char* text, const int64_t* offs,
 int tok_write(rse_index* h, int32_t slot, int n, int special, int cap, int32_t* ids) {
   if (h->tok[slot].bpe)
     bpe_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-        h->tok[slot].bt, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n,
-        special, cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
+        h->tok[slot].bt, h->tk_src_text, h->tk_src_offs, n, special, cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
   else
     wp_write_kernel<<<(n + kWpThreads - 1) / kWpThreads, kWpThreads, 0, h->stream>>>(
-        h->tok[slot].t, static_cast<const uint8_t*>(h->tk_text.p), static_cast<const int64_t*>(h->tk_offs.p), n, special,
-        cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
+        h->tok[slot].t, h->tk_src_text, h->tk_src_offs, n, special, cap, static_cast<const int64_t*>(h->tk_cu64.p), ids);
   LAUNCHED(h);
   return RSE_OK;
 }
@@ -3843,6 +3859,177 @@ int rse_tokens_fetch_dev(rse_index* h, int32_t* ids_dev, int32_t* cu_seqlens_dev
   CK(cudaMemcpyAsync(cu_seqlens_dev, h->tk_cu32.p, 4 * static_cast<size_t>(h->tk_n + 1), cudaMemcpyDeviceToDevice, h->stream));
   if (h->tk_total > 0)
     CK(cudaMemcpyAsync(ids_dev, h->tk_ids.p, 4 * static_cast<size_t>(h->tk_total), cudaMemcpyDeviceToDevice, h->stream));
+  return RSE_OK;
+}
+
+namespace {
+// offsets_dev[0 .. n] of a device text of text_bytes bytes, checked on the device (one small copy back, synchronises)
+int check_dev_offsets(rse_index* h, const std::string& w, const int64_t* offsets_dev, int64_t n, int64_t text_bytes) {
+  ENSURE(h->ck_meta, 8);
+  if (!h->tk_pin_meta) CK(cudaMallocHost(reinterpret_cast<void**>(&h->tk_pin_meta), 8 * (kWpMeta + 1)));
+  auto* bad = static_cast<unsigned long long*>(h->ck_meta.p);
+  CK(cudaMemsetAsync(bad, 0xFF, 8, h->stream));
+  dev_offsets_check_kernel<<<static_cast<unsigned>((n + 256) / 256), 256, 0, h->stream>>>(offsets_dev, n, text_bytes, bad);
+  LAUNCHED(h);
+  CK(cudaMemcpyAsync(h->tk_pin_meta, bad, 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  if (h->tk_pin_meta[0] != ~0ull)
+    return fail(h, RSE_ERR_INVALID, w + ": offsets[" + std::to_string(h->tk_pin_meta[0]) + "] is out of order or outside "
+                                        "the text (offsets must go from 0 up to at most text_bytes)");
+  return RSE_OK;
+}
+
+int chunk_args(rse_index* h, const std::string& w, const char* text_dev, int64_t text_bytes, const int64_t* offsets_dev,
+               int32_t n_movies, int32_t max_chunk_size) {
+  if (max_chunk_size < 1) return fail(h, RSE_ERR_INVALID, w + ": max_chunk_size must be >= 1");
+  if (n_movies < 1 || !offsets_dev || text_bytes < 0 || (text_bytes > 0 && !text_dev))
+    return fail(h, RSE_ERR_INVALID, w + ": bad arguments (n_movies < 1, offsets or text NULL, or text_bytes < 0)");
+  CK(cudaSetDevice(h->device));
+  return check_dev_offsets(h, w, offsets_dev, 2 * static_cast<int64_t>(n_movies), text_bytes);
+}
+
+int chunk_carry(int32_t size, int32_t overlap) { return overlap > 0 && overlap < size ? overlap : 0; }
+}  // namespace
+
+int rse_tokenize_dev(rse_index* h, int32_t slot, const char* text_dev, int64_t text_bytes, const int64_t* offsets_dev,
+                     int32_t n, int32_t add_special, int32_t max_length, int64_t* out_total, int32_t* out_max_len) {
+  if (!h) return RSE_ERR_INVALID;
+  h->tk_n = 0;
+  const std::string w("rse_tokenize_dev");
+  if (add_special != 0 && add_special != 1) return fail(h, RSE_ERR_INVALID, w + ": add_special must be 0 or 1");
+  if (slot < 0 || slot >= RSE_MAX_TOKENIZERS) return fail(h, RSE_ERR_INVALID, w + ": tokenizer slot out of range");
+  if (!h->tok[slot].loaded) return fail(h, RSE_ERR_STATE, w + ": no tokenizer in this slot (rse_tokenizer_load)");
+  if (n < 1 || !offsets_dev || text_bytes < 0 || (text_bytes > 0 && !text_dev))
+    return fail(h, RSE_ERR_INVALID, w + ": bad arguments (n < 1, offsets or text NULL, or text_bytes < 0)");
+  if (add_special && max_length > 0 && max_length < 2)
+    return fail(h, RSE_ERR_UNSUPPORTED, w + ": max_length must be >= 2 with [CLS] / [SEP]");
+  const int cap = max_length > 0 ? max_length - 2 * add_special : INT_MAX;
+  CK(cudaSetDevice(h->device));
+  int rc = check_dev_offsets(h, w, offsets_dev, n, text_bytes);
+  if (rc != RSE_OK) return rc;
+  h->tk_src_text = reinterpret_cast<const uint8_t*>(text_dev);
+  h->tk_src_offs = offsets_dev;
+  unsigned long long m[kWpMeta];
+  rc = tok_count_dev(h, slot, n, add_special, cap, w, m);
+  if (rc != RSE_OK) return rc;
+  ENSURE(h->tk_ids, 4 * std::max<size_t>(m[4], 1));
+  rc = tok_write(h, slot, n, add_special, cap, static_cast<int32_t*>(h->tk_ids.p));
+  if (rc != RSE_OK) return rc;
+  h->tk_n = n; h->tk_total = static_cast<int64_t>(m[4]);
+  if (out_total) *out_total = h->tk_total;
+  if (out_max_len) *out_max_len = static_cast<int32_t>(m[5]);
+  return RSE_OK;
+}
+
+int rse_encode_tokens_dev(rse_index* h, int32_t enc_slot, int64_t max_tokens_per_call, float* out_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  const std::string w("rse_encode_tokens_dev");
+  int rc = enc_check(h, enc_slot, true);
+  if (rc != RSE_OK) return rc;
+  Encoder& e = h->enc[enc_slot];
+  if (e.clip || e.cfg.head != 0) return fail(h, RSE_ERR_INVALID, w + ": the slot does not hold a sentence encoder (head 0)");
+  if (h->tk_n < 1) return fail(h, RSE_ERR_STATE, w + ": nothing tokenized (rse_tokenize / rse_tokenize_dev)");
+  if (!out_dev || max_tokens_per_call < 1) return fail(h, RSE_ERR_INVALID, w + ": bad arguments");
+  if (h->tk_max_id >= static_cast<unsigned long long>(e.cfg.vocab_size))
+    return fail(h, RSE_ERR_INVALID, w + ": token id " + std::to_string(h->tk_max_id) + " >= the encoder's vocab_size " +
+                                        std::to_string(e.cfg.vocab_size));
+  const int n = h->tk_n;
+  CK(cudaSetDevice(h->device));
+  std::vector<int32_t> cu(static_cast<size_t>(n) + 1);
+  CK(cudaMemcpyAsync(cu.data(), h->tk_cu32.p, 4 * (static_cast<size_t>(n) + 1), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->stats.d2h_bytes += 4 * (static_cast<int64_t>(n) + 1);
+  for (int s = 0; s < n; ++s) {
+    const int len = cu[s + 1] - cu[s];
+    if (len < 1) return fail(h, RSE_ERR_INVALID, w + ": text " + std::to_string(s) + " has no ids (tokenize with add_special 1)");
+    if (len > e.cfg.max_positions)
+      return fail(h, RSE_ERR_UNSUPPORTED, w + ": text " + std::to_string(s) + " is longer than max_positions (tokenize with max_length)");
+  }
+  // slices of at most max_tokens_per_call tokens, greedy in text order at the real lengths (a text alone when it is
+  // longer): GpuSentenceEncoder.encode's cut, which does not change any row (every kernel of the encoder works per
+  // token or per sequence)
+  int n_max = 0;
+  std::vector<int> bound{0};
+  for (int lo = 0; lo < n;) {
+    int hi = lo + 1;
+    while (hi < n && static_cast<int64_t>(cu[hi + 1]) - cu[lo] <= max_tokens_per_call) ++hi;
+    bound.push_back(hi);
+    n_max = std::max(n_max, hi - lo);
+    lo = hi;
+  }
+  ENSURE(e.cu, sizeof(int32_t) * (n_max + 1));
+  const int H = e.cfg.hidden;
+  for (size_t k = 0; k + 1 < bound.size(); ++k) {
+    const int lo = bound[k], hi = bound[k + 1], ns = hi - lo, Ts = cu[hi] - cu[lo];
+    int max_len = 1;
+    for (int s = lo; s < hi; ++s) max_len = std::max(max_len, cu[s + 1] - cu[s]);
+    bpe_rebase_kernel<<<(ns + 256) / 256, 256, 0, h->stream>>>(static_cast<const int32_t*>(h->tk_cu32.p) + lo, ns,
+                                                               static_cast<int32_t*>(e.cu.p));
+    LAUNCHED(h);
+    rc = enc_forward(h, e, static_cast<const int32_t*>(h->tk_ids.p) + cu[lo], nullptr, static_cast<const int32_t*>(e.cu.p),
+                     ns, Ts, max_len, out_dev + static_cast<size_t>(lo) * H);
+    if (rc != RSE_OK) return rc;
+  }
+  return RSE_OK;
+}
+
+int rse_chunk_count(rse_index* h, const char* text_dev, int64_t text_bytes, const int64_t* offsets_dev, int32_t n_movies,
+                    int32_t max_chunk_size, int32_t overlap, int64_t* chunk_cu_dev, int64_t* byte_cu_dev,
+                    int64_t* out_n_chunks, int64_t* out_n_bytes) {
+  if (!h) return RSE_ERR_INVALID;
+  int rc = chunk_args(h, "rse_chunk_count", text_dev, text_bytes, offsets_dev, n_movies, max_chunk_size);
+  if (rc != RSE_OK) return rc;
+  if (!chunk_cu_dev || !byte_cu_dev) return fail(h, RSE_ERR_INVALID, "rse_chunk_count: chunk_cu / byte_cu NULL");
+  const int64_t n = n_movies;
+  ENSURE(h->ck_chunks, 4 * static_cast<size_t>(n));
+  ENSURE(h->ck_bytes, 4 * static_cast<size_t>(n));
+  ENSURE(h->ck_cu32, 4 * static_cast<size_t>(n + 1));
+  ENSURE(h->ck_meta, 8 * (kChunkMeta + 2 * kWpMeta));
+  auto* dm = static_cast<unsigned long long*>(h->ck_meta.p);
+  CK(cudaMemsetAsync(dm, 0, 8 * (kChunkMeta + 2 * kWpMeta), h->stream));
+  CK(cudaMemsetAsync(dm + 1, 0xFF, 8, h->stream));
+  const auto* t = reinterpret_cast<const uint8_t*>(text_dev);
+  const int grid = static_cast<int>((n + kChunkThreads - 1) / kChunkThreads);
+  chunk_count_kernel<<<grid, kChunkThreads, 0, h->stream>>>(t, offsets_dev, n_movies, max_chunk_size,
+                                                            chunk_carry(max_chunk_size, overlap),
+                                                            static_cast<int32_t*>(h->ck_chunks.p),
+                                                            static_cast<int32_t*>(h->ck_bytes.p), dm);
+  LAUNCHED(h);
+  wp_scan_kernel<<<1, kWpScanThreads, 0, h->stream>>>(static_cast<const int32_t*>(h->ck_chunks.p), n_movies, chunk_cu_dev,
+                                                      static_cast<int32_t*>(h->ck_cu32.p), dm + kChunkMeta);
+  LAUNCHED(h);
+  wp_scan_kernel<<<1, kWpScanThreads, 0, h->stream>>>(static_cast<const int32_t*>(h->ck_bytes.p), n_movies, byte_cu_dev,
+                                                      static_cast<int32_t*>(h->ck_cu32.p), dm + kChunkMeta + kWpMeta);
+  LAUNCHED(h);
+  unsigned long long m[kChunkMeta + 2 * kWpMeta];
+  CK(cudaMemcpyAsync(m, dm, sizeof(m), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(sizeof(m));
+  if (m[0])
+    return fail(h, RSE_ERR_UNSUPPORTED, "rse_chunk_count: movie " + std::to_string(m[1]) + " has more than 2^31 bytes of "
+                                        "chunk text (" + std::to_string(m[0]) + " movie(s))");
+  if (out_n_chunks) *out_n_chunks = static_cast<int64_t>(m[kChunkMeta + 4]);
+  if (out_n_bytes) *out_n_bytes = static_cast<int64_t>(m[kChunkMeta + kWpMeta + 4]);
+  return RSE_OK;
+}
+
+int rse_chunk_write(rse_index* h, const char* text_dev, int64_t text_bytes, const int64_t* offsets_dev, int32_t n_movies,
+                    int32_t max_chunk_size, int32_t overlap, const int64_t* chunk_cu_dev, const int64_t* byte_cu_dev,
+                    int32_t movie_base, char* out_text_dev, int64_t* out_offsets_dev, int32_t* out_movie_dev,
+                    int32_t* out_index_dev) {
+  if (!h) return RSE_ERR_INVALID;
+  if (!chunk_cu_dev || !byte_cu_dev || !out_offsets_dev || !out_movie_dev || !out_index_dev || !out_text_dev)
+    return fail(h, RSE_ERR_INVALID, "rse_chunk_write: an output or a scan is NULL");
+  if (movie_base < 0 || static_cast<int64_t>(movie_base) + n_movies > INT_MAX)
+    return fail(h, RSE_ERR_INVALID, "rse_chunk_write: movie_base + n_movies must fit 31 bits");
+  int rc = chunk_args(h, "rse_chunk_write", text_dev, text_bytes, offsets_dev, n_movies, max_chunk_size);
+  if (rc != RSE_OK) return rc;
+  const int grid = (n_movies + kChunkThreads - 1) / kChunkThreads;
+  chunk_write_kernel<<<grid, kChunkThreads, 0, h->stream>>>(
+      reinterpret_cast<const uint8_t*>(text_dev), offsets_dev, n_movies, max_chunk_size, chunk_carry(max_chunk_size, overlap),
+      chunk_cu_dev, byte_cu_dev, movie_base, reinterpret_cast<uint8_t*>(out_text_dev), out_offsets_dev, out_movie_dev,
+      out_index_dev);
+  LAUNCHED(h);
   return RSE_OK;
 }
 

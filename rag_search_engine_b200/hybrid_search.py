@@ -39,7 +39,7 @@ class HybridSearch:
         self.cross_encoder = cross_encoder
         self.tie_mode = {"reference": _lib.TIE_REFERENCE, "id": _lib.TIE_BY_ID}[tie_mode]
         kw_extra = {k: v for k, v in retriever_kwargs.items() if k in ("tokenizer",)}
-        sem_extra = {k: v for k, v in retriever_kwargs.items() if k in ("encoder", "fallback_build")}
+        sem_extra = {k: v for k, v in retriever_kwargs.items() if k in ("encoder", "fallback_build", "device_build")}
         if KeywordSearch.__module__.startswith(__package__):
             kw_extra["device"] = device
         if SemanticSearch.__module__.startswith(__package__):

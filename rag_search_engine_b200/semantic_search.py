@@ -8,7 +8,9 @@ chunk text / titles for the ≤k hits still come from SQLite (:262-279, :321-328
 """
 from __future__ import annotations
 
+import json
 import sqlite3
+import time
 from pathlib import Path
 from typing import Any, Dict, List, Optional
 
@@ -27,10 +29,23 @@ def _default_encoder():
     return SentenceTransformer("all-MiniLM-L6-v2")              # semantic_search.py:45
 
 
+def _vec0_rows_in_order(conn: sqlite3.Connection, n: int) -> bool:
+    """Rows 0 .. n-1 of a freshly filled vec0 table sit at positions 0 .. n-1 of store.export_embeddings: ceil(n /
+    1024) consecutive blocks, and every rowid at (block - first block) * 1024 + its offset."""
+    t = store.VEC_TABLE
+    n_blocks, lo, hi = conn.execute(f"SELECT COUNT(*), MIN(chunk_id), MAX(chunk_id) FROM {t}_chunks").fetchone()
+    if n_blocks != (n + store.VEC0_BLOCK - 1) // store.VEC0_BLOCK or hi - lo + 1 != n_blocks:
+        return False
+    (n_rows,) = conn.execute(f"SELECT COUNT(*) FROM {t}_rowids").fetchone()
+    (bad,) = conn.execute(f"SELECT COUNT(*) FROM {t}_rowids WHERE (chunk_id - ?) * ? + chunk_offset != rowid",
+                          (lo, store.VEC0_BLOCK)).fetchone()
+    return n_rows == n and bad == 0
+
+
 class SemanticSearch:
     def __init__(self, docs_path: Path | str | None = None, db_path: Path | str | None = None,
                  max_chunk_size: int = 3, overlap: int = 1, force: bool = False, *, encoder=None,
-                 device: int = 0, fallback_build: bool = False) -> None:
+                 device: int = 0, fallback_build: bool = False, device_build: bool = False) -> None:
         self.model = encoder if encoder is not None else _default_encoder()
         self.max_chunk_size = max_chunk_size
         self.overlap = overlap
@@ -39,8 +54,9 @@ class SemanticSearch:
         self.docs_path = Path(docs_path) if docs_path else None
         self.device = device
         self.fallback_build = fallback_build
+        self.device_build = device_build
         if self.docs_path is not None:
-            self._build(force)
+            self._build_device(force) if device_build else self._build(force)
         self.conn = sqlite3.connect(self.db_path)
         self.conn.execute("PRAGMA journal_mode=WAL")
         self.conn.execute("PRAGMA synchronous=NORMAL")
@@ -72,23 +88,12 @@ class SemanticSearch:
         if self.model is None:
             raise RuntimeError("SemanticSearch build needs an encoder (sentence-transformers is not installed): "
                                "pass encoder=<object with .encode(texts)>")
-        import json
-        data = json.loads(Path(self.docs_path).read_text(encoding="utf-8"))["movies"]
         conn = sqlite3.connect(self.db_path)
         try:
             store._init_schema(conn)
+            self._sync_movies_json(conn)
             cur = conn.cursor()
-            (n_movies,) = cur.execute("SELECT COUNT(*) FROM movies").fetchone()
-            if n_movies != len(data):
-                cur.execute("DELETE FROM movies")
-                cur.executemany("INSERT INTO movies(id, title, description) VALUES (?, ?, ?)",
-                                [(int(d["id"]), d["title"], d["description"]) for d in data])
-                conn.commit()
-            (n_chunks,) = cur.execute("SELECT COUNT(*) FROM chunks").fetchone()
-            params = cur.execute("SELECT DISTINCT max_chunk_size, overlap FROM chunks").fetchall()
-            in_sync = (n_chunks > 0 and len(params) == 1 and params[0] == (self.max_chunk_size, self.overlap)
-                       and store._table_exists(conn, f"{store.VEC_TABLE}_chunks"))          # :145-154
-            if force or not in_sync:
+            if force or not self._in_sync(conn):
                 movies = cur.execute("SELECT id, title, description FROM movies ORDER BY id").fetchall()
                 rows, texts = store.plan_chunks(movies, self.max_chunk_size, self.overlap)
                 cur.execute("DELETE FROM chunks")
@@ -100,14 +105,162 @@ class SemanticSearch:
         finally:
             conn.close()
 
+    def _sync_movies_json(self, conn: sqlite3.Connection) -> None:
+        """The fallback build's movies sync: the JSON rows replace the table when the counts differ."""
+        data = json.loads(Path(self.docs_path).read_text(encoding="utf-8"))["movies"]
+        cur = conn.cursor()
+        (n_movies,) = cur.execute("SELECT COUNT(*) FROM movies").fetchone()
+        if n_movies != len(data):
+            cur.execute("DELETE FROM movies")
+            cur.executemany("INSERT INTO movies(id, title, description) VALUES (?, ?, ?)",
+                            [(int(d["id"]), d["title"], d["description"]) for d in data])
+            conn.commit()
+
+    def _in_sync(self, conn: sqlite3.Connection) -> bool:
+        """semantic_search.py:145-154: chunks exist, all of this (max_chunk_size, overlap), and vec0 exists."""
+        cur = conn.cursor()
+        (n_chunks,) = cur.execute("SELECT COUNT(*) FROM chunks").fetchone()
+        params = cur.execute("SELECT DISTINCT max_chunk_size, overlap FROM chunks").fetchall()
+        return (n_chunks > 0 and len(params) == 1 and params[0] == (self.max_chunk_size, self.overlap)
+                and store._table_exists(conn, f"{store.VEC_TABLE}_chunks"))
+
+    def _sync_movies(self, conn: sqlite3.Connection) -> None:
+        """The movies table for the device build: the reference's own sync when the reference is importable — its
+        BaseSearchDB, constructed like the reference's search classes (docs_path=, db_path=), loads the docs and
+        syncs the table (basesearch_db.py:24-49, :81-92) and may fix the texts it stores, so the build reads the rows
+        back from the table — else the fallback build's JSON sync."""
+        try:
+            from rag_search_engine.utils.basesearch_db import BaseSearchDB  # type: ignore
+        except ImportError:
+            self._sync_movies_json(conn)
+            return
+        BaseSearchDB(docs_path=self.docs_path, db_path=self.db_path).close()
+
+    def _build_device(self, force: bool) -> None:
+        """``device_build=True``: the chunk texts, their ids and their embeddings are made on the device
+        (device_build.build_embeddings) and the matrix stays in HBM as this handle's corpus; the ``chunks`` rows, vec0
+        and the ``.rse-emb`` sidecar are written from the one host copy.  vec0 goes through the real ``vec0`` virtual
+        table when ``sqlite_vec`` is importable (the reference can open the file), else, under ``fallback_build=True``
+        only, into the shadow tables ``store.write_vec0_shadow`` writes."""
+        from . import device_build
+        from .encoder import DeviceWordPiece, GpuSentenceEncoder
+        if self.max_chunk_size < 1:
+            raise ValueError(f"max_chunk_size must be >= 1 (got {self.max_chunk_size})")
+        try:
+            import sqlite_vec  # type: ignore
+        except ImportError:
+            sqlite_vec = None
+        if sqlite_vec is None and not self.fallback_build:
+            raise RuntimeError("device_build writes vec0 through sqlite-vec, which is not importable here; pass "
+                               "fallback_build=True as well to write a GPU-ONLY database (vec0 shadow tables without the "
+                               "virtual table: sqlite-vec / the reference cannot open it)")
+        index = runtime.acquire(self.db_path, self.device)
+        try:
+            enc = self.model
+            if not isinstance(enc, GpuSentenceEncoder) or not isinstance(enc.tokenizer, DeviceWordPiece):
+                raise TypeError("device_build needs encoder=GpuSentenceEncoder(...) with a DeviceWordPiece tokenizer")
+            if enc.index is not index or enc.tokenizer.index is not index:
+                raise ValueError("device_build: the encoder (and its DeviceWordPiece) must live on this database's "
+                                 "handle, runtime.acquire(db_path, device)")
+            conn = sqlite3.connect(self.db_path)
+            try:
+                store._init_schema(conn)
+                self._sync_movies(conn)
+                cur = conn.cursor()
+                if self._in_sync(conn) and not force:
+                    return
+                movies = cur.execute("SELECT id, title, description FROM movies ORDER BY id").fetchall()
+                built = device_build.build_embeddings(enc, movies, self.max_chunk_size, self.overlap)
+                self._write_device_build(conn, index, movies, built, sqlite_vec)
+            finally:
+                conn.close()
+        finally:
+            runtime.release(self.db_path, self.device)
+
+    def _write_device_build(self, conn, index, movies, built, sqlite_vec) -> None:
+        """The chunks rows, vec0 and (through _load) the sidecar from the one host copy; the device matrix becomes the
+        handle's corpus.  ``self.build_timings``: seconds per stage, the device stages of build_embeddings first."""
+        import torch
+        t = self.build_timings = dict(built.timings)
+        ts = time.perf_counter()
+        emb = built.emb.cpu().numpy()                                    # the one host copy
+        t["device_to_host"] = time.perf_counter() - ts
+        ts = time.perf_counter()
+        n = int(built.movie_idx.shape[0])
+        movie_ids = np.array([m[0] for m in movies], np.int64)
+        per = built.chunks_per_movie
+        first = np.repeat(np.cumsum(per) - per, per)
+        chunk_ids = np.arange(n, dtype=np.int64)
+        rows = zip(chunk_ids.tolist(), np.repeat(movie_ids, per).tolist(), (chunk_ids - first).tolist(),
+                   [self.max_chunk_size] * n, [self.overlap] * n)
+        cur = conn.cursor()
+        cur.execute("DELETE FROM chunks")
+        cur.executemany("INSERT INTO chunks(id, movie_id, chunk_index, max_chunk_size, overlap) VALUES (?,?,?,?,?)",
+                        rows)
+        conn.commit()
+        t["sqlite_chunks"] = time.perf_counter() - ts
+        ts = time.perf_counter()
+        if sqlite_vec is not None:
+            conn.enable_load_extension(True)
+            sqlite_vec.load(conn)                                        # semantic_search.py:68-72
+            conn.enable_load_extension(False)
+            for x in ("_chunks", "_vector_chunks00", "_rowids", "_info"):  # a shadow-only layout from an earlier build
+                if not store._table_exists(conn, store.VEC_TABLE) and store._table_exists(conn, store.VEC_TABLE + x):
+                    cur.execute(f"DROP TABLE {store.VEC_TABLE}{x}")
+            if store._table_exists(conn, "rse_meta"):
+                cur.execute("DELETE FROM rse_meta WHERE key = 'vec0_shadow_writer'")
+            cur.execute(f"DROP TABLE IF EXISTS {store.VEC_TABLE}")
+            cur.execute(f"CREATE VIRTUAL TABLE IF NOT EXISTS {store.VEC_TABLE} USING vec0("
+                        f"embedding float[{emb.shape[1]}] distance_metric=cosine)")      # :94-101
+            cur.executemany(f"INSERT INTO {store.VEC_TABLE}(rowid, embedding) VALUES (?, ?)",   # :203-206
+                            ((i, emb[i]) for i in range(n)))
+        else:
+            store.write_vec0_shadow(conn, chunk_ids, emb)
+        conn.commit()
+        t["sqlite_vec0"] = time.perf_counter() - ts
+        if n == 0:                                                        # an empty index: _load exports it as usual
+            return
+        ts = time.perf_counter()
+        keep = None
+        if not _vec0_rows_in_order(conn, n):
+            # vec0 placed the rows elsewhere than positions 0 .. n-1: serve what the file holds, as a fresh open would
+            arr = store.export_embeddings(conn)
+            index.load_embeddings(arr.emb, valid=arr.valid, rowid=arr.rowid, movie_idx=arr.movie_idx)
+        else:
+            # rows inserted 0, 1, ... into a fresh table sit at positions 0, 1, ...: these are the arrays
+            # store.export_embeddings reads back from the file
+            arr = store.EmbArrays(emb=emb, valid=None, rowid=chunk_ids, movie_idx=built.movie_idx,
+                                  movie_ids=movie_ids, dim=int(emb.shape[1]))
+            rowid_dev = torch.from_numpy(chunk_ids).to(built.emb.device)
+            midx_dev = torch.from_numpy(built.movie_idx).to(built.emb.device)
+            torch.cuda.synchronize(built.emb.device)
+            index.attach_embeddings_dev(built.emb.data_ptr(), n, int(emb.shape[1]), rowid_ptr=rowid_dev.data_ptr(),
+                                        movie_idx_ptr=midx_dev.data_ptr(), keepalive=built.emb)
+            index.synchronize()
+            keep = built.emb                                             # the registry keeps the borrowed matrix
+        t["attach"] = time.perf_counter() - ts
+        # the sidecar is written by _load, with the fingerprint of the connection a later open compares against
+        self._device_built = arr
+        full = store._db_fingerprint(conn, self.db_path)
+        reg = runtime.parts(self.db_path, self.device)
+        reg["emb"], reg["emb_fp"] = arr, store.part_fingerprint(full, "emb")
+        reg["emb_dev"] = keep
+        reg.pop("ids", None)
+
     def _load(self) -> None:
         reg = runtime.parts(self.db_path, self.device)
         full = store._db_fingerprint(self.conn, self.db_path)
         fp = store.part_fingerprint(full, "emb")
+        built = self.__dict__.pop("_device_built", None)
+        if built is not None:                                     # the device build's host copy: no export
+            ts = time.perf_counter()
+            store.write_sidecar(self.db_path, "emb", built, json.dumps(full, sort_keys=True))
+            self.build_timings["sidecar"] = time.perf_counter() - ts
         if "emb" not in reg or reg.get("emb_fp") != fp:          # first open, or re-embedded under a live handle
             arr = store.load_or_export(self.conn, self.db_path, "emb", fingerprint=full)
             if arr.emb.shape[0] > 0:
                 self._index.load_embeddings(arr.emb, valid=arr.valid, rowid=arr.rowid, movie_idx=arr.movie_idx)
+                reg.pop("emb_dev", None)                         # a device-built matrix this load replaced
             else:
                 # no chunk embeddings (keyword-only / fresh database): query_top_k returns [] like the reference;
                 # the handle still needs a dimension for the batch entry points' reshape

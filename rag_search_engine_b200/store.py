@@ -314,6 +314,13 @@ def load_or_export(conn: sqlite3.Connection, db_path, part: str, use_cache: bool
         except Exception as e:                        # unreadable sidecar → re-export, but say so
             logger.warning("sidecar %s rejected (%s: %s): re-exporting", sc, type(e).__name__, e)
     arr = exporter(conn)
+    write_sidecar(db_path, part, arr, fp)
+    return arr
+
+
+def write_sidecar(db_path, part: str, arr, fp: str) -> None:
+    """The sidecar of ``part`` for the arrays ``arr`` of the database whose fingerprint (json) is ``fp``."""
+    sc = sidecar_path(db_path, part)
 
     def atomic(path: Path, write) -> None:
         # tmp + os.replace: a concurrent opener sees the old file or the new one, never a half-written one
@@ -345,7 +352,6 @@ def load_or_export(conn: sqlite3.Connection, db_path, part: str, use_cache: bool
                                            dim=np.int64(arr.dim)))
     except OSError as e:
         logger.info("sidecar for %s not written (%s): read-only location?", db_path, e)
-    return arr
 
 
 # ----------------------------------------------------------------------------- writer (reference on-disk format)
