@@ -125,6 +125,20 @@ int rse_knn_movies(rse_index *h, const float *q_host, int32_t nq, int32_t k, int
                    float *out_dist, int64_t *out_chunk_rowid, int32_t *out_movie_idx,
                    int32_t *out_count);
 
+/* Exact movie-level KNN: the k nearest movies by best chunk over EVERY row (DESIGN §11).  Outputs [nq, k] as
+ * rse_knn_movies; out_scanned (may be NULL) = queries that needed the full segmented scan.  1 <= k <= 4096.
+ * A movie's best chunk is its row with the smallest (distance, block asc, slot desc) key; rows with valid = 0 or
+ * movie_idx = -1 never compete; movies are ordered by their best key and the first min(k, movies) are returned,
+ * each distance bit-identical to rse_knn's for that row (rse_set_fma honoured).  Prefix property: where
+ * rse_knn_movies(k, K') returns k movies for a query the two results are identical, and where it returns fewer its
+ * list is a prefix of this one.  RSE_ERR_UNSUPPORTED for k > 4096; RSE_ERR_STATE without a corpus or movie_idx.
+ * RSE_MOVIES_EXACT_BUDGET (bytes, read by rse_create; default 512 MB) bounds the [queries, movies] u64 key buffer
+ * of the segmented scan, i.e. how many queries one pass over the corpus serves.  With rse_set_timing on, the call's
+ * H2D → D2H time lands in last_knn_total_ms and its scan launches in scan_ms_total. */
+int rse_knn_movies_exact(rse_index *h, const float *q_host, int32_t nq, int32_t k, float *out_dist,
+                         int64_t *out_chunk_rowid, int32_t *out_movie_idx, int32_t *out_count,
+                         int32_t *out_scanned);
+
 /* Device-pointer building blocks for the row-sharded multi-GPU path (SURVEY §8e).
  * Local top-kprime as packed candidates: cand_dev is [nq, kprime, 3] int64 =
  * {key, rowid, movie_idx}; key = (orderable(distance) << 32) | (global_pos ^ 1023),

@@ -118,6 +118,8 @@ _SIGNATURES = {
                                POINTER(c_int64), POINTER(c_int32), POINTER(c_int32)]),
     "rse_knn_movies": (ctypes.c_int, [c_void_p, POINTER(c_float), c_int32, c_int32, c_int32, POINTER(c_float),
                                       POINTER(c_int64), POINTER(c_int32), POINTER(c_int32)]),
+    "rse_knn_movies_exact": (ctypes.c_int, [c_void_p, POINTER(c_float), c_int32, c_int32, POINTER(c_float),
+                                            POINTER(c_int64), POINTER(c_int32), POINTER(c_int32), POINTER(c_int32)]),
     "rse_knn_local_dev": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
     "rse_set_defer_flags": (ctypes.c_int, [c_void_p, c_int32]),
     "rse_knn_flags_dev": (ctypes.c_int, [c_void_p, c_void_p]),
@@ -368,6 +370,23 @@ class Index:
         self._check(self._L.rse_knn_movies(self._h, _ptr(Q, c_float), nq, int(k), int(kprime), _ptr(dist, c_float),
                                            _ptr(rowid, c_int64), _ptr(movie, c_int32), _ptr(cnt, c_int32)))
         return dist, rowid, movie, cnt
+
+    def knn_movies_exact(self, Q, k: int):
+        """The k nearest movies by best chunk over every row (rse_knn_movies_exact) →
+        (dist, rowid, movie, count, scanned); scanned = queries that took the full segmented scan."""
+        Q = _c(Q, np.float32)
+        Q = Q.reshape(-1, self.dim or Q.shape[-1])
+        nq = Q.shape[0]
+        kk = max(int(k), 1)
+        dist = np.zeros((nq, kk), np.float32)
+        rowid = np.zeros((nq, kk), np.int64)
+        movie = np.zeros((nq, kk), np.int32)
+        cnt = np.zeros(nq, np.int32)
+        scanned = c_int32(0)
+        self._check(self._L.rse_knn_movies_exact(self._h, _ptr(Q, c_float), nq, int(k), _ptr(dist, c_float),
+                                                 _ptr(rowid, c_int64), _ptr(movie, c_int32), _ptr(cnt, c_int32),
+                                                 ctypes.byref(scanned)))
+        return dist, rowid, movie, cnt, int(scanned.value)
 
     def knn_local_dev(self, q_ptr: int, nq: int, kprime: int, cand_ptr: int):
         self._check(self._L.rse_knn_local_dev(self._h, c_void_p(q_ptr), int(nq), int(kprime), c_void_p(cand_ptr)))

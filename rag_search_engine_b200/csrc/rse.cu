@@ -28,6 +28,7 @@
 #include "wordpiece.cuh"
 #include "bpe.cuh"
 #include "chunk.cuh"
+#include "knn_movies_exact.cuh"
 
 using namespace rse;
 
@@ -221,6 +222,13 @@ struct rse_index {
   DevBuf sb, sel, hist, selkeys, cand, dist, o_dist, o_pos, o_rowid, o_movie, o_count;
   int64_t dist_ld = 0;
 
+  // ---- rse_knn_movies_exact (knn_movies_exact.cuh): the corpus's movie layout, checked once per load (-1 = not
+  // yet), and the per-(query, movie) key buffer's budget, which sets how many queries one segmented scan serves
+  int movies_sorted = -1;
+  int64_t movie_slots = 0;
+  size_t mx_budget = size_t(512) << 20;   // RSE_MOVIES_EXACT_BUDGET (bytes)
+  DevBuf mx_span, mx_meta, mx_best, mx_list, mx_q, mx_sb, mx_keys, mx_cand, mx_dist, mx_rowid, mx_movie, mx_count;
+
   // ---- a6: BM25
   int64_t n_terms = 0, n_postings = 0, n_docs = 0, n_movies = 0;
   double avgdl = 0.0;
@@ -369,6 +377,8 @@ void release_embeddings(rse_index* h) {
   free_buf(h->tc_sample);
   h->sample_tiles = 0;
   h->shadow_state = 0;
+  h->movies_sorted = -1;
+  h->movie_slots = 0;
 }
 
 void release_bm25(rse_index* h) {
@@ -1047,6 +1057,119 @@ int merge_candidates(rse_index* h, const long long* gathered, int n_lists, int n
   return RSE_OK;
 }
 
+// ---- exact movie-level KNN (knn_movies_exact.cuh, DESIGN §11)
+// The corpus's movie layout, once per load: n_movie_slots and whether the competing rows are sorted by movie_idx.
+int movies_layout(rse_index* h) {
+  if (h->movies_sorted >= 0) return RSE_OK;
+  const int n_spans = static_cast<int>(std::max<int64_t>(1, (h->n_rows + kLayoutRowsPerThread - 1) / kLayoutRowsPerThread));
+  ENSURE(h->mx_span, sizeof(int4) * n_spans);
+  ENSURE(h->mx_meta, sizeof(unsigned int) * 2);
+  unsigned int* meta = static_cast<unsigned int*>(h->mx_meta.p);   // [0] n_movie_slots, [1] sorted
+  CK(cudaMemsetAsync(meta, 0, sizeof(unsigned int) * 2, h->stream));
+  if (h->n_rows > 0) {
+    movies_layout_kernel<<<(n_spans + 127) / 128, 128, 0, h->stream>>>(h->movie_idx, h->amag, h->n_rows, n_spans,
+                                                                      static_cast<int4*>(h->mx_span.p), meta);
+    LAUNCHED(h);
+    movies_layout_join_kernel<<<1, 1, 0, h->stream>>>(static_cast<const int4*>(h->mx_span.p), n_spans,
+                                                      reinterpret_cast<int*>(meta + 1));
+    LAUNCHED(h);
+  }
+  unsigned int host[2] = {0u, 0u};
+  CK(cudaMemcpyAsync(host, meta, sizeof(host), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->movie_slots = host[0];
+  h->movies_sorted = (h->n_rows == 0 || host[1]) ? 1 : 0;
+  return RSE_OK;
+}
+
+// The k nearest movies of nq device-resident queries (|q| factors sb ready) over every row: the exact scan of
+// knn_scan.cuh per group of 16 queries, the segmented minimum into best[query][movie], then the radix select over
+// the movie keys per group of <= 256 queries.  Outputs are device [nq, k] in rse_knn_movies' layout.  Queries go in
+// chunks whose best buffer fits mx_budget.
+int movies_exact_scan(rse_index* h, const float* q, const double* sb, int nq, int k, float* o_dist,
+                      long long* o_rowid, int* o_movie, int* o_count) {
+  const int QB = kScanMaxQB;
+  const int64_t n_slots = std::max<int64_t>(h->movie_slots, 1);   // no movie at all: one empty slot, nothing found
+  const size_t per_q = sizeof(unsigned long long) * static_cast<size_t>(n_slots);
+  int64_t chunk = std::max<int64_t>(1, static_cast<int64_t>(h->mx_budget / per_q));
+  if (chunk >= QB) chunk -= chunk % QB;
+  chunk = std::min<int64_t>(chunk, nq);
+  const int sel_q = std::min(nq, kTcBN);
+  ENSURE(h->mx_best, per_q * static_cast<size_t>(chunk));
+  ENSURE(h->dist, sizeof(float) * static_cast<size_t>(QB) * h->dist_ld);
+  ENSURE(h->sel, sizeof(SelState) * std::max(nq, kTcBN));
+  ENSURE(h->mx_keys, sizeof(unsigned long long) * static_cast<size_t>(sel_q) * k);
+  ENSURE(h->mx_cand, sizeof(long long) * static_cast<size_t>(sel_q) * k * 3);
+  if (h->hist.bytes < sizeof(unsigned int) * kSelBins * kTcBN) {
+    ENSURE(h->hist, sizeof(unsigned int) * kSelBins * kTcBN);
+    CK(cudaMemsetAsync(h->hist.p, 0, h->hist.bytes, h->stream));
+  }
+  unsigned long long* best = static_cast<unsigned long long*>(h->mx_best.p);
+  float* dist = static_cast<float*>(h->dist.p);
+  SelState* sel = static_cast<SelState*>(h->sel.p);
+  unsigned int* hist = static_cast<unsigned int*>(h->hist.p);
+  unsigned long long* keys = static_cast<unsigned long long*>(h->mx_keys.p);
+  long long* cand = static_cast<long long*>(h->mx_cand.p);
+  static const int shifts[6] = {53, 42, 32, 21, 10, 0};
+  static const int widths[6] = {11, 11, 10, 11, 11, 10};
+  const int sel_blocks = static_cast<int>(std::min<int64_t>((n_slots + 4095) / 4096, h->sm_count * 2));
+  const int kp2 = next_pow2(k);
+  const size_t fsmem = static_cast<size_t>(kp2) * 12;
+  if (fsmem > 48 * 1024) CK(cudaFuncSetAttribute(select_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  for (int c0 = 0; c0 < nq; c0 += static_cast<int>(chunk)) {
+    const int nc = std::min(static_cast<int>(chunk), nq - c0);
+    CK(cudaMemsetAsync(best, 0xFF, per_q * nc, h->stream));
+    for (int g0 = c0; g0 < c0 + nc; g0 += QB) {
+      const int ng = std::min(QB, c0 + nc - g0);
+      cudaEvent_t e0 = nullptr, e1 = nullptr;                    // rse_set_timing: the scan's share of the call
+      if (h->timing && h->scan_ev_used + 2 <= (1u << 16)) {
+        int rc = scan_event(h, &e0);
+        if (rc != RSE_OK) return rc;
+      }
+      int rc = h->fma ? launch_scan<true>(h, q + static_cast<int64_t>(g0) * h->dim, sb + g0, ng, dist)
+                      : launch_scan<false>(h, q + static_cast<int64_t>(g0) * h->dim, sb + g0, ng, dist);
+      if (rc != RSE_OK) return rc;
+      if (e0) {
+        rc = scan_event(h, &e1);
+        if (rc != RSE_OK) return rc;
+        h->scan_ev_passes.push_back(1);
+      }
+      const int seg_blocks = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(
+          (h->n_rows + kSegThreads - 1) / kSegThreads, std::max(1, h->sm_count * 16 / ng))));
+      unsigned long long* bg = best + static_cast<int64_t>(g0 - c0) * n_slots;
+      const uint32_t* d32 = reinterpret_cast<const uint32_t*>(dist);
+      if (h->movies_sorted)
+        movies_segmin_kernel<true><<<dim3(seg_blocks, ng), kSegThreads, 0, h->stream>>>(
+            d32, h->dist_ld, h->n_rows, h->pos_base, h->movie_idx, n_slots, bg);
+      else
+        movies_segmin_kernel<false><<<dim3(seg_blocks, ng), kSegThreads, 0, h->stream>>>(
+            d32, h->dist_ld, h->n_rows, h->pos_base, h->movie_idx, n_slots, bg);
+      LAUNCHED(h);
+    }
+    for (int s0 = c0; s0 < c0 + nc; s0 += kTcBN) {
+      const int ns = std::min(kTcBN, c0 + nc - s0);
+      const unsigned long long* bs = best + static_cast<int64_t>(s0 - c0) * n_slots;
+      select_init_kernel<<<(ns + 127) / 128, 128, 0, h->stream>>>(sel, ns, static_cast<unsigned int>(k));
+      LAUNCHED(h);
+      const dim3 grid(std::max(sel_blocks, 1), ns);
+      for (int p = 0; p < 6; ++p) {
+        select_keys_pass_kernel<<<grid, kSelThreads, 0, h->stream>>>(bs, n_slots, n_slots, sel, hist, shifts[p], widths[p]);
+        LAUNCHED(h);
+      }
+      select_keys_collect_kernel<<<grid, kSelThreads, 0, h->stream>>>(bs, n_slots, n_slots, sel, keys, k);
+      LAUNCHED(h);
+      select_finish_kernel<<<ns, kSelThreads, fsmem, h->stream>>>(keys, sel, k, kp2, h->pos_base, h->rowid,
+                                                                 h->movie_idx, cand);
+      LAUNCHED(h);
+      const int64_t o = static_cast<int64_t>(s0) * k;
+      knn_unpack_kernel<<<ns, 128, 0, h->stream>>>(cand, ns, k, o_dist + o, nullptr, o_rowid + o, o_movie + o,
+                                                   o_count + s0);
+      LAUNCHED(h);
+    }
+  }
+  return RSE_OK;
+}
+
 int upload_queries(rse_index* h, const float* q_host, int nq) {
   ENSURE(h->staged.q, sizeof(float) * static_cast<size_t>(nq) * h->dim);
   CK(cudaMemcpyAsync(h->staged.q.p, q_host, sizeof(float) * static_cast<size_t>(nq) * h->dim, cudaMemcpyHostToDevice,
@@ -1127,6 +1250,7 @@ int rse_create(int32_t device, rse_index** out) {
   if (const char* ev = std::getenv("RSE_TC_SAMPLE_STRIDE")) { const int v = std::atoi(ev); if (v >= 2 && v <= 256) h->sample_stride = v; }
   if (const char* ev = std::getenv("RSE_TC_SAMPLE_MIN_TILES")) { const int v = std::atoi(ev); if (v >= 1) h->sample_min_tiles = v; }
   if (const char* ev = std::getenv("RSE_TC_PROBE_RANK")) { const int v = std::atoi(ev); if (v >= 1) h->probe_rank = v; }
+  if (const char* ev = std::getenv("RSE_MOVIES_EXACT_BUDGET")) { const long long v = std::atoll(ev); if (v >= 1) h->mx_budget = static_cast<size_t>(v); }
   if (const char* ev = std::getenv("RSE_TC_SURVIVOR_DIV")) { const int v = std::atoi(ev); if (v >= 1 && v <= 64) h->survivor_div = v; }
   *out = h;
   return RSE_OK;
@@ -1145,7 +1269,8 @@ void rse_destroy(rse_index* h) {
                     &h->f_bid, &h->f_bsc, &h->f_bcnt, &h->f_sid, &h->f_sds, &h->f_scnt, &h->f_oid, &h->f_osc, &h->f_oa,
                     &h->f_ob, &h->f_ocnt, &h->tc_thr,
                     &h->tc_rows, &h->tc_cnt, &h->tc_status, &h->fb_list, &h->fb_q, &h->fb_sb, &h->fb_cand, &h->tc_q16, &h->b_shi, &h->b_slo, &h->b_scnt,
-                    &h->b_status, &h->b_flagged})
+                    &h->b_status, &h->b_flagged, &h->mx_span, &h->mx_meta, &h->mx_best, &h->mx_list, &h->mx_q,
+                    &h->mx_sb, &h->mx_keys, &h->mx_cand, &h->mx_dist, &h->mx_rowid, &h->mx_movie, &h->mx_count})
     free_buf(*b);
   if (h->pin_status.p) cudaFreeHost(h->pin_status.p);
   if (h->pin_stage) cudaFreeHost(h->pin_stage);
@@ -1496,6 +1621,100 @@ int rse_knn_movies(rse_index* h, const float* q_host, int32_t nq, int32_t k, int
     CK(cudaEventElapsedTime(&ms, h->ev[2], h->ev[3]));
     h->stats.last_knn_total_ms = ms;
   }
+  return RSE_OK;
+}
+
+int rse_knn_movies_exact(rse_index* h, const float* q_host, int32_t nq, int32_t k, float* out_dist,
+                         int64_t* out_chunk_rowid, int32_t* out_movie_idx, int32_t* out_count, int32_t* out_scanned) {
+  if (!h) return RSE_ERR_INVALID;
+  if (nq < 0 || k < 1 || (nq > 0 && (!q_host || !out_dist || !out_chunk_rowid || !out_movie_idx || !out_count)))
+    return fail(h, RSE_ERR_INVALID, "rse_knn_movies_exact: bad arguments");
+  if (k > RSE_MAX_KPRIME) return fail(h, RSE_ERR_UNSUPPORTED, "rse_knn_movies_exact: k must be in [1, 4096]");
+  if (!h->emb) return fail(h, RSE_ERR_STATE, "rse_knn_movies_exact: no embeddings loaded");
+  if (!h->movie_idx) return fail(h, RSE_ERR_STATE, "rse_knn_movies_exact: embeddings were loaded without movie_idx");
+  if (out_scanned) *out_scanned = 0;
+  if (nq == 0) return RSE_OK;
+  CK(cudaSetDevice(h->device));
+  if (h->timing) CK(cudaEventRecord(h->ev[2], h->stream));
+  int rc = upload_queries(h, q_host, nq);
+  if (rc != RSE_OK) return rc;
+  rc = movies_layout(h);
+  if (rc != RSE_OK) return rc;
+  const size_t n = static_cast<size_t>(nq) * k;
+  ENSURE(h->o_dist, sizeof(float) * n);
+  ENSURE(h->o_rowid, sizeof(long long) * n);
+  ENSURE(h->o_movie, sizeof(int) * n);
+  ENSURE(h->o_count, sizeof(int) * nq);
+  float* o_dist = static_cast<float*>(h->o_dist.p);
+  long long* o_rowid = static_cast<long long*>(h->o_rowid.p);
+  int* o_movie = static_cast<int*>(h->o_movie.p);
+  int* o_count = static_cast<int*>(h->o_count.p);
+  const float* q = static_cast<const float*>(h->staged.q.p);
+  // Staging (DESIGN §11): where the tensor-core filter serves K' = kMoviesExactStageMult * k, rse_knn_movies runs
+  // first; a query it gives k movies is final (prefix property), and only the short ones take the segmented scan.
+  // A corpus whose fp16 shadow cannot be built (shadow_state -1) would answer the first stage with the exact scan:
+  // it goes straight to the segmented scan instead
+  const int kprime = kMoviesExactStageMult * k;
+  int n_scan = nq;
+  if (kprime <= RSE_MAX_KPRIME && h->shadow_state >= 0 && tc_eligible(h, nq, kprime)) {
+    ENSURE(h->cand, sizeof(long long) * static_cast<size_t>(nq) * kprime * 3);
+    rc = knn_local(h, q, nq, kprime, static_cast<long long*>(h->cand.p));
+    if (rc == RSE_OK) rc = aggregate(h, static_cast<const long long*>(h->cand.p), nq, k, kprime, o_dist, o_rowid, o_movie, o_count);
+    if (rc != RSE_OK) return rc;
+    std::vector<int> cnt(nq), list;
+    CK(cudaMemcpyAsync(cnt.data(), o_count, sizeof(int) * nq, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int i = 0; i < nq; ++i)
+      if (cnt[i] < k) list.push_back(i);
+    n_scan = static_cast<int>(list.size());
+    if (n_scan > 0) {
+      const size_t ns = static_cast<size_t>(n_scan);
+      ENSURE(h->mx_list, sizeof(int) * ns);
+      ENSURE(h->mx_q, sizeof(float) * ns * h->dim);
+      ENSURE(h->mx_sb, sizeof(double) * ns);
+      ENSURE(h->mx_dist, sizeof(float) * ns * k);
+      ENSURE(h->mx_rowid, sizeof(long long) * ns * k);
+      ENSURE(h->mx_movie, sizeof(int) * ns * k);
+      ENSURE(h->mx_count, sizeof(int) * ns);
+      CK(cudaMemcpyAsync(h->mx_list.p, list.data(), sizeof(int) * ns, cudaMemcpyHostToDevice, h->stream));
+      CK(cudaStreamSynchronize(h->stream));                      // `list` is a pageable temporary
+      const int* dl = static_cast<const int*>(h->mx_list.p);
+      knn_gather_queries_kernel<<<n_scan, 128, 0, h->stream>>>(q, static_cast<const double*>(h->sb.p), dl, h->dim,
+                                                              static_cast<float*>(h->mx_q.p), static_cast<double*>(h->mx_sb.p));
+      LAUNCHED(h);
+      float* s_dist = static_cast<float*>(h->mx_dist.p);
+      long long* s_rowid = static_cast<long long*>(h->mx_rowid.p);
+      int* s_movie = static_cast<int*>(h->mx_movie.p);
+      int* s_count = static_cast<int*>(h->mx_count.p);
+      rc = movies_exact_scan(h, static_cast<const float*>(h->mx_q.p), static_cast<const double*>(h->mx_sb.p), n_scan, k,
+                             s_dist, s_rowid, s_movie, s_count);
+      if (rc != RSE_OK) return rc;
+      movies_scatter_kernel<<<n_scan, 128, 0, h->stream>>>(s_dist, s_rowid, s_movie, s_count, dl, k, o_dist, o_rowid,
+                                                          o_movie, o_count);
+      LAUNCHED(h);
+    }
+  } else {
+    ENSURE(h->sb, sizeof(double) * nq);
+    double* sb = static_cast<double*>(h->sb.p);
+    if (h->fma) knn_query_prep_kernel<true><<<(nq + 3) / 4, 128, 0, h->stream>>>(q, nq, h->dim, sb);
+    else knn_query_prep_kernel<false><<<(nq + 3) / 4, 128, 0, h->stream>>>(q, nq, h->dim, sb);
+    LAUNCHED(h);
+    rc = movies_exact_scan(h, q, sb, nq, k, o_dist, o_rowid, o_movie, o_count);
+    if (rc != RSE_OK) return rc;
+  }
+  CK(cudaMemcpyAsync(out_dist, o_dist, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(out_chunk_rowid, o_rowid, sizeof(long long) * n, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(out_movie_idx, o_movie, sizeof(int) * n, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(out_count, o_count, sizeof(int) * nq, cudaMemcpyDeviceToHost, h->stream));
+  h->stats.d2h_bytes += static_cast<int64_t>(n) * 16 + static_cast<int64_t>(nq) * 4;
+  if (h->timing) CK(cudaEventRecord(h->ev[3], h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  if (h->timing) {
+    float ms = 0.f;
+    CK(cudaEventElapsedTime(&ms, h->ev[2], h->ev[3]));
+    h->stats.last_knn_total_ms = ms;
+  }
+  if (out_scanned) *out_scanned = n_scan;
   return RSE_OK;
 }
 

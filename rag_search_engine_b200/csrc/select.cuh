@@ -40,6 +40,74 @@ __global__ void select_init_kernel(SelState* st, int nq, unsigned int kprime) {
   st[q] = s;
 }
 
+// The histogram -> digit step of one radix pass, shared by select_pass_kernel (keys derived
+// from distances) and select_keys_pass_kernel (stored keys, knn_movies_exact.cuh): merge
+// this CTA's histogram h into the query's global one gh, and let the last CTA of the
+// query locate the digit holding the `need`-th smallest key.
+__device__ __forceinline__ void select_pass_pick(const SelState s, SelState* __restrict__ st, int q,
+                                                 unsigned int* __restrict__ h, unsigned int* __restrict__ gh,
+                                                 unsigned int* s_part, int* s_last, int shift, unsigned int dmask) {
+  for (int i = threadIdx.x; i < kSelBins; i += blockDim.x)
+    if (h[i]) atomicAdd(&gh[i], h[i]);
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned int t = atomicAdd(&st[q].ticket, 1u);
+    *s_last = (t == gridDim.x - 1);
+  }
+  __syncthreads();
+  if (!*s_last) return;
+  __threadfence();
+
+  // ---- last CTA of this query: locate the digit that contains the need-th key
+  constexpr int per = kSelBins / kSelThreads;   // 8 consecutive bins per thread
+  unsigned int loc[per];
+  unsigned int mysum = 0u;
+#pragma unroll
+  for (int i = 0; i < per; ++i) {
+    loc[i] = __ldcg(&gh[threadIdx.x * per + i]);
+    mysum += loc[i];
+  }
+  s_part[threadIdx.x] = mysum;
+  __syncthreads();
+  // exclusive prefix over 256 partial sums (Hillis-Steele in smem; once per pass)
+  for (int off = 1; off < kSelThreads; off <<= 1) {
+    unsigned int v = (threadIdx.x >= off) ? s_part[threadIdx.x - off] : 0u;
+    __syncthreads();
+    s_part[threadIdx.x] += v;
+    __syncthreads();
+  }
+  const unsigned int incl = s_part[threadIdx.x];
+  const unsigned int excl = incl - mysum;
+  const unsigned int total = s_part[kSelThreads - 1];
+  if (total < s.need) {
+    // fewer matching keys than requested (only possible before any bit is
+    // resolved: fewer valid rows than K') → take everything.
+    if (threadIdx.x == 0) {
+      st[q].done = 1u; st[q].mask = 0ull; st[q].prefix = 0ull;
+      st[q].total = total; st[q].ticket = 0u;
+    }
+  } else if (excl < s.need && s.need <= incl) {   // exactly one thread owns the crossing
+    unsigned int run = excl, below = 0u, in_bucket = 0u;
+    int digit = -1;
+#pragma unroll
+    for (int i = 0; i < per; ++i) {
+      if (digit < 0) {
+        if (run + loc[i] >= s.need) { digit = threadIdx.x * per + i; below = run; in_bucket = loc[i]; }
+        else run += loc[i];
+      }
+    }
+    const unsigned int need2 = s.need - below;
+    st[q].prefix = s.prefix | (static_cast<unsigned long long>(digit) << shift);
+    st[q].mask = s.mask | (static_cast<unsigned long long>(dmask) << shift);
+    st[q].need = need2;
+    st[q].ticket = 0u;
+    if (in_bucket == need2 || shift == 0) st[q].done = 1u;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kSelBins; i += blockDim.x) gh[i] = 0u;
+}
+
 // One radix pass: histogram the digit [shift, shift+bits) of every key that matches
 // the resolved prefix; the last CTA of each query picks the digit holding the
 // `need`-th smallest key and refines the state.  `hist` is [nq][kSelBins], zero on
@@ -95,66 +163,7 @@ select_pass_kernel(const uint32_t* __restrict__ dist, int64_t ld, int64_t n_rows
   }
   if (run_cnt) atomicAdd(&h[run_digit], run_cnt);
   __syncthreads();
-  unsigned int* gh = hist + static_cast<int64_t>(q) * kSelBins;
-  for (int i = threadIdx.x; i < kSelBins; i += blockDim.x)
-    if (h[i]) atomicAdd(&gh[i], h[i]);
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned int t = atomicAdd(&st[q].ticket, 1u);
-    s_last = (t == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-
-  // ---- last CTA of this query: locate the digit that contains the need-th key
-  constexpr int per = kSelBins / kSelThreads;   // 8 consecutive bins per thread
-  unsigned int loc[per];
-  unsigned int mysum = 0u;
-#pragma unroll
-  for (int i = 0; i < per; ++i) {
-    loc[i] = __ldcg(&gh[threadIdx.x * per + i]);
-    mysum += loc[i];
-  }
-  s_part[threadIdx.x] = mysum;
-  __syncthreads();
-  // exclusive prefix over 256 partial sums (Hillis-Steele in smem; once per pass)
-  for (int off = 1; off < kSelThreads; off <<= 1) {
-    unsigned int v = (threadIdx.x >= off) ? s_part[threadIdx.x - off] : 0u;
-    __syncthreads();
-    s_part[threadIdx.x] += v;
-    __syncthreads();
-  }
-  const unsigned int incl = s_part[threadIdx.x];
-  const unsigned int excl = incl - mysum;
-  const unsigned int total = s_part[kSelThreads - 1];
-  if (total < s.need) {
-    // fewer matching keys than requested (only possible before any bit is
-    // resolved: fewer valid rows than K') → take everything.
-    if (threadIdx.x == 0) {
-      st[q].done = 1u; st[q].mask = 0ull; st[q].prefix = 0ull;
-      st[q].total = total; st[q].ticket = 0u;
-    }
-  } else if (excl < s.need && s.need <= incl) {   // exactly one thread owns the crossing
-    unsigned int run = excl, below = 0u, in_bucket = 0u;
-    int digit = -1;
-#pragma unroll
-    for (int i = 0; i < per; ++i) {
-      if (digit < 0) {
-        if (run + loc[i] >= s.need) { digit = threadIdx.x * per + i; below = run; in_bucket = loc[i]; }
-        else run += loc[i];
-      }
-    }
-    const unsigned int need2 = s.need - below;
-    st[q].prefix = s.prefix | (static_cast<unsigned long long>(digit) << shift);
-    st[q].mask = s.mask | (static_cast<unsigned long long>(dmask) << shift);
-    st[q].need = need2;
-    st[q].ticket = 0u;
-    if (in_bucket == need2 || shift == 0) st[q].done = 1u;
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < kSelBins; i += blockDim.x) gh[i] = 0u;
+  select_pass_pick(s, st, q, h, hist + static_cast<int64_t>(q) * kSelBins, s_part, &s_last, shift, dmask);
 }
 
 // Gather the selected keys: everything whose resolved bits are <= the threshold prefix.

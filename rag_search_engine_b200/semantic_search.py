@@ -20,6 +20,8 @@ from . import runtime, store
 from .keyword_search import DEFAULT_DB_PATH
 from .textutil import chunk_text
 
+MAX_EXACT_K = 4096                                              # rse_knn_movies_exact's bound on k (include/rse.h)
+
 
 def _default_encoder():
     try:
@@ -309,14 +311,24 @@ class SemanticSearch:
         return np.asarray(self.model.encode(texts), dtype=np.float32)
 
     # ------------------------------------------------------------------ query
-    def query_top_k_vec(self, query_vecs, k: int = 5, knn_multiplier: int = 10) -> List[List[Dict[str, Any]]]:
-        """Batch entry point on frozen query vectors [B, dim] → one reference-shaped result list per query."""
+    def query_top_k_vec(self, query_vecs, k: int = 5, knn_multiplier: int = 10, *,
+                        exact_movies: bool = False) -> List[List[Dict[str, Any]]]:
+        """Batch entry point on frozen query vectors [B, dim] → one reference-shaped result list per query.
+
+        exact_movies=True: the k nearest movies by best chunk over every chunk (rse_knn_movies_exact), not only
+        over the top k * knn_multiplier chunks, so a query gets min(k, movies) hits; knn_multiplier is ignored
+        and k may go up to 4096.  Where the default call returns k movies, the exact one returns the same list."""
+        if exact_movies and not 1 <= int(k) <= MAX_EXACT_K:
+            raise ValueError(f"exact_movies: k must be in [1, {MAX_EXACT_K}], got {k}")
         Q = np.atleast_2d(np.ascontiguousarray(query_vecs, np.float32))
         if self._arr.emb.shape[0] == 0:                         # no chunk embeddings: [] per query, like the reference
             return [[] for _ in range(Q.shape[0])]
         Q = Q.reshape(-1, self._arr.dim)
-        internal_k = max(k * knn_multiplier, k)                 # semantic_search.py:251
-        dist, rowid, movie, cnt = self._index.knn_movies(Q, k, internal_k)
+        if exact_movies:
+            dist, rowid, movie, cnt, _ = self._index.knn_movies_exact(Q, int(k))
+        else:
+            internal_k = max(k * knn_multiplier, k)             # semantic_search.py:251
+            dist, rowid, movie, cnt = self._index.knn_movies(Q, k, internal_k)
         # the two JOINs of semantic_search.py:262-279 for the <= k final hits of every query: ONE lookup per table
         # for the whole batch (a point query per hit costs more than the device call from ~100 hits on)
         movie_ids = self._arr.movie_ids
@@ -350,10 +362,14 @@ class SemanticSearch:
                 got[row[0]] = row[1:]
         return got
 
-    def query_top_k(self, query_text: str, k: int = 5, knn_multiplier: int = 10) -> List[Dict[str, Any]]:
-        """semantic_search.py:225-340."""
+    def query_top_k(self, query_text: str, k: int = 5, knn_multiplier: int = 10, *,
+                    exact_movies: bool = False) -> List[Dict[str, Any]]:
+        """semantic_search.py:225-340; exact_movies as in query_top_k_vec."""
+        if exact_movies and not 1 <= int(k) <= MAX_EXACT_K:
+            raise ValueError(f"exact_movies: k must be in [1, {MAX_EXACT_K}], got {k}")
         query_vec = self.generate_embedding(query_text)[0]
-        return self.query_top_k_vec(query_vec[None, :], k=k, knn_multiplier=knn_multiplier)[0]
+        return self.query_top_k_vec(query_vec[None, :], k=k, knn_multiplier=knn_multiplier,
+                                    exact_movies=exact_movies)[0]
 
     def _reconstruct_chunk_text(self, title, description, chunk_index, max_chunk_size, overlap) -> str:
         return chunk_text(title, description, chunk_index, max_chunk_size, overlap)
